@@ -2,6 +2,7 @@
 """Benchmark of the guided denoising loop (BASELINE.json metric: guided img-steps/s; DDPM-256, 50-step schedules).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl native|reference] [--config 1|2|3|4]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline workload (BASELINE.json configs[1], per GPU): DDPM-256 UNet2DModel (random-init, seed 0), batch 8, the guided
@@ -210,7 +211,14 @@ def main():
     ap.add_argument("--profile-out", default=None, help="write the per-op CUDA-event profile (JSON) here")
     ap.add_argument("--precision", default=None, choices=["fp16", "bf16", "fp32"],
                     help="noise predictor: 16-bit operands (default: what the library is built for, fp16) or the fp32-accurate split mode")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last timed pass of the headline returned as DIR/<name>.npy "
+                         "(float32, rank 0's shard; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the native arm's outputs; --impl reference has none")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -246,13 +254,15 @@ def main():
         return v
 
     def timed(fn, passes):
-        """passes x fn() between CUDA events on the launching (current) stream, barrier + synchronize on both sides, max over ranks."""
+        """passes x fn() between CUDA events on the launching (current) stream, barrier + synchronize on both sides, max over ranks.
+        -> (ms, launches, what the final pass returned)."""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         n0 = _C.launch_count()
         e0.record()
-        for _ in range(passes):
+        for _ in range(passes - 1):
             fn()
+        last = fn()     # each earlier pass's result is freed as it returns; only the final one is kept
         e1.record()
         barrier()
         launches = _C.launch_count() - n0
@@ -260,12 +270,16 @@ def main():
             lt = torch.tensor([launches], device=dev, dtype=torch.int64)
             dist.all_reduce(lt)
             launches = int(lt.item())
-        return max_over_ranks(e0.elapsed_time(e1)), launches
+        return max_over_ranks(e0.elapsed_time(e1)), launches, last
     c.barrier, c.timed = barrier, timed
 
     headline = {1: config1, 2: config2, 3: config3, 4: config4}[args.config]
     with ClockSampler(local_rank, enabled=(rank == 0)) as clk:
         res = headline(c, precision, args.batch if args.config == 2 else None, args.steps, args.warmup, headline=True)
+    last_output = res.pop("last_output", None)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last_output, args.dump_outputs)
+    del last_output
     line = None
     if rank == 0:
         line = {"metric": METRIC if args.config == 2 else res["metric"], "value": res["value"], "unit": UNIT, "n_gpus": world,
@@ -340,6 +354,22 @@ def pass_result(c, name, B, D, K, ms_dev, ms_e2e, launches, h2d, d2h, cfg, flops
     return out
 
 
+def dump_outputs(out, out_dir, max_elems=4 << 20):
+    """Writes the EditorOutput of the last timed pass as out_dir/<field>.npy in float32: ``imgs`` and the per-step histories
+    ``pred_original_samples`` / ``model_outputs`` stacked to (steps, ...).  An array of more than max_elems elements (16 MB)
+    is replaced by a fixed sample: the same seeded element positions of every step, shape (steps, n) ((1, n) for ``imgs``),
+    so that two builds compare element for element and the three files stay under 48 MB together."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        a = (v if torch.is_tensor(v) else torch.stack(list(v))).detach().float()
+        if a.numel() > max_elems:
+            rows = a.reshape(a.shape[0] if not torch.is_tensor(v) else 1, -1)
+            pick = torch.randperm(rows.shape[1], generator=torch.Generator().manual_seed(0))[:max_elems // rows.shape[0]]
+            a = rows[:, pick.sort().values.to(rows.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
+
+
 # ----- BASELINE configs[1]: the headline
 def config2(c, precision, B, K, W, headline=False):
     from attr_functions import SingleColorAttrFunc
@@ -384,8 +414,8 @@ def config2(c, precision, B, K, W, headline=False):
     for _ in range(W):      # W untimed passes of each shape (plans, function attributes, allocator growth, lazy NCCL setup)
         run(False)
     run(True)
-    ms_dev, launches = c.timed(lambda: run(False), K)
-    ms_e2e, _ = c.timed(lambda: run(True), K)
+    ms_dev, launches, _ = c.timed(lambda: run(False), K)
+    ms_e2e, _, last = c.timed(lambda: run(True), K)
     h2d = (x_host.numel() + zs_host.numel()) * 4
     d2h = (out_host.numel() + x0_host.numel()) * 4
     res = pass_result(c, "BASELINE configs[1]", B, D, K, ms_dev, ms_e2e, launches, h2d, d2h, workload_config(args, B, D),
@@ -394,6 +424,8 @@ def config2(c, precision, B, K, W, headline=False):
                       "step on a side stream, overlapped with the next UNet forward, joined before the end event) and the final "
                       "images land in pinned host memory inside the timed region; bytes are per bench step (pass)")
     res["precision"] = precision
+    if headline and c.args.dump_outputs:
+        res["last_output"] = last
     if headline and rank == 0:
         res["rooflines"] = rooflines(c, wrapper, sch, x_dev, precision)
     del pipe, wrapper
@@ -534,18 +566,21 @@ def config1(c, precision, B, K, W, headline=False):
                               x0_history_out=x0_host if from_host else None)
         if from_host:
             out_host.copy_(out.imgs, non_blocking=True)
+        return out
     for _ in range(W):
         run(False)
     run(True)
     D = max(T_INFER, D)    # eta = 0 walks the whole schedule
-    ms_dev, launches = c.timed(lambda: run(False), K)
-    ms_e2e, _ = c.timed(lambda: run(True), K)
+    ms_dev, launches, _ = c.timed(lambda: run(False), K)
+    ms_e2e, _, last = c.timed(lambda: run(True), K)
     cfg = {"workload": f"BASELINE configs[0] on the GPU: DDPM-256, colour-guided DDIM (eta=0, clip_sample) {D} steps, batch {B}",
            "batch_per_gpu": B, "guidance": "SingleColorAttrFunc(target=0.8,color_idx=0,loss_scale=100)"}
     res = pass_result(c, "BASELINE configs[0] (GPU)", B, D, K, ms_dev, ms_e2e, launches, x_host.numel() * 4,
                       (out_host.numel() + x0_host.numel()) * 4, cfg, w.unet.flops_per_sample, "as the headline")
     res["metric"] = "guided img-steps/s (DDPM-256, colour-guided DDIM-50, batch 1)"
     res["precision"] = precision
+    if headline and c.args.dump_outputs:
+        res["last_output"] = last
     res["cuda_graph"] = bool(w.unet._graph_on)
     del pipe, w
     return res
@@ -567,7 +602,7 @@ def batch_sweep(c, precision, batches=(2, 4, 16, 32, 64, 128, 256), D=4, K=2):
         x = torch.randn(B, 3, 256, 256, generator=torch.Generator().manual_seed(77 + c.rank)).to(c.dev)
         run = lambda: pipe.edit_image(xt=x, eta=0.0, attr_func=f, prog_bar=False, output_type="tensor")   # noqa: E731
         run()
-        ms, _ = c.timed(run, K)
+        ms, _, _ = c.timed(run, K)
         points.append({"batch_per_gpu": B, "value": c.world * B * D * K / (ms * 1e-3), "ms_per_denoising_step": ms / (K * D),
                        "achieved_tflops_per_gpu": B * w.unet.flops_per_sample / (ms / (K * D) * 1e-3) / 1e12})
         del pipe, w, x
@@ -601,11 +636,12 @@ def config3(c, precision, B, K, W, headline=False):
         out = pipe.edit_image(xt=x, attr_func=f, prog_bar=False, output_type="tensor", mask=mask)
         if from_host:
             out_host.copy_(out.imgs, non_blocking=True)
+        return out
     for _ in range(W):
         run(False)
     run(True)
-    ms_dev, launches = c.timed(lambda: run(False), K)
-    ms_e2e, _ = c.timed(lambda: run(True), K)
+    ms_dev, launches, _ = c.timed(lambda: run(False), K)
+    ms_e2e, _, last = c.timed(lambda: run(True), K)
     fl = w.unet.flops_per_sample + w.vqvae.flops_per_sample   # gradient mode: the decoder figure counts forward + backward
     cfg = {"workload": f"BASELINE configs[2]: LDM-CelebAHQ layout (64x64x3 latent, random-init), masked colour guidance through the "
                        f"native VQ decoder (forward + latent gradient), batch {B}, {D} DDIM steps per pass + one final decode",
@@ -614,6 +650,8 @@ def config3(c, precision, B, K, W, headline=False):
                       "edit_image from a pinned host latent batch; decoded images copied to pinned host memory")
     res["metric"] = "guided img-steps/s (LDM 64x64x3 latent, mask guidance through the VQ decoder)"
     res["precision"] = precision
+    if headline and c.args.dump_outputs:
+        res["last_output"] = last
     res["max_memory_gb"] = torch.cuda.max_memory_allocated() / 1e9
     del pipe, w
     return res
@@ -645,11 +683,12 @@ def config4(c, precision, B, K, W, headline=False):
             out_host.copy_(out.imgs, non_blocking=True)
         if c.world > 1:
             c.gather(out.imgs, c.world * B)
+        return out
     for _ in range(W):
         run(False)
     run(True)
-    ms_dev, launches = c.timed(lambda: run(False), K)
-    ms_e2e, _ = c.timed(lambda: run(True), K)
+    ms_dev, launches, _ = c.timed(lambda: run(False), K)
+    ms_e2e, _, last = c.timed(lambda: run(True), K)
     fl = 2 * w.unet.flops_per_sample + w.vae.flops_per_sample
     cfg = {"workload": f"BASELINE configs[3]: Stable Diffusion 1.x layout (64x64x4 latent, random-init), CFG 7.5 (doubled latent batch, "
                        f"precomputed (2,77,768) text embedding) + classifier guidance through the native KL decoder and ResNet-50 "
@@ -660,6 +699,8 @@ def config4(c, precision, B, K, W, headline=False):
                       "edit_image from a pinned host latent batch; decoded 512x512 images copied to pinned host memory")
     res["metric"] = "guided img-steps/s (SD-1.x 64x64x4 latent, CFG + classifier guidance)"
     res["precision"] = precision
+    if headline and c.args.dump_outputs:
+        res["last_output"] = last
     res["max_memory_gb"] = torch.cuda.max_memory_allocated() / 1e9
     del pipe, w, predictor
     return res
