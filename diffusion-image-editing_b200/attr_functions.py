@@ -12,6 +12,10 @@ predicted clean image:  x <- x + (-d(loss_scale*loss)/dx) * alphas_cumprod[t]**2
 * Any other strategy (user subclasses, network losses) evaluates ``loss`` with torch autograd on the device - exactly the
   reference's procedure - and the resulting gradient is applied by a CUDA kernel.  That is the extension contract of the
   reference: subclass, implement ``loss``, register.
+* ``mask_pred_original_sample=True, use_lpips=True`` needs the distance network as ``lpips_model=`` (``models.get_lpips``,
+  the native LPIPS-vgg, or any callable ``(in0, in1) -> (B, 1, 1, 1)``): the loss is ``loss(mask * x0') +
+  lambda_ * LPIPS(1 - mask * x0', x_0)``, differentiated by autograd through the native LPIPS node.  Without
+  ``lpips_model`` ``use_lpips`` raises, as it must without VGG weights.
 """
 from abc import ABC, abstractmethod
 
@@ -62,15 +66,19 @@ class AttrFunc(ABC):
 
     def __init__(self, loss_scale: float = 1, t1: int = 0, t2: int = 50, nudge_xt=True, nudge_zt=False,
                  per_sample: bool = False, **kwargs) -> None:
+        lpips_model = kwargs.pop("lpips_model", None)
         self.kwargs = kwargs
         self.loss_scale = loss_scale
         self.t1, self.t2 = t1, t2
         self.nudge_xt, self.nudge_zt = nudge_xt, nudge_zt
         self.per_sample = per_sample
         if kwargs.get("use_lpips", False):
-            raise NotImplementedError("LPIPS regularisation needs the lpips package and VGG weights, "
-                                      "neither of which is available offline; use use_l2=True")
-        if kwargs.get("use_l2", False):
+            if lpips_model is None:
+                raise NotImplementedError("LPIPS regularisation needs the lpips package and VGG weights, "
+                                          "neither of which is available offline; pass lpips_model= "
+                                          "(models.get_lpips) or use use_l2=True")
+            self.metric = lpips_model
+        elif kwargs.get("use_l2", False):
             self.metric = l2_norm
 
     @property
@@ -90,12 +98,22 @@ class AttrFunc(ABC):
         if kwargs.get("mask_pred_original_sample", False):
             lambda_, mask, x_0 = kwargs.get("lambda_"), kwargs.get("mask"), kwargs.get("x_0")
             if kwargs.get("use_lpips", False):
-                raise NotImplementedError("LPIPS is unavailable offline")
+                return self.loss(mask * pred_original_sample) + lambda_ * apply_lpips(
+                    1 - mask * pred_original_sample, x_0, self._lpips_model())
             if kwargs.get("use_l2", False):
                 return self.loss(mask * pred_original_sample) + lambda_ * l2_norm(
                     1 - mask * pred_original_sample, x_0)
             raise ValueError("No metric specified")
         return self.loss(pred_original_sample, **kwargs)
+
+    def _has_lpips(self) -> bool:
+        m = getattr(self, "metric", None)
+        return m is not None and m is not l2_norm
+
+    def _lpips_model(self):
+        if not self._has_lpips():
+            raise NotImplementedError("LPIPS is unavailable offline without lpips_model= (models.get_lpips)")
+        return self.metric
 
     def edit_attr_grad(self, attr_grad, **kwargs):
         if kwargs.get("mask_attr_grad", False):
@@ -142,6 +160,8 @@ class AttrFunc(ABC):
                   mask_grad=bool(kwargs.get("mask_attr_grad", False)),
                   n_mean=(xt.shape[-1] * xt.shape[-2]) if self.per_sample else None)
         if kwargs.get("mask_pred_original_sample", False):
+            if kwargs.get("use_lpips", False) and self._has_lpips():
+                return None             # LPIPS regulariser: not one of the fused kernels
             if not kwargs.get("use_l2", False):
                 if kwargs.get("use_lpips", False):
                     raise NotImplementedError("LPIPS is unavailable offline")
@@ -192,6 +212,59 @@ class AttrFunc(ABC):
             return None                # a mask that does not match the latent: the generic path reports it
         return ops.apply_latent_guidance(xt, d_lat, chain, coeffs.sqrt_a_t, coeffs.a_t_sq, mask=gmask)
 
+    def _apply_native_lpips(self, xt, model_output, coeffs, model, **kwargs):
+        """Built-in colour strategies with the LPIPS regulariser (mask_pred_original_sample + use_lpips) on the native
+        LPIPS network: x0' kernel (-> native decoder forward) -> LPIPS forward on 1 - mask * img (formed by its input
+        packer) and backward -> one kernel for mask * d colour(mask * img) + lambda_ * d LPIPS -> (native decoder backward)
+        -> update kernel.  No autograd.  With B > 1 images the regulariser is lambda_ * sum_b LPIPS_b (the reference's
+        autograd call accepts only one image, its loss being (B, 1, 1, 1)).  Returns None when the strategy / model / shapes
+        do not qualify (autograd path)."""
+        from b200edit.lpips import LPIPS
+        spec, lp = self.colour_spec(), getattr(self, "metric", None)
+        if (spec is None or not isinstance(lp, LPIPS) or self.nudge_zt or not self.nudge_xt or self.per_sample
+                or not kwargs.get("mask_pred_original_sample", False) or not kwargs.get("use_lpips", False)):
+            return None
+        mask, x_0, lam = kwargs.get("mask"), kwargs.get("x_0"), kwargs.get("lambda_")
+        if kwargs.get("mask_attr_grad", False) and mask is None:
+            raise ValueError("No mask specified")
+        if mask is None or x_0 is None or lam is None or not torch.is_tensor(mask) or not torch.is_tensor(x_0):
+            return None
+        dec, chain = None, 1.0
+        if not _identity_decoder(model):
+            nd = getattr(model, "native_decoder", None)
+            nd = nd() if callable(nd) else None
+            if nd is None:
+                return None
+            dec, chain = nd
+            if xt.shape[0] > dec.max_batch:
+                return None
+        S = lp.config.input_size
+        B = xt.shape[0]
+        if (B > lp.max_batch or mask.dim() != 4 or mask.shape[0] not in (1, B) or mask.shape[1] not in (1, 3)
+                or tuple(mask.shape[2:]) != (S, S) or x_0.dim() != 4 or tuple(x_0.shape[1:]) != (3, S, S)
+                or x_0.shape[0] not in (1, B)):
+            return None
+        targets, weights = spec
+        lat = ops.pred_x0(xt, model_output, coeffs.sqrt_a_t, coeffs.sqrt_b_t)
+        if dec is None:
+            img = lat
+        else:
+            if chain != 1.0:
+                lat = ops.axpby(lat, lat, chain, 0.0)
+            img = dec.decode_keep(lat)
+        if tuple(img.shape[1:]) != (3, S, S):
+            return None
+        with torch.no_grad():
+            lp(img, x_0, mask=mask)
+            d_lp = lp.input_grad(torch.ones(B, dtype=torch.float32, device=img.device))
+        d_img = ops.lpips_guidance_grad(img, mask, d_lp, targets, weights, self.loss_scale,
+                                        img.shape[-1] * img.shape[-2] * B, lam)
+        d_lat = d_img if dec is None else dec.latent_grad(d_img)
+        gmask = mask if kwargs.get("mask_attr_grad", False) else None
+        if gmask is not None and tuple(gmask.shape[1:]) != tuple(xt.shape[1:]):
+            return None                # a mask that does not match the sample: the generic path reports it
+        return ops.apply_latent_guidance(xt, d_lat, chain, coeffs.sqrt_a_t, coeffs.a_t_sq, mask=gmask)
+
     def in_window(self, step_idx: int) -> bool:
         return self.t1 <= step_idx < self.t2
 
@@ -203,6 +276,9 @@ class AttrFunc(ABC):
         coeffs = model.scheduler.coeffs(int(timestep), 0.0, "ddim")
         fk = self.fused_kwargs(xt, model, **kwargs)
         if fk is None:
+            out = self._apply_native_lpips(xt, model_output, coeffs, model, **kwargs)
+            if out is not None:
+                return out, zt
             out = self._apply_native_decoder(xt, model_output, coeffs, model, **kwargs)
             if out is not None:
                 return out, zt

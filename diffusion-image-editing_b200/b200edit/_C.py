@@ -67,6 +67,10 @@ class ResNetConfig(C.Structure):
                 ("precision", C.c_int32)]
 
 
+class LpipsConfig(C.Structure):
+    _fields_ = [("input_size", C.c_int32), ("precision", C.c_int32)]
+
+
 _P, _I64, _I, _F, _SZ = C.c_void_p, C.c_int64, C.c_int, C.c_float, C.c_size_t
 
 # name -> (restype, argtypes); every symbol include/b200edit.h declares
@@ -83,6 +87,7 @@ PROTOTYPES = {
     "b2e_apply_guidance_grad_f32": (_I, [_P, _P, _P, _I64, _I64, _I, _F, _P]),
     "b2e_color_loss_grad_workspace_bytes": (_SZ, []),
     "b2e_color_loss_grad_f32": (_I, [_P, _P, _P, _P, _I64, _I64, _I64, C.POINTER(ColorGradParams), _P, _SZ, _P]),
+    "b2e_lpips_guidance_grad_f32": (_I, [_P, _P, _P, _P, _I64, _I64, _I64, C.POINTER(ColorGradParams), _P]),
     "b2e_apply_latent_guidance_f32": (_I, [_P, _P, _P, _I64, _I64, _I, _F, _F, _F, _P]),
     "b2e_pred_x0_f32": (_I, [_P, _P, _P, _I64, _F, _F, _P]),
     "b2e_renoise_f32": (_I, [_P, _P, _P, _I64, _F, _F, _F, _F, _P]),
@@ -110,6 +115,10 @@ PROTOTYPES = {
     "b2e_clip_forward": (_I, [_P, _P, _I64, _P, _I64, _P]),
     "b2e_resnet_create": (_I, [C.POINTER(ResNetConfig), _I64, C.POINTER(_P)]),
     "b2e_resnet_backward": (_I, [_P, _P, _P, _I64, _P]),
+    "b2e_lpips_create": (_I, [C.POINTER(LpipsConfig), _I64, C.POINTER(_P)]),
+    "b2e_lpips_set_reference": (_I, [_P, _P, _I64, _P]),
+    "b2e_lpips_forward": (_I, [_P, _P, _P, _I64, _P, _I64, _P]),
+    "b2e_lpips_backward": (_I, [_P, _P, _P, _I64, _P]),
     "b2e_unet_enable_grad": (_I, [_P, _I]),
     "b2e_vqdec_backward": (_I, [_P, _P, _P, _I64, _P]),
     "b2e_unet_destroy": (None, [_P]),

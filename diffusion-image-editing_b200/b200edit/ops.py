@@ -176,12 +176,7 @@ def apply_guidance_grad(x, neg_grad, a_t_sq: float, mask=None):
     return x
 
 
-def color_loss_grad(img, targets, weights, loss_scale, n_mean, mask=None, x_ref=None, lambda_=None):
-    """d(loss_scale * colour loss)/d(decoded image) in closed form (guidance through a latent decoder; the result feeds the
-    decoder's native backward pass).  targets / weights as in guided_step; n_mean = elements the loss mean runs over.
-    mask + x_ref + lambda_: the masked-prediction + L2-regularised variant (mask_pred_original_sample, use_l2)."""
-    img = _f32(img, "decoded image")
-    B, Cc, H, W = img.shape
+def _color_grad_params(targets, weights, loss_scale, n_mean, Cc):
     p = _C.ColorGradParams()
     for c in range(4):
         t = targets[c] if c < len(targets) else None
@@ -190,6 +185,33 @@ def color_loss_grad(img, targets, weights, loss_scale, n_mean, mask=None, x_ref=
         p.target[c] = float(t) if t is not None else 0.0
         p.k[c] = float(torch.tensor(float(loss_scale), dtype=torch.float32) * torch.tensor(float(w), dtype=torch.float32)
                        / torch.tensor(float(n_mean), dtype=torch.float32)) if t is not None else 0.0
+    return p
+
+
+def lpips_guidance_grad(img, mask, d_lpips, targets, weights, loss_scale, n_mean, lambda_):
+    """d(loss_scale * (colour loss(mask * img) + lambda_ * LPIPS(1 - mask * img, x_0))) / d(img) in one kernel, given
+    d_lpips = d(LPIPS) / d(img) from the native LPIPS backward (its -mask chain included).  mask (1 | B, C, H, W)."""
+    img, d_lpips = _f32(img, "decoded image"), _f32(d_lpips, "d_lpips")
+    B, Cc, H, W = img.shape
+    mask = _f32(mask, "mask")
+    if mask.shape[1:] != img.shape[1:]:
+        mask = mask.expand(mask.shape[0], Cc, H, W).contiguous()
+    p = _color_grad_params(targets, weights, loss_scale, n_mean, Cc)
+    p.lam_scale = float(loss_scale) * float(lambda_)
+    p.mask_batched = int(mask.shape[0] == B and B > 1)
+    out = torch.empty_like(img)
+    check(lib.b2e_lpips_guidance_grad_f32(_p(img), _p(mask), _p(d_lpips), _p(out), B, Cc, H * W, C.byref(p), _stream()),
+          "lpips_guidance_grad")
+    return out
+
+
+def color_loss_grad(img, targets, weights, loss_scale, n_mean, mask=None, x_ref=None, lambda_=None):
+    """d(loss_scale * colour loss)/d(decoded image) in closed form (guidance through a latent decoder; the result feeds the
+    decoder's native backward pass).  targets / weights as in guided_step; n_mean = elements the loss mean runs over.
+    mask + x_ref + lambda_: the masked-prediction + L2-regularised variant (mask_pred_original_sample, use_l2)."""
+    img = _f32(img, "decoded image")
+    B, Cc, H, W = img.shape
+    p = _color_grad_params(targets, weights, loss_scale, n_mean, Cc)
     ws = None
     ws_bytes = 0
     if x_ref is not None:

@@ -135,6 +135,18 @@ struct b2e_unet {
     float *f1_w = nullptr, *f2_w = nullptr;
   } bs;
   const float* in_dlogits = nullptr;
+  // LPIPS mode (b2e_lpips_create): scaling layer -> VGG-16 features[0:30] (conv1_1 as a 1x1 convolution over the im2col
+  // input, ReLU in every epilogue) -> distance head at relu1_2 .. relu5_3 against the reference's cached normalised
+  // features; backward: d(dist) -> d(input).  The regulariser of the masked-prediction guidance (use_lpips)
+  bool lpips = false;
+  b2e_lpips_config lcfg{};
+  std::vector<ConvL> vgg;                 // the thirteen convolutions; vgg[0] reads the im2col tensor
+  float* lin_w[5] = {};                   // lin{k}.model.1.weight, C_k floats
+  float* lp_const = nullptr;              // shift[3], scale[3], diag(1 / scale) (3 x 3): scaling layer and its adjoint
+  size_t lp_ref_off[5] = {};             // reference cache (workspace offset 0): normalised tap features, fp32 [max_batch][HW_k][C_k]
+  int64_t lp_ref_B = -1;                  // images in the cache (-1: none)
+  bool lp_ref_mode = false;               // the forward fills the cache instead of computing distances
+  const float* lp_mask = nullptr; int lp_mask_batched = 0;   // per call: input 1 - mask * x
   int enc_q = 0;
   float *qc_w = nullptr, *qc_b = nullptr;   // [enc_q][enc_q], [enc_q]
   float *codebook = nullptr, *pq_w = nullptr, *pq_b = nullptr;   // [n_codes][latent], [latent][latent], [latent]
@@ -222,7 +234,7 @@ struct b2e_unet {
     ConvL dd;
     const int PL = this->PL;
     // (a <= 16-channel output, i.e. conv_out, receives its gradient as a 64-channel padded NHWC tensor)
-    if (decoder || resnet) { c.dg = make_dgrad(cin, cout > 16 ? c.cout_pad : kConvBlockK, k); dd = dgrads[c.dg]; cc.dg = c.dg; }
+    if (decoder || resnet || lpips) { c.dg = make_dgrad(cin, cout > 16 ? c.cout_pad : kConvBlockK, k); dd = dgrads[c.dg]; cc.dg = c.dg; }
     add_param(name + ".weight", (int64_t)cout * cin * k * k, (int64_t)cin * k * k, [cc, dd, PL, src0](const float* src, cudaStream_t st) {
       int rc;
       if (PL == 3 && src0 > 0 && cc.k == 1) {
@@ -1019,6 +1031,242 @@ int build_program_resnet(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* 
   return B2E_OK;
 }
 
+// LPIPS (lpips v0.1, net='vgg') trunk: VGG-16 features[0:30] under lpips.LPIPS().state_dict() names.  conv1_1 is a 1x1
+// convolution over the im2col input (27 of 64 columns) that the packer forms from the scaled input, because the zero
+// padding of the convolution belongs to the scaled space.  Every convolution has its dgrad twin.
+constexpr int kVggStages = 5;
+constexpr int kVggConvs[kVggStages] = {2, 2, 3, 3, 3};
+constexpr int kVggWidth[kVggStages] = {64, 128, 256, 512, 512};
+
+int build_model_lpips(b2e_unet* m) {
+  const int PL = m->PL;
+  m->in_im2col = true;
+  int idx = 0, cin = 3, n = 0;
+  for (int s = 0; s < kVggStages; ++s) {
+    for (int j = 0; j < kVggConvs[s]; ++j, ++n) {
+      const std::string name = "net.slice" + std::to_string(s + 1) + "." + std::to_string(idx);
+      const int cout = kVggWidth[s];
+      if (n == 0) {
+        ConvL ci;
+        ci.cin = ci.cin_pad = kConvBlockK; ci.cout = cout; ci.k = 1; ci.cout_pad = conv_cout_pad(cout); ci.row_len = kConvBlockK * PL;
+        ci.w = m->dmalloc<f16>((size_t)ci.cout_pad * ci.row_len);
+        ci.b = m->dmalloc<float>(ci.cout_pad);
+        ci.dg = m->make_dgrad(kConvBlockK, ci.cout_pad, 1);   // gradient w.r.t. the 64 im2col columns
+        const ConvL cd = m->dgrads[ci.dg];
+        m->add_param(name + ".weight", (int64_t)cout * 27, 27, [ci, cd, PL](const float* src, cudaStream_t st) {
+          const float ws = PL == 3 ? b2e_unet::kSplitWScale : 1.f;
+          int rc = conv_pack_weight(src, ci.w, ci.cout, 3, 3, 3, ci.row_len, 0, st, 0, 0, 0, ws);
+          if (!rc && PL == 3) rc = conv_pack_weight(src, ci.w, ci.cout, 3, 3, 3, ci.row_len, kConvBlockK, st, 0, 0, 0, ws);
+          if (!rc && PL == 3) rc = conv_pack_weight(src, ci.w, ci.cout, 3, 3, 3, ci.row_len, 2 * kConvBlockK, st, 0, 0, 1, ws);
+          if (!rc) rc = conv_pack_weight_im2col_T(src, cd.w, ci.cout, 3, cd.row_len, st);
+          return rc;
+        });
+        m->add_f32(name + ".bias", ci.b, cout, 27);
+        m->vgg.push_back(ci);
+      } else {
+        m->vgg.push_back(m->make_conv(name, cin, cout, 3));
+      }
+      cin = cout;
+      idx += 2;                  // conv, ReLU
+    }
+    idx += 1;                    // max pool
+  }
+  for (int k = 0; k < kVggStages; ++k) {
+    m->lin_w[k] = m->dmalloc<float>(kVggWidth[k]);
+    m->add_f32("lin" + std::to_string(k) + ".model.1.weight", m->lin_w[k], kVggWidth[k], kVggWidth[k]);
+  }
+  const float shift[3] = {-.030f, -.088f, -.188f}, scale[3] = {.458f, .448f, .450f};
+  float c[15] = {};
+  for (int i = 0; i < 3; ++i) { c[i] = shift[i]; c[3 + i] = scale[i]; c[6 + 4 * i] = 1.f / scale[i]; }
+  m->lp_const = m->dmalloc<float>(15);
+  if (m->lp_const && cudaMemcpy(m->lp_const, c, sizeof(c), cudaMemcpyHostToDevice) != cudaSuccess) m->build_error = B2E_CUDA_ERROR;
+  return m->build_error;
+}
+
+// Launch lists of the LPIPS network for batch B.  Forward: input packing (1 - mask * x, scaling layer, im2col) -> VGG
+// trunk -> one head launch per tap -> fixed-order final sum.  In reference mode (b2e_lpips_set_reference) the same list
+// writes the normalised tap features to the cache instead.  Backward: head gradients joined tap by tap (relu5_3 ->
+// relu1_2) into the dgrad chain, max-pool backward, im2col / scaling-layer / mask adjoint.
+int build_program_lpips(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
+  Arena ar;
+  ar.reset(ws, ws_bytes);
+  const bool dry = ar.dry;
+  std::vector<b2e_unet::Op> fwd, bwd;
+  std::vector<b2e_unet::Op>* cur = &fwd;
+  double flops = 0;
+  int rc = B2E_OK;
+  const int PL = m->PL, S = m->lcfg.input_size;
+  int tap_hw[kVggStages];
+  for (int k = 0; k < kVggStages; ++k) tap_hw[k] = (S >> k) * (S >> k);
+  // the reference cache comes first, sized for max_batch: same offset for every batch the program is rebuilt for
+  size_t ref_floats = 0;
+  for (int k = 0; k < kVggStages; ++k) { m->lp_ref_off[k] = ref_floats; ref_floats += (size_t)m->max_batch * tap_hw[k] * kVggWidth[k]; }
+  float* ref = (float*)ar.alloc(ref_floats * sizeof(float));
+  auto talloc = [&](int N, int H, int W, int C, int planes = 1) {
+    Tensor t; t.N = N; t.H = H; t.W = W; t.C = C; t.Cr = C; t.bytes = (size_t)N * H * W * C * planes * sizeof(f16);
+    t.p = (f16*)ar.alloc(t.bytes);
+    return t;
+  };
+  const size_t split_bytes = (size_t)kNumSMs * kConvBlockM * 128 * sizeof(float);
+  float* split_ws = (float*)ar.alloc(split_bytes);
+  int* split_cnt = (int*)ar.alloc(sizeof(int) * 1024);
+  if (!dry) cudaMemset(split_cnt, 0, sizeof(int) * 1024);
+  LpipsTaps taps{};
+  int nslots = 0;
+  for (int k = 0; k < kVggStages; ++k) { taps.n[k] = lpips_head_blocks(tap_hw[k]); taps.off[k] = nslots; taps.hw[k] = tap_hw[k]; nslots += taps.n[k]; }
+  double* partial = (double*)ar.alloc(sizeof(double) * B * nslots);
+  float* hmax = (float*)ar.alloc(sizeof(float) * B);      // largest head-gradient element per image (gradient scale)
+  auto conv = [&](const ConvL& L, const Tensor& x, Tensor* out, const char* what) {
+    if (rc) return;
+    *out = talloc(B, x.H, x.W, L.cout_pad, PL);
+    flops += 2.0 * B * x.H * x.W * (double)L.cout_pad * L.k * L.k * x.C * PL;
+    if (dry) return;
+    if (PL * L.k * L.k * x.C != L.row_len) {
+      rc = B2E_INVALID_ARG; set_error("lpips: operand widths do not match the packed weights (%s)", what); return;
+    }
+    ConvDesc d;
+    d.s0 = ConvSrc{x.p, x.C * PL};
+    d.out_planes = PL;
+    d.N = B; d.H = x.H; d.W = x.W; d.ksize = L.k; d.stride = 1;
+    d.w_packed = L.w; d.Cout = L.cout_pad; d.out_f16 = out->p;
+    d.split_ws = split_ws; d.split_ws_bytes = split_bytes; d.split_counters = split_cnt;
+    ConvPlan pl;
+    rc = conv_plan_build(&pl, d);
+    if (rc) return;
+    ConvEpilogue ep;
+    ep.bias = L.b; ep.relu = 1;
+    if (PL == 3) ep.acc_scale = 1.f / b2e_unet::kSplitWScale;
+    char desc[160];
+    snprintf(desc, sizeof(desc), "%s: conv%dx%d %dx%d cin%d cout%d bn%d%s +relu", what, L.k, L.k, x.H, x.W, x.C, L.cout, pl.block_n,
+             pl.halo ? " halo" : pl.pair ? " pair" : "");
+    cur->push_back({[pl, ep](cudaStream_t st) { return conv_launch(pl, ep, st); }, 0, pl.flops, 0.0, desc});
+  };
+  auto ew = [&](std::function<int(cudaStream_t)> fn, double bytes, const char* what) {
+    if (!dry && !rc) cur->push_back({std::move(fn), 3, 0.0, bytes, what});
+  };
+
+  // ---------------- forward
+  ew([hmax, B](cudaStream_t st) -> int { B2E_CUDA(cudaMemsetAsync(hmax, 0, sizeof(float) * B, st)); return (int)B2E_OK; }, 4.0 * B,
+     "lpips: clear the head-gradient bound");
+  Tensor cols = talloc(B, S, S, kConvBlockK, PL);
+  ew([m, cols, B, S, PL](cudaStream_t st) {
+       return pack_input_launch(m->in_x, cols.p, B, 3, S, S, kConvBlockK, true, st, PL, nullptr, m->lp_const, m->lp_const + 3,
+                                m->lp_mask, m->lp_mask_batched); },
+     (double)B * S * S * 12.0 + (double)cols.bytes, "input: 1 - mask * x, scaling layer, im2col");
+  std::vector<Tensor> acts(m->vgg.size());
+  Tensor tap[kVggStages], h = cols;
+  uint16_t* pidx[kVggStages] = {};
+  int li = 0;
+  for (int s = 0; s < kVggStages && !rc; ++s) {
+    if (s > 0) {
+      Tensor p = talloc(B, h.H / 2, h.W / 2, h.C, PL);
+      pidx[s - 1] = (uint16_t*)ar.alloc(sizeof(uint16_t) * (size_t)B * p.H * p.W * (p.C / 8));
+      const Tensor hh = h;
+      uint16_t* ix = pidx[s - 1];
+      ew([hh, p, ix, B, PL](cudaStream_t st) { return maxpool2x2_launch(hh.p, p.p, ix, B, hh.H, hh.W, hh.C, st, PL); },
+         1.25 * (double)hh.bytes, "maxpool 2x2");
+      h = p;
+    }
+    for (int j = 0; j < kVggConvs[s]; ++j, ++li) {
+      conv(m->vgg[li], h, &acts[li], "vgg");
+      h = acts[li];
+    }
+    tap[s] = h;
+  }
+  for (int k = 0; k < kVggStages && !rc; ++k) {
+    const Tensor t = tap[k];
+    const int slot0 = taps.off[k];
+    float* rk = ref + m->lp_ref_off[k];
+    ew([m, t, k, rk, partial, nslots, slot0, hmax, B, PL](cudaStream_t st) {
+         const bool rmode = m->lp_ref_mode;
+         return lpips_head_launch(t.p, B, t.C, t.H * t.W, PL, m->lin_w[k], rk, rmode ? 0 : m->lp_ref_B != 1, partial, nslots, slot0,
+                                  rmode ? 0 : 1, hmax, st); },
+       (double)t.bytes + 4.0 * B * t.H * t.W * t.C, "lpips head (normalise, lin, spatial sum)");
+  }
+  ew([m, partial, nslots, taps, B](cudaStream_t st) {
+       return m->lp_ref_mode ? (int)B2E_OK : lpips_finalize_launch(partial, nslots, taps, m->out_eps, B, st); },
+     8.0 * B * nslots, "lpips: sum over taps");
+
+  // ---------------- backward: d(dist) -> d(input)
+  if (!rc && m->grad) {
+    cur = &bwd;
+    auto dconv = [&](const ConvL& L, const Tensor& dy, Tensor* dx) {
+      if (rc) return;
+      const ConvL& D = m->dgrads[L.dg];
+      *dx = talloc(B, dy.H, dy.W, D.cout_pad);
+      flops += 2.0 * B * dy.H * dy.W * (double)D.cout_pad * D.row_len;
+      if (dry) return;
+      if (D.k * D.k * dy.C != D.row_len) { rc = B2E_INVALID_ARG; set_error("lpips backward: operand widths do not match"); return; }
+      ConvDesc d;
+      d.s0 = ConvSrc{dy.p, dy.C};
+      d.N = B; d.H = dy.H; d.W = dy.W; d.ksize = D.k; d.stride = 1;
+      d.w_packed = D.w; d.Cout = D.cout_pad; d.out_f16 = dx->p;
+      d.split_ws = split_ws; d.split_ws_bytes = split_bytes; d.split_counters = split_cnt;
+      ConvPlan pl;
+      rc = conv_plan_build(&pl, d);
+      if (rc) return;
+      char desc[160];
+      snprintf(desc, sizeof(desc), "vgg: dgrad conv%dx%d %dx%d cin%d cout%d", D.k, D.k, dy.H, dy.W, dy.C, D.cout);
+      cur->push_back({[pl](cudaStream_t st) { return conv_launch(pl, ConvEpilogue{}, st); }, 0, pl.flops, 0.0, desc});
+    };
+    // gradient scale record (grad_scale_launch) from the largest head-gradient element the forward measured (it includes
+    // the 1 / ||f|| of the normalisation Jacobian, so the scale follows the feature norms of the actual weights)
+    float* gsc = (float*)ar.alloc(sizeof(float) * 4);
+    float* gprod = (float*)ar.alloc(sizeof(float) * B);
+    if (!dry) cudaMemset(gsc, 0, sizeof(float) * 4);
+    ew([m, hmax, gprod, gsc, B](cudaStream_t st) { return lpips_grad_scale_launch(m->in_dlogits, hmax, gprod, B, gsc, st); },
+       8.0 * B, "max |d(dist)| x head-gradient bound -> power-of-two gradient scale");
+    Tensor gp;      // gradient arriving at the current tap through the max pool above it (none at relu5_3)
+    li = (int)m->vgg.size() - 1;
+    for (int s = kVggStages - 1; s >= 0 && !rc; --s) {
+      const Tensor t = tap[s];
+      Tensor g = talloc(B, t.H, t.W, t.C);
+      const f16* gpp = s == kVggStages - 1 ? nullptr : gp.p;
+      float* rk = ref + m->lp_ref_off[s];
+      ew([m, t, s, rk, gsc, gpp, g, B, PL](cudaStream_t st) {
+           return lpips_head_bwd_launch(t.p, B, t.C, t.H * t.W, PL, m->lin_w[s], rk, m->lp_ref_B != 1, m->in_dlogits, gsc, gpp, g.p, st); },
+         (double)t.bytes + 4.0 * B * t.H * t.W * t.C + 2.0 * (double)g.bytes, "lpips head backward (+ pooled path, relu mask)");
+      for (int j = kVggConvs[s] - 1; j >= 0 && !rc; --j, --li) {
+        Tensor dx;
+        dconv(m->vgg[li], g, &dx);
+        if (j > 0) {
+          const Tensor gg = dx, yy = acts[li - 1];
+          ew([gg, yy, PL](cudaStream_t st) { return relu_bwd_launch(gg.p, yy.p, gg.p, (int64_t)(gg.bytes / sizeof(f16)), st, PL, gg.C); },
+             3.0 * (double)gg.bytes, "relu backward");
+        }
+        g = dx;
+      }
+      if (rc) break;
+      if (s > 0) {
+        // g = d(pool output): to the arg-max positions of the tap below (+ its ReLU mask)
+        const Tensor tb = tap[s - 1], gy = g;
+        gp = talloc(B, tb.H, tb.W, tb.C);
+        const Tensor gx = gp;
+        uint16_t* ix = pidx[s - 1];
+        ew([tb, ix, gy, gx, B, PL](cudaStream_t st) { return maxpool2x2_bwd_launch(tb.p, ix, gy.p, gx.p, B, tb.H, tb.W, tb.C, st, PL); },
+           2.5 * (double)gx.bytes, "maxpool 2x2 backward (+ relu mask)");
+      } else {
+        const Tensor dc = g;
+        ew([m, dc, gsc, B, S](cudaStream_t st) {
+             return vq_col2im_bwd_launch(dc.p, m->lp_const + 6, m->out_dz, B, 3, S, S, st, gsc, m->lp_mask, m->lp_mask_batched); },
+           (double)dc.bytes + 12.0 * B * S * S, "col2im + scaling layer + input mask backward");
+      }
+    }
+    cur = &fwd;
+  }
+  if (rc) return rc;
+  if (need) *need = ar.peak;
+  if (!dry) {
+    B2E_REQUIRE(ar.peak <= ws_bytes, B2E_WORKSPACE_TOO_SMALL, "lpips: workspace too small (%zu > %zu)", ar.peak, ws_bytes);
+    m->ops = std::move(fwd);
+    m->bops = std::move(bwd);
+    m->fwd_B = -1;
+    m->cur_B = B;
+  }
+  m->flops = flops;
+  return B2E_OK;
+}
+
 int build_model_clip(b2e_unet* m) {
   const b2e_clip_config& c = m->ccfg;
   const int D = c.hidden_size;
@@ -1044,6 +1292,7 @@ int build_model_clip(b2e_unet* m) {
 int build_model(b2e_unet* m) {
   if (m->clip) return build_model_clip(m);
   if (m->resnet) return build_model_resnet(m);
+  if (m->lpips) return build_model_lpips(m);
   if (m->decoder) return build_model_decoder(m);
   if (m->encoder) return build_model_encoder(m);
   const b2e_unet_config& c = m->cfg;
@@ -1165,6 +1414,7 @@ int finish_forward_only(b2e_unet* m, std::vector<b2e_unet::Op>& fwd, size_t peak
 // arena base this is a dry run that only measures the arena size.
 int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
   if (m->resnet) return build_program_resnet(m, B, ws, ws_bytes, need);
+  if (m->lpips) return build_program_lpips(m, B, ws, ws_bytes, need);
   const b2e_unet_config& c = m->cfg;
   Arena ar;
   ar.reset(ws, ws_bytes);
@@ -2179,6 +2429,76 @@ int b2e_resnet_backward(b2e_unet* m, const float* d_logits, float* d_image, int6
   return B2E_OK;
 }
 
+static int unet_forward_impl(b2e_unet* m, const float* x, const int64_t* timesteps, float* eps, int64_t B, void* stream);
+
+int b2e_lpips_create(const b2e_lpips_config* cfg, int64_t max_batch, b2e_unet** out) {
+  B2E_REQUIRE(cfg && out && max_batch > 0, B2E_INVALID_ARG, "lpips_create: bad argument");
+  B2E_REQUIRE(cfg->input_size >= 32 && cfg->input_size % 16 == 0 && cfg->input_size <= 4096, B2E_UNSUPPORTED_SHAPE,
+              "lpips_create: input_size must be a multiple of 16 in 32..4096 (got %d)", cfg->input_size);
+  B2E_REQUIRE(cfg->precision == 0 || cfg->precision == 1, B2E_INVALID_ARG, "lpips_create: precision must be 0 or 1");
+  b2e_unet* m = new b2e_unet();
+  m->lpips = true;
+  m->grad = true;    // the regulariser exists for its input gradient
+  m->PL = cfg->precision == 1 ? 3 : 1;
+  m->lcfg = *cfg;
+  m->cfg = b2e_unet_config{};
+  m->cfg.sample_size = cfg->input_size; m->cfg.in_channels = 3; m->cfg.out_channels = 1;
+  m->max_batch = max_batch;
+  int rc = build_model(m);
+  if (!rc && cudaDeviceSynchronize() != cudaSuccess) { set_error("lpips_create: device error"); rc = B2E_CUDA_ERROR; }
+  if (!rc) rc = build_program(m, (int)max_batch, nullptr, 0, &m->ws_need);
+  if (rc) { delete m; return rc; }
+  *out = m;
+  return B2E_OK;
+}
+
+int b2e_lpips_set_reference(b2e_unet* m, const float* x_ref, int64_t B_ref, void* stream) {
+  B2E_REQUIRE(m && x_ref, B2E_INVALID_ARG, "lpips_set_reference: null pointer");
+  B2E_REQUIRE(m->lpips, B2E_INVALID_ARG, "lpips_set_reference: not an LPIPS handle");
+  B2E_REQUIRE(m->ws, B2E_INVALID_ARG, "lpips_set_reference: no workspace bound");
+  B2E_REQUIRE(B_ref >= 1 && B_ref <= m->max_batch, B2E_UNSUPPORTED_SHAPE, "lpips_set_reference: batch %lld (1..%lld)",
+              (long long)B_ref, (long long)m->max_batch);
+  if (B_ref != m->cur_B) {
+    int rc = build_program(m, (int)B_ref, m->ws, m->ws_bytes, nullptr);
+    if (rc) return rc;
+  }
+  m->in_x = x_ref; m->lp_mask = nullptr; m->lp_mask_batched = 0;
+  m->lp_ref_mode = true;
+  m->lp_ref_B = -1;
+  m->fwd_B = -1;     // the activations now belong to the reference pass: no backward over them
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = B2E_OK;
+  for (size_t i = 0; i < m->ops.size() && !rc; ++i) rc = m->ops[i].fn(st);
+  m->lp_ref_mode = false;
+  if (rc) return rc;
+  m->lp_ref_B = B_ref;
+  return B2E_OK;
+}
+
+int b2e_lpips_forward(b2e_unet* m, const float* x, const float* mask, int64_t mask_batch, float* dist, int64_t B, void* stream) {
+  B2E_REQUIRE(m && x && dist, B2E_INVALID_ARG, "lpips_forward: null pointer");
+  B2E_REQUIRE(m->lpips, B2E_INVALID_ARG, "lpips_forward: not an LPIPS handle");
+  B2E_REQUIRE(!mask || mask_batch == 1 || mask_batch == B, B2E_UNSUPPORTED_SHAPE,
+              "lpips_forward: the mask batch must be 1 or %lld (got %lld)", (long long)B, (long long)mask_batch);
+  m->lp_mask = mask; m->lp_mask_batched = mask && mask_batch > 1;
+  return unet_forward_impl(m, x, nullptr, dist, B, stream);
+}
+
+int b2e_lpips_backward(b2e_unet* m, const float* d_dist, float* d_x, int64_t B, void* stream) {
+  B2E_REQUIRE(m && d_dist && d_x, B2E_INVALID_ARG, "lpips_backward: null pointer");
+  B2E_REQUIRE(m->lpips, B2E_INVALID_ARG, "lpips_backward: not an LPIPS handle");
+  B2E_REQUIRE(m->grad, B2E_INVALID_ARG, "lpips_backward: gradient mode is off (b2e_unet_enable_grad)");
+  B2E_REQUIRE(m->fwd_B == B && m->cur_B == B, B2E_INVALID_ARG,
+              "lpips_backward: no live forward pass of batch %lld (last forward: %lld)", (long long)B, (long long)m->fwd_B);
+  m->in_dlogits = d_dist; m->out_dz = d_x;
+  cudaStream_t st = (cudaStream_t)stream;
+  for (auto& op : m->bops) {
+    int rc = op.fn(st);
+    if (rc) return rc;
+  }
+  return B2E_OK;
+}
+
 void b2e_unet_destroy(b2e_unet* m) { delete m; }
 
 int b2e_unet_num_params(const b2e_unet* m) { return m ? (int)m->params.size() : 0; }
@@ -2209,11 +2529,18 @@ int b2e_unet_bind_workspace(b2e_unet* m, void* workspace, size_t workspace_bytes
               m->ws_need, workspace_bytes);
   B2E_REQUIRE(((uintptr_t)workspace & 255) == 0, B2E_INVALID_ARG, "bind_workspace: workspace must be 256-byte aligned");
   m->ws = workspace; m->ws_bytes = workspace_bytes;
+  m->lp_ref_B = -1;
   return build_program(m, (int)m->max_batch, workspace, workspace_bytes, nullptr);
 }
 
 int b2e_unet_forward(b2e_unet* m, const float* x, const int64_t* timesteps, float* eps, int64_t B, void* stream) {
-  B2E_REQUIRE(m && x && (timesteps || m->decoder || m->encoder || m->resnet || m->clip) && eps, B2E_INVALID_ARG, "unet_forward: null pointer");
+  // an LPIPS handle called directly (profiling): no input mask - the last b2e_lpips_forward's may be gone
+  if (m && m->lpips) { m->lp_mask = nullptr; m->lp_mask_batched = 0; }
+  return unet_forward_impl(m, x, timesteps, eps, B, stream);
+}
+
+static int unet_forward_impl(b2e_unet* m, const float* x, const int64_t* timesteps, float* eps, int64_t B, void* stream) {
+  B2E_REQUIRE(m && x && (timesteps || m->decoder || m->encoder || m->resnet || m->clip || m->lpips) && eps, B2E_INVALID_ARG, "unet_forward: null pointer");
   B2E_REQUIRE(m->ws, B2E_INVALID_ARG, "unet_forward: no workspace bound");
   B2E_REQUIRE(B > 0 && B <= m->max_batch, B2E_UNSUPPORTED_SHAPE, "unet_forward: batch %lld exceeds max_batch %lld",
               (long long)B, (long long)m->max_batch);
@@ -2223,6 +2550,8 @@ int b2e_unet_forward(b2e_unet* m, const float* x, const int64_t* timesteps, floa
   }
   B2E_REQUIRE(m->cfg.cross_attention_dim <= 0 || m->in_ctx, B2E_INVALID_ARG,
               "unet_forward: a conditional UNet needs b2e_unet_forward_cond");
+  B2E_REQUIRE(!m->lpips || m->lp_ref_B == 1 || m->lp_ref_B == B, B2E_INVALID_ARG,
+              "lpips_forward: %s", m->lp_ref_B < 0 ? "no reference (b2e_lpips_set_reference)" : "the reference batch must be 1 or B");
   m->in_x = x; m->in_t = timesteps; m->out_eps = eps;
   cudaStream_t st = (cudaStream_t)stream;
   for (auto& op : m->ops) {
@@ -2245,12 +2574,13 @@ int b2e_unet_forward_cond(b2e_unet* m, const float* x, const int64_t* timesteps,
 
 int b2e_unet_enable_grad(b2e_unet* m, int enable) {
   B2E_REQUIRE(m, B2E_INVALID_ARG, "unet_enable_grad: null handle");
-  B2E_REQUIRE(!enable || m->decoder || m->resnet, B2E_UNSUPPORTED_SHAPE,
-              "unet_enable_grad: gradient mode is implemented for the VQ / KL decoder and the classifier");
-  B2E_REQUIRE(!enable || m->PL == 1 || m->resnet, B2E_UNSUPPORTED_SHAPE, "unet_enable_grad: the fp32-accurate mode is forward-only");
+  B2E_REQUIRE(!enable || m->decoder || m->resnet || m->lpips, B2E_UNSUPPORTED_SHAPE,
+              "unet_enable_grad: gradient mode is implemented for the VQ / KL decoder, the classifier and LPIPS");
+  B2E_REQUIRE(!enable || m->PL == 1 || m->resnet || m->lpips, B2E_UNSUPPORTED_SHAPE, "unet_enable_grad: the fp32-accurate mode is forward-only");
   if ((enable != 0) == m->grad) return B2E_OK;
   m->grad = enable != 0;
   m->cur_B = -1; m->fwd_B = -1; m->ws = nullptr; m->ws_bytes = 0;   // the workspace must be re-queried and re-bound
+  m->lp_ref_B = -1;
   return build_program(m, (int)m->max_batch, nullptr, 0, &m->ws_need);
 }
 
@@ -2293,7 +2623,7 @@ const char* b2e_unet_op_desc(const b2e_unet* m, int idx) {
 
 int b2e_unet_profile(b2e_unet* m, const float* x, const int64_t* timesteps, float* eps, int64_t B, void* stream,
                      int max_ops, int* n_ops, float* ms, double* flops, double* bytes, int* kind) {
-  B2E_REQUIRE(m && x && (timesteps || m->decoder || m->encoder || m->resnet || m->clip) && eps && n_ops && ms && flops && bytes && kind, B2E_INVALID_ARG,
+  B2E_REQUIRE(m && x && (timesteps || m->decoder || m->encoder || m->resnet || m->clip || m->lpips) && eps && n_ops && ms && flops && bytes && kind, B2E_INVALID_ARG,
               "unet_profile: null pointer");
   // one plain pass first (plan rebuild / lazy function attributes), then the instrumented pass
   int rc = b2e_unet_forward(m, x, timesteps, eps, B, stream);

@@ -884,9 +884,13 @@ __global__ void pack_input_kernel(const float* __restrict__ x, f16* __restrict__
 
 // im2col variant: one thread per pixel gathers its 9 x C neighbourhood (coalesced across the warp, neighbours hit
 // L1) and writes the pixel's 64 channels (128 B)
+// mask / shift: the optional input transform (1 - mask * x, then (v - shift) / scale) of pack_input_launch; none of it
+// is evaluated without them, so the plain packing keeps its arithmetic
 template <int C>
 __global__ void __launch_bounds__(256) pack_input_im2col_kernel(const float* __restrict__ x, f16* __restrict__ out, int B,
-                                                                int H, int W, int planes) {
+                                                                int H, int W, int planes, const float* __restrict__ shift,
+                                                                const float* __restrict__ scale, const float* __restrict__ mask,
+                                                                int mask_batched) {
   pdl_wait();
   const int HW = H * W;
   const int64_t total = (int64_t)B * HW;
@@ -901,7 +905,12 @@ __global__ void __launch_bounds__(256) pack_input_im2col_kernel(const float* __r
       const bool in = hh >= 0 && hh < H && ww >= 0 && ww < W;
 #pragma unroll
       for (int c = 0; c < C; ++c)
-        if (in) f[t * C + c] = __ldg(x + ((int64_t)b * C + c) * HW + hh * W + ww);
+        if (in) {
+          float v = __ldg(x + ((int64_t)b * C + c) * HW + hh * W + ww);
+          if (mask) v = __fsub_rn(1.f, __fmul_rn(__ldg(mask + ((int64_t)(mask_batched ? b : 0) * C + c) * HW + hh * W + ww), v));
+          if (shift) v = __fdiv_rn(__fsub_rn(v, __ldg(shift + c)), __ldg(scale + c));
+          f[t * C + c] = v;
+        }
     }
     uint4* o = reinterpret_cast<uint4*>(out + p * 64 * planes);
 #pragma unroll
@@ -920,7 +929,9 @@ __global__ void __launch_bounds__(256) pack_input_im2col_kernel(const float* __r
 }
 
 int pack_input_launch(const float* x, f16* out, int B, int C, int H, int W, int cpad, bool im2col, cudaStream_t st,
-                      int planes, const float* gs) {
+                      int planes, const float* gs, const float* shift, const float* scale, const float* mask, int mask_batched) {
+  B2E_REQUIRE(im2col || (!shift && !mask), B2E_UNSUPPORTED_SHAPE, "pack_input: the input transform needs the im2col layout");
+  B2E_REQUIRE(!shift == !scale, B2E_INVALID_ARG, "pack_input: shift and scale go together");
   const int HW = H * W;
   int64_t total = (int64_t)B * HW;
   int grid = (int)((total + 255) / 256);
@@ -928,9 +939,9 @@ int pack_input_launch(const float* x, f16* out, int B, int C, int H, int W, int 
   if (im2col) {
     B2E_REQUIRE(9 * C <= 64 && cpad == 64 && !gs, B2E_UNSUPPORTED_SHAPE, "pack_input: im2col needs 9*C <= 64 (and takes no gradient scale)");
     switch (C) {
-      case 1: launch_pdl(pack_input_im2col_kernel<1>, dim3(grid), dim3(256), 0, st, x, out, B, H, W, planes); break;
-      case 3: launch_pdl(pack_input_im2col_kernel<3>, dim3(grid), dim3(256), 0, st, x, out, B, H, W, planes); break;
-      case 4: launch_pdl(pack_input_im2col_kernel<4>, dim3(grid), dim3(256), 0, st, x, out, B, H, W, planes); break;
+      case 1: launch_pdl(pack_input_im2col_kernel<1>, dim3(grid), dim3(256), 0, st, x, out, B, H, W, planes, shift, scale, mask, mask_batched); break;
+      case 3: launch_pdl(pack_input_im2col_kernel<3>, dim3(grid), dim3(256), 0, st, x, out, B, H, W, planes, shift, scale, mask, mask_batched); break;
+      case 4: launch_pdl(pack_input_im2col_kernel<4>, dim3(grid), dim3(256), 0, st, x, out, B, H, W, planes, shift, scale, mask, mask_batched); break;
       default: B2E_REQUIRE(false, B2E_UNSUPPORTED_SHAPE, "pack_input: im2col supports 1, 3 or 4 input channels (got %d)", C);
     }
     return check_launch("pack_input_im2col");
@@ -1680,7 +1691,8 @@ int softmax_bwd_rows_launch(const f16* p, f16* dp, int64_t rows, int T, float sc
 // w.r.t. im2col column t*L + c of every pixel; dz[b][k][h][w] = sum_c pq_w[c][k] * sum_t dcols[(h,w) - tap_t][t*L + c]
 __global__ void __launch_bounds__(256) vq_col2im_bwd_kernel(const f16* __restrict__ dcols, const float* __restrict__ pq_w,
                                                             float* __restrict__ dz, int B, int L, int H, int W,
-                                                            const float* __restrict__ gs) {
+                                                            const float* __restrict__ gs, const float* __restrict__ mask,
+                                                            int mask_batched) {
   pdl_wait();
   const float unscale = gs ? gs[1] : 1.f;
   const int64_t total = (int64_t)B * H * W;
@@ -1699,15 +1711,17 @@ __global__ void __launch_bounds__(256) vq_col2im_bwd_kernel(const f16* __restric
   for (int k = 0; k < L; ++k) {
     float acc = 0.f;
     for (int c = 0; c < L; ++c) acc += pq_w[c * L + k] * g[c];
-    dz[((int64_t)b * L + k) * HW + q] = acc * unscale;
+    float v = acc * unscale;
+    if (mask) v = -__ldg(mask + ((int64_t)(mask_batched ? b : 0) * L + k) * HW + q) * v;
+    dz[((int64_t)b * L + k) * HW + q] = v;
   }
 }
 
 int vq_col2im_bwd_launch(const f16* dcols, const float* pq_w, float* dz, int B, int L, int H, int W, cudaStream_t st,
-                         const float* gs) {
+                         const float* gs, const float* mask, int mask_batched) {
   B2E_REQUIRE(L >= 1 && L <= 4 && 9 * L <= 64, B2E_UNSUPPORTED_SHAPE, "vq_col2im_bwd: latent channels %d", L);
   const int64_t total = (int64_t)B * H * W;
-  launch_pdl(vq_col2im_bwd_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, st, dcols, pq_w, dz, B, L, H, W, gs);
+  launch_pdl(vq_col2im_bwd_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, st, dcols, pq_w, dz, B, L, H, W, gs, mask, mask_batched);
   return check_launch("vq_col2im_bwd");
 }
 

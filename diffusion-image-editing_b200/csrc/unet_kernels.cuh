@@ -61,8 +61,11 @@ int gn_finalize_launch(const float* tile_stats, float* chan_stats, int N, int C,
 // x[c] at 3x3 tap t (zero outside the image), so that a 3x3 convolution becomes a 1x1 one
 // planes = 3 (im2col only): split-f16 output [hi | lo | hi] of cpad channels each (fp32-accurate mode)
 // gs (plain layout only): gradient scale record of grad_scale_launch, x is multiplied by gs[0]
+// im2col only: mask (fp32 (1 | B, C, H, W), mask_batched) replaces x by 1 - mask * x, and shift / scale (C floats each,
+// device) apply (v - shift[c]) / scale[c] (the LPIPS scaling layer) before the zero padding of the taps
 int pack_input_launch(const float* x, f16* out, int B, int C, int H, int W, int cpad, bool im2col, cudaStream_t st,
-                      int planes = 1, const float* gs = nullptr);
+                      int planes = 1, const float* gs = nullptr, const float* shift = nullptr, const float* scale = nullptr,
+                      const float* mask = nullptr, int mask_batched = 0);
 // gs[0] = s = 2^e, gs[1] = 1 / s with max|x| * mult * s in [4, 8) (B2E_GRAD_LOG2 moves the target); gs = 3 floats, gs[2] zero
 // before the first launch (the kernels re-arm it).  Keeps fp16 gradients in range; exact (powers of two).
 int grad_scale_launch(const float* x, int64_t n, float* gs, float mult, cudaStream_t st);
@@ -108,8 +111,9 @@ int unpad_rows_f32_launch(const f16* x, float* out, int B, int L, int Lpad, int 
 int downsum2x_launch(const f16* dy, f16* dx, int N, int H, int W, int C, cudaStream_t st);
 int transpose_window_launch(const f16* src, f16* dst, int N, int R, int Cc, int src_pitch, int col0, cudaStream_t st);
 int softmax_bwd_rows_launch(const f16* p, f16* dp, int64_t rows, int T, float scale, cudaStream_t st);
+// mask (fp32 (1 | B, L, H, W), mask_batched): the chain of an input x -> 1 - mask * x, dz *= -mask
 int vq_col2im_bwd_launch(const f16* dcols, const float* pq_w, float* dz, int B, int L, int H, int W, cudaStream_t st,
-                         const float* gs = nullptr);
+                         const float* gs = nullptr, const float* mask = nullptr, int mask_batched = 0);
 
 // VQModel.decode front: nearest codebook entry + 1x1 post_quant_conv; z, out fp32 NCHW (B, L <= 4, HW)
 int vq_quantize_launch(const float* z, const float* codebook, int n_codes, const float* pq_w, const float* pq_b, float* out,
@@ -133,6 +137,22 @@ int avgpool_fc_launch(const f16* x, float* feat, const float* w, const float* b,
                       cudaStream_t st, int planes = 1);
 int avgpool_fc_bwd_launch(const float* dlogits, const float* w, float* dfeat, const f16* y, f16* g, int N, int HW, int C, int K,
                           cudaStream_t st, const float* gs = nullptr, int yplanes = 1);
+
+// LPIPS (VGG-16) kernels, csrc/lpips_kernels.cu; planes / xplanes = 3: split tensors of the fp32-accurate forward
+int maxpool2x2_launch(const f16* x, f16* y, uint16_t* idx, int N, int H, int W, int C, cudaStream_t st, int planes = 1);
+int maxpool2x2_bwd_launch(const f16* x, const uint16_t* idx, const f16* gy, f16* gx, int N, int H, int W, int C, cudaStream_t st,
+                          int xplanes = 1);
+struct LpipsTaps { int n[5], off[5], hw[5]; };   // partial slots per tap, their offset in a row of partials, pixels per image
+int lpips_head_blocks(int HW);
+// mode 0: ref <- normalised features of x; mode 1: partial[b][slot0 ..] <- distance partial sums against ref
+// hmax (mode 1): per-image running max of the head-gradient elements for d(dist) = 1 (zeroed by the caller per forward)
+int lpips_head_launch(const f16* x, int B, int C, int HW, int planes, const float* w, float* ref, int ref_batched, double* partial,
+                      int part_pitch, int slot0, int mode, float* hmax, cudaStream_t st);
+// gs (grad_scale_launch record) from max_b |d_dist[b]| * hmax[b]; prod = B floats of scratch
+int lpips_grad_scale_launch(const float* d_dist, const float* hmax, float* prod, int B, float* gs, cudaStream_t st);
+int lpips_finalize_launch(const double* partial, int part_pitch, const LpipsTaps& taps, float* dist, int B, cudaStream_t st);
+int lpips_head_bwd_launch(const f16* x, int B, int C, int HW, int planes, const float* w, const float* ref, int ref_batched,
+                          const float* d_dist, const float* gs, const f16* gp, f16* gout, cudaStream_t st);
 
 // face parser (BiSeNet) helpers
 int avgpool_launch(const f16* x, float* feat, int N, int HW, int C, cudaStream_t st, int planes = 1);

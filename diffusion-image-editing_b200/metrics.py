@@ -6,7 +6,8 @@ harness is exercised for its contract (shapes, keys, determinism).
 
 Deviations from the reference: ``num_inference_steps`` and ``predictor`` are parameters (the reference hard-codes 50 steps
 and reloads the checkpoint inside every call), tensors follow the model's device instead of the literal "cuda", and
-``lpips`` raises (no LPIPS package / VGG weights offline; the reference's own function shadows the module it needs)."""
+``lpips`` takes the distance network as ``model=`` (``models.get_lpips``: the native LPIPS-vgg; the reference's own
+function shadows the ``lpips`` module it needs); without one it raises."""
 from collections import defaultdict
 from typing import Dict, Optional, Tuple
 
@@ -19,8 +20,15 @@ from transforms import pil_to_tensor
 from utils import generate_random_samples
 
 
-def lpips(original: torch.Tensor, edited: torch.Tensor):
-    raise NotImplementedError("LPIPS needs the lpips package and VGG weights, neither of which is available offline")
+def lpips(original: torch.Tensor, edited: torch.Tensor, model=None):
+    """LPIPS(original, edited), (B, 1, 1, 1) (src/metrics.py: ``lpips.LPIPS(net='vgg')(original, edited)``).  ``model``:
+    the distance network, e.g. ``models.get_lpips(input_size=...)``; there is no default because no VGG / lin weights
+    ship offline."""
+    if model is None:
+        raise NotImplementedError("metrics.lpips needs model= (e.g. models.get_lpips(input_size=...)): the lpips package "
+                                  "and its VGG weights are not available offline")
+    with torch.no_grad():
+        return model(original, edited)
 
 
 def _predictor_for(img_t: torch.Tensor, predictor=None):

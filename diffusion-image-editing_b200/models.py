@@ -143,6 +143,22 @@ def get_pretrained_anyGAN(input_size: int = 256, max_batch: int = 1, state_dict_
     return resnet50_predictor(80, input_size, max_batch=max_batch, state_dict=sd, seed=seed, precision=precision)
 
 
+def get_lpips(input_size: int = 256, max_batch: int = 1, state_dict: Optional[dict] = None, seed: int = 0,
+              precision: Optional[str] = "fp32"):
+    """The LPIPS (vgg) distance of ``use_lpips`` guidance and ``metrics.lpips`` (the reference's ``lpips.LPIPS(net='vgg')``)
+    on the native engine: forward and input gradient on the tcgen05 kernels.  ``state_dict``: the full
+    ``lpips.LPIPS(net='vgg').state_dict()``; without it the weights are seeded random (no pretrained VGG offline).
+    ``precision`` "fp32" (default) runs the fp32-accurate forward because guidance differentiates the network (the
+    ReLU / max-pool masks of the input gradient then agree with an fp32 evaluation); "fp16" is the 16-bit forward."""
+    from b200edit.lpips import LPIPS
+    net = LPIPS("vgg", input_size=input_size, max_batch=max_batch, device=get_device(), precision=precision)
+    if state_dict is not None:
+        net.load_state_dict(state_dict)
+    else:
+        net.init_random(seed)
+    return net
+
+
 class SegmentationModel:
     """Face parser front-end (src/models.py:80-118), same leading positional arguments as the reference:
     ``SegmentationModel(ckpt, n_classes, image_size)``.  The network is the native BiSeNet (b200edit.bisenet) for ANY

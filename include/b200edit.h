@@ -136,6 +136,12 @@ size_t b2e_color_loss_grad_workspace_bytes(void);
 int b2e_color_loss_grad_f32(const float* img, const float* mask, const float* x_ref, float* d_img, int64_t B, int64_t C,
                             int64_t HW, const b2e_color_grad_params* p, void* workspace, size_t workspace_bytes,
                             void* stream);
+/* The same colour gradient in the masked-prediction mode with the LPIPS regulariser instead of L2 (use_lpips):
+ *   d_img = mask * k_c * sign(mask * img - target_c) + lam_scale * d_lpips
+ * d_lpips = b2e_lpips_backward's d(LPIPS(1 - mask * img, x_0)) / d(img) (the -mask chain included); reads has_target,
+ * target, k, lam_scale (= loss_scale * lambda_) and mask_batched of p; mask (1 | B, C, HW) is required. */
+int b2e_lpips_guidance_grad_f32(const float* img, const float* mask, const float* d_lpips, float* d_img, int64_t B, int64_t C,
+                                int64_t HW, const b2e_color_grad_params* p, void* stream);
 /* ... and the update on the latent after the decoder's backward pass returned d_latent = dL/d(decoder input):
  *   g = -(d_latent * chain) / sqrt_a_t ;  x <- x + (mask? mask*g : g) * a_t_sq
  * chain = d(decoder input)/d(x0 prediction): 1 for LDM, 1/0.18215 for SD (src/diffusion_classes.py:33). */
@@ -381,6 +387,29 @@ typedef struct {
 } b2e_resnet_config;
 int b2e_resnet_create(const b2e_resnet_config* cfg, int64_t max_batch, b2e_unet** out);
 int b2e_resnet_backward(b2e_unet* m, const float* d_logits, float* d_image, int64_t B, void* stream);
+
+/* ------------------------------------------------------------------ LPIPS distance (use_lpips regulariser, metrics.lpips)
+ * lpips v0.1 with net='vgg' (lpips.LPIPS(net='vgg'), normalize=False): scaling layer (x - shift) / scale, VGG-16
+ * features[0:30] (thirteen 3x3 convolutions + ReLU, 2x2 max pools), taps relu1_2 .. relu5_3, per tap and pixel
+ * sum_c w_k[c] (u0_c - u1_c)^2 of the channel-normalised features u = f / (||f|| + 1e-10), spatial mean, sum over taps.
+ * Parameters under lpips.LPIPS().state_dict() names: "net.slice1.0.weight/.bias" .. "net.slice5.28.weight/.bias",
+ * "lin0.model.1.weight" .. "lin4.model.1.weight" (the scaling layer's constants are built in).
+ * b2e_lpips_set_reference: runs the network on x_ref (B_ref, 3, S, S) fp32 (B_ref = 1 or the batch of later forwards)
+ *   and keeps its normalised tap features in a part of the workspace no forward overwrites.  Binding a workspace or
+ *   toggling gradient mode drops the reference.
+ * b2e_lpips_forward: dist[b] = LPIPS(mask ? 1 - mask * x : x, reference); x (B, 3, S, S) fp32, mask NULL or fp32
+ *   (mask_batch = 1 or B, 3, S, S), dist (B) fp32.  Bit-deterministic (fixed-order fp64 reductions).
+ * b2e_lpips_backward: d_x = d(sum_b d_dist[b] * dist[b]) / dx through the input transform of the last forward
+ *   (b2e_lpips_forward of batch B; the gradient mode of b2e_unet_enable_grad is on after create).
+ * Workspace, parameters and profiling through the b2e_unet_* entry points. */
+typedef struct {
+  int32_t input_size;   /* image height = width: a multiple of 16, >= 32 */
+  int32_t precision;    /* 0: f16 operands; 1: fp32-accurate forward (backward on f16 operands), as b2e_resnet_config */
+} b2e_lpips_config;
+int b2e_lpips_create(const b2e_lpips_config* cfg, int64_t max_batch, b2e_unet** out);
+int b2e_lpips_set_reference(b2e_unet* m, const float* x_ref, int64_t B_ref, void* stream);
+int b2e_lpips_forward(b2e_unet* m, const float* x, const float* mask, int64_t mask_batch, float* dist, int64_t B, void* stream);
+int b2e_lpips_backward(b2e_unet* m, const float* d_dist, float* d_x, int64_t B, void* stream);
 
 /* The 16-bit storage / tensor-core operand type the library was built for: 0 = IEEE fp16 (default), 1 = bf16
  * (-DB2E_ACT_BF16 builds).  Accumulation is fp32 either way. */
