@@ -12,6 +12,10 @@ predicted clean image:  x <- x + (-d(loss_scale*loss)/dx) * alphas_cumprod[t]**2
 * Any other strategy (user subclasses, network losses) evaluates ``loss`` with torch autograd on the device - exactly the
   reference's procedure - and the resulting gradient is applied by a CUDA kernel.  That is the extension contract of the
   reference: subclass, implement ``loss``, register.
+* The network strategies (``NetAttrFunc`` / ``ClassifierAttrFunc``) with ``per_sample=True`` on a native parser / predictor
+  (and an identity or native decoder) run kernel to kernel as well: x0' kernel -> (decoder forward) -> network forward ->
+  batched loss head (value and gradient of every image) -> network input gradient -> (decoder backward) -> update kernel
+  (``_apply_native_network``).
 * ``mask_pred_original_sample=True, use_lpips=True`` needs the distance network as ``lpips_model=`` (``models.get_lpips``,
   the native LPIPS-vgg, or any callable ``(in0, in1) -> (B, 1, 1, 1)``): the loss is ``loss(mask * x0') +
   lambda_ * LPIPS(1 - mask * x0', x_0)``, differentiated by autograd through the native LPIPS node.  Without
@@ -61,8 +65,9 @@ def _identity_decoder(model) -> bool:
 class AttrFunc(ABC):
     """Base class of the guidance strategies.  kwargs understood by ``apply`` (also stored at
     construction and splatted back by the pipeline): use_mask, mask, mask_attr_grad,
-    mask_pred_original_sample, use_l2, use_lpips, lambda_, x_0.  ``per_sample=True`` (extension)
-    averages the loss per image instead of over the whole batch."""
+    mask_pred_original_sample, use_l2, use_lpips, lambda_, x_0.  ``per_sample=True`` (extension) makes every image of
+    a batch its own problem: the colour losses average per image instead of over the whole batch, the network losses
+    are sum_b L_b with L_b the reference's loss on image b alone (the reference's heads read batch element 0 only)."""
 
     def __init__(self, loss_scale: float = 1, t1: int = 0, t2: int = 50, nudge_xt=True, nudge_zt=False,
                  per_sample: bool = False, **kwargs) -> None:
@@ -92,6 +97,14 @@ class AttrFunc(ABC):
     # ---- fused-kernel description of the loss; None -> generic autograd path
     def colour_spec(self):
         return None
+
+    # ---- native network strategies (per_sample): the engine that evaluates the loss network on (B, 3, size, size)
+    # images with forward_keep / input_grad, or None; and the batched head: d(loss_scale * sum_b L_b) / d(logits)
+    def native_network(self, size: int):
+        return None
+
+    def native_head_grad(self, logits):
+        raise NotImplementedError
 
     # ---- generic (autograd) pieces, same structure as the reference
     def calculate_loss(self, pred_original_sample: torch.Tensor, **kwargs) -> torch.Tensor:
@@ -265,6 +278,46 @@ class AttrFunc(ABC):
             return None                # a mask that does not match the sample: the generic path reports it
         return ops.apply_latent_guidance(xt, d_lat, chain, coeffs.sqrt_a_t, coeffs.a_t_sq, mask=gmask)
 
+    def _apply_native_network(self, xt, model_output, coeffs, model, **kwargs):
+        """Network strategies with per_sample=True on a native network: x0' kernel (-> chain scaling, native decoder
+        forward) -> network forward_keep -> batched loss head (every image's gradient, scaled by loss_scale) -> network
+        input_grad (-> native decoder backward) -> update kernel.  No autograd graph, no torch arithmetic.  Image b's nudge
+        is the batch-1 nudge of image b.  Returns None when the strategy / model / shapes do not qualify (autograd path)."""
+        if (not self.per_sample or self.nudge_zt or not self.nudge_xt
+                or kwargs.get("mask_pred_original_sample", False)):
+            return None
+        mask = kwargs.get("mask")
+        if kwargs.get("mask_attr_grad", False) and mask is None:
+            raise ValueError("No mask specified")
+        B = xt.shape[0]
+        dec, chain, size = None, 1.0, xt.shape[-1]
+        if not _identity_decoder(model):
+            nd = getattr(model, "native_decoder", None)
+            nd = nd() if callable(nd) else None
+            if nd is None:
+                return None
+            dec, chain = nd
+            size = getattr(dec, "out_size", None)
+            if size is None or B > dec.max_batch:
+                return None
+        gmask = mask if kwargs.get("mask_attr_grad", False) else None
+        if gmask is not None and (not torch.is_tensor(gmask) or gmask.dim() != 4 or gmask.shape[0] not in (1, B)
+                                  or gmask.shape[1] not in (1, xt.shape[1]) or gmask.shape[2:] != xt.shape[2:]):
+            return None                # a mask that does not match the sample: the generic path reports it
+        net = self.native_network(int(size))
+        if net is None or B > net.max_batch:
+            return None
+        lat = ops.pred_x0(xt, model_output, coeffs.sqrt_a_t, coeffs.sqrt_b_t)
+        if dec is None:
+            img = lat
+        else:
+            if chain != 1.0:
+                lat = ops.axpby(lat, lat, chain, 0.0)
+            img = dec.decode_keep(lat)
+        d_img = net.input_grad(self.native_head_grad(net.forward_keep(img)))
+        d_lat = d_img if dec is None else dec.latent_grad(d_img)
+        return ops.apply_latent_guidance(xt, d_lat, chain, coeffs.sqrt_a_t, coeffs.a_t_sq, mask=gmask)
+
     def in_window(self, step_idx: int) -> bool:
         return self.t1 <= step_idx < self.t2
 
@@ -276,6 +329,9 @@ class AttrFunc(ABC):
         coeffs = model.scheduler.coeffs(int(timestep), 0.0, "ddim")
         fk = self.fused_kwargs(xt, model, **kwargs)
         if fk is None:
+            out = self._apply_native_network(xt, model_output, coeffs, model, **kwargs)
+            if out is not None:
+                return out, zt
             out = self._apply_native_lpips(xt, model_output, coeffs, model, **kwargs)
             if out is not None:
                 return out, zt
@@ -341,11 +397,24 @@ class NetAttrFunc(AttrFunc):
         if hasattr(net, "enable_grad") and not getattr(net, "differentiable", True):
             net.enable_grad()
 
+    def _head_ids(self):
+        """The class ids when the fused head can evaluate the loss (a list of distinct ids), else None."""
+        if not isinstance(self.idx_for_class, (list, tuple)):
+            return None
+        ids = [int(c) for c in self.idx_for_class]
+        return ids if len(set(ids)) == len(ids) else None
+
     def loss(self, img, **kwargs):
         out = self.segmentation_model.net(img)[0]
-        ids = [int(c) for c in (self.idx_for_class if isinstance(self.idx_for_class, (list, tuple)) else [self.idx_for_class])]
-        if (out.is_cuda and out.dtype == torch.float32 and out.dim() == 4 and out.shape[0] == 1 and out.shape[1] <= 32
-                and len(set(ids)) == len(ids) and isinstance(self.idx_for_class, (list, tuple))):
+        ids = self._head_ids()
+        if self.per_sample:
+            # sum_b of the reference's loss on image b alone
+            if ids is not None and out.is_cuda and out.dtype == torch.float32 and out.dim() == 4 and out.shape[1] <= 32:
+                return ops.seg_area_loss(out, ids, per_sample=True)
+            area = out.softmax(dim=1).sum(dim=(2, 3)) / (256 * 256)
+            return area[:, self.idx_for_class].sum()
+        if (ids is not None and out.is_cuda and out.dtype == torch.float32 and out.dim() == 4 and out.shape[0] == 1
+                and out.shape[1] <= 32):
             # fused head: softmax + selected-class area and its analytic gradient in one kernel; the parser
             # itself (the user's torch module) is differentiated by autograd as in the reference
             return ops.seg_area_loss(out, ids)
@@ -353,9 +422,28 @@ class NetAttrFunc(AttrFunc):
         out = out.sum(dim=(1, 2)) / (256 * 256)
         return out[self.idx_for_class].sum()
 
+    def native_network(self, size):
+        from b200edit.bisenet import BiSeNet, MultiResBiSeNet
+        net = getattr(self.segmentation_model, "net", None)
+        ids = self._head_ids()
+        if ids is None:
+            return None
+        if isinstance(net, MultiResBiSeNet):
+            if size % 32 or size < 64 or net.n_classes > 32:
+                return None
+            net = net.engine(size, grad=True)
+        if (not isinstance(net, BiSeNet) or not net.differentiable or net.config.input_size != size
+                or net.config.n_classes > 32):
+            return None
+        return net
+
+    def native_head_grad(self, logits):
+        _, grad = ops.seg_area_head(logits, self._head_ids(), per_sample=True, grad_scale=self.loss_scale)
+        return grad
+
 
 class ClassifierAttrFunc(AttrFunc):
-    """Classifier guidance on an 80-logit (40 attributes x 2) predictor; uses batch element 0."""
+    """Classifier guidance on an 80-logit (40 attributes x 2) predictor; uses batch element 0 (per_sample: every image)."""
 
     def __init__(self, predictor, idx_for_class, idx_of_interest=0, regularize_idx_idx_score=(None, None, None),
                  **kwargs) -> None:
@@ -364,18 +452,45 @@ class ClassifierAttrFunc(AttrFunc):
         self.idx_for_class, self.idx_of_interest = idx_for_class, idx_of_interest
         self.regularize_idx_idx_score = regularize_idx_idx_score
 
+    def _fused_head(self):
+        return isinstance(self.idx_for_class, int) and self.idx_of_interest in (0, 1)
+
     def loss(self, xt, **kwargs):
         logits = self.predictor(xt)
-        if (logits.is_cuda and logits.dtype == torch.float32 and logits.numel() % 80 == 0
-                and isinstance(self.idx_for_class, int) and self.idx_of_interest in (0, 1)):
+        r_idx, r_pred, r_score = self.regularize_idx_idx_score
+        if self.per_sample:
+            # sum_b of the reference's loss on image b alone (its first 80 logits)
+            if (self._fused_head() and logits.is_cuda and logits.dtype == torch.float32 and logits.dim() == 2
+                    and logits.shape[1] == 80):
+                return ops.classifier_logit_loss(logits, self.idx_for_class, self.idx_of_interest,
+                                                 self.regularize_idx_idx_score, per_sample=True)
+            attr = logits.reshape(logits.shape[0], -1)[:, :80].reshape(-1, 40, 2)
+            value = attr[:, self.idx_for_class, self.idx_of_interest]
+            if r_idx is not None:
+                value = value + (attr[:, r_idx, r_pred] + r_score[r_pred]) ** 2
+            return value.sum()
+        if (logits.is_cuda and logits.dtype == torch.float32 and logits.numel() % 80 == 0 and self._fused_head()):
             return ops.classifier_logit_loss(logits, self.idx_for_class, self.idx_of_interest,
                                              self.regularize_idx_idx_score)
         attr = logits.view(-1, 40, 2)
         value = attr[0][self.idx_for_class][self.idx_of_interest]
-        r_idx, r_pred, r_score = self.regularize_idx_idx_score
         if r_idx is not None:
             value = value + (attr[0][r_idx][r_pred] + r_score[r_pred]) ** 2
         return value
+
+    def native_network(self, size):
+        from b200edit.resnet import ResNet
+        net = self.predictor
+        cfg = getattr(net, "config", None)
+        if (not self._fused_head() or not isinstance(net, ResNet) or cfg.num_classes != 80 or cfg.in_channels != 3
+                or cfg.input_size != size):
+            return None
+        return net
+
+    def native_head_grad(self, logits):
+        _, grad = ops.classifier_head(logits, self.idx_for_class, self.idx_of_interest, self.regularize_idx_idx_score,
+                                      per_sample=True, grad_scale=self.loss_scale)
+        return grad
 
 
 class AnyGANAttrFunc(ClassifierAttrFunc):

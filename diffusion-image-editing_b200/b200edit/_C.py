@@ -101,6 +101,9 @@ PROTOTYPES = {
     "b2e_seg_area_head_workspace_bytes": (_SZ, []),
     "b2e_seg_area_head_f32": (_I, [_P, _I64, _I64, C.POINTER(C.c_int32), _I, _F, _P, _P, _P, _SZ, _P]),
     "b2e_classifier_head_f32": (_I, [_P, _I64, _I, _I, _I, _I, _F, _P, _P, _P]),
+    "b2e_seg_area_head_batched_workspace_bytes": (_SZ, [_I64]),
+    "b2e_seg_area_head_batched_f32": (_I, [_P, _I64, _I64, _I64, C.POINTER(C.c_int32), _I, _F, _F, _P, _P, _P, _SZ, _P]),
+    "b2e_classifier_head_batched_f32": (_I, [_P, _I64, _I, _I, _I, _I, _F, _F, _P, _P, _P]),
     "b2e_sample_xts_f32": (_I, [_P, _P, _P, _P, _P, _I64, _I64, _P]),
     "b2e_extract_noise_f32": (_I, [_P, _P, _P, _P, _I64, C.POINTER(StepCoeffs), _P]),
     "b2e_mask_workspace_bytes": (_SZ, [_I64, _I64, _I64, _I64]),

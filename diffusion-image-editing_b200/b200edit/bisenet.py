@@ -22,8 +22,8 @@ from .unet import UNet2DModel
 class _BiSeNetFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, image, model):
-        ctx.model, ctx.shape = model, tuple(image.shape)
-        out = model._forward(image)
+        ctx.model = model
+        out = model.forward_keep(image)
         ctx.gen = model._fwd_gen      # the activations of THIS forward live in the engine's single workspace
         return out
 
@@ -33,11 +33,7 @@ class _BiSeNetFn(torch.autograd.Function):
         if m._fwd_gen != ctx.gen:
             raise _C.B2EError("BiSeNet backward: the engine ran another forward since this graph was built (its activations "
                               "were overwritten); differentiate before the next call on the same network")
-        g = d_logits.to(torch.float32).contiguous()
-        dx = torch.empty(ctx.shape, dtype=torch.float32, device=g.device)
-        check(lib.b2e_resnet_backward(m._h, C.c_void_p(g.data_ptr()), C.c_void_p(dx.data_ptr()), ctx.shape[0],
-                                      C.c_void_p(torch.cuda.current_stream().cuda_stream)), "bisenet_backward")
-        return dx, None
+        return m.input_grad(d_logits), None
 
 
 def _fold(w, sd, bn, eps=1e-5):
@@ -133,17 +129,40 @@ class BiSeNet(UNet2DModel):
     def load_reference_state_dict(self, sd, eps=1e-5):
         return self.load_state_dict(self.fold_reference_state_dict(sd, eps))
 
-    def __call__(self, image):
+    def _check_input(self, image):
         if not image.is_cuda:
             raise _C.B2EError("BiSeNet: image must be a CUDA tensor (no CPU fallback)")
         cfg = self.config
         if tuple(image.shape[1:]) != (3, cfg.input_size, cfg.input_size):
             raise ValueError(f"BiSeNet: expected (B,3,{cfg.input_size},{cfg.input_size}), got {tuple(image.shape)}")
+
+    def forward_keep(self, image):
+        """Logits (B, n_classes, S, S) - ``net(image)[0]`` - with the activations kept in the engine's workspace for
+        ``input_grad`` (no autograd graph).  Needs gradient mode (``enable_grad()``) and B <= max_batch."""
+        self._check_input(image)
+        if not self.differentiable:
+            raise _C.B2EError("BiSeNet: call enable_grad() before differentiating through the native face parser")
+        if image.shape[0] > self.max_batch:
+            raise ValueError(f"BiSeNet with gradient: batch {image.shape[0]} > max_batch {self.max_batch}")
+        x = image.detach().to(torch.float32).contiguous()
+        out = self._forward(x)
+        self._keep_gen, self._keep_shape = self._fwd_gen, tuple(x.shape)
+        return out
+
+    def input_grad(self, d_logits):
+        """d(loss)/d(image) of the last ``forward_keep`` given d(loss)/d(logits) (native dgrad of the whole parser)."""
+        if getattr(self, "_keep_gen", None) != self._fwd_gen:
+            raise _C.B2EError("BiSeNet.input_grad: the engine ran another forward since forward_keep (activations overwritten)")
+        g = d_logits.detach().to(torch.float32).contiguous()
+        dx = torch.empty(self._keep_shape, dtype=torch.float32, device=g.device)
+        check(lib.b2e_resnet_backward(self._h, C.c_void_p(g.data_ptr()), C.c_void_p(dx.data_ptr()), self._keep_shape[0],
+                                      C.c_void_p(torch.cuda.current_stream().cuda_stream)), "bisenet_backward")
+        return dx
+
+    def __call__(self, image):
+        self._check_input(image)
+        cfg = self.config
         if image.requires_grad and torch.is_grad_enabled():
-            if not self.differentiable:
-                raise _C.B2EError("BiSeNet: call enable_grad() before differentiating through the native face parser")
-            if image.shape[0] > self.max_batch:
-                raise ValueError(f"BiSeNet with gradient: batch {image.shape[0]} > max_batch {self.max_batch}")
             xx = image if (image.dtype == torch.float32 and image.is_contiguous()) else image.to(torch.float32).contiguous()
             return (_BiSeNetFn.apply(xx, self), None, None)
         x = image.detach().to(torch.float32).contiguous()

@@ -300,10 +300,25 @@ def channel_l1(img, targets):
     return out[:Cc]
 
 
-def seg_area_head(logits, classes, area_divisor=256.0 * 256.0, want_grad=True):
+def seg_area_head(logits, classes, area_divisor=256.0 * 256.0, want_grad=True, per_sample=False, grad_scale=1.0):
     """NetAttrFunc.loss head (src/attr_functions.py:213-219) on the parser logits of ONE image, (C,H,W) or
-    (1,C,H,W): returns (loss 0-d tensor, dL/dlogits with the shape of ``logits`` or None)."""
+    (1,C,H,W): returns (loss 0-d tensor, dL/dlogits with the shape of ``logits`` or None).
+    ``per_sample=True``: logits (B,C,H,W), the head of every image on its own -> (loss (B,), dL_b/dlogits_b * grad_scale);
+    image b's values are bit-identical to a B = 1 call on image b."""
     lg = _f32(logits, "logits")
+    ids = [int(c) for c in classes]
+    arr = (C.c_int32 * max(1, len(ids)))(*ids)
+    if per_sample:
+        if lg.dim() != 4:
+            raise ValueError(f"seg_area_head(per_sample=True): expected (B,C,H,W) logits, got {tuple(lg.shape)}")
+        B, Cc, H, W = lg.shape
+        n = lib.b2e_seg_area_head_batched_workspace_bytes(B)
+        ws = torch.empty(n, dtype=torch.uint8, device=lg.device)
+        loss = torch.empty(B, dtype=torch.float32, device=lg.device)
+        grad = torch.empty_like(lg) if want_grad else None
+        check(lib.b2e_seg_area_head_batched_f32(_p(lg), B, Cc, H * W, arr, len(ids), float(area_divisor), float(grad_scale),
+                                                _p(loss), _p(grad), _p(ws), n, _stream()), "seg_area_head")
+        return loss, grad
     if lg.dim() == 4:
         if lg.shape[0] != 1:
             raise ValueError("seg_area_head: the reference head squeezes batch dimension 0 (batch 1 only)")
@@ -311,8 +326,6 @@ def seg_area_head(logits, classes, area_divisor=256.0 * 256.0, want_grad=True):
     else:
         core = lg
     Cc, H, W = core.shape
-    ids = [int(c) for c in classes]
-    arr = (C.c_int32 * max(1, len(ids)))(*ids)
     n = lib.b2e_seg_area_head_workspace_bytes()
     ws = torch.empty(n, dtype=torch.uint8, device=lg.device)
     loss = torch.empty(1, dtype=torch.float32, device=lg.device)
@@ -322,15 +335,28 @@ def seg_area_head(logits, classes, area_divisor=256.0 * 256.0, want_grad=True):
     return loss[0], grad
 
 
-def classifier_head(logits, idx_for_class: int, idx_of_interest: int = 0, reg=(None, None, None), want_grad=True):
-    """ClassifierAttrFunc.loss head (src/attr_functions.py:237-257) on (B,80) logits: (loss 0-d, dL/dlogits)."""
-    lg = _f32(logits, "logits")
+def _classifier_reg(reg):
     r_idx, r_pred, r_score = reg
     if r_idx is None:
-        ri, rp, rs = -1, 0, 0.0
-    else:
-        ri, rp = int(r_idx), int(r_pred)
-        rs = float(r_score[rp])
+        return -1, 0, 0.0
+    return int(r_idx), int(r_pred), float(r_score[int(r_pred)])
+
+
+def classifier_head(logits, idx_for_class: int, idx_of_interest: int = 0, reg=(None, None, None), want_grad=True,
+                    per_sample=False, grad_scale=1.0):
+    """ClassifierAttrFunc.loss head (src/attr_functions.py:237-257) on (B,80) logits: (loss 0-d, dL/dlogits).
+    ``per_sample=True``: the head of every row on its own -> (loss (B,), dL_b/dlogits_b * grad_scale)."""
+    lg = _f32(logits, "logits")
+    ri, rp, rs = _classifier_reg(reg)
+    if per_sample:
+        if lg.dim() != 2 or lg.shape[1] != 80:
+            raise ValueError(f"classifier_head(per_sample=True): expected (B,80) logits, got {tuple(lg.shape)}")
+        B = lg.shape[0]
+        loss = torch.empty(B, dtype=torch.float32, device=lg.device)
+        grad = torch.empty_like(lg) if want_grad else None
+        check(lib.b2e_classifier_head_batched_f32(_p(lg), B, int(idx_for_class), int(idx_of_interest), ri, rp, rs,
+                                                  float(grad_scale), _p(loss), _p(grad), _stream()), "classifier_head")
+        return loss, grad
     loss = torch.empty(1, dtype=torch.float32, device=lg.device)
     grad = torch.empty_like(lg) if want_grad else None
     check(lib.b2e_classifier_head_f32(_p(lg), lg.numel(), int(idx_for_class), int(idx_of_interest), ri, rp, rs,
@@ -340,26 +366,13 @@ def classifier_head(logits, idx_for_class: int, idx_of_interest: int = 0, reg=(N
 
 class _SegAreaHeadFn(torch.autograd.Function):
     """loss = head(logits) with the analytic gradient from the same kernel launch (the network below it is the
-    user's torch module and is differentiated by autograd, exactly as in the reference)."""
+    user's torch module and is differentiated by autograd, exactly as in the reference).  per_sample: sum_b L_b."""
 
     @staticmethod
-    def forward(ctx, logits, classes, area_divisor):
-        loss, grad = seg_area_head(logits.detach(), classes, area_divisor, want_grad=True)
+    def forward(ctx, logits, classes, area_divisor, per_sample=False):
+        loss, grad = seg_area_head(logits.detach(), classes, area_divisor, want_grad=True, per_sample=per_sample)
         ctx.save_for_backward(grad)
-        return loss
-
-    @staticmethod
-    def backward(ctx, g):
-        (grad,) = ctx.saved_tensors
-        return grad * g, None, None
-
-
-class _ClassifierHeadFn(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, logits, idx_for_class, idx_of_interest, reg):
-        loss, grad = classifier_head(logits.detach(), idx_for_class, idx_of_interest, reg, want_grad=True)
-        ctx.save_for_backward(grad)
-        return loss
+        return loss.sum() if per_sample else loss
 
     @staticmethod
     def backward(ctx, g):
@@ -367,14 +380,28 @@ class _ClassifierHeadFn(torch.autograd.Function):
         return grad * g, None, None, None
 
 
-def seg_area_loss(logits, classes, area_divisor=256.0 * 256.0):
-    """Differentiable NetAttrFunc head (fused value + analytic gradient)."""
-    return _SegAreaHeadFn.apply(logits, tuple(int(c) for c in classes), float(area_divisor))
+class _ClassifierHeadFn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, logits, idx_for_class, idx_of_interest, reg, per_sample=False):
+        loss, grad = classifier_head(logits.detach(), idx_for_class, idx_of_interest, reg, want_grad=True,
+                                     per_sample=per_sample)
+        ctx.save_for_backward(grad)
+        return loss.sum() if per_sample else loss
+
+    @staticmethod
+    def backward(ctx, g):
+        (grad,) = ctx.saved_tensors
+        return grad * g, None, None, None, None
 
 
-def classifier_logit_loss(logits, idx_for_class, idx_of_interest=0, reg=(None, None, None)):
-    """Differentiable ClassifierAttrFunc head (fused value + analytic gradient)."""
-    return _ClassifierHeadFn.apply(logits, int(idx_for_class), int(idx_of_interest), reg)
+def seg_area_loss(logits, classes, area_divisor=256.0 * 256.0, per_sample=False):
+    """Differentiable NetAttrFunc head (fused value + analytic gradient); per_sample: sum_b of each image's head."""
+    return _SegAreaHeadFn.apply(logits, tuple(int(c) for c in classes), float(area_divisor), bool(per_sample))
+
+
+def classifier_logit_loss(logits, idx_for_class, idx_of_interest=0, reg=(None, None, None), per_sample=False):
+    """Differentiable ClassifierAttrFunc head (fused value + analytic gradient); per_sample: sum_b of each row's head."""
+    return _ClassifierHeadFn.apply(logits, int(idx_for_class), int(idx_of_interest), reg, bool(per_sample))
 
 
 def cfg_combine(e_first, e_second, scale: float):

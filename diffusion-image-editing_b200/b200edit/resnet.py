@@ -22,8 +22,8 @@ RESNET50_LAYERS = (3, 4, 6, 3)
 class _ResNetFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, image, model):
-        ctx.model, ctx.shape = model, tuple(image.shape)
-        out = model._forward(image)
+        ctx.model = model
+        out = model.forward_keep(image)
         ctx.gen = model._fwd_gen      # the activations of THIS forward live in the engine's single workspace
         return out
 
@@ -33,11 +33,7 @@ class _ResNetFn(torch.autograd.Function):
         if m._fwd_gen != ctx.gen:
             raise _C.B2EError("ResNet backward: the engine ran another forward since this graph was built (its activations "
                               "were overwritten); differentiate before the next call on the same network")
-        g = d_logits.to(torch.float32).contiguous()
-        dx = torch.empty(ctx.shape, dtype=torch.float32, device=g.device)
-        check(lib.b2e_resnet_backward(m._h, C.c_void_p(g.data_ptr()), C.c_void_p(dx.data_ptr()), ctx.shape[0],
-                                      C.c_void_p(torch.cuda.current_stream().cuda_stream)), "resnet_backward")
-        return dx, None
+        return m.input_grad(d_logits), None
 
 
 class ResNet(UNet2DModel):
@@ -109,7 +105,7 @@ class ResNet(UNet2DModel):
                                    C.c_void_p(torch.cuda.current_stream().cuda_stream)), "resnet_forward")
         return logits
 
-    def __call__(self, image):
+    def _check_input(self, image):
         if not image.is_cuda:
             raise _C.B2EError("ResNet: image must be a CUDA tensor (no CPU fallback)")
         cfg = self.config
@@ -117,6 +113,27 @@ class ResNet(UNet2DModel):
             raise ValueError(f"ResNet: expected (B,{cfg.in_channels},{cfg.input_size},{cfg.input_size}), got {tuple(image.shape)}")
         if image.shape[0] > self.max_batch:
             raise ValueError(f"ResNet: batch {image.shape[0]} > max_batch {self.max_batch}")
+
+    def forward_keep(self, image):
+        """``net(image)`` with the activations kept in the engine's workspace for ``input_grad`` (no autograd graph)."""
+        self._check_input(image)
+        x = image.detach().to(torch.float32).contiguous()
+        logits = self._forward(x)
+        self._keep_gen, self._keep_shape = self._fwd_gen, tuple(x.shape)
+        return logits
+
+    def input_grad(self, d_logits):
+        """d(loss)/d(image) of the last ``forward_keep`` given d(loss)/d(logits) (native dgrad of the whole network)."""
+        if getattr(self, "_keep_gen", None) != self._fwd_gen:
+            raise _C.B2EError("ResNet.input_grad: the engine ran another forward since forward_keep (activations overwritten)")
+        g = d_logits.detach().to(torch.float32).contiguous()
+        dx = torch.empty(self._keep_shape, dtype=torch.float32, device=g.device)
+        check(lib.b2e_resnet_backward(self._h, C.c_void_p(g.data_ptr()), C.c_void_p(dx.data_ptr()), self._keep_shape[0],
+                                      C.c_void_p(torch.cuda.current_stream().cuda_stream)), "resnet_backward")
+        return dx
+
+    def __call__(self, image):
+        self._check_input(image)
         x = image if (image.dtype == torch.float32 and image.is_contiguous()) else image.to(torch.float32).contiguous()
         if x.requires_grad and torch.is_grad_enabled():
             return _ResNetFn.apply(x, self)

@@ -165,10 +165,11 @@ class SegmentationModel:
     square input resolution - mask creation feeds it 512x512, ``NetAttrFunc`` the decoded 256x256 image, both through
     this one object as in the reference - loaded from ``ckpt`` (the reference's Segmentation/res/cp/79999_iter.pth, a blob
     missing from the checkout) when the file exists, else seeded random-init weights.  ``net=`` (keyword-only)
-    substitutes any callable mapping a (1,3,S,S) image to ([1,19,S,S] logits, ...)."""
+    substitutes any callable mapping a (1,3,S,S) image to ([1,19,S,S] logits, ...).  ``max_batch`` (keyword-only) is the
+    largest batch the default parser differentiates at once (``NetAttrFunc(per_sample=True)`` on a batch of images)."""
 
     def __init__(self, ckpt: str = "Segmentation/res/cp/79999_iter.pth", n_classes: int = 19, image_size: tuple = (512, 512),
-                 *, net=None, seed: int = 0, precision: Optional[str] = None) -> None:
+                 *, net=None, seed: int = 0, precision: Optional[str] = None, max_batch: int = 1) -> None:
         self.device = get_device()
         if not (ckpt is None or isinstance(ckpt, (str, bytes)) or hasattr(ckpt, "__fspath__")):
             raise TypeError("SegmentationModel: the first argument is the checkpoint path (as in the reference); pass a "
@@ -176,7 +177,7 @@ class SegmentationModel:
         if net is None:
             import os
             from b200edit.bisenet import MultiResBiSeNet
-            net = MultiResBiSeNet(n_classes, max_batch=1, device=self.device, seed=seed, precision=precision)
+            net = MultiResBiSeNet(n_classes, max_batch=max_batch, device=self.device, seed=seed, precision=precision)
             if ckpt and os.path.exists(ckpt):
                 net.load_reference_state_dict(torch.load(ckpt, map_location="cpu"))
         self.net = net

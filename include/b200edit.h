@@ -193,6 +193,20 @@ int b2e_seg_area_head_f32(const float* logits, int64_t C, int64_t HW, const int3
  * dlogits (n) = the matching one-hot(s), zero elsewhere (may be NULL; loss may be NULL). */
 int b2e_classifier_head_f32(const float* logits, int64_t n, int idx_for_class, int idx_of_interest, int reg_idx,
                             int reg_pred, float reg_score, float* loss, float* dlogits, void* stream);
+/* Per-sample heads (AttrFunc per_sample=True): the loss is sum_b L_b with L_b the head above on image b alone.
+ * loss: DEVICE fp32 [B] (L_b); dlogits = dL_b/dlogits_b * grad_scale, the multiply being the last rounding step (the
+ * rounding autograd applies when it seeds loss_scale into the head's backward; grad_scale 1 is exact).
+ * Seg-area: logits (B,C,HW); the blocks and partial sums of one image depend on HW only, so image b's loss and gradient
+ * bits are those of a B = 1 call on image b (b2e_seg_area_head_f32 IS the B = 1, grad_scale 1 case).
+ * workspace: b2e_seg_area_head_batched_workspace_bytes(B). */
+size_t b2e_seg_area_head_batched_workspace_bytes(int64_t B);
+int b2e_seg_area_head_batched_f32(const float* logits, int64_t B, int64_t C, int64_t HW, const int32_t* classes,
+                                  int n_classes, float area_divisor, float grad_scale, float* loss, float* dlogits,
+                                  void* workspace, size_t workspace_bytes, void* stream);
+/* Classifier: logits (B,80), one row per image; dlogits (B,80) holds every image's gradient row. */
+int b2e_classifier_head_batched_f32(const float* logits, int64_t B, int idx_for_class, int idx_of_interest, int reg_idx,
+                                    int reg_pred, float reg_score, float grad_scale, float* loss, float* dlogits,
+                                    void* stream);
 
 /* ------------------------------------------------------------------ edit-friendly inversion
  * sample_xts_from_x0, src/ddpm_inversion.py:31-55: xts[i] = x0*sa[i] + noise[i]*sb[i], i<T;
