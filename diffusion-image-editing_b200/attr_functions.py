@@ -62,6 +62,37 @@ def _identity_decoder(model) -> bool:
     return bool(getattr(model, "decode_is_identity", False))
 
 
+def _native_decoder(model, B):
+    """The decoder of a nudge of B samples without autograd, as (decoder, chain): (None, 1.0) for an identity decoder;
+    a latent model's native decoder in gradient mode and chain = d(decoder input) / d(x0 prediction); None when the
+    model's decoder is not native or B exceeds its max_batch."""
+    if _identity_decoder(model):
+        return None, 1.0
+    nd = getattr(model, "native_decoder", None)
+    nd = nd() if callable(nd) else None
+    if nd is None or B > nd[0].max_batch:
+        return None
+    return nd
+
+
+def _decode_x0(xt, model_output, coeffs, dec, chain):
+    """x0' = (x - sqrt(1-a) eps) / sqrt(a), then the wrapper's decode scaling (SD: 1 / 0.18215 * latent) as its own rounding
+    step - the reference's op order, so the decoder sees bit-identical input on both paths - and the decoder forward,
+    kept for the backward of ``_guide``."""
+    lat = ops.pred_x0(xt, model_output, coeffs.sqrt_a_t, coeffs.sqrt_b_t)
+    if dec is None:
+        return lat
+    if chain != 1.0:
+        lat = ops.axpby(lat, lat, chain, 0.0)
+    return dec.decode_keep(lat)
+
+
+def _guide(xt, d_img, dec, chain, coeffs, gmask):
+    """The nudged sample from d(loss)/d(image) of ``_decode_x0``'s image: decoder backward, then the update kernel."""
+    d_lat = d_img if dec is None else dec.latent_grad(d_img)
+    return ops.apply_latent_guidance(xt, d_lat, chain, coeffs.sqrt_a_t, coeffs.a_t_sq, mask=gmask)
+
+
 class AttrFunc(ABC):
     """Base class of the guidance strategies.  kwargs understood by ``apply`` (also stored at
     construction and splatted back by the pipeline): use_mask, mask, mask_attr_grad,
@@ -190,9 +221,8 @@ class AttrFunc(ABC):
         kernel -> decoder backward (dgrad twins) -> fused update kernel.  No autograd graph, no torch arithmetic.
         Returns None when the strategy / model does not qualify (the caller falls back to autograd, as the reference)."""
         spec = self.colour_spec()
-        nd = getattr(model, "native_decoder", None)
-        nd = nd() if callable(nd) else None
-        if spec is None or nd is None or self.nudge_zt or not self.nudge_xt:
+        nd = _native_decoder(model, xt.shape[0])
+        if spec is None or nd is None or nd[0] is None or self.nudge_zt or not self.nudge_xt:
             return None
         dec, chain = nd
         targets, weights = spec
@@ -207,23 +237,15 @@ class AttrFunc(ABC):
             x_0, lam = kwargs.get("x_0"), kwargs.get("lambda_")
             if mask is None or x_0 is None or lam is None or mask.shape[-1] != out_size or x_0.shape[-1] != out_size:
                 return None            # shapes that do not broadcast against the decoded image: let torch report it
-        if xt.shape[0] > dec.max_batch:
-            return None
-        # x0' = (x - sqrt(1-a) eps) / sqrt(a), then the wrapper's decode scaling (SD: 1 / 0.18215 * latent) as its own
-        # rounding step - the reference's op order, so the decoder sees bit-identical input on both paths
-        lat = ops.pred_x0(xt, model_output, coeffs.sqrt_a_t, coeffs.sqrt_b_t)
-        if chain != 1.0:
-            lat = ops.axpby(lat, lat, chain, 0.0)
-        img = dec.decode_keep(lat)
+        gmask = mask if kwargs.get("mask_attr_grad", False) else None
+        if gmask is not None and gmask.shape[-1] != xt.shape[-1]:
+            return None                # a mask that does not match the latent: the generic path reports it
+        img = _decode_x0(xt, model_output, coeffs, dec, chain)
         n_mean = img.shape[-1] * img.shape[-2] * (1 if self.per_sample else img.shape[0])
         d_img = ops.color_loss_grad(img, targets, weights, self.loss_scale, n_mean,
                                     mask=mask if mask_pred else None, x_ref=kwargs.get("x_0") if mask_pred else None,
                                     lambda_=kwargs.get("lambda_") if mask_pred else None)
-        d_lat = dec.latent_grad(d_img)
-        gmask = mask if kwargs.get("mask_attr_grad", False) else None
-        if gmask is not None and gmask.shape[-1] != xt.shape[-1]:
-            return None                # a mask that does not match the latent: the generic path reports it
-        return ops.apply_latent_guidance(xt, d_lat, chain, coeffs.sqrt_a_t, coeffs.a_t_sq, mask=gmask)
+        return _guide(xt, d_img, dec, chain, coeffs, gmask)
 
     def _apply_native_lpips(self, xt, model_output, coeffs, model, **kwargs):
         """Built-in colour strategies with the LPIPS regulariser (mask_pred_original_sample + use_lpips) on the native
@@ -242,29 +264,21 @@ class AttrFunc(ABC):
             raise ValueError("No mask specified")
         if mask is None or x_0 is None or lam is None or not torch.is_tensor(mask) or not torch.is_tensor(x_0):
             return None
-        dec, chain = None, 1.0
-        if not _identity_decoder(model):
-            nd = getattr(model, "native_decoder", None)
-            nd = nd() if callable(nd) else None
-            if nd is None:
-                return None
-            dec, chain = nd
-            if xt.shape[0] > dec.max_batch:
-                return None
+        nd = _native_decoder(model, xt.shape[0])
+        if nd is None:
+            return None
+        dec, chain = nd
         S = lp.config.input_size
         B = xt.shape[0]
         if (B > lp.max_batch or mask.dim() != 4 or mask.shape[0] not in (1, B) or mask.shape[1] not in (1, 3)
                 or tuple(mask.shape[2:]) != (S, S) or x_0.dim() != 4 or tuple(x_0.shape[1:]) != (3, S, S)
                 or x_0.shape[0] not in (1, B)):
             return None
+        gmask = mask if kwargs.get("mask_attr_grad", False) else None
+        if gmask is not None and tuple(gmask.shape[1:]) != tuple(xt.shape[1:]):
+            return None                # a mask that does not match the sample: the generic path reports it
         targets, weights = spec
-        lat = ops.pred_x0(xt, model_output, coeffs.sqrt_a_t, coeffs.sqrt_b_t)
-        if dec is None:
-            img = lat
-        else:
-            if chain != 1.0:
-                lat = ops.axpby(lat, lat, chain, 0.0)
-            img = dec.decode_keep(lat)
+        img = _decode_x0(xt, model_output, coeffs, dec, chain)
         if tuple(img.shape[1:]) != (3, S, S):
             return None
         with torch.no_grad():
@@ -272,11 +286,7 @@ class AttrFunc(ABC):
             d_lp = lp.input_grad(torch.ones(B, dtype=torch.float32, device=img.device))
         d_img = ops.lpips_guidance_grad(img, mask, d_lp, targets, weights, self.loss_scale,
                                         img.shape[-1] * img.shape[-2] * B, lam)
-        d_lat = d_img if dec is None else dec.latent_grad(d_img)
-        gmask = mask if kwargs.get("mask_attr_grad", False) else None
-        if gmask is not None and tuple(gmask.shape[1:]) != tuple(xt.shape[1:]):
-            return None                # a mask that does not match the sample: the generic path reports it
-        return ops.apply_latent_guidance(xt, d_lat, chain, coeffs.sqrt_a_t, coeffs.a_t_sq, mask=gmask)
+        return _guide(xt, d_img, dec, chain, coeffs, gmask)
 
     def _apply_native_network(self, xt, model_output, coeffs, model, **kwargs):
         """Network strategies with per_sample=True on a native network: x0' kernel (-> chain scaling, native decoder
@@ -290,16 +300,13 @@ class AttrFunc(ABC):
         if kwargs.get("mask_attr_grad", False) and mask is None:
             raise ValueError("No mask specified")
         B = xt.shape[0]
-        dec, chain, size = None, 1.0, xt.shape[-1]
-        if not _identity_decoder(model):
-            nd = getattr(model, "native_decoder", None)
-            nd = nd() if callable(nd) else None
-            if nd is None:
-                return None
-            dec, chain = nd
-            size = getattr(dec, "out_size", None)
-            if size is None or B > dec.max_batch:
-                return None
+        nd = _native_decoder(model, B)
+        if nd is None:
+            return None
+        dec, chain = nd
+        size = xt.shape[-1] if dec is None else getattr(dec, "out_size", None)
+        if size is None:
+            return None
         gmask = mask if kwargs.get("mask_attr_grad", False) else None
         if gmask is not None and (not torch.is_tensor(gmask) or gmask.dim() != 4 or gmask.shape[0] not in (1, B)
                                   or gmask.shape[1] not in (1, xt.shape[1]) or gmask.shape[2:] != xt.shape[2:]):
@@ -307,16 +314,9 @@ class AttrFunc(ABC):
         net = self.native_network(int(size))
         if net is None or B > net.max_batch:
             return None
-        lat = ops.pred_x0(xt, model_output, coeffs.sqrt_a_t, coeffs.sqrt_b_t)
-        if dec is None:
-            img = lat
-        else:
-            if chain != 1.0:
-                lat = ops.axpby(lat, lat, chain, 0.0)
-            img = dec.decode_keep(lat)
+        img = _decode_x0(xt, model_output, coeffs, dec, chain)
         d_img = net.input_grad(self.native_head_grad(net.forward_keep(img)))
-        d_lat = d_img if dec is None else dec.latent_grad(d_img)
-        return ops.apply_latent_guidance(xt, d_lat, chain, coeffs.sqrt_a_t, coeffs.a_t_sq, mask=gmask)
+        return _guide(xt, d_img, dec, chain, coeffs, gmask)
 
     def in_window(self, step_idx: int) -> bool:
         return self.t1 <= step_idx < self.t2

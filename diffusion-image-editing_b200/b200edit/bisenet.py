@@ -9,31 +9,13 @@ the tcgen05 implicit-GEMM kernel with ReLU in the epilogue, the channel-attentio
 convolutions -> sigmoid) as small fp32 kernels, the final align_corners bilinear upsampling as one kernel."""
 from __future__ import annotations
 
-import ctypes as C
 from types import SimpleNamespace
 
 import torch
 
 from . import _C
-from ._C import ResNetConfig, check, lib
-from .unet import UNet2DModel
-
-
-class _BiSeNetFn(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, image, model):
-        ctx.model = model
-        out = model.forward_keep(image)
-        ctx.gen = model._fwd_gen      # the activations of THIS forward live in the engine's single workspace
-        return out
-
-    @staticmethod
-    def backward(ctx, d_logits):
-        m = ctx.model
-        if m._fwd_gen != ctx.gen:
-            raise _C.B2EError("BiSeNet backward: the engine ran another forward since this graph was built (its activations "
-                              "were overwritten); differentiate before the next call on the same network")
-        return m.input_grad(d_logits), None
+from ._C import ResNetConfig, lib
+from .engine import Engine
 
 
 def _fold(w, sd, bn, eps=1e-5):
@@ -43,7 +25,9 @@ def _fold(w, sd, bn, eps=1e-5):
     return (w.double() * s.view(-1, 1, 1, 1)).float(), (b - mu * s).float()
 
 
-class BiSeNet(UNet2DModel):
+class BiSeNet(Engine):
+    differentiable = False
+
     def __init__(self, n_classes=19, input_size=512, max_batch=1, device="cuda", precision=None):
         """precision: None / "fp16" - f16 operands throughout; "fp32" - fp32-accurate FORWARD (split f16 operands), so
         the ReLU / max-pool masks the backward pass routes gradients with are those of the fp32 network (see
@@ -52,47 +36,25 @@ class BiSeNet(UNet2DModel):
         self.precision, precision_cfg = _C.resolve_precision(precision, "BiSeNet")
         self.config = SimpleNamespace(n_classes=n_classes, input_size=input_size, in_channels=3, sample_size=input_size,
                                       out_channels=n_classes)
-        self.device = torch.device(device)
-        self.dtype = torch.float32
-        self.max_batch = int(max_batch)
         cfg = ResNetConfig()
         cfg.input_size, cfg.in_channels, cfg.bottleneck, cfg.width, cfg.num_classes, cfg.head = input_size, 3, 0, 64, n_classes, 1
         for i in range(4):
             cfg.layers[i] = 2
         cfg.precision = precision_cfg
-        h = C.c_void_p()
-        with torch.cuda.device(self.device):
-            check(lib.b2e_resnet_create(C.byref(cfg), self.max_batch, C.byref(h)), "bisenet_create")
-            self._h = h
-            nbytes = lib.b2e_unet_workspace_bytes(h)
-            self._ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
-            base = (self._ws.data_ptr() + 255) // 256 * 256
-            check(lib.b2e_unet_bind_workspace(h, C.c_void_p(base), nbytes), "unet_bind_workspace")
-        self._t_cache = {}
-        self.differentiable = False
+        self._create(lib.b2e_resnet_create, cfg, max_batch, device)
 
     def enable_grad(self, enable: bool = True):
         """Gradient mode: ``net(x)[0]`` becomes differentiable w.r.t. the image (native dgrad of the whole parser;
         batches <= max_batch).  Costs workspace: the backward pass has its own buffers."""
-        with torch.cuda.device(self.device):
-            check(lib.b2e_unet_enable_grad(self._h, int(enable)), "unet_enable_grad")
-            nbytes = lib.b2e_unet_workspace_bytes(self._h)
-            self._ws = None
-            self._ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
-            base = (self._ws.data_ptr() + 255) // 256 * 256
-            check(lib.b2e_unet_bind_workspace(self._h, C.c_void_p(base), nbytes), "unet_bind_workspace")
+        self._enable_grad(enable)
         self.differentiable = bool(enable)
         return self
 
-    _fwd_gen = 0   # bumped by every forward: a backward over a stale workspace is detected (see _BiSeNetFn)
+    _backward_fn = lib.b2e_resnet_backward
 
-    def _forward(self, x):
+    def _out_shape(self, B):
         cfg = self.config
-        self._fwd_gen += 1
-        o = torch.empty((x.shape[0], cfg.n_classes, cfg.input_size, cfg.input_size), dtype=torch.float32, device=x.device)
-        check(lib.b2e_unet_forward(self._h, C.c_void_p(x.data_ptr()), None, C.c_void_p(o.data_ptr()), x.shape[0],
-                                   C.c_void_p(torch.cuda.current_stream().cuda_stream)), "bisenet_forward")
-        return o
+        return (B, cfg.n_classes, cfg.input_size, cfg.input_size)
 
     @staticmethod
     def fold_reference_state_dict(sd, eps=1e-5):
@@ -129,55 +91,39 @@ class BiSeNet(UNet2DModel):
     def load_reference_state_dict(self, sd, eps=1e-5):
         return self.load_state_dict(self.fold_reference_state_dict(sd, eps))
 
-    def _check_input(self, image):
+    def _check_input(self, image, keep=False):
         if not image.is_cuda:
             raise _C.B2EError("BiSeNet: image must be a CUDA tensor (no CPU fallback)")
         cfg = self.config
         if tuple(image.shape[1:]) != (3, cfg.input_size, cfg.input_size):
             raise ValueError(f"BiSeNet: expected (B,3,{cfg.input_size},{cfg.input_size}), got {tuple(image.shape)}")
+        if keep and not self.differentiable:
+            raise _C.B2EError("BiSeNet: call enable_grad() before differentiating through the native face parser")
+        if keep and image.shape[0] > self.max_batch:
+            raise ValueError(f"BiSeNet with gradient: batch {image.shape[0]} > max_batch {self.max_batch}")
 
     def forward_keep(self, image):
         """Logits (B, n_classes, S, S) - ``net(image)[0]`` - with the activations kept in the engine's workspace for
         ``input_grad`` (no autograd graph).  Needs gradient mode (``enable_grad()``) and B <= max_batch."""
-        self._check_input(image)
-        if not self.differentiable:
-            raise _C.B2EError("BiSeNet: call enable_grad() before differentiating through the native face parser")
-        if image.shape[0] > self.max_batch:
-            raise ValueError(f"BiSeNet with gradient: batch {image.shape[0]} > max_batch {self.max_batch}")
-        x = image.detach().to(torch.float32).contiguous()
-        out = self._forward(x)
-        self._keep_gen, self._keep_shape = self._fwd_gen, tuple(x.shape)
-        return out
+        self._check_input(image, keep=True)
+        return self._keep(image.detach().to(torch.float32).contiguous())
 
     def input_grad(self, d_logits):
         """d(loss)/d(image) of the last ``forward_keep`` given d(loss)/d(logits) (native dgrad of the whole parser)."""
-        if getattr(self, "_keep_gen", None) != self._fwd_gen:
-            raise _C.B2EError("BiSeNet.input_grad: the engine ran another forward since forward_keep (activations overwritten)")
-        g = d_logits.detach().to(torch.float32).contiguous()
-        dx = torch.empty(self._keep_shape, dtype=torch.float32, device=g.device)
-        check(lib.b2e_resnet_backward(self._h, C.c_void_p(g.data_ptr()), C.c_void_p(dx.data_ptr()), self._keep_shape[0],
-                                      C.c_void_p(torch.cuda.current_stream().cuda_stream)), "bisenet_backward")
-        return dx
+        return self._keep_grad(d_logits)
 
     def __call__(self, image):
-        self._check_input(image)
-        cfg = self.config
-        if image.requires_grad and torch.is_grad_enabled():
+        grad = image.requires_grad and torch.is_grad_enabled()
+        self._check_input(image, keep=grad)
+        if grad:
             xx = image if (image.dtype == torch.float32 and image.is_contiguous()) else image.to(torch.float32).contiguous()
-            return (_BiSeNetFn.apply(xx, self), None, None)
-        x = image.detach().to(torch.float32).contiguous()
-        outs = []
-        for b0 in range(0, x.shape[0], self.max_batch):
-            self._fwd_gen += 1
-            xb = x[b0:b0 + self.max_batch]
-            o = torch.empty((xb.shape[0], cfg.n_classes, cfg.input_size, cfg.input_size), dtype=torch.float32, device=x.device)
-            check(lib.b2e_unet_forward(self._h, C.c_void_p(xb.data_ptr()), None, C.c_void_p(o.data_ptr()), xb.shape[0],
-                                       C.c_void_p(torch.cuda.current_stream().cuda_stream)), "bisenet_forward")
-            outs.append(o)
-        return (outs[0] if len(outs) == 1 else torch.cat(outs), None, None)
+            return (self._keep_node(xx), None, None)
+        return (self._forward_sliced(image.detach().to(torch.float32).contiguous()), None, None)
 
-    def eval(self):
-        return self
+    def profile(self, image, timestep=None):
+        """Per-op CUDA-event timings of one forward (``timestep`` is ignored: the face parser has none)."""
+        x = image.detach().to(torch.float32).contiguous()
+        return self._profile(x, None, torch.empty(self._out_shape(x.shape[0]), dtype=torch.float32, device=x.device))
 
 
 class MultiResBiSeNet:

@@ -5,14 +5,13 @@ attention kernel, quick-GELU MLP, every linear layer on the implicit-GEMM kernel
 Parameters load from a transformers ``state_dict`` unchanged.  The tokenizer (BPE files) stays the caller's."""
 from __future__ import annotations
 
-import ctypes as C
 from types import SimpleNamespace
 
 import torch
 
 from . import _C
-from ._C import ClipConfig, check, lib
-from .unet import UNet2DModel
+from ._C import ClipConfig, lib
+from .engine import Engine, _ptr, _stream
 
 # openai/clip-vit-large-patch14 text tower (the text encoder of Stable Diffusion 1.x)
 SD15_CLIP_CONFIG = dict(vocab_size=49408, hidden_size=768, intermediate_size=3072, num_hidden_layers=12,
@@ -25,7 +24,7 @@ class TextEncoderOutput(tuple):
         return self[0]
 
 
-class CLIPTextModel(UNet2DModel):
+class CLIPTextModel(Engine):
     def __init__(self, vocab_size=49408, hidden_size=768, intermediate_size=3072, num_hidden_layers=12,
                  num_attention_heads=12, max_position_embeddings=77, max_batch=2, device="cuda"):
         _C.require_device()
@@ -33,37 +32,25 @@ class CLIPTextModel(UNet2DModel):
                                       num_hidden_layers=num_hidden_layers, num_attention_heads=num_attention_heads,
                                       max_position_embeddings=max_position_embeddings, in_channels=1, sample_size=8,
                                       out_channels=1)
-        self.device = torch.device(device)
-        self.dtype = torch.float32
-        self.max_batch = int(max_batch)
         cfg = ClipConfig()
         cfg.vocab_size, cfg.hidden_size, cfg.intermediate_size = vocab_size, hidden_size, intermediate_size
         cfg.num_layers, cfg.num_heads, cfg.max_positions = num_hidden_layers, num_attention_heads, max_position_embeddings
-        h = C.c_void_p()
-        with torch.cuda.device(self.device):
-            check(lib.b2e_clip_create(C.byref(cfg), self.max_batch, C.byref(h)), "clip_create")
-            self._h = h
-            nbytes = lib.b2e_unet_workspace_bytes(h)
-            self._ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
-            base = (self._ws.data_ptr() + 255) // 256 * 256
-            check(lib.b2e_unet_bind_workspace(h, C.c_void_p(base), nbytes), "unet_bind_workspace")
-        self._t_cache = {}
+        self._create(lib.b2e_clip_create, cfg, max_batch, device)
 
     def load_state_dict(self, sd, strict=True):
         sd = {k: v for k, v in sd.items() if not k.endswith("position_ids")}   # a buffer of older transformers versions
         return super().load_state_dict(sd, strict)
 
+    def _forward(self, ids):
+        ids = ids.contiguous()
+        o = torch.empty((ids.shape[0], ids.shape[1], self.config.hidden_size), dtype=torch.float32, device=self.device)
+        self._launch(lib.b2e_clip_forward, _ptr(ids), ids.shape[1], _ptr(o), ids.shape[0], _stream())
+        return o
+
     def __call__(self, input_ids, **_):
         ids = input_ids.to(self.device, torch.int64).contiguous()
         if ids.dim() != 2 or ids.shape[1] > self.config.max_position_embeddings:
             raise ValueError(f"CLIPTextModel: input_ids must be (B, L <= {self.config.max_position_embeddings}), got {tuple(ids.shape)}")
-        outs = []
-        for b0 in range(0, ids.shape[0], self.max_batch):
-            ib = ids[b0:b0 + self.max_batch].contiguous()
-            o = torch.empty((ib.shape[0], ib.shape[1], self.config.hidden_size), dtype=torch.float32, device=self.device)
-            check(lib.b2e_clip_forward(self._h, C.c_void_p(ib.data_ptr()), ib.shape[1], C.c_void_p(o.data_ptr()), ib.shape[0],
-                                       C.c_void_p(torch.cuda.current_stream().cuda_stream)), "clip_forward")
-            outs.append(o)
-        return TextEncoderOutput((outs[0] if len(outs) == 1 else torch.cat(outs),))
+        return TextEncoderOutput((self._forward_sliced(ids),))
 
     forward = __call__

@@ -8,14 +8,13 @@ kernels, the input gradient on the dgrad twins of the same convolutions.  The se
 its normalised features are computed once and cached in the engine (re-run only when that tensor changes)."""
 from __future__ import annotations
 
-import ctypes as C
 from types import SimpleNamespace
 
 import torch
 
 from . import _C
-from ._C import LpipsConfig, check, lib
-from .unet import UNet2DModel
+from ._C import LpipsConfig, lib
+from .engine import Engine, _ptr, _stream
 
 # (slice, index in vgg16().features, in channels, out channels) of the thirteen convolutions
 VGG16_CONVS = ((1, 0, 3, 64), (1, 2, 64, 64), (2, 5, 64, 128), (2, 7, 128, 128), (3, 10, 128, 256), (3, 12, 256, 256),
@@ -26,27 +25,12 @@ SCALING_SHIFT = (-.030, -.088, -.188)
 SCALING_SCALE = (.458, .448, .450)
 
 
-class _LPIPSFn(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, in0, model, mask):
-        ctx.model, ctx.shape = model, tuple(in0.shape)
-        out = model._forward(in0, mask)
-        ctx.gen = model._fwd_gen      # the activations of THIS forward live in the engine's single workspace
-        return out
-
-    @staticmethod
-    def backward(ctx, d_out):
-        m = ctx.model
-        if m._fwd_gen != ctx.gen:
-            raise _C.B2EError("LPIPS backward: the engine ran another forward since this graph was built (its activations "
-                              "were overwritten); differentiate before the next call on the same network")
-        return m._backward(d_out.reshape(ctx.shape[0])), None, None
-
-
-class LPIPS(UNet2DModel):
+class LPIPS(Engine):
     """``d = LPIPS(...)(in0, in1)``: (B, 1, 1, 1), like ``lpips.LPIPS.forward``; in0 (B, 3, S, S) and in1 (1 | B, 3, S, S)
-    fp32 CUDA tensors in [-1, 1].  Autograd node in ``in0`` only.  Shares parameter loading / profiling with the UNet
-    wrapper (same engine handle type); parameters under ``lpips.LPIPS().state_dict()`` names."""
+    fp32 CUDA tensors in [-1, 1].  Autograd node in ``in0`` only; parameters under ``lpips.LPIPS().state_dict()`` names."""
+
+    _ref = None             # the reference tensor whose features the engine holds (kept alive: identity check)
+    _mask = None            # the mask the engine reads in the backward of the last forward (kept alive)
 
     def __init__(self, net="vgg", input_size=256, max_batch=1, device="cuda", precision="fp32"):
         """precision: "fp32" (default) - fp32-accurate FORWARD (split 16-bit operands, three tensor-core products per
@@ -57,22 +41,9 @@ class LPIPS(UNet2DModel):
         _C.require_device()
         self.precision, precision_cfg = _C.resolve_precision(precision, "LPIPS")
         self.config = SimpleNamespace(net=net, input_size=input_size, sample_size=input_size, in_channels=3, out_channels=1)
-        self.device = torch.device(device)
-        self.dtype = torch.float32
-        self.max_batch = int(max_batch)
         cfg = LpipsConfig()
         cfg.input_size, cfg.precision = input_size, precision_cfg
-        h = C.c_void_p()
-        with torch.cuda.device(self.device):
-            check(lib.b2e_lpips_create(C.byref(cfg), self.max_batch, C.byref(h)), "lpips_create")
-            self._h = h
-            nbytes = lib.b2e_unet_workspace_bytes(h)
-            self._ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
-            base = (self._ws.data_ptr() + 255) // 256 * 256
-            check(lib.b2e_unet_bind_workspace(h, C.c_void_p(base), nbytes), "unet_bind_workspace")
-        self._t_cache = {}
-        self._ref = None            # the reference tensor whose features the engine holds (kept alive: identity check)
-        self._mask = None           # the mask the engine reads in the backward of the last forward (kept alive)
+        self._create(lib.b2e_lpips_create, cfg, max_batch, device)
 
     # ------------------------------------------------------------------ parameters
     def load_state_dict(self, sd, strict=True):
@@ -107,16 +78,10 @@ class LPIPS(UNet2DModel):
         return lpips_random_state_dict(seed)
 
     # ------------------------------------------------------------------ forward / backward
-    _fwd_gen = 0   # bumped by every forward: a backward over a stale workspace is detected (see _LPIPSFn)
+    _backward_fn = lib.b2e_lpips_backward
 
     def enable_grad(self, enable: bool = True):
-        with torch.cuda.device(self.device):
-            check(lib.b2e_unet_enable_grad(self._h, int(enable)), "unet_enable_grad")
-            nbytes = lib.b2e_unet_workspace_bytes(self._h)
-            self._ws = None
-            self._ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
-            base = (self._ws.data_ptr() + 255) // 256 * 256
-            check(lib.b2e_unet_bind_workspace(self._h, C.c_void_p(base), nbytes), "unet_bind_workspace")
+        self._enable_grad(enable)
         self._ref = None                # the engine dropped the cached reference with the workspace
         return self
 
@@ -136,29 +101,16 @@ class LPIPS(UNet2DModel):
             return
         x = self._check(in1, "in1", lambda b: 1 <= b <= self.max_batch).detach()
         self._ref = None
-        self._fwd_gen += 1
-        check(lib.b2e_lpips_set_reference(self._h, C.c_void_p(x.data_ptr()), x.shape[0],
-                                          C.c_void_p(torch.cuda.current_stream().cuda_stream)), "lpips_set_reference")
+        self._launch(lib.b2e_lpips_set_reference, _ptr(x), x.shape[0], _stream())
         self._ref = (in1, in1._version)
 
     def _forward(self, x, mask=None):
-        self._fwd_gen += 1
         self._mask = mask           # the backward's -mask chain reads this memory: it lives until the next forward
         B = x.shape[0]
         dist = torch.empty((B, 1, 1, 1), dtype=torch.float32, device=x.device)
-        mp, mb = (None, 0) if mask is None else (C.c_void_p(mask.data_ptr()), mask.shape[0])
-        check(lib.b2e_lpips_forward(self._h, C.c_void_p(x.data_ptr()), mp, mb, C.c_void_p(dist.data_ptr()), B,
-                                    C.c_void_p(torch.cuda.current_stream().cuda_stream)), "lpips_forward")
+        self._launch(lib.b2e_lpips_forward, _ptr(x), _ptr(mask), 0 if mask is None else mask.shape[0], _ptr(dist), B,
+                     _stream())
         return dist
-
-    def _backward(self, d_dist):
-        g = d_dist.to(torch.float32).contiguous()
-        B = g.shape[0]
-        S = self.config.input_size
-        dx = torch.empty((B, 3, S, S), dtype=torch.float32, device=g.device)
-        check(lib.b2e_lpips_backward(self._h, C.c_void_p(g.data_ptr()), C.c_void_p(dx.data_ptr()), B,
-                                     C.c_void_p(torch.cuda.current_stream().cuda_stream)), "lpips_backward")
-        return dx
 
     def __call__(self, in0, in1, normalize=False, mask=None):
         """LPIPS(in0, in1) (B, 1, 1, 1).  ``mask`` (extension, 1 | B, 3, S, S): the distance of ``1 - mask * in0`` -
@@ -176,30 +128,19 @@ class LPIPS(UNet2DModel):
                                else mask, "mask", lambda b: b in (1, B)).detach()
         self.set_reference(in1)
         if x.requires_grad and torch.is_grad_enabled():
-            return _LPIPSFn.apply(x, self, mask)
-        return self._forward(x.detach(), mask)
+            return self._keep_node(x, mask)
+        return self._keep(x.detach(), mask)
 
     forward = __call__
 
     def input_grad(self, d_dist):
         """d(sum_b d_dist[b] * dist[b]) / d(in0) of the last forward (through its mask transform), without autograd."""
-        return self._backward(d_dist.reshape(-1))
+        return self._keep_grad(d_dist)
 
     def profile(self, in0):
         x = self._check(in0, "in0", lambda b: 1 <= b <= self.max_batch).detach()
-        B = x.shape[0]
-        out = torch.empty((B,), dtype=torch.float32, device=x.device)
-        self._fwd_gen += 1          # profiling forwards overwrite the activations (and run without a mask)
-        self._mask = None
-        cap = 1024
-        n = C.c_int()
-        ms, fl, by, kd = (C.c_float * cap)(), (C.c_double * cap)(), (C.c_double * cap)(), (C.c_int * cap)()
-        check(lib.b2e_unet_profile(self._h, C.c_void_p(x.data_ptr()), None, C.c_void_p(out.data_ptr()), B,
-                                   C.c_void_p(torch.cuda.current_stream().cuda_stream), cap, C.byref(n), ms, fl, by, kd),
-              "lpips_profile")
-        names = {0: "conv_igemm", 1: "groupnorm", 2: "attention", 3: "other"}
-        return [dict(kind=names[kd[i]], ms=ms[i], flops=fl[i], bytes=by[i],
-                     desc=lib.b2e_unet_op_desc(self._h, i).decode()) for i in range(n.value)]
+        self._mask = None           # profiling forwards run without a mask
+        return self._profile(x, None, torch.empty((x.shape[0],), dtype=torch.float32, device=x.device))
 
 
 def lpips_random_state_dict(seed=0):

@@ -7,38 +7,19 @@ convolution runs on the tcgen05 implicit-GEMM kernel (bf16 operands, fp32 accumu
 the block shortcut fused as a K segment; the input gradient runs on the dgrad twins of the same kernel."""
 from __future__ import annotations
 
-import ctypes as C
 from types import SimpleNamespace
 
 import torch
 
 from . import _C
-from ._C import ResNetConfig, check, lib
-from .unet import UNet2DModel
+from ._C import ResNetConfig, lib
+from .engine import Engine
 
 RESNET50_LAYERS = (3, 4, 6, 3)
 
 
-class _ResNetFn(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, image, model):
-        ctx.model = model
-        out = model.forward_keep(image)
-        ctx.gen = model._fwd_gen      # the activations of THIS forward live in the engine's single workspace
-        return out
-
-    @staticmethod
-    def backward(ctx, d_logits):
-        m = ctx.model
-        if m._fwd_gen != ctx.gen:
-            raise _C.B2EError("ResNet backward: the engine ran another forward since this graph was built (its activations "
-                              "were overwritten); differentiate before the next call on the same network")
-        return m.input_grad(d_logits), None
-
-
-class ResNet(UNet2DModel):
-    """``logits = net(image)``; image (B, C, S, S) fp32 CUDA, S a power of two >= 64.  Shares parameter loading /
-    random init / profiling with the UNet wrapper (same engine handle type)."""
+class ResNet(Engine):
+    """``logits = net(image)``; image (B, C, S, S) fp32 CUDA, S a power of two >= 64."""
 
     def __init__(self, block="bottleneck", layers=RESNET50_LAYERS, num_classes=80, input_size=256, in_channels=3, width=64,
                  max_batch=8, device="cuda", precision=None):
@@ -51,24 +32,13 @@ class ResNet(UNet2DModel):
             raise ValueError("ResNet: block must be 'bottleneck' or 'basic'")
         self.config = SimpleNamespace(block=block, layers=tuple(layers), num_classes=num_classes, input_size=input_size,
                                       in_channels=in_channels, sample_size=input_size, out_channels=num_classes, width=width)
-        self.device = torch.device(device)
-        self.dtype = torch.float32
-        self.max_batch = int(max_batch)
         cfg = ResNetConfig()
         cfg.input_size, cfg.in_channels, cfg.bottleneck = input_size, in_channels, int(block == "bottleneck")
         for i in range(4):
             cfg.layers[i] = layers[i]
         cfg.width, cfg.num_classes = width, num_classes
         cfg.precision = precision_cfg
-        h = C.c_void_p()
-        with torch.cuda.device(self.device):
-            check(lib.b2e_resnet_create(C.byref(cfg), self.max_batch, C.byref(h)), "resnet_create")
-            self._h = h
-            nbytes = lib.b2e_unet_workspace_bytes(h)
-            self._ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
-            base = (self._ws.data_ptr() + 255) // 256 * 256
-            check(lib.b2e_unet_bind_workspace(h, C.c_void_p(base), nbytes), "unet_bind_workspace")
-        self._t_cache = {}
+        self._create(lib.b2e_resnet_create, cfg, max_batch, device)
 
     # ------------------------------------------------------------------ parameters
     @staticmethod
@@ -96,14 +66,10 @@ class ResNet(UNet2DModel):
         return self.load_state_dict(self.fold_batchnorm(sd, eps))
 
     # ------------------------------------------------------------------ forward / backward
-    _fwd_gen = 0   # bumped by every forward: a backward over a stale workspace is detected (see _ResNetFn)
+    _backward_fn = lib.b2e_resnet_backward
 
-    def _forward(self, x):
-        self._fwd_gen += 1
-        logits = torch.empty((x.shape[0], self.config.num_classes), dtype=torch.float32, device=x.device)
-        check(lib.b2e_unet_forward(self._h, C.c_void_p(x.data_ptr()), None, C.c_void_p(logits.data_ptr()), x.shape[0],
-                                   C.c_void_p(torch.cuda.current_stream().cuda_stream)), "resnet_forward")
-        return logits
+    def _out_shape(self, B):
+        return (B, self.config.num_classes)
 
     def _check_input(self, image):
         if not image.is_cuda:
@@ -117,43 +83,24 @@ class ResNet(UNet2DModel):
     def forward_keep(self, image):
         """``net(image)`` with the activations kept in the engine's workspace for ``input_grad`` (no autograd graph)."""
         self._check_input(image)
-        x = image.detach().to(torch.float32).contiguous()
-        logits = self._forward(x)
-        self._keep_gen, self._keep_shape = self._fwd_gen, tuple(x.shape)
-        return logits
+        return self._keep(image.detach().to(torch.float32).contiguous())
 
     def input_grad(self, d_logits):
         """d(loss)/d(image) of the last ``forward_keep`` given d(loss)/d(logits) (native dgrad of the whole network)."""
-        if getattr(self, "_keep_gen", None) != self._fwd_gen:
-            raise _C.B2EError("ResNet.input_grad: the engine ran another forward since forward_keep (activations overwritten)")
-        g = d_logits.detach().to(torch.float32).contiguous()
-        dx = torch.empty(self._keep_shape, dtype=torch.float32, device=g.device)
-        check(lib.b2e_resnet_backward(self._h, C.c_void_p(g.data_ptr()), C.c_void_p(dx.data_ptr()), self._keep_shape[0],
-                                      C.c_void_p(torch.cuda.current_stream().cuda_stream)), "resnet_backward")
-        return dx
+        return self._keep_grad(d_logits)
 
     def __call__(self, image):
         self._check_input(image)
         x = image if (image.dtype == torch.float32 and image.is_contiguous()) else image.to(torch.float32).contiguous()
         if x.requires_grad and torch.is_grad_enabled():
-            return _ResNetFn.apply(x, self)
+            return self._keep_node(x)
         return self._forward(x.detach())
 
     forward = __call__
 
     def profile(self, image):
         x = image.detach().to(torch.float32).contiguous()
-        B = x.shape[0]
-        out = torch.empty((B, self.config.num_classes), dtype=torch.float32, device=x.device)
-        cap = 1024
-        n = C.c_int()
-        ms, fl, by, kd = (C.c_float * cap)(), (C.c_double * cap)(), (C.c_double * cap)(), (C.c_int * cap)()
-        check(lib.b2e_unet_profile(self._h, C.c_void_p(x.data_ptr()), None, C.c_void_p(out.data_ptr()), B,
-                                   C.c_void_p(torch.cuda.current_stream().cuda_stream), cap, C.byref(n), ms, fl, by, kd),
-              "resnet_profile")
-        names = {0: "conv_igemm", 1: "groupnorm", 2: "attention", 3: "other"}
-        return [dict(kind=names[kd[i]], ms=ms[i], flops=fl[i], bytes=by[i],
-                     desc=lib.b2e_unet_op_desc(self._h, i).decode()) for i in range(n.value)]
+        return self._profile(x, None, torch.empty(self._out_shape(x.shape[0]), dtype=torch.float32, device=x.device))
 
 
 def resnet50_predictor(num_classes=80, input_size=256, max_batch=8, state_dict=None, seed=0, precision=None):

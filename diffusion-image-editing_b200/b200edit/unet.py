@@ -4,15 +4,14 @@ direct attributes - src/diffusion_utils.py:72, src/utils.py:68-70, src/ddpm_inve
 executed by libb200edit.so: bf16 tcgen05 implicit-GEMM convolutions, fp32 accumulation."""
 from __future__ import annotations
 
-import ctypes as C
-import math
 from types import SimpleNamespace
 from typing import Dict, Optional
 
 import torch
 
 from . import _C
-from ._C import UNetConfig, check, lib
+from ._C import UNetConfig, lib
+from .engine import Engine, _ptr, _stream
 
 DDPM256_CONFIG = dict(
     sample_size=256, in_channels=3, out_channels=3,
@@ -40,7 +39,7 @@ class UNetOutput(dict):
         return self["sample"]
 
 
-class UNet2DModel:
+class UNet2DModel(Engine):
     def __init__(self, sample_size=256, in_channels=3, out_channels=3,
                  block_out_channels=(128, 128, 256, 256, 512, 512), layers_per_block=2,
                  down_block_types=None, up_block_types=None, norm_num_groups=32, norm_eps=1e-6,
@@ -61,9 +60,6 @@ class UNet2DModel:
             norm_num_groups=norm_num_groups, norm_eps=norm_eps, attention_head_dim=attention_head_dim,
             flip_sin_to_cos=flip_sin_to_cos, freq_shift=freq_shift, downsample_padding=downsample_padding)
         self.in_channels, self.sample_size = in_channels, sample_size   # deprecated aliases
-        self.device = torch.device(device)
-        self.dtype = torch.float32
-        self.max_batch = int(max_batch)
         cfg = UNetConfig()
         cfg.sample_size, cfg.in_channels, cfg.out_channels, cfg.n_blocks = sample_size, in_channels, out_channels, n
         for i in range(n):
@@ -75,97 +71,19 @@ class UNet2DModel:
         cfg.flip_sin_to_cos, cfg.freq_shift = int(flip_sin_to_cos), float(freq_shift)
         cfg.downsample_padding = int(downsample_padding)
         cfg.precision = self._precision_cfg
-        h = C.c_void_p()
-        with torch.cuda.device(self.device):
-            check(lib.b2e_unet_create(C.byref(cfg), self.max_batch, C.byref(h)), "unet_create")
-            self._h = h
-            nbytes = lib.b2e_unet_workspace_bytes(h)
-            self._ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
-            base = (self._ws.data_ptr() + 255) // 256 * 256
-            check(lib.b2e_unet_bind_workspace(h, C.c_void_p(base), nbytes), "unet_bind_workspace")
+        self._create(lib.b2e_unet_create, cfg, max_batch, device)
         self._t_cache: Dict[tuple, torch.Tensor] = {}
 
-    def __del__(self):
-        h = getattr(self, "_h", None)
-        if h:
-            lib.b2e_unet_destroy(h)
-            self._h = None
-
-    # ------------------------------------------------------------------ parameters
-    def param_info(self):
-        out = []
-        name, numel, fan = C.c_char_p(), C.c_int64(), C.c_int64()
-        for i in range(lib.b2e_unet_num_params(self._h)):
-            check(lib.b2e_unet_param_info(self._h, i, C.byref(name), C.byref(numel), C.byref(fan)))
-            out.append((name.value.decode(), numel.value, fan.value))
-        return out
-
-    def load_state_dict(self, sd, strict=True):
-        """sd: mapping diffusers-name -> fp32 tensor (any device)."""
-        stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
-        names = {n for n, _, _ in self.param_info()}
-        missing = sorted(names - set(sd))
-        unexpected = sorted(set(sd) - names)
-        if strict and (missing or unexpected):
-            raise KeyError(f"load_state_dict: missing {missing[:5]}..., unexpected {unexpected[:5]}...")
-        with torch.cuda.device(self.device):
-            for k in names & set(sd):
-                t = sd[k].detach().to(self.device, torch.float32).contiguous()
-                check(lib.b2e_unet_set_param(self._h, k.encode(), C.c_void_p(t.data_ptr()), t.numel(), stream),
-                      f"set_param({k})")
-            torch.cuda.current_stream().synchronize()   # temporaries above must outlive the copies
-        return missing, unexpected
-
-    def init_random(self, seed=0):
-        """PyTorch-default-style init (U(-1/sqrt(fan_in), 1/sqrt(fan_in)); norm scale 1, shift 0)."""
-        self.load_state_dict(self.random_state_dict(seed))
-        return self
-
-    def random_state_dict(self, seed=0):
-        """The state dict ``init_random(seed)`` loads (so that a second engine can be given the same weights)."""
-        g = torch.Generator().manual_seed(seed)
-        sd = {}
-        for name, numel, fan in self.param_info():
-            if fan == 0:
-                sd[name] = torch.ones(numel) if name.endswith(".weight") else torch.zeros(numel)
-            elif fan < 0:   # codebook: U(-1/n, 1/n) with n = -fan (diffusers VectorQuantizer init)
-                sd[name] = (torch.rand(numel, generator=g) * 2 - 1) / float(-fan)
-            else:
-                bound = 1.0 / math.sqrt(fan)
-                sd[name] = (torch.rand(numel, generator=g) * 2 - 1) * bound
-        return sd
-
-    def to(self, *a, **k):
-        return self
-
-    def eval(self):
-        return self
-
-    @property
-    def flops_per_sample(self) -> float:
-        return float(lib.b2e_unet_flops(self._h, 1))
-
-    @property
-    def launches_per_forward(self) -> int:
-        return int(lib.b2e_unet_launches_per_forward(self._h))
+    def _out_shape(self, B):
+        cfg = self.config
+        return (B, cfg.out_channels, cfg.sample_size, cfg.sample_size)
 
     def profile(self, sample, timestep):
         """Per-op CUDA-event timings of one forward: list of dicts(kind, ms, flops, bytes)."""
         x = sample.to(torch.float32).contiguous()
         B = x.shape[0]
-        t = self._timesteps(timestep, B)
-        eps = torch.empty((B, self.config.out_channels, self.config.sample_size, self.config.sample_size),
-                          dtype=torch.float32, device=x.device)
-        cap = 1024
-        n = C.c_int()
-        ms, fl, by, kd = (C.c_float * cap)(), (C.c_double * cap)(), (C.c_double * cap)(), (C.c_int * cap)()
-        check(lib.b2e_unet_profile(self._h, C.c_void_p(x.data_ptr()), C.c_void_p(t.data_ptr()),
-                                   C.c_void_p(eps.data_ptr()), B,
-                                   C.c_void_p(torch.cuda.current_stream().cuda_stream), cap, C.byref(n), ms, fl, by, kd),
-              "unet_profile")
-        names = {0: "conv_igemm", 1: "groupnorm", 2: "attention", 3: "other"}
-        return [dict(kind=names[kd[i]], ms=ms[i], flops=fl[i], bytes=by[i],
-                     desc=lib.b2e_unet_op_desc(self._h, i).decode()) for i in range(n.value)]
+        eps = torch.empty(self._out_shape(B), dtype=torch.float32, device=x.device)
+        return self._profile(x, self._timesteps(timestep, B), eps)
 
     # ------------------------------------------------------------------ forward
     def _timesteps(self, timestep, B):
@@ -189,15 +107,12 @@ class UNet2DModel:
             raise ValueError(f"UNet2DModel: expected (B,{cfg.in_channels},{cfg.sample_size},{cfg.sample_size}), "
                              f"got {tuple(x.shape)}")
         t = self._timesteps(timestep, B)
-        eps = out if out is not None else torch.empty(
-            (B, cfg.out_channels, cfg.sample_size, cfg.sample_size), dtype=torch.float32, device=x.device)
+        eps = out if out is not None else torch.empty(self._out_shape(B), dtype=torch.float32, device=x.device)
         if self._graph_on and B == self.max_batch and not torch.cuda.is_current_stream_capturing():
             return UNetOutput(sample=self._replay(x, t, eps))
         if self._graph_on and self._graphs:
             self._graphs.clear()      # an eager forward at another batch re-plans the workspace: captured launches are stale
-        check(lib.b2e_unet_forward(self._h, C.c_void_p(x.data_ptr()), C.c_void_p(t.data_ptr()),
-                                   C.c_void_p(eps.data_ptr()), B,
-                                   C.c_void_p(torch.cuda.current_stream().cuda_stream)), "unet_forward")
+        self._launch(lib.b2e_unet_forward, _ptr(x), _ptr(t), _ptr(eps), B, _stream())
         return UNetOutput(sample=eps)
 
     # ------------------------------------------------------------------ CUDA-graph replay (launch-bound regime)
@@ -219,16 +134,12 @@ class UNet2DModel:
         if g is None:
             sx, st, se = torch.empty_like(x), torch.empty_like(t), torch.empty_like(eps)
             sx.copy_(x); st.copy_(t)
-            stream = C.c_void_p
             # warm-up outside capture (plan rebuild for this batch, lazy function attributes), then capture
-            check(lib.b2e_unet_forward(self._h, C.c_void_p(sx.data_ptr()), C.c_void_p(st.data_ptr()), C.c_void_p(se.data_ptr()), B,
-                                       stream(torch.cuda.current_stream().cuda_stream)), "unet_forward")
+            self._launch(lib.b2e_unet_forward, _ptr(sx), _ptr(st), _ptr(se), B, _stream())
             torch.cuda.synchronize()
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
-                check(lib.b2e_unet_forward(self._h, C.c_void_p(sx.data_ptr()), C.c_void_p(st.data_ptr()),
-                                           C.c_void_p(se.data_ptr()), B, stream(torch.cuda.current_stream().cuda_stream)),
-                      "unet_forward (capture)")
+                self._launch(lib.b2e_unet_forward, _ptr(sx), _ptr(st), _ptr(se), B, _stream())
             g = self._graphs[B] = (graph, sx, st, se)
         graph, sx, st, se = g
         sx.copy_(x)

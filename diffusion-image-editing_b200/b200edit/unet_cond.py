@@ -5,13 +5,13 @@ libb200edit.so.  ResNet blocks and down/up-sampling are the UNet2DModel ones; at
 LayerNorm + GEGLU feed-forward, 1x1 proj_out), all linear layers and attention products on the tcgen05 GEMM kernel."""
 from __future__ import annotations
 
-import ctypes as C
 from types import SimpleNamespace
 
 import torch
 
 from . import _C
-from ._C import UNetConfig, check, lib
+from ._C import UNetConfig, lib
+from .engine import _ptr, _stream
 from .unet import UNet2DModel, UNetOutput
 
 SD15_CONFIG = dict(sample_size=64, in_channels=4, out_channels=4, block_out_channels=(320, 640, 1280, 1280),
@@ -34,9 +34,6 @@ class UNet2DConditionModel(UNet2DModel):
             norm_num_groups=norm_num_groups, norm_eps=norm_eps, down_block_types=down_block_types,
             up_block_types=up_block_types)
         self.in_channels, self.sample_size = in_channels, sample_size
-        self.device = torch.device(device)
-        self.dtype = torch.float32
-        self.max_batch = int(max_batch)
         cfg = UNetConfig()
         cfg.sample_size, cfg.in_channels, cfg.out_channels, cfg.n_blocks = sample_size, in_channels, out_channels, n
         for i in range(n):
@@ -48,14 +45,7 @@ class UNet2DConditionModel(UNet2DModel):
         cfg.flip_sin_to_cos, cfg.freq_shift, cfg.downsample_padding = 1, 0.0, 1
         cfg.cross_attention_dim, cfg.num_attention_heads = cross_attention_dim, attention_head_dim   # SD 1.x: 8 heads
         cfg.precision = self._precision_cfg   # 1: fp32-accurate mode (split-f16 operands, fp32 attention)
-        h = C.c_void_p()
-        with torch.cuda.device(self.device):
-            check(lib.b2e_unet_create(C.byref(cfg), self.max_batch, C.byref(h)), "unet_create")
-            self._h = h
-            nbytes = lib.b2e_unet_workspace_bytes(h)
-            self._ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
-            base = (self._ws.data_ptr() + 255) // 256 * 256
-            check(lib.b2e_unet_bind_workspace(h, C.c_void_p(base), nbytes), "unet_bind_workspace")
+        self._create(lib.b2e_unet_create, cfg, max_batch, device)
         self._t_cache = {}
 
     def __call__(self, sample, timestep, encoder_hidden_states=None, out=None, **_):
@@ -82,7 +72,5 @@ class UNet2DConditionModel(UNet2DModel):
         t = self._timesteps(timestep, B)
         eps = out if out is not None else torch.empty_like(x[:, :cfg.out_channels]) if cfg.out_channels == cfg.in_channels \
             else torch.empty((B, cfg.out_channels, cfg.sample_size, cfg.sample_size), dtype=torch.float32, device=x.device)
-        check(lib.b2e_unet_forward_cond(self._h, C.c_void_p(x.data_ptr()), C.c_void_p(t.data_ptr()), C.c_void_p(ctx.data_ptr()),
-                                        ctx.shape[1], C.c_void_p(eps.data_ptr()), B,
-                                        C.c_void_p(torch.cuda.current_stream().cuda_stream)), "unet_forward_cond")
+        self._launch(lib.b2e_unet_forward_cond, _ptr(x), _ptr(t), _ptr(ctx), ctx.shape[1], _ptr(eps), B, _stream())
         return UNetOutput(sample=eps)

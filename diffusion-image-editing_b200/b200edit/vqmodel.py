@@ -8,46 +8,19 @@ decoder (AttrFunc.apply with no_grad=False) uses.  ``with_encoder=True`` adds th
 (``vqvae.encode(img).latents`` / ``vae.encode(img).latent_dist.mode()``, src/diffusion_classes.py:27-30, 55-60)."""
 from __future__ import annotations
 
-import ctypes as C
 from types import SimpleNamespace
 
 import torch
 
 from . import _C
-from ._C import VQDecConfig, VQEncConfig, check, lib
-from .unet import UNet2DModel
+from ._C import VQDecConfig, VQEncConfig, lib
+from .engine import Engine
 
 LDM_VQ_CONFIG = dict(latent_channels=3, out_channels=3, block_out_channels=(128, 256, 512), layers_per_block=2,
                      norm_num_groups=32, norm_eps=1e-6, num_vq_embeddings=8192, sample_size=64)
 
 
-class _DecodeFn(torch.autograd.Function):
-    """decode as an autograd node: forward = native decoder (activations stay in the engine's workspace), backward =
-    native dgrad of the whole decoder (straight-through quantiser)."""
-
-    @staticmethod
-    def forward(ctx, latent, model):
-        ctx.model = model
-        ctx.B = latent.shape[0]
-        out = model._forward(latent)
-        ctx.gen = model._fwd_gen      # the activations of THIS forward live in the engine's single workspace
-        return out
-
-    @staticmethod
-    def backward(ctx, grad_img):
-        m = ctx.model
-        if m._fwd_gen != ctx.gen:
-            raise _C.B2EError("VQModel.decode backward: the engine ran another forward since this graph was built (its "
-                              "activations were overwritten); differentiate before the next decode() on the same model")
-        g = grad_img.to(torch.float32).contiguous()
-        dz = torch.empty((ctx.B, m.config.latent_channels, m.config.sample_size, m.config.sample_size),
-                         dtype=torch.float32, device=g.device)
-        check(lib.b2e_vqdec_backward(m._h, C.c_void_p(g.data_ptr()), C.c_void_p(dz.data_ptr()), ctx.B,
-                                     C.c_void_p(torch.cuda.current_stream().cuda_stream)), "vqdec_backward")
-        return dz, None
-
-
-class _EncoderEngine(UNet2DModel):
+class _EncoderEngine(Engine):
     """diffusers ``Encoder`` + ``quant_conv`` on the engine (b2e_vqenc_create): image (B, C, S, S) -> (B, Q, s, s)."""
 
     def __init__(self, image_size, in_channels, latent_channels, block_out_channels, layers_per_block, norm_num_groups,
@@ -56,24 +29,16 @@ class _EncoderEngine(UNet2DModel):
         self.image_size, self.q = image_size, latent_channels * (2 if double_z else 1)
         self.out_size = image_size >> (n - 1)
         self.config = SimpleNamespace(in_channels=in_channels, sample_size=image_size, out_channels=self.q)
-        self.device = torch.device(device)
-        self.dtype = torch.float32
-        self.max_batch = int(max_batch)
         cfg = VQEncConfig()
         cfg.sample_size, cfg.in_channels, cfg.latent_channels, cfg.n_blocks = image_size, in_channels, latent_channels, n
         for i in range(n):
             cfg.block_out_channels[i] = block_out_channels[i]
         cfg.layers_per_block, cfg.norm_num_groups, cfg.norm_eps = layers_per_block, norm_num_groups, norm_eps
         cfg.double_z = int(double_z)
-        h = C.c_void_p()
-        with torch.cuda.device(self.device):
-            check(lib.b2e_vqenc_create(C.byref(cfg), self.max_batch, C.byref(h)), "vqenc_create")
-            self._h = h
-            nbytes = lib.b2e_unet_workspace_bytes(h)
-            self._ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
-            base = (self._ws.data_ptr() + 255) // 256 * 256
-            check(lib.b2e_unet_bind_workspace(h, C.c_void_p(base), nbytes), "unet_bind_workspace")
-        self._t_cache = {}
+        self._create(lib.b2e_vqenc_create, cfg, max_batch, device)
+
+    def _out_shape(self, B):
+        return (B, self.q, self.out_size, self.out_size)
 
     def __call__(self, image):
         if not image.is_cuda:
@@ -82,14 +47,7 @@ class _EncoderEngine(UNet2DModel):
         if tuple(x.shape[1:]) != (self.config.in_channels, self.image_size, self.image_size):
             raise ValueError(f"encode: expected (B,{self.config.in_channels},{self.image_size},{self.image_size}), "
                              f"got {tuple(x.shape)}")
-        outs = []
-        for b0 in range(0, x.shape[0], self.max_batch):
-            xb = x[b0:b0 + self.max_batch]
-            o = torch.empty((xb.shape[0], self.q, self.out_size, self.out_size), dtype=torch.float32, device=x.device)
-            check(lib.b2e_unet_forward(self._h, C.c_void_p(xb.data_ptr()), None, C.c_void_p(o.data_ptr()), xb.shape[0],
-                                       C.c_void_p(torch.cuda.current_stream().cuda_stream)), "vqenc_forward")
-            outs.append(o)
-        return outs[0] if len(outs) == 1 else torch.cat(outs)
+        return self._forward_sliced(x)
 
 
 class DiagonalGaussianDistribution:
@@ -113,8 +71,7 @@ def _is_encoder_key(k: str) -> bool:
     return k.startswith("encoder.") or k.startswith("quant_conv.")
 
 
-class VQModel(UNet2DModel):
-    """Shares parameter loading / random init / profiling with the UNet wrapper (same engine handle type)."""
+class VQModel(Engine):
 
     forward_only = True   # until enable_grad(): no autograd graph through decode (see LDM.decode)
 
@@ -131,9 +88,6 @@ class VQModel(UNet2DModel):
                                       num_vq_embeddings=num_vq_embeddings, sample_size=sample_size,
                                       in_channels=latent_channels)
         self.out_size = sample_size << (n - 1)
-        self.device = torch.device(device)
-        self.dtype = torch.float32
-        self.max_batch = int(max_batch)
         cfg = VQDecConfig()
         cfg.sample_size, cfg.latent_channels, cfg.out_channels, cfg.n_blocks = sample_size, latent_channels, out_channels, n
         for i in range(n):
@@ -141,15 +95,7 @@ class VQModel(UNet2DModel):
         cfg.layers_per_block, cfg.norm_num_groups, cfg.norm_eps = layers_per_block, norm_num_groups, norm_eps
         cfg.num_vq_embeddings = num_vq_embeddings
         cfg.precision = self._precision_cfg      # 1: fp32-accurate decode (split-f16 operands), forward only
-        h = C.c_void_p()
-        with torch.cuda.device(self.device):
-            check(lib.b2e_vqdec_create(C.byref(cfg), self.max_batch, C.byref(h)), "vqdec_create")
-            self._h = h
-            nbytes = lib.b2e_unet_workspace_bytes(h)
-            self._ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
-            base = (self._ws.data_ptr() + 255) // 256 * 256
-            check(lib.b2e_unet_bind_workspace(h, C.c_void_p(base), nbytes), "unet_bind_workspace")
-        self._t_cache = {}
+        self._create(lib.b2e_vqdec_create, cfg, max_batch, device)
         if with_encoder:
             self._enc = _EncoderEngine(self.out_size, out_channels, latent_channels, block_out_channels, layers_per_block,
                                        norm_num_groups, norm_eps, num_vq_embeddings == 0, max_batch, device)
@@ -173,79 +119,47 @@ class VQModel(UNet2DModel):
     def enable_grad(self, enable: bool = True):
         """Gradient mode: decode() becomes differentiable w.r.t. the latent (native dgrad; batches <= max_batch).
         Costs workspace: every activation of a forward pass is kept until the backward pass."""
-        with torch.cuda.device(self.device):
-            check(lib.b2e_unet_enable_grad(self._h, int(enable)), "unet_enable_grad")
-            nbytes = lib.b2e_unet_workspace_bytes(self._h)
-            self._ws = None
-            self._ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
-            base = (self._ws.data_ptr() + 255) // 256 * 256
-            check(lib.b2e_unet_bind_workspace(self._h, C.c_void_p(base), nbytes), "unet_bind_workspace")
+        self._enable_grad(enable)
         self.forward_only = not enable
         return self
 
-    _fwd_gen = 0   # bumped by every forward: a backward over a stale workspace is detected (see _DecodeFn)
+    _backward_fn = lib.b2e_vqdec_backward
 
-    def _forward(self, z):
-        cfg = self.config
-        self._fwd_gen += 1
-        img = torch.empty((z.shape[0], cfg.out_channels, self.out_size, self.out_size), dtype=torch.float32, device=z.device)
-        check(lib.b2e_unet_forward(self._h, C.c_void_p(z.data_ptr()), None, C.c_void_p(img.data_ptr()), z.shape[0],
-                                   C.c_void_p(torch.cuda.current_stream().cuda_stream)), "vqdec_forward")
-        return img
+    def _out_shape(self, B):
+        return (B, self.config.out_channels, self.out_size, self.out_size)
 
     # ---- decode + latent gradient WITHOUT an autograd graph (analytic guidance: the caller supplies d(loss)/d(image))
-    def decode_keep(self, latent: torch.Tensor) -> torch.Tensor:
-        """decode(latent).sample with the activations kept in the engine's workspace for ``latent_grad``."""
-        if self.forward_only:
-            raise _C.B2EError(f"{type(self).__name__}.decode_keep: call enable_grad() first")
+    def _check_latent(self, latent, keep):
         cfg = self.config
         if latent.dim() != 4 or tuple(latent.shape[1:]) != (cfg.latent_channels, cfg.sample_size, cfg.sample_size):
             raise ValueError(f"VQModel.decode: expected (B,{cfg.latent_channels},{cfg.sample_size},{cfg.sample_size}), "
                              f"got {tuple(latent.shape)}")
-        if latent.shape[0] > self.max_batch:
+        if keep and latent.shape[0] > self.max_batch:
             raise ValueError(f"VQModel.decode with gradient: batch {latent.shape[0]} > max_batch {self.max_batch}")
-        z = latent.detach().to(torch.float32).contiguous()
-        img = self._forward(z)
-        self._keep_gen, self._keep_B = self._fwd_gen, z.shape[0]
-        return img
+
+    def decode_keep(self, latent: torch.Tensor) -> torch.Tensor:
+        """decode(latent).sample with the activations kept in the engine's workspace for ``latent_grad``."""
+        if self.forward_only:
+            raise _C.B2EError(f"{type(self).__name__}.decode_keep: call enable_grad() first")
+        self._check_latent(latent, keep=True)
+        return self._keep(latent.detach().to(torch.float32).contiguous())
 
     def latent_grad(self, d_image: torch.Tensor) -> torch.Tensor:
         """d(loss)/d(latent) for the last ``decode_keep`` given d(loss)/d(image) (native dgrad of the whole decoder)."""
-        if getattr(self, "_keep_gen", None) != self._fwd_gen:
-            raise _C.B2EError("VQModel.latent_grad: the engine ran another forward since decode_keep (activations overwritten)")
-        g = d_image.detach().to(torch.float32).contiguous()
-        cfg = self.config
-        dz = torch.empty((self._keep_B, cfg.latent_channels, cfg.sample_size, cfg.sample_size), dtype=torch.float32, device=g.device)
-        check(lib.b2e_vqdec_backward(self._h, C.c_void_p(g.data_ptr()), C.c_void_p(dz.data_ptr()), self._keep_B,
-                                     C.c_void_p(torch.cuda.current_stream().cuda_stream)), "vqdec_backward")
-        return dz
+        return self._keep_grad(d_image)
 
     def decode(self, latent: torch.Tensor, force_not_quantize: bool = False):
         if force_not_quantize:
             raise NotImplementedError("VQModel.decode(force_not_quantize=True) is not on the native engine")
         if not latent.is_cuda:
             raise _C.B2EError("VQModel.decode: latent must be a CUDA tensor (no CPU fallback)")
-        cfg = self.config
-        if latent.dim() != 4 or tuple(latent.shape[1:]) != (cfg.latent_channels, cfg.sample_size, cfg.sample_size):
-            raise ValueError(f"VQModel.decode: expected (B,{cfg.latent_channels},{cfg.sample_size},{cfg.sample_size}), "
-                             f"got {tuple(latent.shape)}")
-        if not self.forward_only and latent.requires_grad and torch.is_grad_enabled():
-            if latent.shape[0] > self.max_batch:
-                raise ValueError(f"VQModel.decode with gradient: batch {latent.shape[0]} > max_batch {self.max_batch}")
+        grad = not self.forward_only and latent.requires_grad and torch.is_grad_enabled()
+        self._check_latent(latent, keep=grad)
+        if grad:
             zz = latent if (latent.dtype == torch.float32 and latent.is_contiguous()) else latent.to(torch.float32).contiguous()
-            return SimpleNamespace(sample=_DecodeFn.apply(zz, self))
-        z = latent.detach().to(torch.float32).contiguous()
-        B = z.shape[0]
-        outs = []
-        for b0 in range(0, B, self.max_batch):      # histories can be longer than max_batch
-            self._fwd_gen += 1
-            zb = z[b0:b0 + self.max_batch]
-            img = torch.empty((zb.shape[0], cfg.out_channels, self.out_size, self.out_size), dtype=torch.float32,
-                              device=z.device)
-            check(lib.b2e_unet_forward(self._h, C.c_void_p(zb.data_ptr()), None, C.c_void_p(img.data_ptr()), zb.shape[0],
-                                       C.c_void_p(torch.cuda.current_stream().cuda_stream)), "vqdec_forward")
-            outs.append(img)
-        return SimpleNamespace(sample=outs[0] if len(outs) == 1 else torch.cat(outs))
+            return SimpleNamespace(sample=self._keep_node(zz))
+        # histories can be longer than max_batch
+        return SimpleNamespace(sample=self._forward_sliced(latent.detach().to(torch.float32).contiguous()))
 
     def _encode_raw(self, x):
         if self._enc is None:
@@ -261,17 +175,7 @@ class VQModel(UNet2DModel):
 
     def profile(self, latent):
         z = latent.to(torch.float32).contiguous()
-        B = z.shape[0]
-        img = torch.empty((B, self.config.out_channels, self.out_size, self.out_size), dtype=torch.float32, device=z.device)
-        cap = 1024
-        n = C.c_int()
-        ms, fl, by, kd = (C.c_float * cap)(), (C.c_double * cap)(), (C.c_double * cap)(), (C.c_int * cap)()
-        check(lib.b2e_unet_profile(self._h, C.c_void_p(z.data_ptr()), None, C.c_void_p(img.data_ptr()), B,
-                                   C.c_void_p(torch.cuda.current_stream().cuda_stream), cap, C.byref(n), ms, fl, by, kd),
-              "vqdec_profile")
-        names = {0: "conv_igemm", 1: "groupnorm", 2: "attention", 3: "other"}
-        return [dict(kind=names[kd[i]], ms=ms[i], flops=fl[i], bytes=by[i],
-                     desc=lib.b2e_unet_op_desc(self._h, i).decode()) for i in range(n.value)]
+        return self._profile(z, None, torch.empty(self._out_shape(z.shape[0]), dtype=torch.float32, device=z.device))
 
 
 # CompVis/stable-diffusion-v1-x `vae` decode path: 64x64x4 latent -> 512x512x3 image (x8), no quantiser

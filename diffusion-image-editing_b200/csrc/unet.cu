@@ -2246,6 +2246,26 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
   return B2E_OK;
 }
 
+// the common tail of every b2e_*_create: upload the weights, plan for max_batch (workspace size only), hand out the handle
+int finish_create(b2e_unet* m, b2e_unet** out, const char* who) {
+  int rc = build_model(m);
+  if (!rc && cudaDeviceSynchronize() != cudaSuccess) { set_error("%s: device error", who); rc = B2E_CUDA_ERROR; }
+  if (!rc) rc = build_program(m, (int)m->max_batch, nullptr, 0, &m->ws_need);
+  if (rc) { delete m; return rc; }
+  *out = m;
+  return B2E_OK;
+}
+
+// the input-gradient op list of a classifier / face parser / LPIPS handle, over the live forward's activations
+int run_backward(b2e_unet* m, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  for (auto& op : m->bops) {
+    int rc = op.fn(st);
+    if (rc) return rc;
+  }
+  return B2E_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -2285,12 +2305,7 @@ int b2e_unet_create(const b2e_unet_config* cfg, int64_t max_batch, b2e_unet** ou
   m->cfg = *cfg;
   m->PL = cfg->precision == 1 ? 3 : 1;
   m->max_batch = max_batch;
-  int rc = build_model(m);
-  if (!rc && cudaDeviceSynchronize() != cudaSuccess) { set_error("unet_create: device error"); rc = B2E_CUDA_ERROR; }
-  if (!rc) rc = build_program(m, (int)max_batch, nullptr, 0, &m->ws_need);
-  if (rc) { delete m; return rc; }
-  *out = m;
-  return B2E_OK;
+  return finish_create(m, out, "unet_create");
 }
 
 int b2e_vqdec_create(const b2e_vqdec_config* cfg, int64_t max_batch, b2e_unet** out) {
@@ -2317,12 +2332,7 @@ int b2e_vqdec_create(const b2e_vqdec_config* cfg, int64_t max_batch, b2e_unet** 
   u.layers_per_block = cfg->layers_per_block; u.norm_num_groups = cfg->norm_num_groups; u.norm_eps = cfg->norm_eps;
   u.attention_head_dim = 0;
   m->max_batch = max_batch;
-  int rc = build_model(m);
-  if (!rc && cudaDeviceSynchronize() != cudaSuccess) { set_error("vqdec_create: device error"); rc = B2E_CUDA_ERROR; }
-  if (!rc) rc = build_program(m, (int)max_batch, nullptr, 0, &m->ws_need);
-  if (rc) { delete m; return rc; }
-  *out = m;
-  return B2E_OK;
+  return finish_create(m, out, "vqdec_create");
 }
 
 int b2e_vqenc_create(const b2e_vqenc_config* cfg, int64_t max_batch, b2e_unet** out) {
@@ -2348,12 +2358,7 @@ int b2e_vqenc_create(const b2e_vqenc_config* cfg, int64_t max_batch, b2e_unet** 
   u.layers_per_block = cfg->layers_per_block; u.norm_num_groups = cfg->norm_num_groups; u.norm_eps = cfg->norm_eps;
   u.attention_head_dim = 0; u.downsample_padding = 0;
   m->max_batch = max_batch;
-  int rc = build_model(m);
-  if (!rc && cudaDeviceSynchronize() != cudaSuccess) { set_error("vqenc_create: device error"); rc = B2E_CUDA_ERROR; }
-  if (!rc) rc = build_program(m, (int)max_batch, nullptr, 0, &m->ws_need);
-  if (rc) { delete m; return rc; }
-  *out = m;
-  return B2E_OK;
+  return finish_create(m, out, "vqenc_create");
 }
 
 int b2e_clip_create(const b2e_clip_config* cfg, int64_t max_batch, b2e_unet** out) {
@@ -2370,12 +2375,7 @@ int b2e_clip_create(const b2e_clip_config* cfg, int64_t max_batch, b2e_unet** ou
   m->cfg = b2e_unet_config{};
   m->cfg.sample_size = 8; m->cfg.in_channels = 1; m->cfg.out_channels = 1; m->cfg.norm_num_groups = 1;
   m->max_batch = max_batch;
-  int rc = build_model(m);
-  if (!rc && cudaDeviceSynchronize() != cudaSuccess) { set_error("clip_create: device error"); rc = B2E_CUDA_ERROR; }
-  if (!rc) rc = build_program(m, (int)max_batch, nullptr, 0, &m->ws_need);
-  if (rc) { delete m; return rc; }
-  *out = m;
-  return B2E_OK;
+  return finish_create(m, out, "clip_create");
 }
 
 int b2e_clip_forward(b2e_unet* m, const int64_t* input_ids, int64_t seq_len, float* hidden, int64_t B, void* stream) {
@@ -2406,12 +2406,7 @@ int b2e_resnet_create(const b2e_resnet_config* cfg, int64_t max_batch, b2e_unet*
   m->cfg = b2e_unet_config{};
   m->cfg.sample_size = cfg->input_size; m->cfg.in_channels = cfg->in_channels; m->cfg.out_channels = cfg->num_classes;
   m->max_batch = max_batch;
-  int rc = build_model(m);
-  if (!rc && cudaDeviceSynchronize() != cudaSuccess) { set_error("resnet_create: device error"); rc = B2E_CUDA_ERROR; }
-  if (!rc) rc = build_program(m, (int)max_batch, nullptr, 0, &m->ws_need);
-  if (rc) { delete m; return rc; }
-  *out = m;
-  return B2E_OK;
+  return finish_create(m, out, "resnet_create");
 }
 
 int b2e_resnet_backward(b2e_unet* m, const float* d_logits, float* d_image, int64_t B, void* stream) {
@@ -2421,12 +2416,7 @@ int b2e_resnet_backward(b2e_unet* m, const float* d_logits, float* d_image, int6
   B2E_REQUIRE(m->fwd_B == B && m->cur_B == B, B2E_INVALID_ARG,
               "resnet_backward: no live forward pass of batch %lld (last forward: %lld)", (long long)B, (long long)m->fwd_B);
   m->in_dlogits = d_logits; m->out_dz = d_image;
-  cudaStream_t st = (cudaStream_t)stream;
-  for (auto& op : m->bops) {
-    int rc = op.fn(st);
-    if (rc) return rc;
-  }
-  return B2E_OK;
+  return run_backward(m, stream);
 }
 
 static int unet_forward_impl(b2e_unet* m, const float* x, const int64_t* timesteps, float* eps, int64_t B, void* stream);
@@ -2444,12 +2434,7 @@ int b2e_lpips_create(const b2e_lpips_config* cfg, int64_t max_batch, b2e_unet** 
   m->cfg = b2e_unet_config{};
   m->cfg.sample_size = cfg->input_size; m->cfg.in_channels = 3; m->cfg.out_channels = 1;
   m->max_batch = max_batch;
-  int rc = build_model(m);
-  if (!rc && cudaDeviceSynchronize() != cudaSuccess) { set_error("lpips_create: device error"); rc = B2E_CUDA_ERROR; }
-  if (!rc) rc = build_program(m, (int)max_batch, nullptr, 0, &m->ws_need);
-  if (rc) { delete m; return rc; }
-  *out = m;
-  return B2E_OK;
+  return finish_create(m, out, "lpips_create");
 }
 
 int b2e_lpips_set_reference(b2e_unet* m, const float* x_ref, int64_t B_ref, void* stream) {
@@ -2491,12 +2476,7 @@ int b2e_lpips_backward(b2e_unet* m, const float* d_dist, float* d_x, int64_t B, 
   B2E_REQUIRE(m->fwd_B == B && m->cur_B == B, B2E_INVALID_ARG,
               "lpips_backward: no live forward pass of batch %lld (last forward: %lld)", (long long)B, (long long)m->fwd_B);
   m->in_dlogits = d_dist; m->out_dz = d_x;
-  cudaStream_t st = (cudaStream_t)stream;
-  for (auto& op : m->bops) {
-    int rc = op.fn(st);
-    if (rc) return rc;
-  }
-  return B2E_OK;
+  return run_backward(m, stream);
 }
 
 void b2e_unet_destroy(b2e_unet* m) { delete m; }
