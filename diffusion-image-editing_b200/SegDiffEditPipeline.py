@@ -16,7 +16,7 @@ from b200edit import ops
 from b200edit.outputs import BaseOutput
 from constants import ATTRS
 from ddim_inversion import ddim_inversion
-from ddpm_inversion import invert, reverse_step  # noqa: F401  (reverse_step re-exported like the reference)
+from ddpm_inversion import check_batch, invert, reverse_step  # noqa: F401  (reverse_step re-exported like the reference)
 from diffusion_classes import DDPM, LDM, SD
 from diffusion_utils import diffusion_loop, get_noise_pred, get_variance_noise
 from mask_creator import MaskCreator
@@ -54,12 +54,25 @@ class SegDiffEditPipeline:
         if attr_func is None and (mask is None or resynthesize is None):
             raise ValueError("attr_func is None and classes and mask is None implies no edit")
 
+    def check_batch_shapes(self, xt, zs, xts, mask):
+        """Batched edits (extension): 5-D xts (T+1,B,C,H,W) go with 5-D zs (T,B,C,H,W); a mask's batch is 1 or B."""
+        if xts is not None and xts.dim() == 5:
+            if zs is None or zs.dim() != 5 or tuple(zs.shape[1:]) != tuple(xts.shape[1:]):
+                raise ValueError(f"xts of shape {tuple(xts.shape)} (T+1, B, C, H, W) needs zs of shape (T, B, C, H, W), got "
+                                 f"{None if zs is None else tuple(zs.shape)}")
+            B = xts.shape[1]
+        else:
+            B = xt.shape[0] if xt is not None and xt.dim() == 4 else 1
+        if mask is not None and mask.dim() == 4 and mask.shape[0] not in (1, B):
+            raise ValueError(f"the mask batch must be 1 or the image batch {B}, got a mask of shape {tuple(mask.shape)}")
+
     # ------------------------------------------------------------------ preparation
     def create_mask(self, classes, dilate_mask, segmentation, dim):
         return MaskCreator(dilate_mask=dilate_mask, resize_size=(dim, dim)).create_mask(segmentation, classes=classes)
 
     def prepare_for_edit(self, img: torch.Tensor, classes: Optional[List[int]] = None, dilate_mask: bool = False):
-        """Returns (latent, mask, segmentation).  Call before edit_image."""
+        """Returns (latent, mask, segmentation).  Call before edit_image.  A batch of B > 1 images gives (B, ...) latents,
+        (B, S, S) parsing maps and (B, C, d, d) masks."""
         self.check_classes(classes)
         segmentation = mask = None
         if classes is not None:
@@ -70,8 +83,10 @@ class SegDiffEditPipeline:
         return self.diffusion_wrapper.encode(img), mask, segmentation
 
     def edit_noise_map(self, noise_map: torch.Tensor, mask: torch.Tensor):
-        fresh = generate_random_samples(noise_map.shape[0], self.diffusion_wrapper.model.unet).to(noise_map.device)
-        return apply_mask(mask, noise_map, fresh)
+        """Fresh noise of the map's own shape ((B,C,H,W) or (T',B,C,H,W)) inside the mask."""
+        n = noise_map.shape[:-3].numel()
+        fresh = generate_random_samples(n, self.diffusion_wrapper.model.unet).to(noise_map.device)
+        return apply_mask(mask, noise_map, fresh.reshape(noise_map.shape))
 
     def edit_noise_maps(self, xt, zs, mask, resynthesize):
         if mask is not None and resynthesize:
@@ -94,11 +109,14 @@ class SegDiffEditPipeline:
                                 classes: Optional[List[int]] = None, dilate_mask: bool = False,
                                 prompt: Optional[str] = None, cfg_scale: Optional[float] = None,
                                 prog_bar: bool = True):
-        """Invert a real image: returns (xt, zs, xts, mask, segmentation)."""
+        """Invert a real image: returns (xt, zs, xts, mask, segmentation).  A batch of B > 1 images is inverted in one
+        pass (``ddpm_inversion.invert``): xt (B, ...), zs (T, B, ...), xts (T+1, B, ...)."""
         if inversion_method == "ddim" and eta > 0:
             raise ValueError("eta > 0 and inversion_method == 'ddim' is not possible")
-        latent, mask, segmentation = self.prepare_for_edit(img, classes, dilate_mask)
         w = self.diffusion_wrapper
+        if inversion_method == "ddpm" and img.dim() == 4:
+            check_batch(w.model, img.shape[0], prompt is not None)     # before any network runs
+        latent, mask, segmentation = self.prepare_for_edit(img, classes, dilate_mask)
         if type(w) in (DDPM, LDM):
             assert w.model.scheduler.config.clip_sample is False
         if inversion_method == "ddim":
@@ -111,7 +129,7 @@ class SegDiffEditPipeline:
             raise ValueError(f"Unknown inversion method: {inversion_method}")
         if type(w) == SD and mask is not None:
             # one extra all-ones channel for the 4th latent channel (the reference hard-codes 32x32)
-            ones = torch.ones((1, 1) + tuple(mask.shape[-2:]), device=xt.device)
+            ones = torch.ones((mask.shape[0], 1) + tuple(mask.shape[-2:]), device=xt.device)
             mask = torch.cat((mask, ones), dim=1)
         return xt, zs, xts, mask, segmentation
 
@@ -132,13 +150,14 @@ class SegDiffEditPipeline:
         blocks the host until the last of those copies has landed (the final decode has to be consumed anyway), so the
         slices are safe to read as soon as it returns."""
         self.check_inputs(attr_func=attr_func, eta=eta, mask=mask, resynthesize=resynthesize, zs=zs)
+        self.check_batch_shapes(xt, zs, xts, mask)
         xt, zs = self.edit_noise_maps(xt, zs, mask, resynthesize)
         text_emb = self.prepare_text_emb(prompt)
         w = self.diffusion_wrapper
         sch = w.model.scheduler
         eps_hist, x0_hist = [], []
         if xts is not None:
-            xt = xts[Tskip].unsqueeze(0)
+            xt = xts[Tskip] if xts.dim() == 5 else xts[Tskip].unsqueeze(0)
             zs = zs[Tskip:]
         mode = "ddpm" if (inversion_method == "ddpm" and Tskip is not None) else "ddim"
         clip = bool(sch.config.clip_sample) if mode == "ddim" else False

@@ -109,6 +109,9 @@ PROTOTYPES = {
     "b2e_mask_workspace_bytes": (_SZ, [_I64, _I64, _I64, _I64]),
     "b2e_mask_from_seg": (_I, [_P, _I64, _I64, C.POINTER(C.c_int32), _I, _I, _I, _I64, _I64, _I, _I,
                                _P, _P, _SZ, _P]),
+    "b2e_mask_batched_workspace_bytes": (_SZ, [_I64, _I64, _I64, _I64, _I64]),
+    "b2e_mask_from_seg_batched": (_I, [_P, _I64, _I64, _I64, C.POINTER(C.c_int32), _I, _I, _I, _I64, _I64, _I, _I,
+                                       _P, _P, _SZ, _P]),
     "b2e_resize_bilinear_aa_f32": (_I, [_P, _I64, _I64, _P, _I64, _I64, _P, _SZ, _P]),
     "b2e_morphology2d_f32": (_I, [_P, _P, _P, _I64, _I64, _I64, _I64, _I64, _I, _I, _I, _F, _P]),
     "b2e_unet_create": (_I, [C.POINTER(UNetConfig), _I64, C.POINTER(_P)]),
@@ -118,6 +121,7 @@ PROTOTYPES = {
     "b2e_clip_forward": (_I, [_P, _P, _I64, _P, _I64, _P]),
     "b2e_resnet_create": (_I, [C.POINTER(ResNetConfig), _I64, C.POINTER(_P)]),
     "b2e_resnet_backward": (_I, [_P, _P, _P, _I64, _P]),
+    "b2e_resnet_forward_labels": (_I, [_P, _P, _P, _I64, _P]),
     "b2e_lpips_create": (_I, [C.POINTER(LpipsConfig), _I64, C.POINTER(_P)]),
     "b2e_lpips_set_reference": (_I, [_P, _P, _I64, _P]),
     "b2e_lpips_forward": (_I, [_P, _P, _P, _I64, _P, _I64, _P]),
@@ -140,6 +144,7 @@ PROTOTYPES = {
     "b2e_act_dtype": (_I, []),
     "b2e_conv2d_nhwc_f16": (_I, [_P, _P, _P, _P, _P, _I64, _I64, _I64, _I64, _I64, _I, _I, _P]),
     "b2e_conv2d_bench_f16": (_I, [_I64, _I64, _I64, _I64, _I64, _I, _I, _I, _I, _P, _P]),
+    "b2e_bilinear_ac_argmax_f16": (_I, [_P, _P, _I64, _I64, _I64, _I64, _I64, _I64, _I, _P]),
     "b2e_upsample_conv3x3_nhwc_f16": (_I, [_P, _P, _P, _P, _I64, _I64, _I64, _I64, _I64, _P]),
 }
 

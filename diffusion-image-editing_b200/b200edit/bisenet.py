@@ -15,7 +15,7 @@ import torch
 
 from . import _C
 from ._C import ResNetConfig, lib
-from .engine import Engine
+from .engine import Engine, _ptr, _stream
 
 
 def _fold(w, sd, bn, eps=1e-5):
@@ -120,6 +120,19 @@ class BiSeNet(Engine):
             return (self._keep_node(xx), None, None)
         return (self._forward_sliced(image.detach().to(torch.float32).contiguous()), None, None)
 
+    def labels(self, image):
+        """Parsing map (B, S, S) int64 = ``net(image)[0].argmax(1)``, bit for bit: the last kernel upsamples the logits
+        and takes their argmax per pixel, so no (B, n_classes, S, S) logits are written.  Batches above max_batch run
+        in slices.  The call overwrites the activations, so a gradient of an earlier kept forward is refused after it."""
+        self._check_input(image)
+        x = image.detach().to(torch.float32).contiguous()
+        S = self.config.input_size
+        out = torch.empty((x.shape[0], S, S), dtype=torch.int64, device=x.device)
+        for b0 in range(0, x.shape[0], self.max_batch):
+            xs, ls = x[b0:b0 + self.max_batch], out[b0:b0 + self.max_batch]
+            self._launch(lib.b2e_resnet_forward_labels, _ptr(xs), _ptr(ls), xs.shape[0], _stream())
+        return out
+
     def profile(self, image, timestep=None):
         """Per-op CUDA-event timings of one forward (``timestep`` is ignored: the face parser has none)."""
         x = image.detach().to(torch.float32).contiguous()
@@ -168,10 +181,19 @@ class MultiResBiSeNet:
             self._engines[(size, grad)] = e
         return e
 
-    def __call__(self, image):
+    @staticmethod
+    def _check_shape(image):
         if image.dim() != 4 or image.shape[1] != 3 or image.shape[-1] != image.shape[-2]:
             raise ValueError(f"BiSeNet: expected (B,3,S,S), got {tuple(image.shape)}")
+
+    def __call__(self, image):
+        self._check_shape(image)
         return self.engine(int(image.shape[-1]), grad=image.requires_grad and torch.is_grad_enabled())(image)
+
+    def labels(self, image):
+        """Parsing map (B, S, S) int64 on the forward-only engine of the input's resolution (``BiSeNet.labels``)."""
+        self._check_shape(image)
+        return self.engine(int(image.shape[-1])).labels(image)
 
     def eval(self):
         return self

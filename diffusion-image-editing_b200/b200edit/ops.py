@@ -416,11 +416,13 @@ def apply_mask(mask, zo, zv):
     mask, zo, zv = _f32(mask, "mask"), _f32(zo, "zo"), _f32(zv, "zv")
     if zo.shape != zv.shape:
         raise ValueError("apply_mask: zo and zv must have the same shape")
-    chw = zo[0].numel()
-    if mask.numel() != chw:
+    rows, chw = zo.shape[0], zo[0].numel()
+    if mask.numel() == zo.numel() and mask.numel() != chw:
+        rows, chw = 1, zo.numel()                 # one mask per image of a (B,C,H,W) batch
+    elif mask.numel() != chw:
         mask = mask.expand(1, *zo.shape[1:]).contiguous()
     out = torch.empty_like(zo)
-    check(lib.b2e_apply_mask_f32(_p(mask), _p(zo), _p(zv), _p(out), zo.shape[0], chw, _stream()), "apply_mask")
+    check(lib.b2e_apply_mask_f32(_p(mask), _p(zo), _p(zv), _p(out), rows, chw, _stream()), "apply_mask")
     return out
 
 
@@ -455,6 +457,8 @@ def extract_noise(x_t, eps, x_tm1: torch.Tensor, z_out: torch.Tensor, c: StepCoe
 # ----------------------------------------------------------------------------- masks
 def mask_from_seg(seg: torch.Tensor, classes: Sequence[int], dilate: bool, size, channels=3, ksize=7,
                   antialias=True):
+    """(H,W) parsing map -> (1,channels,oh,ow) mask; an (N,H,W) stack of N > 1 maps -> (N,channels,oh,ow) in one call,
+    map n bit-identical to the single-map result."""
     if not seg.is_cuda:
         raise _C.B2EError("mask_from_seg: segmentation must be a CUDA tensor (no CPU fallback)")
     _C.require_device()
@@ -462,6 +466,14 @@ def mask_from_seg(seg: torch.Tensor, classes: Sequence[int], dilate: bool, size,
     H, W = seg.shape[-2:]
     oh, ow = int(size[0]), int(size[1])
     cls = (C.c_int32 * max(1, len(classes)))(*[int(c) for c in classes])
+    if seg.dim() == 3 and seg.shape[0] > 1:
+        N = seg.shape[0]
+        nbytes = lib.b2e_mask_batched_workspace_bytes(N, H, W, oh, ow)
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=seg.device)
+        out = torch.empty((N, channels, oh, ow), dtype=torch.float32, device=seg.device)
+        check(lib.b2e_mask_from_seg_batched(_p(seg), N, H, W, cls, len(classes), int(bool(dilate)), ksize, oh, ow, channels,
+                                            int(bool(antialias)), _p(out), _p(ws), nbytes, _stream()), "mask_from_seg")
+        return out
     nbytes = lib.b2e_mask_workspace_bytes(H, W, oh, ow)
     ws = torch.empty(nbytes, dtype=torch.uint8, device=seg.device)
     out = torch.empty((1, channels, oh, ow), dtype=torch.float32, device=seg.device)
@@ -483,6 +495,19 @@ def resize_bilinear_aa(x: torch.Tensor, size):
         check(lib.b2e_resize_bilinear_aa_f32(_p(planes[i]), H, W, _p(out[i]), oh, ow, _p(ws), nbytes, _stream()),
               "resize_bilinear_aa")
     return out.reshape(*lead, oh, ow)
+
+
+def bilinear_argmax(x_nhwc: torch.Tensor, K: int, S: int, planes: int = 1) -> torch.Tensor:
+    """Test hook for the face parser's label kernel: x (N,Hi,Wi,planes*P) in the engine's 16-bit type (``act_dtype()``)
+    -> (N,S,S) int64, the argmax over the first K channels of the align_corners bilinear upsampling to S x S."""
+    _C.require_device()
+    if not x_nhwc.is_cuda or x_nhwc.dtype != act_dtype() or x_nhwc.dim() != 4 or x_nhwc.shape[-1] % planes:
+        raise ValueError(f"bilinear_argmax: x must be a CUDA {act_dtype()} (N,Hi,Wi,planes*P) tensor")
+    N, Hi, Wi, PP = x_nhwc.shape
+    out = torch.empty((N, S, S), dtype=torch.int64, device=x_nhwc.device)
+    check(lib.b2e_bilinear_ac_argmax_f16(_p(x_nhwc.contiguous()), _p(out), N, Hi, Wi, PP // planes, K, S, planes, _stream()),
+          "bilinear_argmax")
+    return out
 
 
 def morphology2d(x, weight, op: str, soft_max=False, beta=20.0):

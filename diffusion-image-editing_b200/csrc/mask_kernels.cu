@@ -22,12 +22,14 @@ struct ClassSet {
   float mult[kMaxClasses];  // multiplicity of a repeated class id
 };
 
-// m(y,x) = sum_c mult_c * max_{window}(seg == c), zero padding
+// m(y,x) = sum_c mult_c * max_{window}(seg == c), zero padding; map blockIdx.z of a batch of (H,W) maps
 __global__ void class_dilate_sum_kernel(const int64_t* __restrict__ seg, float* __restrict__ out,
                                         int H, int W, int r, ClassSet cs) {
   const int x = blockIdx.x * blockDim.x + threadIdx.x;
   const int y = blockIdx.y * blockDim.y + threadIdx.y;
   if (x >= W || y >= H) return;
+  seg += (int64_t)blockIdx.z * H * W;
+  out += (int64_t)blockIdx.z * H * W;
   unsigned bits = 0;
   for (int dy = -r; dy <= r; ++dy) {
     const int yy = y + dy;
@@ -101,23 +103,27 @@ __device__ __forceinline__ float aa_accumulate(const float* __restrict__ src, in
   return acc;
 }
 
-// horizontal: in (H,W) -> tmp (H,ow)
+// horizontal: in (H,W) -> tmp (H,ow); plane blockIdx.z of a batch
 __global__ void aa_resize_h_kernel(const float* __restrict__ in, float* __restrict__ tmp, int H,
                                    int W, int ow, AATable t) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   const int y = blockIdx.y * blockDim.y + threadIdx.y;
   if (i >= ow || y >= H) return;
+  in += (int64_t)blockIdx.z * H * W;
+  tmp += (int64_t)blockIdx.z * H * ow;
   const int n = t.xsize[i];
   tmp[(int64_t)y * ow + i] =
       n > 0 ? aa_accumulate(in + (int64_t)y * W + t.xmin[i], 1, t.w + (size_t)i * t.max_taps, n) : 0.f;
 }
 
-// vertical: tmp (H,ow) -> out; threshold != 0: out = (r >= 1) replicated over `channels`
+// vertical: tmp (H,ow) -> out; threshold != 0: out = (r >= 1) replicated over `channels`; plane blockIdx.z
 __global__ void aa_resize_v_kernel(const float* __restrict__ tmp, float* __restrict__ out, int H,
                                    int ow, int oh, AATable t, int threshold, int channels) {
   const int x = blockIdx.x * blockDim.x + threadIdx.x;
   const int i = blockIdx.y * blockDim.y + threadIdx.y;
   if (x >= ow || i >= oh) return;
+  tmp += (int64_t)blockIdx.z * H * ow;
+  out += (int64_t)blockIdx.z * (threshold ? channels : 1) * oh * ow;
   const int n = t.xsize[i];
   float r = n > 0 ? aa_accumulate(tmp + (int64_t)t.xmin[i] * ow + x, ow, t.w + (size_t)i * t.max_taps, n)
                   : 0.f;
@@ -175,20 +181,22 @@ __global__ void morphology_kernel(const float* __restrict__ x, const float* __re
 
 static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+// N maps: one (H,W) class-sum plane and one (H,ow) intermediate each; the weight tables depend only on the sizes
+// and are shared.  N = 1 is the single-map layout.
 struct MaskWs {
-  float* plane;  // (H,W) class-sum
-  float* tmp;    // (H,ow)
+  float* plane;  // (N,H,W) class-sum
+  float* tmp;    // (N,H,ow)
   AATable th, tv;
   size_t bytes;
 };
 
-static MaskWs carve(void* ws, int64_t H, int64_t W, int64_t oh, int64_t ow) {
+static MaskWs carve(void* ws, int64_t N, int64_t H, int64_t W, int64_t oh, int64_t ow) {
   MaskWs m;
   char* p = (char*)ws;
   size_t off = 0;
   auto take = [&](size_t n) { char* q = p ? p + off : nullptr; off += align_up(n, 256); return q; };
-  m.plane = (float*)take(sizeof(float) * H * W);
-  m.tmp = (float*)take(sizeof(float) * H * ow);
+  m.plane = (float*)take(sizeof(float) * N * H * W);
+  m.tmp = (float*)take(sizeof(float) * N * H * ow);
   m.th.max_taps = aa_max_taps(W, ow);
   m.tv.max_taps = aa_max_taps(H, oh);
   m.th.xmin = (int*)take(sizeof(int) * ow);
@@ -201,7 +209,7 @@ static MaskWs carve(void* ws, int64_t H, int64_t W, int64_t oh, int64_t ow) {
   return m;
 }
 
-static int run_resize(const float* in, int64_t H, int64_t W, float* out, int64_t oh, int64_t ow,
+static int run_resize(const float* in, int64_t N, int64_t H, int64_t W, float* out, int64_t oh, int64_t ow,
                       const MaskWs& m, int threshold, int channels, cudaStream_t st) {
   aa_weights_kernel<<<(unsigned)((ow + 127) / 128), 128, 0, st>>>((int)W, (int)ow, m.th);
   int rc = check_launch("aa_weights(h)");
@@ -210,11 +218,11 @@ static int run_resize(const float* in, int64_t H, int64_t W, float* out, int64_t
   rc = check_launch("aa_weights(v)");
   if (rc) return rc;
   dim3 blk(32, 8);
-  aa_resize_h_kernel<<<dim3((unsigned)((ow + 31) / 32), (unsigned)((H + 7) / 8)), blk, 0, st>>>(
+  aa_resize_h_kernel<<<dim3((unsigned)((ow + 31) / 32), (unsigned)((H + 7) / 8), (unsigned)N), blk, 0, st>>>(
       in, m.tmp, (int)H, (int)W, (int)ow, m.th);
   rc = check_launch("aa_resize_h");
   if (rc) return rc;
-  aa_resize_v_kernel<<<dim3((unsigned)((ow + 31) / 32), (unsigned)((oh + 7) / 8)), blk, 0, st>>>(
+  aa_resize_v_kernel<<<dim3((unsigned)((ow + 31) / 32), (unsigned)((oh + 7) / 8), (unsigned)N), blk, 0, st>>>(
       m.tmp, out, (int)H, (int)ow, (int)oh, m.tv, threshold, channels);
   return check_launch("aa_resize_v");
 }
@@ -227,15 +235,28 @@ extern "C" {
 
 size_t b2e_mask_workspace_bytes(int64_t H, int64_t W, int64_t out_h, int64_t out_w) {
   if (H <= 0 || W <= 0 || out_h <= 0 || out_w <= 0) return 0;
-  return carve(nullptr, H, W, out_h, out_w).bytes;
+  return carve(nullptr, 1, H, W, out_h, out_w).bytes;
+}
+
+size_t b2e_mask_batched_workspace_bytes(int64_t N, int64_t H, int64_t W, int64_t out_h, int64_t out_w) {
+  if (N <= 0 || H <= 0 || W <= 0 || out_h <= 0 || out_w <= 0) return 0;
+  return carve(nullptr, N, H, W, out_h, out_w).bytes;
 }
 
 int b2e_mask_from_seg(const int64_t* seg, int64_t H, int64_t W, const int32_t* classes,
                       int n_classes, int dilate, int ksize, int64_t out_h, int64_t out_w,
                       int channels, int antialias, float* out, void* workspace,
                       size_t workspace_bytes, void* stream) {
+  return b2e_mask_from_seg_batched(seg, 1, H, W, classes, n_classes, dilate, ksize, out_h, out_w, channels, antialias, out,
+                                   workspace, workspace_bytes, stream);
+}
+
+int b2e_mask_from_seg_batched(const int64_t* seg, int64_t N, int64_t H, int64_t W, const int32_t* classes,
+                              int n_classes, int dilate, int ksize, int64_t out_h, int64_t out_w,
+                              int channels, int antialias, float* out, void* workspace,
+                              size_t workspace_bytes, void* stream) {
   B2E_REQUIRE(seg && out && workspace, B2E_INVALID_ARG, "mask_from_seg: null pointer");
-  B2E_REQUIRE(H > 0 && W > 0 && out_h > 0 && out_w > 0 && channels > 0, B2E_UNSUPPORTED_SHAPE,
+  B2E_REQUIRE(N > 0 && N < 65536 && H > 0 && W > 0 && out_h > 0 && out_w > 0 && channels > 0, B2E_UNSUPPORTED_SHAPE,
               "mask_from_seg: bad shape");
   B2E_REQUIRE(H < (1 << 15) && W < (1 << 15), B2E_UNSUPPORTED_SHAPE, "mask_from_seg: map too large");
   B2E_REQUIRE(n_classes >= 0 && (n_classes == 0 || classes), B2E_INVALID_ARG, "mask_from_seg: classes");
@@ -243,7 +264,7 @@ int b2e_mask_from_seg(const int64_t* seg, int64_t H, int64_t W, const int32_t* c
               "mask_from_seg: dilation kernel size must be odd and <= 31 (got %d)", ksize);
   B2E_REQUIRE(antialias, B2E_UNSUPPORTED_SHAPE,
               "mask_from_seg: only the antialiased resize (torchvision >= 0.17 default) is implemented");
-  B2E_REQUIRE(workspace_bytes >= b2e_mask_workspace_bytes(H, W, out_h, out_w), B2E_WORKSPACE_TOO_SMALL,
+  B2E_REQUIRE(workspace_bytes >= b2e_mask_batched_workspace_bytes(N, H, W, out_h, out_w), B2E_WORKSPACE_TOO_SMALL,
               "mask_from_seg: workspace too small");
   ClassSet cs;
   cs.n = 0;
@@ -261,13 +282,13 @@ int b2e_mask_from_seg(const int64_t* seg, int64_t H, int64_t W, const int32_t* c
     cs.mult[j] += 1.f;
   }
   cudaStream_t st = (cudaStream_t)stream;
-  MaskWs m = carve(workspace, H, W, out_h, out_w);
+  MaskWs m = carve(workspace, N, H, W, out_h, out_w);
   dim3 blk(32, 8);
-  class_dilate_sum_kernel<<<dim3((unsigned)((W + 31) / 32), (unsigned)((H + 7) / 8)), blk, 0, st>>>(
+  class_dilate_sum_kernel<<<dim3((unsigned)((W + 31) / 32), (unsigned)((H + 7) / 8), (unsigned)N), blk, 0, st>>>(
       seg, m.plane, (int)H, (int)W, dilate ? ksize / 2 : 0, cs);
   int rc = check_launch("class_dilate_sum");
   if (rc) return rc;
-  return run_resize(m.plane, H, W, out, out_h, out_w, m, 1, channels, st);
+  return run_resize(m.plane, N, H, W, out, out_h, out_w, m, 1, channels, st);
 }
 
 int b2e_resize_bilinear_aa_f32(const float* in, int64_t H, int64_t W, float* out, int64_t out_h,
@@ -276,8 +297,8 @@ int b2e_resize_bilinear_aa_f32(const float* in, int64_t H, int64_t W, float* out
   B2E_REQUIRE(H > 0 && W > 0 && out_h > 0 && out_w > 0, B2E_UNSUPPORTED_SHAPE, "resize: bad shape");
   B2E_REQUIRE(workspace_bytes >= b2e_mask_workspace_bytes(H, W, out_h, out_w), B2E_WORKSPACE_TOO_SMALL,
               "resize: workspace too small");
-  MaskWs m = carve(workspace, H, W, out_h, out_w);
-  return run_resize(in, H, W, out, out_h, out_w, m, 0, 1, (cudaStream_t)stream);
+  MaskWs m = carve(workspace, 1, H, W, out_h, out_w);
+  return run_resize(in, 1, H, W, out, out_h, out_w, m, 0, 1, (cudaStream_t)stream);
 }
 
 int b2e_morphology2d_f32(const float* x, const float* weight, float* out, int64_t B, int64_t Cin,

@@ -646,8 +646,40 @@ int bilinear_ac_bwd_launch(const float* g, f16* dx, int N, int Hi, int Wi, int P
   return check_launch("bilinear_ac_bwd");
 }
 
-// F.interpolate(x, (Ho, Wo), mode="bilinear", align_corners=True): x f16 NHWC (N,Hi,Wi,P), first K channels ->
-// out fp32 NCHW (N,K,Ho,Wo).  ATen's arithmetic: src = dst * (in-1)/(out-1); weights (1-l, l).
+// F.interpolate(x, (Ho, Wo), mode="bilinear", align_corners=True) at one output pixel: the four source pixels and the
+// weights.  ATen's arithmetic: src = dst * (in-1)/(out-1); weights (1-l, l).
+struct BilinearTap {
+  const f16 *p00, *p01, *p10, *p11;
+  float lh, lw;
+};
+
+__device__ __forceinline__ BilinearTap bilinear_ac_tap(const f16* x, int n, int oh, int ow, int Hi, int Wi, int PP, float sh,
+                                                       float sw) {
+  const float fh = sh * (float)oh, fw = sw * (float)ow;
+  const int h0 = (int)fh, w0 = (int)fw;
+  const int h1 = h0 + (h0 < Hi - 1 ? 1 : 0), w1 = w0 + (w0 < Wi - 1 ? 1 : 0);
+  BilinearTap t;
+  t.lh = fh - (float)h0;
+  t.lw = fw - (float)w0;
+  t.p00 = x + (((int64_t)n * Hi + h0) * Wi + w0) * PP;
+  t.p01 = x + (((int64_t)n * Hi + h0) * Wi + w1) * PP;
+  t.p10 = x + (((int64_t)n * Hi + h1) * Wi + w0) * PP;
+  t.p11 = x + (((int64_t)n * Hi + h1) * Wi + w1) * PP;
+  return t;
+}
+
+// Channel k of the upsampled value.  The logits kernel and the label kernel both call this, so a label is the argmax of
+// exactly the logits; the roundings are spelled out (they are the contraction the compiler chose for the original
+// expression (1-lh)((1-lw) v00 + lw v01) + lh((1-lw) v10 + lw v11)) so that no kernel can contract them differently.
+__device__ __forceinline__ float bilinear_ac_value(const BilinearTap& t, int k, int P, int planes) {
+  auto val = [&](const f16* q) { return planes == 3 ? __fadd_rn(f16_to_float(q[k]), f16_to_float(q[P + k])) : f16_to_float(q[k]); };
+  const float r0 = __fmaf_rn(1.f - t.lw, val(t.p00), __fmul_rn(t.lw, val(t.p01)));
+  const float r1 = __fmaf_rn(1.f - t.lw, val(t.p10), __fmul_rn(t.lw, val(t.p11)));
+  return __fmaf_rn(1.f - t.lh, r0, __fmul_rn(t.lh, r1));
+}
+
+// x f16 NHWC (N,Hi,Wi,P), first K channels -> out fp32 NCHW (N,K,Ho,Wo).  planes = 3: split tensor [hi | lo | hi] per
+// pixel, value = hi + lo.
 __global__ void __launch_bounds__(256) bilinear_ac_kernel(const f16* __restrict__ x, float* __restrict__ out, int N, int Hi,
                                                           int Wi, int P, int K, int Ho, int Wo, float sh, float sw, int planes) {
   pdl_wait();
@@ -656,28 +688,61 @@ __global__ void __launch_bounds__(256) bilinear_ac_kernel(const f16* __restrict_
     const int ow = (int)(i % Wo);
     const int oh = (int)((i / Wo) % Ho);
     const int n = (int)(i / ((int64_t)Wo * Ho));
-    const float fh = sh * (float)oh, fw = sw * (float)ow;
-    const int h0 = (int)fh, w0 = (int)fw;
-    const int h1 = h0 + (h0 < Hi - 1 ? 1 : 0), w1 = w0 + (w0 < Wi - 1 ? 1 : 0);
-    const float lh = fh - (float)h0, lw = fw - (float)w0;
-    const int PP = P * planes;     // planes = 3: split tensor [hi | lo | hi] per pixel, value = hi + lo
-    const f16* p00 = x + (((int64_t)n * Hi + h0) * Wi + w0) * PP;
-    const f16* p01 = x + (((int64_t)n * Hi + h0) * Wi + w1) * PP;
-    const f16* p10 = x + (((int64_t)n * Hi + h1) * Wi + w0) * PP;
-    const f16* p11 = x + (((int64_t)n * Hi + h1) * Wi + w1) * PP;
-    auto val = [&](const f16* q, int k) { return planes == 3 ? f16_to_float(q[k]) + f16_to_float(q[P + k]) : f16_to_float(q[k]); };
-    for (int k = 0; k < K; ++k) {
-      const float v = (1.f - lh) * ((1.f - lw) * val(p00, k) + lw * val(p01, k)) +
-                      lh * ((1.f - lw) * val(p10, k) + lw * val(p11, k));
-      out[(((int64_t)n * K + k) * Ho + oh) * Wo + ow] = v;
-    }
+    const BilinearTap t = bilinear_ac_tap(x, n, oh, ow, Hi, Wi, P * planes, sh, sw);
+    for (int k = 0; k < K; ++k) out[(((int64_t)n * K + k) * Ho + oh) * Wo + ow] = bilinear_ac_value(t, k, P, planes);
   }
 }
 
+// The same upsampling followed by argmax over the K channels: labels int64 (N,Ho,Wo), no logits in memory.  torch.argmax
+// semantics: the first maximum wins a tie, and a NaN is the maximum (the first NaN).
+__global__ void __launch_bounds__(256) bilinear_ac_argmax_kernel(const f16* __restrict__ x, int64_t* __restrict__ labels, int N,
+                                                                 int Hi, int Wi, int P, int K, int Ho, int Wo, float sh, float sw,
+                                                                 int planes) {
+  pdl_wait();
+  const int64_t total = (int64_t)N * Ho * Wo;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int ow = (int)(i % Wo);
+    const int oh = (int)((i / Wo) % Ho);
+    const int n = (int)(i / ((int64_t)Wo * Ho));
+    const BilinearTap t = bilinear_ac_tap(x, n, oh, ow, Hi, Wi, P * planes, sh, sw);
+    float best = bilinear_ac_value(t, 0, P, planes);
+    int arg = 0;
+    for (int k = 1; k < K && best == best; ++k) {
+      const float v = bilinear_ac_value(t, k, P, planes);
+      if (v > best || v != v) { best = v; arg = k; }
+    }
+    labels[i] = arg;
+  }
+}
+
+static void bilinear_ac_scales(int Hi, int Wi, int Ho, int Wo, float* sh, float* sw) {
+  *sh = Ho > 1 ? (float)(Hi - 1) / (float)(Ho - 1) : 0.f;
+  *sw = Wo > 1 ? (float)(Wi - 1) / (float)(Wo - 1) : 0.f;
+}
+
 int bilinear_ac_launch(const f16* x, float* out, int N, int Hi, int Wi, int P, int K, int Ho, int Wo, cudaStream_t st, int planes) {
-  const float sh = Ho > 1 ? (float)(Hi - 1) / (float)(Ho - 1) : 0.f, sw = Wo > 1 ? (float)(Wi - 1) / (float)(Wo - 1) : 0.f;
+  float sh, sw;
+  bilinear_ac_scales(Hi, Wi, Ho, Wo, &sh, &sw);
   launch_pdl(bilinear_ac_kernel, dim3(grid_for((int64_t)N * Ho * Wo)), dim3(256), 0, st, x, out, N, Hi, Wi, P, K, Ho, Wo, sh, sw, planes);
   return check_launch("bilinear_ac");
 }
 
+int bilinear_ac_argmax_launch(const f16* x, int64_t* labels, int N, int Hi, int Wi, int P, int K, int Ho, int Wo, cudaStream_t st,
+                              int planes) {
+  float sh, sw;
+  bilinear_ac_scales(Hi, Wi, Ho, Wo, &sh, &sw);
+  launch_pdl(bilinear_ac_argmax_kernel, dim3(grid_for((int64_t)N * Ho * Wo)), dim3(256), 0, st, x, labels, N, Hi, Wi, P, K, Ho, Wo,
+             sh, sw, planes);
+  return check_launch("bilinear_ac_argmax");
+}
+
 }  // namespace b2e
+
+extern "C" int b2e_bilinear_ac_argmax_f16(const void* x, int64_t* labels, int64_t N, int64_t Hi, int64_t Wi, int64_t P, int64_t K,
+                                          int64_t S, int planes, void* stream) {
+  B2E_REQUIRE(x && labels, B2E_INVALID_ARG, "bilinear_ac_argmax: null pointer");
+  B2E_REQUIRE(N > 0 && Hi > 0 && Wi > 0 && S > 0 && K >= 1 && K <= P, B2E_UNSUPPORTED_SHAPE, "bilinear_ac_argmax: bad shape");
+  B2E_REQUIRE(planes == 1 || planes == 3, B2E_INVALID_ARG, "bilinear_ac_argmax: planes must be 1 or 3");
+  return b2e::bilinear_ac_argmax_launch(static_cast<const b2e::f16*>(x), labels, (int)N, (int)Hi, (int)Wi, (int)P, (int)K, (int)S,
+                                        (int)S, (cudaStream_t)stream, planes);
+}

@@ -135,6 +135,7 @@ struct b2e_unet {
     float *f1_w = nullptr, *f2_w = nullptr;
   } bs;
   const float* in_dlogits = nullptr;
+  int64_t* out_labels = nullptr;   // per call of b2e_resnet_forward_labels: argmax labels instead of logits
   // LPIPS mode (b2e_lpips_create): scaling layer -> VGG-16 features[0:30] (conv1_1 as a 1x1 convolution over the im2col
   // input, ReLU in every epilogue) -> distance head at relu1_2 .. relu5_3 against the reference's cached normalised
   // features; backward: d(dist) -> d(input).  The regulariser of the masked-prediction guidance (use_lpips)
@@ -802,7 +803,10 @@ int build_program_resnet(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* 
     conv(bs.out_cls, hs.o1, 1, false, nullptr, &hs.o2, "conv_out.conv_out");
     if (!rc) {
       const Tensor oo = hs.o2;
-      ew([m, oo, B, K, S, PL](cudaStream_t st) { return bilinear_ac_launch(oo.p, m->out_eps, B, oo.H, oo.W, oo.C, K, S, S, st, PL); },
+      // b2e_resnet_forward_labels sets out_labels for its call: the upsampled logits go straight into their argmax
+      ew([m, oo, B, K, S, PL](cudaStream_t st) {
+           return m->out_labels ? bilinear_ac_argmax_launch(oo.p, m->out_labels, B, oo.H, oo.W, oo.C, K, S, S, st, PL)
+                                : bilinear_ac_launch(oo.p, m->out_eps, B, oo.H, oo.W, oo.C, K, S, S, st, PL); },
          (double)oo.bytes + 4.0 * B * K * S * S, "bilinear upsample (align_corners) -> logits");
     }
   }
@@ -2420,6 +2424,16 @@ int b2e_resnet_backward(b2e_unet* m, const float* d_logits, float* d_image, int6
 }
 
 static int unet_forward_impl(b2e_unet* m, const float* x, const int64_t* timesteps, float* eps, int64_t B, void* stream);
+
+int b2e_resnet_forward_labels(b2e_unet* m, const float* x, int64_t* labels, int64_t B, void* stream) {
+  B2E_REQUIRE(m && x && labels, B2E_INVALID_ARG, "resnet_forward_labels: null pointer");
+  B2E_REQUIRE(m->resnet && m->rcfg.head == 1, B2E_INVALID_ARG, "resnet_forward_labels: not a face-parser handle");
+  m->out_labels = labels;
+  const int rc = unet_forward_impl(m, x, nullptr, reinterpret_cast<float*>(labels), B, stream);
+  m->out_labels = nullptr;
+  m->fwd_B = -1;     // no logits were produced: no backward over this pass
+  return rc;
+}
 
 int b2e_lpips_create(const b2e_lpips_config* cfg, int64_t max_batch, b2e_unet** out) {
   B2E_REQUIRE(cfg && out && max_batch > 0, B2E_INVALID_ARG, "lpips_create: bad argument");

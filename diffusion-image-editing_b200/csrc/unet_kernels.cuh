@@ -160,6 +160,9 @@ int fc_act_launch(const float* x, const float* w, const float* b, float* out, in
 int chan_affine_launch(const f16* x, const float* a, const float* b, const f16* y, f16* out, int N, int HW, int C,
                        cudaStream_t st, int planes = 1);
 int bilinear_ac_launch(const f16* x, float* out, int N, int Hi, int Wi, int P, int K, int Ho, int Wo, cudaStream_t st, int planes = 1);
+// the same upsampling, then the argmax over the K channels -> labels int64 (N,Ho,Wo)
+int bilinear_ac_argmax_launch(const f16* x, int64_t* labels, int N, int Hi, int Wi, int P, int K, int Ho, int Wo, cudaStream_t st,
+                              int planes = 1);
 int bilinear_ac_bwd_launch(const float* g, f16* dx, int N, int Hi, int Wi, int P, int K, int Ho, int Wo, cudaStream_t st,
                            const float* gs = nullptr);
 int chan_dot_launch(const f16* x, const f16* y, float* out, int N, int HW, int C, float scale, cudaStream_t st, int yplanes = 1);

@@ -18,7 +18,8 @@ class MaskCreator:
         self.antialias = antialias                # torchvision >= 0.17 default; False is not implemented
 
     def create_mask(self, segmentation: torch.Tensor, classes: list, channels: int = 3) -> torch.Tensor:
-        """(H,W) integer parsing map -> (1,channels,d,d) float mask in {0,1} on the device."""
+        """(H,W) integer parsing map -> (1,channels,d,d) float mask in {0,1} on the device; (N,H,W) maps ->
+        (N,channels,d,d) in one batched call."""
         seg = segmentation.to(self.device) if not segmentation.is_cuda else segmentation
         return ops.mask_from_seg(seg, list(classes), self.dilate_mask, self.resize_size, channels=channels,
                                  ksize=self.kernel_size, antialias=self.antialias)

@@ -190,5 +190,13 @@ class SegmentationModel:
         return ((x - self.mean.to(x.device)) / self.std.to(x.device)).to(self.device)
 
     def __call__(self, image: torch.Tensor) -> torch.Tensor:
-        out = self.net(self.process(image))[0]
+        """(1,3,H,W) -> (S,S) parsing map, as the reference.  (B,3,H,W) with B > 1 -> (B,S,S) int64: on the native parser
+        the labels come from its fused upsample-and-argmax kernel, on a caller's ``net=`` from ``argmax(1)``."""
+        x = self.process(image)
+        if x.shape[0] > 1:
+            from b200edit.bisenet import BiSeNet, MultiResBiSeNet
+            if isinstance(self.net, (BiSeNet, MultiResBiSeNet)):
+                return self.net.labels(x)
+            return self.net(x)[0].argmax(1)
+        out = self.net(x)[0]
         return out.squeeze(0).argmax(0)

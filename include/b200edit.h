@@ -227,6 +227,13 @@ int b2e_mask_from_seg(const int64_t* seg, int64_t H, int64_t W, const int32_t* c
                       int n_classes, int dilate, int ksize, int64_t out_h, int64_t out_w,
                       int channels, int antialias, float* out, void* workspace,
                       size_t workspace_bytes, void* stream);
+/* N maps at once: seg DEVICE int64 (N,H,W) -> out (N,channels,out_h,out_w), the other arguments as b2e_mask_from_seg.
+ * One launch per stage for the whole batch; map n comes out bit-identical to b2e_mask_from_seg on seg[n]. */
+size_t b2e_mask_batched_workspace_bytes(int64_t N, int64_t H, int64_t W, int64_t out_h, int64_t out_w);
+int b2e_mask_from_seg_batched(const int64_t* seg, int64_t N, int64_t H, int64_t W, const int32_t* classes,
+                              int n_classes, int dilate, int ksize, int64_t out_h, int64_t out_w,
+                              int channels, int antialias, float* out, void* workspace,
+                              size_t workspace_bytes, void* stream);
 /* Antialiased bilinear resize of one fp32 plane (H,W)->(out_h,out_w), ATen CPU order. */
 int b2e_resize_bilinear_aa_f32(const float* in, int64_t H, int64_t W, float* out, int64_t out_h,
                                int64_t out_w, void* workspace, size_t workspace_bytes, void* stream);
@@ -401,6 +408,11 @@ typedef struct {
 } b2e_resnet_config;
 int b2e_resnet_create(const b2e_resnet_config* cfg, int64_t max_batch, b2e_unet** out);
 int b2e_resnet_backward(b2e_unet* m, const float* d_logits, float* d_image, int64_t B, void* stream);
+/* Face parser (head 1) only: the forward of b2e_unet_forward, but the last op upsamples the head's logits and takes
+ * their argmax per pixel in one kernel: labels DEVICE int64 (B, input_size, input_size) = torch.argmax(logits, 1) of the
+ * logits b2e_unet_forward returns (first maximum on a tie, NaN counts as the maximum); no logits are written.  The pass
+ * leaves no forward for b2e_resnet_backward.  B2E_INVALID_ARG on a classifier handle. */
+int b2e_resnet_forward_labels(b2e_unet* m, const float* x, int64_t* labels, int64_t B, void* stream);
 
 /* ------------------------------------------------------------------ LPIPS distance (use_lpips regulariser, metrics.lpips)
  * lpips v0.1 with net='vgg' (lpips.LPIPS(net='vgg'), normalize=False): scaling layer (x - shift) / scale, VGG-16
@@ -443,6 +455,12 @@ int b2e_conv2d_nhwc_f16(const void* x, const float* w, const float* bias, const 
  * each writing its sub-grid of the output through a strided TMA map.  Cin, Cout multiples of 64.  Allocates + synchronises. */
 int b2e_upsample_conv3x3_nhwc_f16(const void* x, const float* w, const float* bias, void* out, int64_t N, int64_t H,
                                    int64_t W, int64_t Cin, int64_t Cout, void* stream);
+
+/* Test hook for the face parser's label kernel: x (N,Hi,Wi,planes*P) 16-bit NHWC (b2e_act_dtype; planes = 3: split
+ * [hi | lo | hi] channel planes, value hi + lo) -> labels int64 (N,S,S), the argmax over the first K channels of the
+ * align_corners bilinear upsampling to S x S. */
+int b2e_bilinear_ac_argmax_f16(const void* x, int64_t* labels, int64_t N, int64_t Hi, int64_t Wi, int64_t P, int64_t K,
+                               int64_t S, int planes, void* stream);
 
 /* Measurement hook for the same kernel: `iters` back-to-back launches of one convolution (zero-filled operands of the
  * given shape, `copies` distinct packed weight sets used round-robin so that launches miss the L2 like the layers of a
