@@ -146,6 +146,8 @@ PROTOTYPES = {
     "b2e_conv2d_bench_f16": (_I, [_I64, _I64, _I64, _I64, _I64, _I, _I, _I, _I, _P, _P]),
     "b2e_bilinear_ac_argmax_f16": (_I, [_P, _P, _I64, _I64, _I64, _I64, _I64, _I64, _I, _P]),
     "b2e_upsample_conv3x3_nhwc_f16": (_I, [_P, _P, _P, _P, _I64, _I64, _I64, _I64, _I64, _P]),
+    "b2e_attention_f16": (_I, [_P, _I64, _I64, _P, _I64, _I64, _I64, _P, _I64, _I64, _I64, _I64, _I64, _I64, _I64, _I64,
+                               _I, _I, _I, _P]),
 }
 
 

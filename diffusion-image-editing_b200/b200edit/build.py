@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(os.path.dirname(HERE), "csrc")
 OUT = os.path.join(HERE, "libb200edit.so")
 OBJ = os.path.join(HERE, "_obj")
-SOURCES = ["step_kernels.cu", "guidance_heads.cu", "mask_kernels.cu", "conv_igemm.cu", "flash_attn.cu", "unet_kernels.cu", "resnet_kernels.cu", "lpips_kernels.cu", "unet.cu"]
+SOURCES = ["step_kernels.cu", "guidance_heads.cu", "mask_kernels.cu", "conv_igemm.cu", "flash_attn.cu", "attention.cu", "unet_kernels.cu", "resnet_kernels.cu", "lpips_kernels.cu", "unet.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
          "-Xcompiler", "-fPIC,-ffp-contract=off", "--expt-relaxed-constexpr",

@@ -542,6 +542,60 @@ def upsample_conv3x3_nhwc_f16(x, w, bias):
     return out
 
 
+ATTENTION_PATHS = {"fused": 0, "materialised": 1, "single_head": 2, "cuda_core": 3, "fp32_split": 4, "fp32_tiled": 5}
+
+
+def split_planes(x: torch.Tensor) -> torch.Tensor:
+    """fp32 (..., P) -> the fp32-accurate mode's split tensor (..., 3P): [hi | lo | hi] planes, hi = 16-bit(x),
+    lo = 16-bit(x - hi)."""
+    hi = x.to(act_dtype())
+    lo = (x - hi.float()).to(act_dtype())
+    return torch.cat([hi, lo, hi], dim=-1).contiguous()
+
+
+def merge_planes(x: torch.Tensor) -> torch.Tensor:
+    """Split tensor (..., 3P) -> fp32 hi + lo (..., P)."""
+    P = x.shape[-1] // 3
+    return x[..., :P].float() + x[..., P:2 * P].float()
+
+
+def attention_f16(q, kv, *, hw, heads, head_dim, k_col, v_col, out_pitch, q_col=0, valid_k=None, causal=False,
+                  path="fused", softmax_warps=8, out=None):
+    """Test hook for the attention paths (include/b200edit.h, b2e_attention_f16): softmax(Q K^T / sqrt(head_dim)) V over
+    channel windows, keys >= valid_k (default: all) masked, through the engine's own launch sequence of `path`
+    (one of ATTENTION_PATHS).
+
+    q (B, H*W, q_pitch) and kv (B, Tk, kv_pitch) are token-major tensors in `act_dtype()`; the "fp32_*" paths take fp32
+    tensors and split them into [hi | lo | hi] planes here (q is kv: one packed tensor).  Returns `out` (B, H*W, out_pitch)
+    in `act_dtype()`, or the split output (B, H*W, 3 * out_pitch) of the fp32 paths (``merge_planes`` gives hi + lo)."""
+    _C.require_device()
+    if path not in ATTENTION_PATHS:
+        raise ValueError(f"attention_f16: path must be one of {sorted(ATTENTION_PATHS)}")
+    planes = 3 if path.startswith("fp32") else 1
+    want = torch.float32 if planes == 3 else act_dtype()
+    if (q.dtype != want or kv.dtype != want or q.dim() != 3 or kv.dim() != 3 or not q.is_cuda or not kv.is_cuda
+            or q.shape[1] != hw[0] * hw[1] or q.shape[0] != kv.shape[0]):
+        raise ValueError(f"attention_f16: q (B, H*W, pitch), kv (B, Tk, pitch) must be CUDA {want} tensors for path {path}")
+    packed = q is kv
+    if planes == 3:
+        q = split_planes(q)
+        kv = q if packed else split_planes(kv)
+    else:
+        q = q.contiguous()
+        kv = q if packed else kv.contiguous()
+    B, Tq, qpp = q.shape
+    Tk, kvpp = kv.shape[1], kv.shape[2]
+    H, W = hw
+    if out is None:
+        out = torch.empty((B, Tq, planes * out_pitch), dtype=act_dtype(), device=q.device)
+    if out.shape != (B, Tq, planes * out_pitch) or out.dtype != act_dtype() or not out.is_contiguous():
+        raise ValueError("attention_f16: out must be a contiguous (B, H*W, planes * out_pitch) tensor")
+    check(lib.b2e_attention_f16(_p(q), qpp // planes, q_col, _p(kv), kvpp // planes, k_col, v_col, _p(out), out_pitch,
+                                B, H, W, Tk, Tk if valid_k is None else valid_k, heads, head_dim, int(bool(causal)),
+                                ATTENTION_PATHS[path], softmax_warps, _stream()), "attention_f16")
+    return out
+
+
 def conv2d_nhwc_f16(x, w, bias, stride=1, residual=None):
     """Test hook for the tcgen05 implicit-GEMM convolution (optionally + residual; 16-bit NHWC, `act_dtype()`)."""
     _C.require_device()

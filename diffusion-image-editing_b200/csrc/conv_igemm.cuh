@@ -106,7 +106,9 @@ struct FlashPlan {
   double flops;
 };
 int flash_attn_plan_build(FlashPlan* pl, const f16* qh, const f16* kh, const f16* vht, f16* oh, int NV, int Tq, int Tk, int D);
-int flash_attn_launch(const FlashPlan& pl, int valid_k, float scale, cudaStream_t st, int causal = 0);
+// softmax_warps: 8 (two threads per query row) or 4 (one); the engine uses flash_attn_default_warps() (B2E_FLASH_WARPS)
+int flash_attn_launch(const FlashPlan& pl, int valid_k, float scale, int softmax_warps, cudaStream_t st, int causal = 0);
+int flash_attn_default_warps();
 
 // fp32 [Cout][Cin][k][k] -> f16 out[co*row_len + col_off + t*tap_width + ci]   (t = kh*k + kw)
 // (ci0, cin_total): pack only input channels [ci0, ci0 + Cin) of a weight with cin_total input channels

@@ -14,7 +14,7 @@
 // compute block j+1's scores while the softmax warps work on block j.
 // Warp roles: warp 0 = TMA producer (Q once per item; K (+ V^T) tiles through an smem ring), warp 1 = TMEM allocator +
 // MMA issuer, warps 2-9 = softmax + epilogue (TMEM lane = query row; two threads per row, 64 key columns / half of the D
-// output columns each, row maxima and sums exchanged through smem; B2E_FLASH_WARPS=4 selects one thread per row).
+// output columns each, row maxima and sums exchanged through smem; softmax_warps = 4 selects one thread per row).
 // Measured (r93): SD UNet forward at batch 16 30.45 -> 30.05 ms, LDM UNet at batch 32 14.74 -> 14.61 ms - the softmax
 // warps were not the limiter the clock64 traces suggested; the remaining gap is in the MMA / TMEM hand-shakes.
 #include <cudaTypedefs.h>
@@ -419,13 +419,18 @@ int flash_attn_plan_build(FlashPlan* pl, const f16* qh, const f16* kh, const f16
   return B2E_OK;
 }
 
-int flash_attn_launch(const FlashPlan& pl, int valid_k, float scale, cudaStream_t st, int causal) {
-  B2E_REQUIRE(valid_k >= 1 && valid_k <= pl.Tk, B2E_INVALID_ARG, "flash_attn: valid_k %d of %d", valid_k, pl.Tk);
-  FaParams p;
-  p.NV = pl.NV; p.Tq = pl.Tq; p.Tk = pl.Tk; p.valid_k = valid_k; p.causal = causal; p.scale_log2e = scale * 1.4426950408889634f; p.out = pl.out;
+int flash_attn_default_warps() {
   // B2E_FLASH_WARPS=4: one softmax thread per query row (the original layout); default 8: two threads per row
   static const int sw = getenv("B2E_FLASH_WARPS") ? atoi(getenv("B2E_FLASH_WARPS")) : 8;
-  if (sw == 8) {
+  return sw == 8 ? 8 : 4;
+}
+
+int flash_attn_launch(const FlashPlan& pl, int valid_k, float scale, int softmax_warps, cudaStream_t st, int causal) {
+  B2E_REQUIRE(valid_k >= 1 && valid_k <= pl.Tk, B2E_INVALID_ARG, "flash_attn: valid_k %d of %d", valid_k, pl.Tk);
+  B2E_REQUIRE(softmax_warps == 4 || softmax_warps == 8, B2E_INVALID_ARG, "flash_attn: %d softmax warps (4 or 8)", softmax_warps);
+  FaParams p;
+  p.NV = pl.NV; p.Tq = pl.Tq; p.Tk = pl.Tk; p.valid_k = valid_k; p.causal = causal; p.scale_log2e = scale * 1.4426950408889634f; p.out = pl.out;
+  if (softmax_warps == 8) {
     switch (pl.D) {
       case 64: return flash_launch_t<64, 8>(pl.map_q, pl.map_k, pl.map_v, p, st);
       case 128: return flash_launch_t<128, 8>(pl.map_q, pl.map_k, pl.map_v, p, st);

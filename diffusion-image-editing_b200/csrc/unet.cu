@@ -15,6 +15,7 @@
 #include <unordered_map>
 #include <vector>
 
+#include "attention.cuh"
 #include "unet_kernels.cuh"
 
 using namespace b2e;
@@ -48,7 +49,7 @@ inline int pad64(int c) { return (c + 63) / 64 * 64; }
 // residual fused into the output projection's K segment) -> 1x1 proj_out + block input
 struct LNL { float* g = nullptr; float* b = nullptr; int C = 0; };
 struct XfL {
-  std::string name; int C = 0, heads = 0, d = 0, dpad = 0;
+  std::string name; int C = 0, heads = 0, d = 0;
   NormL gn; LNL ln1, ln2, ln3;
   ConvL proj_in, qkv1, out1, q2, kv2, out2, ff1, ff2, proj_out;
 };
@@ -359,7 +360,7 @@ struct b2e_unet {
   }
   int make_xformer(const std::string& name, int C, int heads, int ctx_dim) {
     XfL x;
-    x.name = name; x.C = C; x.heads = heads; x.d = C / heads; x.dpad = pad64(x.d);
+    x.name = name; x.C = C; x.heads = heads; x.d = C / heads;
     x.gn = make_norm(name + ".norm", C);
     x.proj_in = make_linear(name + ".proj_in", C, C, true);
     const std::string tb = name + ".transformer_blocks.0";
@@ -1708,7 +1709,7 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
   // and V^T (head_dim -> multiple of 64, tokens -> multiple of 128); S = Q K^T and O = P V are batched GEMMs on the
   // tcgen05 kernel with a (masked) fp32 row softmax between them.  valid_k < 0: read m->ctx_len at launch time.
   auto mh_attention = [&](const Tensor& qsrc, int qcol, const Tensor& ksrc, int kcol, int vcol, int Tq, int Tk, int valid_k,
-                          int heads, int d, int dpad, Tensor* out, int Hh, int Ww, int Cc, int causal = 0) {
+                          int heads, int d, Tensor* out, int Hh, int Ww, int Cc, int causal = 0) {
     if (rc) return;
     if (PL == 3) {
       // fp32-accurate mode: tiled fp32 attention straight on the q / k / v channel windows of the split-f16 tensors
@@ -1725,80 +1726,37 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
       return;
     }
     const int NV = B * heads;
-    const int Tqp = Tq < 128 ? 128 : Tq, Tkp = Tk < 128 ? 128 : Tk;
+    MhAttnShape sh;
+    rc = mh_attention_shape(B, heads, Tq, Tk, d, &sh);
+    if (rc) return;
+    const int Tqp = sh.Tqp, Tkp = sh.Tkp, dpad = sh.dpad;
     Tensor qh = talloc(NV, 1, Tqp, dpad), kh = talloc(NV, 1, Tkp, dpad), vht = talloc(NV, 1, dpad, Tkp);
     Tensor oh = talloc(NV, 1, Tqp, dpad);
     *out = talloc(B, Hh, Ww, Cc);
-    if (Tqp % 128 || Tkp % 128 || (Tkp > 1024 && Tkp != 2048 && Tkp != 4096)) {
-      rc = B2E_UNSUPPORTED_SHAPE; set_error("unet: attention over %d x %d tokens is not supported", Tq, Tk); return;
-    }
+    // fused attention unless B2E_FLASH=0 or head_dim > 192: the score matrix never leaves the SM (csrc/flash_attn.cu)
     static const bool flash_on = !(getenv("B2E_FLASH") && atoi(getenv("B2E_FLASH")) == 0);
-    if (flash_on && dpad <= 192) {
-      // fused attention: the score matrix never leaves the SM (csrc/flash_attn.cu)
-      if (!dry) {
-        FlashPlan fp;
-        rc = flash_attn_plan_build(&fp, qh.p, kh.p, vht.p, oh.p, NV, Tqp, Tkp, dpad);
-        if (!rc) {
-          const float scale = 1.0f / sqrtf((float)d);
-          const Tensor q_ = qsrc, k_ = ksrc, o_ = *out;
-          const int qp = qsrc.C, kp = ksrc.C;
-          ops.push_back({[q_, qh, B, Tq, Tqp, qp, qcol, heads, d, dpad](cudaStream_t st) {
-                           return gather_heads_launch(q_.p, qh.p, B, Tq, Tqp, qp, qcol, heads, d, dpad, false, st); }, 3, 0.0, 4.0 * NV * Tqp * dpad, "gather q heads"});
-          ops.push_back({[k_, kh, B, Tk, Tkp, kp, kcol, heads, d, dpad](cudaStream_t st) {
-                           return gather_heads_launch(k_.p, kh.p, B, Tk, Tkp, kp, kcol, heads, d, dpad, false, st); }, 3, 0.0, 4.0 * NV * Tkp * dpad, "gather k heads"});
-          ops.push_back({[k_, vht, B, Tk, Tkp, kp, vcol, heads, d, dpad](cudaStream_t st) {
-                           return gather_heads_launch(k_.p, vht.p, B, Tk, Tkp, kp, vcol, heads, d, dpad, true, st); }, 3, 0.0, 4.0 * NV * Tkp * dpad, "gather V^T heads"});
-          ops.push_back({[m, fp, valid_k, scale, causal](cudaStream_t st) { return flash_attn_launch(fp, valid_k < 0 ? m->ctx_len : valid_k, scale, st, causal); },
-                         2, fp.flops, 0.0, "flash attention (tcgen05, S in TMEM)"});
-          ops.push_back({[oh, o_, B, Tq, Tqp, heads, d, dpad](cudaStream_t st) {
-                           return scatter_heads_launch(oh.p, o_.p, B, Tq, Tqp, o_.C, heads, d, dpad, st); }, 3, 0.0, 4.0 * B * Tq * heads * d, "merge heads"});
-          flops += fp.flops;
-        }
-      } else {
-        flops += 4.0 * NV * (double)Tqp * Tkp * dpad;
-      }
-      tfree(qh); tfree(kh); tfree(vht); tfree(oh);
-      return;
-    }
-    if (causal) { rc = B2E_UNSUPPORTED_SHAPE; set_error("unet: causal attention needs the fused attention kernel"); return; }
-    Tensor sc = talloc(NV, 1, Tqp, Tkp);   // materialised scores (B2E_FLASH=0 or head_dim > 192)
+    const bool fused = flash_on && dpad <= 192;
+    rc = mh_attention_check(sh, fused, causal, valid_k, valid_k < 0);
+    if (rc) return;
+    Tensor sc;
+    if (!fused) sc = talloc(NV, 1, Tqp, Tkp);   // materialised scores
     if (!dry) {
-      ConvDesc d1;
-      d1.s0.ptr = qh.p; d1.s0.C = dpad;
-      d1.N = NV; d1.H = 1; d1.W = Tqp; d1.ksize = 1; d1.stride = 1;
-      d1.w_packed = kh.p; d1.b_batch_rows = Tkp; d1.b_pitch = dpad; d1.Cout = Tkp; d1.out_f16 = sc.p;
-      ConvPlan p1;
-      rc = conv_plan_build(&p1, d1);
-      ConvDesc d2;
-      d2.s0.ptr = sc.p; d2.s0.C = Tkp;
-      d2.N = NV; d2.H = 1; d2.W = Tqp; d2.ksize = 1; d2.stride = 1;
-      d2.w_packed = vht.p; d2.b_batch_rows = dpad; d2.b_pitch = Tkp; d2.Cout = dpad; d2.out_f16 = oh.p;
-      ConvPlan p2;
-      if (!rc) rc = conv_plan_build(&p2, d2);
-      if (!rc) {
-        const float scale = 1.0f / sqrtf((float)d);
-        const int64_t rows = (int64_t)NV * Tqp;
-        const Tensor q_ = qsrc, k_ = ksrc, o_ = *out;
-        const int qp = qsrc.C, kp = ksrc.C;
-        ops.push_back({[q_, qh, B, Tq, Tqp, qp, qcol, heads, d, dpad](cudaStream_t st) {
-                         return gather_heads_launch(q_.p, qh.p, B, Tq, Tqp, qp, qcol, heads, d, dpad, false, st); }, 3, 0.0, 4.0 * NV * Tqp * dpad, "gather q heads"});
-        ops.push_back({[k_, kh, B, Tk, Tkp, kp, kcol, heads, d, dpad](cudaStream_t st) {
-                         return gather_heads_launch(k_.p, kh.p, B, Tk, Tkp, kp, kcol, heads, d, dpad, false, st); }, 3, 0.0, 4.0 * NV * Tkp * dpad, "gather k heads"});
-        ops.push_back({[k_, vht, B, Tk, Tkp, kp, vcol, heads, d, dpad](cudaStream_t st) {
-                         return gather_heads_launch(k_.p, vht.p, B, Tk, Tkp, kp, vcol, heads, d, dpad, true, st); }, 3, 0.0, 4.0 * NV * Tkp * dpad, "gather V^T heads"});
-        ops.push_back({[p1](cudaStream_t st) { return conv_launch(p1, ConvEpilogue{}, st); }, 0, p1.flops, 0.0, "attention QK^T (heads batched)"});
-        ops.push_back({[m, sc, rows, Tkp, valid_k, scale](cudaStream_t st) {
-                         return softmax_rows_masked_launch(sc.p, rows, Tkp, valid_k < 0 ? m->ctx_len : valid_k, scale, st); },
-                       3, 0.0, 4.0 * rows * Tkp, "softmax"});
-        ops.push_back({[p2](cudaStream_t st) { return conv_launch(p2, ConvEpilogue{}, st); }, 0, p2.flops, 0.0, "attention PV (heads batched)"});
-        ops.push_back({[oh, o_, B, Tq, Tqp, heads, d, dpad](cudaStream_t st) {
-                         return scatter_heads_launch(oh.p, o_.p, B, Tq, Tqp, o_.C, heads, d, dpad, st); }, 3, 0.0, 4.0 * B * Tq * heads * d, "merge heads"});
-        flops += p1.flops + p2.flops;
-      }
+      MhAttnArgs aa;
+      aa.q = qsrc.p; aa.q_pitch = qsrc.C; aa.q_col = qcol;
+      aa.kv = ksrc.p; aa.kv_pitch = ksrc.C; aa.k_col = kcol; aa.v_col = vcol;
+      aa.out = out->p; aa.out_pitch = out->C;
+      aa.B = B; aa.Tq = Tq; aa.Tk = Tk; aa.heads = heads; aa.d = d;
+      aa.valid_k = valid_k; aa.valid_k_live = valid_k < 0 ? &m->ctx_len : nullptr; aa.causal = causal;
+      aa.qh = qh.p; aa.kh = kh.p; aa.vht = vht.p; aa.oh = oh.p; aa.sc = fused ? nullptr : sc.p;
+      std::vector<AttnOp> aops;
+      rc = mh_attention_ops(aa, fused, flash_attn_default_warps(), &aops);
+      for (const AttnOp& o : aops) { ops.push_back({o.fn, o.kind, o.flops, o.bytes, o.desc}); flops += o.flops; }
     } else {
       flops += 4.0 * NV * (double)Tqp * Tkp * dpad;
     }
-    tfree(qh); tfree(kh); tfree(vht); tfree(sc); tfree(oh);
+    tfree(qh); tfree(kh); tfree(vht);
+    if (!fused) tfree(sc);
+    tfree(oh);
   };
   if (m->clip) {
     // ---- CLIP text encoder: ids (B, L <= 128) -> (B, 1, 128, D) f16 token rows (rows >= L zero, masked as keys)
@@ -1818,7 +1776,7 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
       lnorm(L.ln1, x, &a);
       conv(L.qkv, a, nullptr, 1, ConvEpilogue{}, &qkv, nullptr, nullptr, nullptr, false);
       tfree(a);
-      mh_attention(qkv, 0, qkv, D, 2 * D, kCtxPad, kCtxPad, -1, heads, d, pad64(d), &o, 1, kCtxPad, D, 1);
+      mh_attention(qkv, 0, qkv, D, 2 * D, kCtxPad, kCtxPad, -1, heads, d, &o, 1, kCtxPad, D, 1);
       tfree(qkv);
       conv(L.out, o, nullptr, 1, ConvEpilogue{}, &x1, nullptr, &x, nullptr, false);
       tfree(o); tfree(x);
@@ -1897,7 +1855,6 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
         o = talloc(B, h.H, h.W, a.P, a.C);
         const int heads = c.attention_head_dim > 0 ? a.C / c.attention_head_dim : 1;
         const int T = h.H * h.W, C = a.P;   // C: padded width of q / k / v (zero tail: no effect on Q K^T, zero rows of V^T)
-        const ConvGeom gq = conv_geometry(B, h.H, h.W, T);
         if (PL == 3) {
           // fp32-accurate mode: fp32 attention core on the CUDA cores over the split-f16 q | k | v planes
           if (!dry) {
@@ -1912,38 +1869,16 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
             }
           }
           flops += 4.0 * B * (double)T * T * a.C;
-        } else if (heads == 1 && T % 128 == 0 && (T <= 1024 || T == 2048 || T == 4096) && gq.Nt == 1) {
+        } else if (heads == 1 && single_head_attention_fits(B, h.H, h.W)) {
           // tensor-core attention: S = Q K^T and O = P V are batched GEMMs on the tcgen05 kernel (the per-image
           // B operand is read straight from the qkv tensor / a transposed copy of V); softmax in fp32 between
           Tensor sc = talloc(B, h.H, h.W, T);
           Tensor vt = talloc(B, 1, C, T);   // V^T: [N][C][T]
           sv.sc = sc;                       // P after the in-place softmax
           if (!dry) {
-            ConvDesc d1;
-            d1.s0.ptr = qkv.p; d1.s0.C = C; d1.s0.pitch = 3 * C;        // Q = channel window [0,C) of qkv
-            d1.N = B; d1.H = h.H; d1.W = h.W; d1.ksize = 1; d1.stride = 1;
-            d1.w_packed = qkv.p + C; d1.b_batch_rows = T; d1.b_pitch = 3 * C;   // K rows of image n
-            d1.Cout = T; d1.out_f16 = sc.p;
-            ConvPlan p1;
-            rc = conv_plan_build(&p1, d1);
-            ConvDesc d2;
-            d2.s0.ptr = sc.p; d2.s0.C = T;                               // P
-            d2.N = B; d2.H = h.H; d2.W = h.W; d2.ksize = 1; d2.stride = 1;
-            d2.w_packed = vt.p; d2.b_batch_rows = C; d2.b_pitch = T;     // V^T rows of image n
-            d2.Cout = C; d2.out_f16 = o.p;
-            ConvPlan p2;
-            if (!rc) rc = conv_plan_build(&p2, d2);
-            if (!rc) {
-              const float scale = 1.0f / sqrtf((float)a.C);
-              const int64_t rows = (int64_t)B * T;
-              ops.push_back({[p1](cudaStream_t st) { return conv_launch(p1, ConvEpilogue{}, st); }, 0, p1.flops, 0.0});
-              ops.push_back({[sc, rows, T, scale](cudaStream_t st) { return softmax_rows_launch(sc.p, rows, T, scale, st); },
-                             3, 0.0, 4.0 * rows * T});
-              ops.push_back({[qkv, vt, B, T, C](cudaStream_t st) { return transpose_v_launch(qkv.p, vt.p, B, T, C, st); },
-                             3, 0.0, 4.0 * B * T * C});
-              ops.push_back({[p2](cudaStream_t st) { return conv_launch(p2, ConvEpilogue{}, st); }, 0, p2.flops, 0.0});
-              flops += p1.flops + p2.flops;
-            }
+            std::vector<AttnOp> aops;
+            rc = single_head_attention_ops(qkv.p, sc.p, vt.p, o.p, B, h.H, h.W, C, a.C, &aops);
+            for (const AttnOp& op : aops) { ops.push_back({op.fn, op.kind, op.flops, op.bytes, op.desc}); flops += op.flops; }
           } else {
             flops += 4.0 * B * (double)T * T * C;
           }
@@ -1955,7 +1890,7 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
           const int d = a.C / heads;
           tfree(o);
           Tensor o2;
-          mh_attention(qkv, 0, qkv, a.P, 2 * a.P, T, T, T, heads, d, pad64(d), &o2, h.H, h.W, a.P);
+          mh_attention(qkv, 0, qkv, a.P, 2 * a.P, T, T, T, heads, d, &o2, h.H, h.W, a.P);
           o2.Cr = a.C;
           o = o2;
         } else if (heads > 1 && (a.C / heads) % 8 == 0 && a.C / heads <= 64 && T % 128 == 0 && T <= 1024 &&
@@ -2026,7 +1961,7 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
         lnorm(x.ln1, t0, &l1);
         conv(x.qkv1, l1, nullptr, 1, ConvEpilogue{}, &qkv, nullptr, nullptr, nullptr, false);
         tfree(l1);
-        mh_attention(qkv, 0, qkv, C, 2 * C, T, T, T, x.heads, x.d, x.dpad, &o1, h.H, h.W, C);
+        mh_attention(qkv, 0, qkv, C, 2 * C, T, T, T, x.heads, x.d, &o1, h.H, h.W, C);
         tfree(qkv);
         conv(x.out1, o1, nullptr, 1, ConvEpilogue{}, &t1, nullptr, &t0, nullptr, false);
         tfree(o1); tfree(t0);
@@ -2035,7 +1970,7 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
         conv(x.q2, l2, nullptr, 1, ConvEpilogue{}, &q2, nullptr, nullptr, nullptr, false);
         tfree(l2);
         conv(x.kv2, ctxp, nullptr, 1, ConvEpilogue{}, &kv, nullptr, nullptr, nullptr, false);
-        mh_attention(q2, 0, kv, 0, C, T, kCtxPad, -1, x.heads, x.d, x.dpad, &o2, h.H, h.W, C);
+        mh_attention(q2, 0, kv, 0, C, T, kCtxPad, -1, x.heads, x.d, &o2, h.H, h.W, C);
         tfree(q2); tfree(kv);
         conv(x.out2, o2, nullptr, 1, ConvEpilogue{}, &t2, nullptr, &t1, nullptr, false);
         tfree(o2); tfree(t1);

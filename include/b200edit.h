@@ -456,6 +456,31 @@ int b2e_conv2d_nhwc_f16(const void* x, const float* w, const float* bias, const 
 int b2e_upsample_conv3x3_nhwc_f16(const void* x, const float* w, const float* bias, void* out, int64_t N, int64_t H,
                                    int64_t W, int64_t Cin, int64_t Cout, void* stream);
 
+/* Test hook for the attention kernels: out = softmax(Q K^T / sqrt(head_dim), keys < valid_k, causal) V per (image, head),
+ * computed by the engine's own launch sequence of the named path (padding rules, shape checks, plans, launch order).
+ * Operands are channel windows of 16-bit (b2e_act_dtype) token-major tensors, as the UNet hands them over:
+ *   q   rows [B][H*W] of q_pitch channels, head h at channels q_col + h*head_dim;
+ *   kv  rows [B][Tk] of kv_pitch channels, key head h at k_col + h*head_dim, value head h at v_col + h*head_dim;
+ *   out rows [B][H*W] of out_pitch channels; the tail [heads*head_dim, out_pitch) is written with zeros.
+ * The fp32 paths read and write split tensors of the fp32-accurate mode: every row is [hi | lo | hi] planes of `pitch`
+ * channels each (value hi + lo); the pitches and columns above are then per plane.
+ * The single-head, CUDA-core and fp32 split paths take one packed tensor (q == kv, q_pitch = kv_pitch = 3 * out_pitch,
+ * columns 0 / out_pitch / 2 * out_pitch) and no key mask (Tk = H*W = valid_k).  causal (query i sees keys <= i) is
+ * fused-only; softmax_warps (4 or 8) selects the fused kernel's softmax layout.  Every unsupported combination returns
+ * an error before anything is launched.  Allocates temporaries itself and synchronises. */
+enum {
+  B2E_ATTN_FUSED = 0,         /* tcgen05 flash kernel (head_dim <= 192) between head gather / scatter */
+  B2E_ATTN_MATERIALISED = 1,  /* batched Q K^T GEMM -> 16-bit scores -> masked row softmax -> P V GEMM */
+  B2E_ATTN_SINGLE_HEAD = 2,   /* single-head GEMM attention straight from the qkv tensor */
+  B2E_ATTN_CUDA_CORE = 3,     /* attention_kernel on the CUDA cores */
+  B2E_ATTN_FP32_SPLIT = 4,    /* fp32-accurate attention_split_kernel */
+  B2E_ATTN_FP32_TILED = 5     /* fp32-accurate attention_split_tiled_kernel (online softmax over key tiles) */
+};
+int b2e_attention_f16(const void* q, int64_t q_pitch, int64_t q_col, const void* kv, int64_t kv_pitch, int64_t k_col,
+                      int64_t v_col, void* out, int64_t out_pitch, int64_t B, int64_t H, int64_t W, int64_t Tk,
+                      int64_t valid_k, int64_t heads, int64_t head_dim, int causal, int path, int softmax_warps,
+                      void* stream);
+
 /* Test hook for the face parser's label kernel: x (N,Hi,Wi,planes*P) 16-bit NHWC (b2e_act_dtype; planes = 3: split
  * [hi | lo | hi] channel planes, value hi + lo) -> labels int64 (N,S,S), the argmax over the first K channels of the
  * align_corners bilinear upsampling to S x S. */
