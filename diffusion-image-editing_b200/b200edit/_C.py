@@ -53,12 +53,12 @@ class VQDecConfig(C.Structure):
 class VQEncConfig(C.Structure):
     _fields_ = [("sample_size", C.c_int32), ("in_channels", C.c_int32), ("latent_channels", C.c_int32),
                 ("n_blocks", C.c_int32), ("block_out_channels", C.c_int32 * 8), ("layers_per_block", C.c_int32),
-                ("norm_num_groups", C.c_int32), ("norm_eps", C.c_float), ("double_z", C.c_int32)]
+                ("norm_num_groups", C.c_int32), ("norm_eps", C.c_float), ("double_z", C.c_int32), ("precision", C.c_int32)]
 
 
 class ClipConfig(C.Structure):
     _fields_ = [("vocab_size", C.c_int32), ("hidden_size", C.c_int32), ("intermediate_size", C.c_int32),
-                ("num_layers", C.c_int32), ("num_heads", C.c_int32), ("max_positions", C.c_int32)]
+                ("num_layers", C.c_int32), ("num_heads", C.c_int32), ("max_positions", C.c_int32), ("precision", C.c_int32)]
 
 
 class ResNetConfig(C.Structure):

@@ -2,7 +2,11 @@
 (``encode_text`` / ``prep_text``, src/diffusion_utils.py:34-52) = ``transformers.CLIPTextModel(...).last_hidden_state``.
 Token + position embedding, pre-LayerNorm transformer layers (causal multi-head self-attention on the fused tcgen05
 attention kernel, quick-GELU MLP, every linear layer on the implicit-GEMM kernel), final LayerNorm - in libb200edit.so.
-Parameters load from a transformers ``state_dict`` unchanged.  The tokenizer (BPE files) stays the caller's."""
+Parameters load from a transformers ``state_dict`` unchanged.  The tokenizer (BPE files) stays the caller's.
+
+``precision="fp32"`` builds the fp32-accurate forward (split hi + lo 16-bit operands, three products per GEMM; the
+embedding sum, LayerNorm, quick-GELU and the causal attention in fp32 on the CUDA cores), the text conditioning an
+fp32-accurate noise predictor wants; ``None`` (default) is the build's 16-bit type."""
 from __future__ import annotations
 
 from types import SimpleNamespace
@@ -26,8 +30,9 @@ class TextEncoderOutput(tuple):
 
 class CLIPTextModel(Engine):
     def __init__(self, vocab_size=49408, hidden_size=768, intermediate_size=3072, num_hidden_layers=12,
-                 num_attention_heads=12, max_position_embeddings=77, max_batch=2, device="cuda"):
+                 num_attention_heads=12, max_position_embeddings=77, max_batch=2, device="cuda", precision=None):
         _C.require_device()
+        self.precision, precision_cfg = _C.resolve_precision(precision, type(self).__name__)
         self.config = SimpleNamespace(vocab_size=vocab_size, hidden_size=hidden_size, intermediate_size=intermediate_size,
                                       num_hidden_layers=num_hidden_layers, num_attention_heads=num_attention_heads,
                                       max_position_embeddings=max_position_embeddings, in_channels=1, sample_size=8,
@@ -35,6 +40,7 @@ class CLIPTextModel(Engine):
         cfg = ClipConfig()
         cfg.vocab_size, cfg.hidden_size, cfg.intermediate_size = vocab_size, hidden_size, intermediate_size
         cfg.num_layers, cfg.num_heads, cfg.max_positions = num_hidden_layers, num_attention_heads, max_position_embeddings
+        cfg.precision = precision_cfg
         self._create(lib.b2e_clip_create, cfg, max_batch, device)
 
     def load_state_dict(self, sd, strict=True):

@@ -542,7 +542,8 @@ def upsample_conv3x3_nhwc_f16(x, w, bias):
     return out
 
 
-ATTENTION_PATHS = {"fused": 0, "materialised": 1, "single_head": 2, "cuda_core": 3, "fp32_split": 4, "fp32_tiled": 5}
+ATTENTION_PATHS = {"fused": 0, "materialised": 1, "single_head": 2, "cuda_core": 3, "fp32_split": 4, "fp32_tiled": 5,
+                   "fp32_tiled_causal": 6}
 
 
 def split_planes(x: torch.Tensor) -> torch.Tensor:
@@ -563,7 +564,7 @@ def attention_f16(q, kv, *, hw, heads, head_dim, k_col, v_col, out_pitch, q_col=
                   path="fused", softmax_warps=8, out=None):
     """Test hook for the attention paths (include/b200edit.h, b2e_attention_f16): softmax(Q K^T / sqrt(head_dim)) V over
     channel windows, keys >= valid_k (default: all) masked, through the engine's own launch sequence of `path`
-    (one of ATTENTION_PATHS).
+    (one of ATTENTION_PATHS; "fp32_tiled_causal" is the causal instantiation of "fp32_tiled" and needs causal=True).
 
     q (B, H*W, q_pitch) and kv (B, Tk, kv_pitch) are token-major tensors in `act_dtype()`; the "fp32_*" paths take fp32
     tensors and split them into [hi | lo | hi] planes here (q is kv: one packed tensor).  Returns `out` (B, H*W, out_pitch)

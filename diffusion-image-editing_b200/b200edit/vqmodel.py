@@ -5,7 +5,9 @@ post_quant_conv and the decoder run in libb200edit.so (bf16 tcgen05 implicit-GEM
 ``decode`` is forward-only by default (post-loop decoding of the final sample and of the x0-prediction history);
 ``enable_grad()`` makes it an autograd node backed by the native decoder dgrad, which is what guidance THROUGH the
 decoder (AttrFunc.apply with no_grad=False) uses.  ``with_encoder=True`` adds the native encoder + quant_conv
-(``vqvae.encode(img).latents`` / ``vae.encode(img).latent_dist.mode()``, src/diffusion_classes.py:27-30, 55-60)."""
+(``vqvae.encode(img).latents`` / ``vae.encode(img).latent_dist.mode()``, src/diffusion_classes.py:27-30, 55-60).
+``precision`` selects the decoder's operands, ``encoder_precision`` the encoder's (``"fp32"``: the fp32-accurate split
+forward; ``None``: the build's 16-bit type - it does not follow ``precision``)."""
 from __future__ import annotations
 
 from types import SimpleNamespace
@@ -24,7 +26,8 @@ class _EncoderEngine(Engine):
     """diffusers ``Encoder`` + ``quant_conv`` on the engine (b2e_vqenc_create): image (B, C, S, S) -> (B, Q, s, s)."""
 
     def __init__(self, image_size, in_channels, latent_channels, block_out_channels, layers_per_block, norm_num_groups,
-                 norm_eps, double_z, max_batch, device):
+                 norm_eps, double_z, max_batch, device, precision=None):
+        self.precision, precision_cfg = _C.resolve_precision(precision, "encoder")
         n = len(block_out_channels)
         self.image_size, self.q = image_size, latent_channels * (2 if double_z else 1)
         self.out_size = image_size >> (n - 1)
@@ -35,6 +38,7 @@ class _EncoderEngine(Engine):
             cfg.block_out_channels[i] = block_out_channels[i]
         cfg.layers_per_block, cfg.norm_num_groups, cfg.norm_eps = layers_per_block, norm_num_groups, norm_eps
         cfg.double_z = int(double_z)
+        cfg.precision = precision_cfg      # 1: fp32-accurate encode (split-f16 operands); quant_conv is fp32 either way
         self._create(lib.b2e_vqenc_create, cfg, max_batch, device)
 
     def _out_shape(self, B):
@@ -77,9 +81,11 @@ class VQModel(Engine):
 
     def __init__(self, latent_channels=3, out_channels=3, block_out_channels=(128, 256, 512), layers_per_block=2,
                  norm_num_groups=32, norm_eps=1e-6, num_vq_embeddings=8192, sample_size=64, max_batch=8,
-                 device="cuda", with_encoder=False, precision=None):
+                 device="cuda", with_encoder=False, precision=None, encoder_precision=None):
         _C.require_device()
         self.precision, self._precision_cfg = _C.resolve_precision(precision, type(self).__name__)
+        # the encoder's own precision (None: the 16-bit type, whatever the decoder's), checked with or without an encoder
+        self.encoder_precision = _C.resolve_precision(encoder_precision, f"{type(self).__name__} encoder")[0]
         n = len(block_out_channels)
         self._enc = None
         self.config = SimpleNamespace(latent_channels=latent_channels, out_channels=out_channels,
@@ -98,7 +104,8 @@ class VQModel(Engine):
         self._create(lib.b2e_vqdec_create, cfg, max_batch, device)
         if with_encoder:
             self._enc = _EncoderEngine(self.out_size, out_channels, latent_channels, block_out_channels, layers_per_block,
-                                       norm_num_groups, norm_eps, num_vq_embeddings == 0, max_batch, device)
+                                       norm_num_groups, norm_eps, num_vq_embeddings == 0, max_batch, device,
+                                       precision=encoder_precision)
 
     # ---- parameters: "encoder.*" / "quant_conv.*" belong to the encoder engine (ignored when there is none)
     def load_state_dict(self, sd, strict=True):
@@ -190,11 +197,11 @@ class AutoencoderKL(VQModel):
 
     def __init__(self, latent_channels=4, out_channels=3, block_out_channels=(128, 256, 512, 512), layers_per_block=2,
                  norm_num_groups=32, norm_eps=1e-6, sample_size=64, max_batch=8, device="cuda", with_encoder=False,
-                 precision=None):
+                 precision=None, encoder_precision=None):
         super().__init__(latent_channels=latent_channels, out_channels=out_channels, block_out_channels=block_out_channels,
                          layers_per_block=layers_per_block, norm_num_groups=norm_num_groups, norm_eps=norm_eps,
                          num_vq_embeddings=0, sample_size=sample_size, max_batch=max_batch, device=device,
-                         with_encoder=with_encoder, precision=precision)
+                         with_encoder=with_encoder, precision=precision, encoder_precision=encoder_precision)
 
     def encode(self, x):
         """``vae.encode(img).latent_dist`` (the reference takes ``.mode()``, src/diffusion_classes.py:29)."""

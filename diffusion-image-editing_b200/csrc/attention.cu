@@ -137,7 +137,11 @@ extern "C" int b2e_attention_f16(const void* q, int64_t q_pitch, int64_t q_col, 
                                  int64_t valid_k, int64_t heads, int64_t head_dim, int causal, int path, int softmax_warps,
                                  void* stream) {
   B2E_REQUIRE(q && kv && out, B2E_INVALID_ARG, "attention: null pointer");
-  B2E_REQUIRE(path >= B2E_ATTN_FUSED && path <= B2E_ATTN_FP32_TILED, B2E_INVALID_ARG, "attention: unknown path %d", path);
+  B2E_REQUIRE(path >= B2E_ATTN_FUSED && path <= B2E_ATTN_FP32_TILED_CAUSAL, B2E_INVALID_ARG, "attention: unknown path %d", path);
+  // path 6 is the causal instantiation of path 5's kernel: without causal = 1 it names no path
+  B2E_REQUIRE(path != B2E_ATTN_FP32_TILED_CAUSAL || causal, B2E_INVALID_ARG,
+              "attention: path %d with causal = 0 is an unknown path (the non-causal fp32 tiled kernel is path %d)", path,
+              (int)B2E_ATTN_FP32_TILED);
   constexpr int64_t kMax = 1 << 30;
   B2E_REQUIRE(B >= 1 && H >= 1 && W >= 1 && Tk >= 1 && heads >= 1 && head_dim >= 1 && B * H * W < kMax && B * Tk < kMax &&
               heads * head_dim < kMax, B2E_INVALID_ARG, "attention: empty or oversized shape");
@@ -147,7 +151,8 @@ extern "C" int b2e_attention_f16(const void* q, int64_t q_pitch, int64_t q_col, 
   B2E_REQUIRE(q_col >= 0 && k_col >= 0 && v_col >= 0 && q_col + C <= q_pitch && k_col + C <= kv_pitch && v_col + C <= kv_pitch &&
               C <= out_pitch && q_pitch < kMax && kv_pitch < kMax && out_pitch < kMax, B2E_INVALID_ARG,
               "attention: channel windows of %lld channels do not fit the pitches", (long long)C);
-  B2E_REQUIRE(!causal || path == B2E_ATTN_FUSED, B2E_UNSUPPORTED_SHAPE, "attention: causal attention needs the fused path");
+  B2E_REQUIRE(!causal || path == B2E_ATTN_FUSED || path == B2E_ATTN_FP32_TILED_CAUSAL, B2E_UNSUPPORTED_SHAPE,
+              "attention: causal attention needs the fused path or the causal fp32 tiled path");
   B2E_REQUIRE(softmax_warps == 4 || softmax_warps == 8, B2E_INVALID_ARG, "attention: %d softmax warps (4 or 8)", softmax_warps);
   // the single-head, CUDA-core and fp32 split kernels read q | k | v blocks of one packed tensor [B][T][3P] and have no
   // key mask (self-attention over all tokens)
@@ -172,10 +177,10 @@ extern "C" int b2e_attention_f16(const void* q, int64_t q_pitch, int64_t q_col, 
     cudaStreamSynchronize(st);
     return rc;
   }
-  if (path == B2E_ATTN_FP32_TILED) {
+  if (path == B2E_ATTN_FP32_TILED || path == B2E_ATTN_FP32_TILED_CAUSAL) {
     rc = attention_split_tiled_launch((const f16*)q, (int)q_pitch, (int)q_col, (const f16*)kv, (int)kv_pitch, (int)k_col, (int)v_col,
                                       (f16*)out, (int)out_pitch, (int)C, (int)B, (int)Tq, (int)Tk, (int)valid_k, (int)heads,
-                                      (int)head_dim, st);
+                                      (int)head_dim, st, path == B2E_ATTN_FP32_TILED_CAUSAL);
     cudaStreamSynchronize(st);
     return rc;
   }

@@ -109,10 +109,12 @@ struct b2e_unet {
   // post_quant_conv (one CUDA-core kernel) -> conv_in; output at sample_size << (n_blocks - 1)
   bool decoder = false;
   // VQ / KL encoder mode (b2e_vqenc_create): image -> conv_in -> down blocks -> mid block -> GroupNorm -> SiLU -> conv_out
-  // (enc_q channels: latent, or 2 x latent moments) -> 1x1 quant_conv in fp32; output at sample_size >> (n_blocks - 1)
+  // (enc_q channels: latent, or 2 x latent moments) -> 1x1 quant_conv in fp32; output at sample_size >> (n_blocks - 1).
+  // Split mode (encoder precision 1, PL = 3): the fp32-accurate forward of the decoder's split mode; quant_conv stays fp32
   bool encoder = false;
   // CLIP text encoder mode (b2e_clip_create): transformers CLIPTextModel - token + position embedding, pre-LN
-  // transformer layers (causal 12-head self-attention on the fused kernel, quick-GELU MLP), final LayerNorm.
+  // transformer layers (causal 12-head self-attention on the fused kernel, quick-GELU MLP), final LayerNorm.  Split mode
+  // (ccfg.precision == 1, PL = 3): the fp32-accurate forward, causal attention on the tiled fp32 kernel.
   // prep_text / encode_text, src/diffusion_utils.py:34-52
   bool clip = false;
   b2e_clip_config ccfg{};
@@ -477,12 +479,19 @@ int build_model_encoder(b2e_unet* m) {
   const int nb = c.n_blocks, cin = c.in_channels, c0 = c.block_out_channels[0], Q = m->enc_q;
   m->in_im2col = true;
   {
+    // conv_in as a 1x1 convolution over the im2col input; split mode (PL = 3): [W_hi | W_hi | W_lo] x 2^10 over the
+    // [hi | lo | hi] planes of the im2col tensor, as the decoder's conv_in
     ConvL ci;
-    ci.cin = ci.cin_pad = kConvBlockK; ci.cout = c0; ci.k = 1; ci.cout_pad = conv_cout_pad(c0); ci.row_len = kConvBlockK;
+    const int PL = m->PL;
+    ci.cin = ci.cin_pad = kConvBlockK; ci.cout = c0; ci.k = 1; ci.cout_pad = conv_cout_pad(c0); ci.row_len = kConvBlockK * PL;
     ci.w = m->dmalloc<f16>((size_t)ci.cout_pad * ci.row_len);
     ci.b = m->dmalloc<float>(ci.cout_pad);
-    m->add_param("encoder.conv_in.weight", (int64_t)c0 * cin * 9, (int64_t)cin * 9, [ci, cin](const float* src, cudaStream_t st) {
-      return conv_pack_weight(src, ci.w, ci.cout, cin, 3, cin, ci.row_len, 0, st);
+    m->add_param("encoder.conv_in.weight", (int64_t)c0 * cin * 9, (int64_t)cin * 9, [ci, cin, PL](const float* src, cudaStream_t st) {
+      const float ws = PL == 3 ? b2e_unet::kSplitWScale : 1.f;
+      int rc = conv_pack_weight(src, ci.w, ci.cout, cin, 3, cin, ci.row_len, 0, st, 0, 0, 0, ws);
+      if (!rc && PL == 3) rc = conv_pack_weight(src, ci.w, ci.cout, cin, 3, cin, ci.row_len, kConvBlockK, st, 0, 0, 0, ws);
+      if (!rc && PL == 3) rc = conv_pack_weight(src, ci.w, ci.cout, cin, 3, cin, ci.row_len, 2 * kConvBlockK, st, 0, 0, 1, ws);
+      return rc;
     });
     m->add_f32("encoder.conv_in.bias", ci.b, c0, (int64_t)cin * 9);
     m->conv_in = ci;
@@ -1713,15 +1722,16 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
     if (rc) return;
     if (PL == 3) {
       // fp32-accurate mode: tiled fp32 attention straight on the q / k / v channel windows of the split-f16 tensors
-      if (causal) { rc = B2E_UNSUPPORTED_SHAPE; set_error("unet: causal attention is not available in the fp32-accurate mode"); return; }
+      // (causal: the CLIP text encoder's self-attention, key tiles above the diagonal skipped)
       *out = talloc(B, Hh, Ww, Cc);
       flops += 4.0 * B * heads * (double)Tq * Tk * d;
       if (!dry) {
         const Tensor q_ = qsrc, k_ = ksrc, o_ = *out;
-        ops.push_back({[m, q_, k_, o_, B, qcol, kcol, vcol, Tq, Tk, valid_k, heads, d, Cc](cudaStream_t st) {
+        ops.push_back({[m, q_, k_, o_, B, qcol, kcol, vcol, Tq, Tk, valid_k, heads, d, Cc, causal](cudaStream_t st) {
                          return attention_split_tiled_launch(q_.p, q_.C, qcol, k_.p, k_.C, kcol, vcol, o_.p, o_.C, Cc, B, Tq, Tk,
-                                                             valid_k < 0 ? m->ctx_len : valid_k, heads, d, st); },
-                       2, 4.0 * B * heads * (double)Tq * Tk * d, 0.0, "attention (fp32, tiled, split-f16 operands)"});
+                                                             valid_k < 0 ? m->ctx_len : valid_k, heads, d, st, causal); },
+                       2, 4.0 * B * heads * (double)Tq * Tk * d, 0.0,
+                       causal ? "attention (fp32, tiled, causal, split-f16 operands)" : "attention (fp32, tiled, split-f16 operands)"});
       }
       return;
     }
@@ -1766,9 +1776,10 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
     Tensor x = talloc(B, 1, kCtxPad, D);
     if (!dry) {
       const Tensor xx = x;
-      ops.push_back({[m, xx, B, D](cudaStream_t st) {
-                       return clip_embed_launch(m->in_ids, m->tok_emb, m->pos_emb, xx.p, B, m->ctx_len, kCtxPad, D, m->ccfg.vocab_size, st); },
-                     3, 0.0, 6.0 * B * kCtxPad * D, "token + position embedding"});
+      ops.push_back({[m, xx, B, D, PL](cudaStream_t st) {
+                       return clip_embed_launch(m->in_ids, m->tok_emb, m->pos_emb, xx.p, B, m->ctx_len, kCtxPad, D, m->ccfg.vocab_size, st,
+                                                PL); },
+                     3, 0.0, (4.0 + 2.0 * PL) * B * kCtxPad * D, "token + position embedding"});
     }
     for (size_t li = 0; li < m->clayers.size() && !rc; ++li) {
       const b2e_unet::ClipL& L = m->clayers[li];
@@ -1785,8 +1796,8 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
       tfree(b2);
       if (!dry && !rc) {
         const Tensor ff = f1;
-        ops.push_back({[ff](cudaStream_t st) { return quick_gelu_launch(ff.p, ff.p, (int64_t)(ff.bytes / sizeof(f16)), st); }, 3, 0.0,
-                       2.0 * (double)ff.bytes, "quick_gelu"});
+        ops.push_back({[ff, PL](cudaStream_t st) { return quick_gelu_launch(ff.p, ff.p, (int64_t)(ff.bytes / sizeof(f16)), st, PL, ff.C); },
+                       3, 0.0, 2.0 * (double)ff.bytes, "quick_gelu"});
       }
       conv(L.fc2, f1, nullptr, 1, ConvEpilogue{}, &x2, nullptr, &x1, nullptr, false);
       tfree(f1); tfree(x1);
@@ -1796,8 +1807,8 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
     lnorm(m->clip_final_ln, x, &y);
     if (!dry && !rc) {
       const Tensor yy = y;
-      ops.push_back({[m, yy, B, D](cudaStream_t st) { return unpad_rows_f32_launch(yy.p, m->out_eps, B, m->ctx_len, kCtxPad, D, st); },
-                     3, 0.0, 6.0 * B * kCtxPad * D, "final hidden states -> fp32"});
+      ops.push_back({[m, yy, B, D, PL](cudaStream_t st) { return unpad_rows_f32_launch(yy.p, m->out_eps, B, m->ctx_len, kCtxPad, D, st, PL); },
+                     3, 0.0, (4.0 + 2.0 * PL) * B * kCtxPad * D, "final hidden states -> fp32"});
     }
     if (rc) return rc;
     return finish_forward_only(m, ops_fwd, ar.peak, ws_bytes, need, dry, flops, B);
@@ -2286,8 +2297,10 @@ int b2e_vqenc_create(const b2e_vqenc_config* cfg, int64_t max_batch, b2e_unet** 
     B2E_REQUIRE(ch % 8 == 0 && ch >= 32 && ch <= 1024 && ch % cfg->norm_num_groups == 0, B2E_UNSUPPORTED_SHAPE,
                 "vqenc_create: block_out_channels must be multiples of 8 and of norm_num_groups, 32..1024 (got %d)", ch);
   }
+  B2E_REQUIRE(cfg->precision == 0 || cfg->precision == 1, B2E_INVALID_ARG, "vqenc_create: precision must be 0 (f16) or 1 (fp32-accurate)");
   b2e_unet* m = new b2e_unet();
   m->encoder = true;
+  m->PL = cfg->precision == 1 ? 3 : 1;
   m->enc_q = cfg->latent_channels * (cfg->double_z ? 2 : 1);
   b2e_unet_config& u = m->cfg;
   u = b2e_unet_config{};
@@ -2308,8 +2321,10 @@ int b2e_clip_create(const b2e_clip_config* cfg, int64_t max_batch, b2e_unet** ou
               B2E_UNSUPPORTED_SHAPE, "clip_create: hidden / intermediate sizes must be multiples of 64, head_dim %% 8 == 0 and <= 192");
   B2E_REQUIRE(cfg->num_layers >= 1 && cfg->num_layers <= 64 && cfg->vocab_size >= 1 && cfg->max_positions >= 1 && cfg->max_positions <= 128,
               B2E_UNSUPPORTED_SHAPE, "clip_create: 1..64 layers, at most 128 positions");
+  B2E_REQUIRE(cfg->precision == 0 || cfg->precision == 1, B2E_INVALID_ARG, "clip_create: precision must be 0 (f16) or 1 (fp32-accurate)");
   b2e_unet* m = new b2e_unet();
   m->clip = true;
+  m->PL = cfg->precision == 1 ? 3 : 1;
   m->ccfg = *cfg;
   m->cfg = b2e_unet_config{};
   m->cfg.sample_size = 8; m->cfg.in_channels = 1; m->cfg.out_channels = 1; m->cfg.norm_num_groups = 1;

@@ -1251,10 +1251,11 @@ int layernorm_rows_launch(const f16* x, f16* y, const float* gamma, const float*
 }
 
 // ---- CLIP text encoder helpers
-// token + position embedding: ids int64 [B][L] -> x f16 [B][Lpad][D] (rows >= L zero)
+// (planes = 3: split-f16 rows [hi | lo | hi] of D channels each, value hi + lo, as layernorm_rows_split_kernel)
+// token + position embedding: ids int64 [B][L] -> x f16 [B][Lpad][D] (rows >= L zero); the sum is taken in fp32
 __global__ void __launch_bounds__(256) clip_embed_kernel(const int64_t* __restrict__ ids, const float* __restrict__ tok,
                                                          const float* __restrict__ pos, f16* __restrict__ out, int B, int L,
-                                                         int Lpad, int D8, int vocab) {
+                                                         int Lpad, int D8, int vocab, int planes) {
   pdl_wait();
   const int64_t total = (int64_t)B * Lpad * D8;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
@@ -1271,15 +1272,26 @@ __global__ void __launch_bounds__(256) clip_embed_kernel(const int64_t* __restri
       f[0] = t0.x + q0.x; f[1] = t0.y + q0.y; f[2] = t0.z + q0.z; f[3] = t0.w + q0.w;
       f[4] = t1.x + q1.x; f[5] = t1.y + q1.y; f[6] = t1.z + q1.z; f[7] = t1.w + q1.w;
     }
-    *reinterpret_cast<uint4*>(out + i * 8) = pack8(f);
+    const uint4 hi = pack8(f);
+    if (planes == 3) {
+      const int64_t r = i / D8;                    // token row
+      uint4* o = reinterpret_cast<uint4*>(out) + r * 3 * D8 + s;
+      float l[8];
+#pragma unroll
+      for (int j = 0; j < 8; ++j) l[j] = __fsub_rn(f[j], f16_to_float(float_to_f16(f[j])));
+      o[0] = hi; o[D8] = pack8(l); o[2 * D8] = hi;
+    } else {
+      *reinterpret_cast<uint4*>(out + i * 8) = hi;
+    }
   }
 }
 
 int clip_embed_launch(const int64_t* ids, const float* tok, const float* pos, f16* out, int B, int L, int Lpad, int D, int vocab,
-                      cudaStream_t st) {
-  B2E_REQUIRE(D % 8 == 0 && L <= Lpad, B2E_UNSUPPORTED_SHAPE, "clip_embed: bad shape");
+                      cudaStream_t st, int planes) {
+  B2E_REQUIRE(D % 8 == 0 && L <= Lpad && (planes == 1 || planes == 3), B2E_UNSUPPORTED_SHAPE, "clip_embed: bad shape");
   const int64_t total = (int64_t)B * Lpad * (D / 8);
-  launch_pdl(clip_embed_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, st, ids, tok, pos, out, B, L, Lpad, D / 8, vocab);
+  launch_pdl(clip_embed_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, st, ids, tok, pos, out, B, L, Lpad, D / 8, vocab,
+             planes);
   return check_launch("clip_embed");
 }
 
@@ -1295,30 +1307,66 @@ __global__ void __launch_bounds__(256) quick_gelu_kernel(const uint4* __restrict
   }
 }
 
-int quick_gelu_launch(const f16* in, f16* out, int64_t numel, cudaStream_t st) {
+// fp32-accurate quick_gelu on split rows of C channels per plane: hi + lo -> x * sigmoid(1.702 x) in fp32 (exact expf,
+// as the split SiLU) -> hi, lo, hi; in place capable
+__global__ void __launch_bounds__(256) quick_gelu_split_kernel(const uint4* __restrict__ in, uint4* __restrict__ out, int64_t rows,
+                                                               int C8) {
+  pdl_wait();
+  const int64_t total = rows * C8;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = i / C8;
+    const int c = (int)(i % C8);
+    const uint4* row = in + r * 3 * C8;
+    float f[8], l[8];
+    unpack8(row[c], f);
+    unpack8(row[C8 + c], l);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      const float v = f[j] + l[j];
+      f[j] = v / (1.f + expf(-1.702f * v));
+      l[j] = __fsub_rn(f[j], f16_to_float(float_to_f16(f[j])));
+    }
+    uint4* orow = out + r * 3 * C8;
+    const uint4 hi = pack8(f);
+    orow[c] = hi; orow[C8 + c] = pack8(l); orow[2 * C8 + c] = hi;
+  }
+}
+
+int quick_gelu_launch(const f16* in, f16* out, int64_t numel, cudaStream_t st, int planes, int C) {
   B2E_REQUIRE(numel % 8 == 0, B2E_UNSUPPORTED_SHAPE, "quick_gelu: numel %% 8 != 0");
+  if (planes == 3) {
+    B2E_REQUIRE(C > 0 && C % 8 == 0 && numel % (3 * (int64_t)C) == 0, B2E_UNSUPPORTED_SHAPE,
+                "quick_gelu: %lld elements are not split rows of 3 x %d channels", (long long)numel, C);
+    const int64_t rows = numel / (3 * (int64_t)C);
+    int64_t g = (rows * (C / 8) + 255) / 256;
+    if (g > kNumSMs * 16) g = kNumSMs * 16;
+    launch_pdl(quick_gelu_split_kernel, dim3((unsigned)g), dim3(256), 0, st, (const uint4*)in, (uint4*)out, rows, C / 8);
+    return check_launch("quick_gelu_split");
+  }
   int64_t g = (numel / 8 + 255) / 256;
   if (g > kNumSMs * 16) g = kNumSMs * 16;
   launch_pdl(quick_gelu_kernel, dim3((unsigned)g), dim3(256), 0, st, (const uint4*)in, (uint4*)out, numel / 8);
   return check_launch("quick_gelu");
 }
 
-// final LayerNorm output: rows [0, L) of every sequence, f16 [B][Lpad][D] -> fp32 [B][L][D]
+// final LayerNorm output: rows [0, L) of every sequence, f16 [B][Lpad][D] -> fp32 [B][L][D] (planes = 3: hi + lo)
 __global__ void __launch_bounds__(256) unpad_rows_f32_kernel(const f16* __restrict__ x, float* __restrict__ out, int B, int L,
-                                                             int Lpad, int D) {
+                                                             int Lpad, int D, int planes) {
   pdl_wait();
   const int64_t total = (int64_t)B * L * D;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
     const int d = (int)(i % D);
     const int l = (int)((i / D) % L);
     const int b = (int)(i / ((int64_t)D * L));
-    out[i] = f16_to_float(x[((int64_t)b * Lpad + l) * D + d]);
+    const f16* row = x + ((int64_t)b * Lpad + l) * planes * D;
+    out[i] = planes == 3 ? f16_to_float(row[d]) + f16_to_float(row[D + d]) : f16_to_float(row[d]);
   }
 }
 
-int unpad_rows_f32_launch(const f16* x, float* out, int B, int L, int Lpad, int D, cudaStream_t st) {
+int unpad_rows_f32_launch(const f16* x, float* out, int B, int L, int Lpad, int D, cudaStream_t st, int planes) {
+  B2E_REQUIRE(planes == 1 || planes == 3, B2E_INVALID_ARG, "unpad_rows_f32: planes must be 1 or 3");
   const int64_t total = (int64_t)B * L * D;
-  launch_pdl(unpad_rows_f32_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, st, x, out, B, L, Lpad, D);
+  launch_pdl(unpad_rows_f32_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, st, x, out, B, L, Lpad, D, planes);
   return check_launch("unpad_rows_f32");
 }
 
@@ -2169,7 +2217,8 @@ int attention_split_launch(const f16* qkv, f16* out, int N, int T, int C, int P,
 // tiles, O accumulated in registers).  q / k / v are channel windows of split-f16 tensors ([hi | lo | hi] planes):
 // q rows [n][tq] of a tensor with `q_plane` channels per plane at column q_col + h*d, k / v rows [n][tk] of a tensor with
 // `k_plane` channels per plane at columns k_col + h*d / v_col + h*d; out rows [n][tq] with o_plane channels per plane.
-// Block = (32 queries, head, image).
+// Block = (32 queries, head, image).  Causal (CLIP text encoder): query row r sees keys <= min(r, valid_k - 1), and the
+// key tiles wholly above the block's diagonal are skipped.
 constexpr int kTaQ = 32, kTaK = 32, kTaThreads = 256;
 struct TiledAttnArgs {
   const f16* q; const f16* kv; f16* out;
@@ -2179,6 +2228,7 @@ struct TiledAttnArgs {
   float scale;
 };
 
+template <bool Causal>
 __global__ void __launch_bounds__(kTaThreads) attention_split_tiled_kernel(TiledAttnArgs a) {
   pdl_wait();
   extern __shared__ __align__(16) uint8_t ta_smem[];
@@ -2211,7 +2261,9 @@ __global__ void __launch_bounds__(kTaThreads) attention_split_tiled_kernel(Tiled
 #pragma unroll
   for (int i = 0; i < kTaQ; ++i) ox[i] = oy[i] = 0.f;
   __syncthreads();
-  for (int k0 = 0; k0 < a.valid_k; k0 += kTaK) {
+  // causal: the block's last query row q0 + kTaQ - 1 sees no key past itself (kTaQ == kTaK: tiles align with the diagonal)
+  const int k_end = Causal ? min(a.valid_k, q0 + kTaQ) : a.valid_k;
+  for (int k0 = 0; k0 < k_end; k0 += kTaK) {
     // ---- K tile -> smem (fp32 = hi + lo)
     for (int i = tid; i < kTaK * d; i += kTaThreads) {
       const int k = i / d, c = i - k * d;
@@ -2230,11 +2282,14 @@ __global__ void __launch_bounds__(kTaThreads) attention_split_tiled_kernel(Tiled
         const float qv = qr[c];
         s0 += qv * k0r[c]; s1 += qv * k0r[ds + c]; s2 += qv * k0r[2 * ds + c]; s3 += qv * k0r[3 * ds + c];
       }
+      // keys this query row may see: the valid prefix, cut at the diagonal for causal attention (every row sees key 0,
+      // so the first tile gives each row a finite running maximum)
+      const int lim = Causal ? min(a.valid_k, q0 + q + 1) : a.valid_k;
       float* sr = S + q * (kTaK + 1) + kk;
-      sr[0] = k0 + kk < a.valid_k ? s0 : -INFINITY;
-      sr[1] = k0 + kk + 1 < a.valid_k ? s1 : -INFINITY;
-      sr[2] = k0 + kk + 2 < a.valid_k ? s2 : -INFINITY;
-      sr[3] = k0 + kk + 3 < a.valid_k ? s3 : -INFINITY;
+      sr[0] = k0 + kk < lim ? s0 : -INFINITY;
+      sr[1] = k0 + kk + 1 < lim ? s1 : -INFINITY;
+      sr[2] = k0 + kk + 2 < lim ? s2 : -INFINITY;
+      sr[3] = k0 + kk + 3 < lim ? s3 : -INFINITY;
     }
     __syncthreads();
     // ---- online softmax per query row (one warp handles 4 rows; lane = key)
@@ -2315,7 +2370,8 @@ __global__ void __launch_bounds__(kTaThreads) attention_split_tiled_kernel(Tiled
 }
 
 int attention_split_tiled_launch(const f16* q, int q_plane, int q_col, const f16* kv, int k_plane, int k_col, int v_col, f16* out,
-                                 int o_plane, int o_real, int N, int Tq, int Tk_rows, int valid_k, int heads, int d, cudaStream_t st) {
+                                 int o_plane, int o_real, int N, int Tq, int Tk_rows, int valid_k, int heads, int d, cudaStream_t st,
+                                 int causal) {
   B2E_REQUIRE(d % 2 == 0 && d >= 8 && d <= 512 && heads >= 1 && valid_k >= 1 && valid_k <= Tk_rows, B2E_UNSUPPORTED_SHAPE,
               "attention (fp32-accurate, tiled): unsupported head_dim %d / keys %d of %d", d, valid_k, Tk_rows);
   TiledAttnArgs a;
@@ -2324,12 +2380,21 @@ int attention_split_tiled_launch(const f16* q, int q_plane, int q_col, const f16
   a.q_img = (int64_t)Tq * 3 * q_plane; a.kv_img = (int64_t)Tk_rows * 3 * k_plane; a.o_img = (int64_t)Tq * 3 * o_plane;
   a.scale = 1.0f / sqrtf((float)d);
   const size_t smem = sizeof(float) * ((size_t)(kTaQ + kTaK) * (d + 1) + kTaQ * (kTaK + 1) + 3 * kTaQ);
-  static size_t attr = 0;
-  if (smem > attr) {
-    B2E_CUDA(cudaFuncSetAttribute(attention_split_tiled_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr = smem;
+  static size_t attr[2] = {0, 0};
+  const dim3 grid((Tq + kTaQ - 1) / kTaQ, heads, N);
+  if (causal) {
+    if (smem > attr[1]) {
+      B2E_CUDA(cudaFuncSetAttribute(attention_split_tiled_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      attr[1] = smem;
+    }
+    launch_pdl(attention_split_tiled_kernel<true>, grid, dim3(kTaThreads), smem, st, a);
+    return check_launch("attention_split_tiled_causal");
   }
-  launch_pdl(attention_split_tiled_kernel, dim3((Tq + kTaQ - 1) / kTaQ, heads, N), dim3(kTaThreads), smem, st, a);
+  if (smem > attr[0]) {
+    B2E_CUDA(cudaFuncSetAttribute(attention_split_tiled_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    attr[0] = smem;
+  }
+  launch_pdl(attention_split_tiled_kernel<false>, grid, dim3(kTaThreads), smem, st, a);
   return check_launch("attention_split_tiled");
 }
 

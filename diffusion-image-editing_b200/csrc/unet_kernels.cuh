@@ -101,11 +101,12 @@ int gather_heads_launch(const f16* src, f16* dst, int N, int Tsrc, int Tpad, int
 int scatter_heads_launch(const f16* oh, f16* out, int N, int T, int Tpad, int pitch, int heads, int d, int dpad, cudaStream_t st);
 int softmax_rows_masked_launch(f16* s, int64_t rows, int T, int valid, float scale, cudaStream_t st);
 
-// CLIP text encoder helpers
+// CLIP text encoder helpers (planes = 3: split-f16 rows [hi | lo | hi] of D (quick_gelu: C) channels per plane; quick_gelu's
+// numel then counts all three planes)
 int clip_embed_launch(const int64_t* ids, const float* tok, const float* pos, f16* out, int B, int L, int Lpad, int D, int vocab,
-                      cudaStream_t st);
-int quick_gelu_launch(const f16* in, f16* out, int64_t numel, cudaStream_t st);
-int unpad_rows_f32_launch(const f16* x, float* out, int B, int L, int Lpad, int D, cudaStream_t st);
+                      cudaStream_t st, int planes = 1);
+int quick_gelu_launch(const f16* in, f16* out, int64_t numel, cudaStream_t st, int planes = 1, int C = 0);
+int unpad_rows_f32_launch(const f16* x, float* out, int B, int L, int Lpad, int D, cudaStream_t st, int planes = 1);
 
 // backward helpers of the decoder (f16 NHWC gradients)
 int downsum2x_launch(const f16* dy, f16* dx, int N, int H, int W, int C, cudaStream_t st);
@@ -180,8 +181,10 @@ int attention_launch(const f16* qkv, f16* out, int N, int T, int C, int P, int h
 // fp32-accurate mode: qkv / out are split-f16 tensors ([hi | lo | hi] planes of 3P / P channels), arithmetic in fp32
 int attention_split_launch(const f16* qkv, f16* out, int N, int T, int C, int P, int heads, cudaStream_t st);
 // any sequence length (online softmax over key tiles); q / k / v are channel windows of split-f16 tensors with q_plane /
-// k_plane channels per plane; keys >= valid_k are masked; out has o_plane channels per plane (o_real of them written)
+// k_plane channels per plane; keys >= valid_k are masked; out has o_plane channels per plane (o_real of them written).
+// causal: query row r also sees no key past r (keys <= min(r, valid_k - 1)), a separate instantiation of the kernel
 int attention_split_tiled_launch(const f16* q, int q_plane, int q_col, const f16* kv, int k_plane, int k_col, int v_col, f16* out,
-                                 int o_plane, int o_real, int N, int Tq, int Tk_rows, int valid_k, int heads, int d, cudaStream_t st);
+                                 int o_plane, int o_real, int N, int Tq, int Tk_rows, int valid_k, int heads, int d, cudaStream_t st,
+                                 int causal = 0);
 
 }  // namespace b2e

@@ -8,6 +8,7 @@ from typing import Optional
 
 import torch
 
+from b200edit import _C
 from b200edit.scheduler import DDIMScheduler
 from b200edit.unet import DDPM256_CONFIG, LDM_CELEBAHQ_CONFIG, UNet2DModel
 from diffusion_classes import DDPM, LDM, SD  # noqa: F401
@@ -26,7 +27,7 @@ def create_diffusion_model(name: str, sample_clipping: bool = True, *, max_batch
                            vq_config: Optional[dict] = None, vq_state_dict: Optional[dict] = None, guidance_module=None,
                            decoder_grad: bool = True, tokenizer=None, text_encoder=None, precision: Optional[str] = None,
                            with_encoder: bool = True, text_encoder_config: Optional[dict] = None,
-                           text_encoder_state_dict: Optional[dict] = None):
+                           text_encoder_state_dict: Optional[dict] = None, encoder_precision: Optional[str] = None):
     """``name``: "ddpm" (google/ddpm-celebahq-256 layout), "sd" (Stable Diffusion 1.x layout: native conditional UNet
     + native KL decoder with gradient; ``vqvae=`` substitutes the vae, ``tokenizer=`` / ``text_encoder=`` are the
     caller's CLIP modules) or "ldm" (CompVis/ldm-celebahq-256 layout: native UNet on
@@ -34,7 +35,11 @@ def create_diffusion_model(name: str, sample_clipping: bool = True, *, max_batch
     (encode().latents / decode().sample, as in the reference's pipeline object); ``guidance_module=`` is the
     differentiable decoder used when guidance runs through decode).  ``precision="fp32"`` selects the fp32-accurate
     (split-f16) noise predictor (all three families) and VQ / KL decoder (forward only: guidance through the decoder uses the fp16 engine).  ``with_encoder`` (default) also builds the native VQ / KL encoder behind
-    ``LDM.encode`` / ``SD.encode``."""
+    ``LDM.encode`` / ``SD.encode``.  ``encoder_precision="fp32"`` selects the fp32-accurate native VQ / KL encoder and
+    native CLIP text encoder (the inputs of a real-image or prompt-conditioned edit); it does not apply to a caller's
+    ``vqvae=`` / ``text_encoder=`` and does not follow ``precision`` (``None``: the 16-bit type)."""
+    if encoder_precision is not None:
+        _C.resolve_precision(encoder_precision, "create_diffusion_model(encoder_precision)")   # refuse before building anything
     device = get_device()
     if name == "ddpm":
         unet = UNet2DModel(**(unet_config or DDPM256_CONFIG), max_batch=max_batch, device=device, precision=precision)
@@ -57,7 +62,7 @@ def create_diffusion_model(name: str, sample_clipping: bool = True, *, max_batch
             # native decoder: forward for the post-loop decoding of the sample / x0 history and, with
             # decoder_grad=True (default), the native dgrad for guidance THROUGH the decoder
             vqvae = VQModel(**(vq_config or LDM_VQ_CONFIG), max_batch=max_batch, device=device, with_encoder=with_encoder,
-                            precision=precision)
+                            precision=precision, encoder_precision=encoder_precision)
             if vq_state_dict is not None:
                 vqvae.load_state_dict(vq_state_dict)
             else:
@@ -91,7 +96,7 @@ def create_diffusion_model(name: str, sample_clipping: bool = True, *, max_batch
             unet.init_random(seed)
         if vqvae is None:
             vae = AutoencoderKL(**(vq_config or SD_VAE_CONFIG), max_batch=max_batch, device=device, with_encoder=with_encoder,
-                                precision=precision)
+                                precision=precision, encoder_precision=encoder_precision)
             if vq_state_dict is not None:
                 vae.load_state_dict(vq_state_dict)
             else:
@@ -114,7 +119,8 @@ def create_diffusion_model(name: str, sample_clipping: bool = True, *, max_batch
         # Prompts need both, precomputed text embeddings (2, 77, 768) need neither.
         if text_encoder is None:
             from b200edit.clip import SD15_CLIP_CONFIG, CLIPTextModel
-            text_encoder = CLIPTextModel(**(text_encoder_config or SD15_CLIP_CONFIG), max_batch=2, device=device)
+            text_encoder = CLIPTextModel(**(text_encoder_config or SD15_CLIP_CONFIG), max_batch=2, device=device,
+                                         precision=encoder_precision)
             if text_encoder_state_dict is not None:
                 text_encoder.load_state_dict(text_encoder_state_dict)
             else:

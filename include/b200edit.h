@@ -345,6 +345,9 @@ typedef struct {
   int32_t norm_num_groups;
   float norm_eps;
   int32_t double_z;          /* 1: AutoencoderKL (conv_out and quant_conv carry 2 * latent_channels) */
+  /* 0: 16-bit operands; 1: fp32-accurate forward (split hi + lo operands, three products per GEMM, GroupNorm / SiLU /
+   * attention in fp32), as b2e_vqdec_config.precision; the 1x1 quant_conv is fp32 either way */
+  int32_t precision;
 } b2e_vqenc_config;
 int b2e_vqenc_create(const b2e_vqenc_config* cfg, int64_t max_batch, b2e_unet** out);
 /* Gradient through the decoder (AttrFunc.apply with decode inside the graph, src/attr_functions.py:147-158):
@@ -360,7 +363,8 @@ int b2e_vqdec_backward(b2e_unet* m, const float* d_image, float* d_latent, int64
  * prep_text / encode_text, src/diffusion_utils.py:34-52: model.text_encoder(input_ids)[0] for the "" and prompt sequences,
  * i.e. transformers CLIPTextModel.last_hidden_state (token + position embedding, pre-LayerNorm transformer layers with
  * causal multi-head self-attention and a quick-GELU MLP, final LayerNorm).  Linear layers on the tcgen05 kernel (q/k/v fused
- * into one GEMM, residual adds as identity K segments), causal attention on the fused attention kernel.  Parameters by
+ * into one GEMM, residual adds as identity K segments), causal attention on the fused attention kernel (fp32-accurate
+ * mode: on the causal tiled fp32 kernel, B2E_ATTN_FP32_TILED_CAUSAL).  Parameters by
  * their transformers names ("text_model.embeddings.token_embedding.weight", "text_model.encoder.layers.0.self_attn.q_proj.weight", ...).
  * b2e_clip_forward: input_ids DEVICE int64 (B, seq_len <= max_positions) -> hidden (B, seq_len, hidden_size) fp32.  The
  * tokenizer (BPE vocabulary files) stays the caller's. */
@@ -371,6 +375,9 @@ typedef struct {
   int32_t num_layers;         /* 12 */
   int32_t num_heads;          /* 12 */
   int32_t max_positions;      /* 77 */
+  /* 0: 16-bit operands; 1: fp32-accurate forward (split hi + lo operands, three products per GEMM, embedding / LayerNorm /
+   * quick-GELU in fp32, causal attention on the tiled fp32 kernel), as b2e_unet_config.precision */
+  int32_t precision;
 } b2e_clip_config;
 int b2e_clip_create(const b2e_clip_config* cfg, int64_t max_batch, b2e_unet** out);
 int b2e_clip_forward(b2e_unet* m, const int64_t* input_ids, int64_t seq_len, float* hidden, int64_t B, void* stream);
@@ -465,16 +472,18 @@ int b2e_upsample_conv3x3_nhwc_f16(const void* x, const float* w, const float* bi
  * The fp32 paths read and write split tensors of the fp32-accurate mode: every row is [hi | lo | hi] planes of `pitch`
  * channels each (value hi + lo); the pitches and columns above are then per plane.
  * The single-head, CUDA-core and fp32 split paths take one packed tensor (q == kv, q_pitch = kv_pitch = 3 * out_pitch,
- * columns 0 / out_pitch / 2 * out_pitch) and no key mask (Tk = H*W = valid_k).  causal (query i sees keys <= i) is
- * fused-only; softmax_warps (4 or 8) selects the fused kernel's softmax layout.  Every unsupported combination returns
- * an error before anything is launched.  Allocates temporaries itself and synchronises. */
+ * columns 0 / out_pitch / 2 * out_pitch) and no key mask (Tk = H*W = valid_k).  causal (query i sees keys
+ * <= min(i, valid_k - 1)) runs on the fused path and on B2E_ATTN_FP32_TILED_CAUSAL, which takes causal = 1 only (with
+ * causal = 0 it is refused as an unknown path); softmax_warps (4 or 8) selects the fused kernel's softmax layout.  Every
+ * unsupported combination returns an error before anything is launched.  Allocates temporaries itself and synchronises. */
 enum {
   B2E_ATTN_FUSED = 0,         /* tcgen05 flash kernel (head_dim <= 192) between head gather / scatter */
   B2E_ATTN_MATERIALISED = 1,  /* batched Q K^T GEMM -> 16-bit scores -> masked row softmax -> P V GEMM */
   B2E_ATTN_SINGLE_HEAD = 2,   /* single-head GEMM attention straight from the qkv tensor */
   B2E_ATTN_CUDA_CORE = 3,     /* attention_kernel on the CUDA cores */
   B2E_ATTN_FP32_SPLIT = 4,    /* fp32-accurate attention_split_kernel */
-  B2E_ATTN_FP32_TILED = 5     /* fp32-accurate attention_split_tiled_kernel (online softmax over key tiles) */
+  B2E_ATTN_FP32_TILED = 5,    /* fp32-accurate attention_split_tiled_kernel (online softmax over key tiles) */
+  B2E_ATTN_FP32_TILED_CAUSAL = 6   /* its causal instantiation (key tiles above the diagonal skipped); causal = 1 */
 };
 int b2e_attention_f16(const void* q, int64_t q_pitch, int64_t q_col, const void* kv, int64_t kv_pitch, int64_t k_col,
                       int64_t v_col, void* out, int64_t out_pitch, int64_t B, int64_t H, int64_t W, int64_t Tk,
