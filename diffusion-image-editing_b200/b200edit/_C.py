@@ -148,6 +148,7 @@ PROTOTYPES = {
     "b2e_upsample_conv3x3_nhwc_f16": (_I, [_P, _P, _P, _P, _I64, _I64, _I64, _I64, _I64, _P]),
     "b2e_attention_f16": (_I, [_P, _I64, _I64, _P, _I64, _I64, _I64, _P, _I64, _I64, _I64, _I64, _I64, _I64, _I64, _I64,
                                _I, _I, _I, _P]),
+    "b2e_attention_bwd_fp32": (_I, [_P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _I64, _P]),
 }
 
 

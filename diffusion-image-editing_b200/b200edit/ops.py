@@ -597,6 +597,27 @@ def attention_f16(q, kv, *, hw, heads, head_dim, k_col, v_col, out_pitch, q_col=
     return out
 
 
+def attention_bwd_fp32(qkv, o, d_o, *, channels):
+    """Test hook for the fp32-accurate single-head attention backward (include/b200edit.h, b2e_attention_bwd_fp32):
+    gradients of O = softmax(Q K^T / sqrt(channels)) V w.r.t. q, k and v, the kernels of the decoders' backward pass.
+
+    Split tensors in `act_dtype()` ([hi | lo | hi] planes, ``split_planes``): qkv (B, T, 9P) holds q | k | v blocks of P
+    columns per plane (``split_planes`` of the fp32 (B, T, 3P) tensor), o and d_o are (B, T, 3P).  Returns the split
+    (dq, dk, dv), each (B, T, 3P) with zero tails beyond `channels` (``merge_planes`` gives hi + lo)."""
+    _C.require_device()
+    B, T, w = qkv.shape
+    P = w // 9
+    for t in (qkv, o, d_o):
+        if t.dtype != act_dtype() or not t.is_cuda or not t.is_contiguous():
+            raise ValueError(f"attention_bwd_fp32: operands must be contiguous CUDA {act_dtype()} split tensors")
+    if w != 9 * P or o.shape != (B, T, 3 * P) or d_o.shape != (B, T, 3 * P):
+        raise ValueError("attention_bwd_fp32: qkv (B, T, 9P), o and d_o (B, T, 3P)")
+    dq, dk, dv = (torch.empty_like(o) for _ in range(3))
+    check(lib.b2e_attention_bwd_fp32(_p(qkv), _p(o), _p(d_o), _p(dq), _p(dk), _p(dv), B, T, channels, P, _stream()),
+          "attention_bwd_fp32")
+    return dq, dk, dv
+
+
 def conv2d_nhwc_f16(x, w, bias, stride=1, residual=None):
     """Test hook for the tcgen05 implicit-GEMM convolution (optionally + residual; 16-bit NHWC, `act_dtype()`)."""
     _C.require_device()

@@ -7,7 +7,9 @@ post_quant_conv and the decoder run in libb200edit.so (bf16 tcgen05 implicit-GEM
 decoder (AttrFunc.apply with no_grad=False) uses.  ``with_encoder=True`` adds the native encoder + quant_conv
 (``vqvae.encode(img).latents`` / ``vae.encode(img).latent_dist.mode()``, src/diffusion_classes.py:27-30, 55-60).
 ``precision`` selects the decoder's operands, ``encoder_precision`` the encoder's (``"fp32"``: the fp32-accurate split
-forward; ``None``: the build's 16-bit type - it does not follow ``precision``)."""
+forward; ``None``: the build's 16-bit type - it does not follow ``precision``).  A ``precision="fp32"`` decoder in gradient
+mode also differentiates at the fp32 bar: split gradients through split dgrad weights, fp32 GroupNorm / upsample /
+attention backward kernels; its forward is the same as in forward-only mode."""
 from __future__ import annotations
 
 from types import SimpleNamespace
@@ -100,7 +102,7 @@ class VQModel(Engine):
             cfg.block_out_channels[i] = block_out_channels[i]
         cfg.layers_per_block, cfg.norm_num_groups, cfg.norm_eps = layers_per_block, norm_num_groups, norm_eps
         cfg.num_vq_embeddings = num_vq_embeddings
-        cfg.precision = self._precision_cfg      # 1: fp32-accurate decode (split-f16 operands), forward only
+        cfg.precision = self._precision_cfg      # 1: fp32-accurate decode and, in gradient mode, latent gradient (split-f16)
         self._create(lib.b2e_vqdec_create, cfg, max_batch, device)
         if with_encoder:
             self._enc = _EncoderEngine(self.out_size, out_channels, latent_channels, block_out_channels, layers_per_block,
@@ -125,7 +127,9 @@ class VQModel(Engine):
 
     def enable_grad(self, enable: bool = True):
         """Gradient mode: decode() becomes differentiable w.r.t. the latent (native dgrad; batches <= max_batch).
-        Costs workspace: every activation of a forward pass is kept until the backward pass."""
+        Costs workspace: every activation of a forward pass is kept until the backward pass.  With
+        ``precision="fp32"`` the gradient is fp32-accurate too (split operands and gradients, fp32 element-wise and
+        attention backward), and the decoded image is the one of forward-only mode bit for bit."""
         self._enable_grad(enable)
         self.forward_only = not enable
         return self

@@ -220,3 +220,19 @@ extern "C" int b2e_attention_f16(const void* q, int64_t q_pitch, int64_t q_col, 
   cudaFree(mem);
   return rc;
 }
+
+// Test hook: the fp32-accurate single-head attention backward alone (include/b200edit.h).
+extern "C" int b2e_attention_bwd_fp32(const void* qkv, const void* o, const void* d_o, void* dq, void* dk, void* dv, int64_t B,
+                                      int64_t T, int64_t C, int64_t P, void* stream) {
+  B2E_REQUIRE(qkv && o && d_o && dq && dk && dv, B2E_INVALID_ARG, "attention_bwd_fp32: null pointer");
+  B2E_REQUIRE(B >= 1 && T >= 1 && C >= 1 && P >= C && B * T < (1 << 30) && P < (1 << 20), B2E_INVALID_ARG,
+              "attention_bwd_fp32: empty or oversized shape");
+  cudaStream_t st = (cudaStream_t)stream;
+  float* stats = nullptr;
+  B2E_CUDA(cudaMalloc(&stats, sizeof(float) * 4 * (size_t)B * T));
+  const int rc = attention_split_bwd_launch((const f16*)qkv, (const f16*)o, (const f16*)d_o, (f16*)dq, (f16*)dk, (f16*)dv, stats,
+                                            (int)B, (int)T, (int)C, (int)P, st);
+  cudaStreamSynchronize(st);
+  cudaFree(stats);
+  return rc;
+}

@@ -978,6 +978,21 @@ __global__ void pack_weight_dgrad_kernel(const float* __restrict__ w, f16* __res
   }
 }
 
+// fp32-accurate mode: the same weights times wscale (a power of two: exact), lo = 1 writes the f16-rounded remainder
+// (the split representation v ~= hi + lo, as pack_weight_kernel)
+__global__ void pack_weight_dgrad_split_kernel(const float* __restrict__ w, f16* __restrict__ out, int Cout, int Cin, int kk,
+                                               int tap_width, int row_len, int col_off, int lo, float wscale) {
+  const int64_t total = (int64_t)Cout * kk * Cin;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int co = (int)(i % Cout);
+    const int t = (int)((i / Cout) % kk);
+    const int ci = (int)(i / ((int64_t)Cout * kk));
+    const float v = w[((int64_t)co * Cin + ci) * kk + (kk - 1 - t)] * wscale;
+    const f16 hi = float_to_f16(v);
+    out[(int64_t)ci * row_len + col_off + (int64_t)t * tap_width + co] = lo ? float_to_f16(__fsub_rn(v, f16_to_float(hi))) : hi;
+  }
+}
+
 // dgrad of conv_in run as a 1x1 convolution over im2col columns: out[(t*Cin + ci)*row_len + co] = w[(co*Cin + ci)*9 + t]
 __global__ void pack_weight_im2col_T_kernel(const float* __restrict__ w, f16* __restrict__ out, int Cout, int Cin, int row_len,
                                             int kk) {
@@ -987,6 +1002,19 @@ __global__ void pack_weight_im2col_T_kernel(const float* __restrict__ w, f16* __
     const int ci = (int)((i / Cout) % Cin);
     const int t = (int)(i / ((int64_t)Cout * Cin));
     out[(int64_t)(t * Cin + ci) * row_len + co] = float_to_f16(w[((int64_t)co * Cin + ci) * kk + t]);
+  }
+}
+
+__global__ void pack_weight_im2col_T_split_kernel(const float* __restrict__ w, f16* __restrict__ out, int Cout, int Cin,
+                                                  int row_len, int kk, int col_off, int lo, float wscale) {
+  const int64_t total = (int64_t)Cout * Cin * kk;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int co = (int)(i % Cout);
+    const int ci = (int)((i / Cout) % Cin);
+    const int t = (int)(i / ((int64_t)Cout * Cin));
+    const float v = w[((int64_t)co * Cin + ci) * kk + t] * wscale;
+    const f16 hi = float_to_f16(v);
+    out[(int64_t)(t * Cin + ci) * row_len + col_off + co] = lo ? float_to_f16(__fsub_rn(v, f16_to_float(hi))) : hi;
   }
 }
 
@@ -1038,19 +1066,38 @@ int conv_pack_weight(const float* w, f16* out, int Cout, int Cin, int ksize, int
 }
 
 int conv_pack_weight_dgrad(const float* w, f16* out, int Cout, int Cin, int ksize, int tap_width, int row_len, int col_off,
-                           cudaStream_t st) {
+                           cudaStream_t st, int planes, float wscale) {
   const int kk = ksize * ksize;
   const int64_t total = (int64_t)Cout * kk * Cin;
   int grid = (int)((total + 255) / 256);
   if (grid > kNumSMs * 16) grid = kNumSMs * 16;
+  if (planes == 3) {   // [W'_hi | W'_hi | W'_lo] x 2^10 per tap: taps 3 * tap_width apart, planes tap_width apart
+    for (int k = 0; k < 3; ++k) {
+      pack_weight_dgrad_split_kernel<<<grid, 256, 0, st>>>(w, out, Cout, Cin, kk, 3 * tap_width, row_len, col_off + k * tap_width,
+                                                           k == 2, wscale);
+      const int rc = check_launch("pack_weight_dgrad_split");
+      if (rc) return rc;
+    }
+    return B2E_OK;
+  }
   pack_weight_dgrad_kernel<<<grid, 256, 0, st>>>(w, out, Cout, Cin, kk, tap_width, row_len, col_off);
   return check_launch("pack_weight_dgrad");
 }
 
-int conv_pack_weight_im2col_T(const float* w, f16* out, int Cout, int Cin, int row_len, cudaStream_t st, int kk) {
+int conv_pack_weight_im2col_T(const float* w, f16* out, int Cout, int Cin, int row_len, cudaStream_t st, int kk, int planes,
+                              float wscale) {
   const int64_t total = (int64_t)Cout * Cin * kk;
   int grid = (int)((total + 255) / 256);
   if (grid > kNumSMs * 16) grid = kNumSMs * 16;
+  if (planes == 3) {   // row_len = 3 * (columns per plane): [W_hi | W_hi | W_lo] x 2^10
+    for (int k = 0; k < 3; ++k) {
+      pack_weight_im2col_T_split_kernel<<<grid, 256, 0, st>>>(w, out, Cout, Cin, row_len, kk, k * (row_len / 3), k == 2,
+                                                              wscale);
+      const int rc = check_launch("pack_weight_im2col_T_split");
+      if (rc) return rc;
+    }
+    return B2E_OK;
+  }
   pack_weight_im2col_T_kernel<<<grid, 256, 0, st>>>(w, out, Cout, Cin, row_len, kk);
   return check_launch("pack_weight_im2col_T");
 }

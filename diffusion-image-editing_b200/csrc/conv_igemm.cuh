@@ -121,11 +121,15 @@ int conv_pack_weight_up2(const float* w, f16* out, int Cout, int Cin, int tap_wi
 int conv_pack_weight(const float* w, f16* out, int Cout, int Cin, int ksize, int tap_width, int row_len,
                      int col_off, cudaStream_t st, int ci0 = 0, int cin_total = 0, int lo = 0, float wscale = 1.f);
 // dgrad weights (flipped taps, transposed channels): out[ci*row_len + col_off + t*tap_width + co] = w[(co*Cin+ci)*kk + kk-1-t]
+// planes = 3 (fp32-accurate mode): split weights [W'_hi | W'_hi | W'_lo] x wscale per tap, taps 3 * tap_width columns apart and
+// the three planes tap_width columns apart (the layout conv_pack_weight gives a split activation operand)
 int conv_pack_weight_dgrad(const float* w, f16* out, int Cout, int Cin, int ksize, int tap_width, int row_len, int col_off,
-                           cudaStream_t st);
+                           cudaStream_t st, int planes = 1, float wscale = 1.f);
 // dgrad of the im2col conv_in: out[(t*Cin + ci)*row_len + co] = w[(co*Cin + ci)*9 + t]
 // (kk taps: 9 for the 3x3 conv_in, 49 for the 7x7 stem of the classifier network)
-int conv_pack_weight_im2col_T(const float* w, f16* out, int Cout, int Cin, int row_len, cudaStream_t st, int kk = 9);
+// planes = 3: row_len / 3 columns per plane, [W_hi | W_hi | W_lo] x wscale
+int conv_pack_weight_im2col_T(const float* w, f16* out, int Cout, int Cin, int row_len, cudaStream_t st, int kk = 9,
+                              int planes = 1, float wscale = 1.f);
 // out[c*row_len + col_off + c] = value for c < C (identity residual segment)
 int conv_fill_identity(f16* out, int C, int row_len, int col_off, cudaStream_t st, float value = 1.f);
 

@@ -239,7 +239,8 @@ struct b2e_unet {
     const int PL = this->PL;
     // (a <= 16-channel output, i.e. conv_out, receives its gradient as a 64-channel padded NHWC tensor)
     if (decoder || resnet || lpips) { c.dg = make_dgrad(cin, cout > 16 ? c.cout_pad : kConvBlockK, k); dd = dgrads[c.dg]; cc.dg = c.dg; }
-    add_param(name + ".weight", (int64_t)cout * cin * k * k, (int64_t)cin * k * k, [cc, dd, PL, src0](const float* src, cudaStream_t st) {
+    const int DPL = dgrad_planes();
+    add_param(name + ".weight", (int64_t)cout * cin * k * k, (int64_t)cin * k * k, [cc, dd, PL, DPL, src0](const float* src, cudaStream_t st) {
       int rc;
       if (PL == 3 && src0 > 0 && cc.k == 1) {
         rc = pack_w(PL, src, cc.w, cc.cout, src0, 1, src0, cc.row_len, 0, src0, st, 0, cc.cin);
@@ -247,7 +248,7 @@ struct b2e_unet {
       } else {
         rc = pack_w(PL, src, cc.w, cc.cout, cc.cin, cc.k, cc.cin_pad, cc.row_len, 0, cc.cin_pad, st);
       }
-      if (!rc && cc.dg >= 0) rc = conv_pack_weight_dgrad(src, dd.w, cc.cout, cc.cin, cc.k, dd.cin_pad, dd.row_len, 0, st);
+      if (!rc && cc.dg >= 0) rc = conv_pack_weight_dgrad(src, dd.w, cc.cout, cc.cin, cc.k, dd.cin_pad, dd.row_len, 0, st, DPL, dgrad_wscale(DPL));
       for (int ph = 0; ph < 4 && !rc && cc.w_up2; ++ph) {
         f16* wp = cc.w_up2 + (size_t)ph * cc.cout_pad * cc.row_len_up2;
         if (PL == 1) {
@@ -263,12 +264,16 @@ struct b2e_unet {
     add_f32(name + ".bias", c.b, cout, (int64_t)cin * k * k);
     return c;
   }
+  // planes of the dgrad twins: the split decoder's gradient is fp32-accurate (split gradients, [W'_hi | W'_hi | W'_lo] x 2^10
+  // weights); the classifier and LPIPS keep a 16-bit backward under their fp32-accurate forward
+  int dgrad_planes() const { return decoder ? PL : 1; }
+  static float dgrad_wscale(int planes) { return planes == 3 ? kSplitWScale : 1.f; }
   // dgrad twin of a stride-1 convolution with `cin` input channels whose output tensor has pitch `dy_pitch`:
   // a convolution dy (dy_pitch channels) -> dx (cin channels), zero bias; the weights are packed by the caller
   int make_dgrad(int cin, int dy_pitch, int k, int extra_k = 0) {
     ConvL d;
     d.cin = dy_pitch; d.cin_pad = dy_pitch; d.cout = cin; d.cout_pad = conv_cout_pad(cin); d.k = k;
-    d.res_c = extra_k; d.row_len = k * k * dy_pitch + extra_k;
+    d.res_c = extra_k; d.row_len = dgrad_planes() * (k * k * dy_pitch + extra_k);
     d.w = dmalloc<f16>((size_t)d.cout_pad * d.row_len);
     d.b = dmalloc<float>(d.cout_pad);
     dgrads.push_back(d);
@@ -305,7 +310,7 @@ struct b2e_unet {
       add_param(name + ".conv_shortcut.weight", (int64_t)cout * cin, cin, [cc, sd, sc_dg, cin, cin0, cin1, p0, p1, PL](const float* src, cudaStream_t st) {
         int rc = pack_w(PL, src, cc.w, cc.cout, cin0, 1, cin0, cc.row_len, PL * 9 * cc.cin_pad, p0, st, 0, cin);
         if (!rc && cin1) rc = pack_w(PL, src, cc.w, cc.cout, cin1, 1, cin1, cc.row_len, PL * (9 * cc.cin_pad + p0), p1, st, cin0, cin);
-        if (!rc && sc_dg >= 0) rc = conv_pack_weight_dgrad(src, sd.w, cc.cout, cin, 1, sd.cin_pad, sd.row_len, 0, st);
+        if (!rc && sc_dg >= 0) rc = conv_pack_weight_dgrad(src, sd.w, cc.cout, cin, 1, sd.cin_pad, sd.row_len, 0, st, PL, dgrad_wscale(PL));
         return rc;
       });
       add_f32(name + ".conv_shortcut.bias", r.c2.b2, cout, cin);
@@ -399,7 +404,7 @@ struct b2e_unet {
       float* bdst = a.qkv.b + (size_t)i * P;
       add_param(name + "." + nm[i] + ".weight", (int64_t)C * C, C, [wdst, qd, qkv_dg, i, C, P, PL](const float* src, cudaStream_t st) {
         int rc = pack_w(PL, src, wdst, C, C, 1, C, P * PL, 0, P, st);
-        if (!rc && qkv_dg >= 0) rc = conv_pack_weight_dgrad(src, qd.w, C, C, 1, P, qd.row_len, i * P, st);
+        if (!rc && qkv_dg >= 0) rc = conv_pack_weight_dgrad(src, qd.w, C, C, 1, P, qd.row_len, PL * i * P, st, PL, dgrad_wscale(PL));
         return rc;
       });
       add_f32(name + "." + nm[i] + ".bias", bdst, C, C);
@@ -443,7 +448,7 @@ int build_model_decoder(b2e_unet* m) {
       int rc = conv_pack_weight(src, ci.w, ci.cout, L, 3, L, ci.row_len, 0, st, 0, 0, 0, ws);
       if (!rc && PL == 3) rc = conv_pack_weight(src, ci.w, ci.cout, L, 3, L, ci.row_len, kConvBlockK, st, 0, 0, 0, ws);
       if (!rc && PL == 3) rc = conv_pack_weight(src, ci.w, ci.cout, L, 3, L, ci.row_len, 2 * kConvBlockK, st, 0, 0, 1, ws);
-      if (!rc) rc = conv_pack_weight_im2col_T(src, cd.w, ci.cout, L, cd.row_len, st);
+      if (!rc) rc = conv_pack_weight_im2col_T(src, cd.w, ci.cout, L, cd.row_len, st, 9, PL, b2e_unet::dgrad_wscale(PL));
       return rc;
     });
     m->add_f32("decoder.conv_in.bias", ci.b, top, (int64_t)L * 9);
@@ -1824,7 +1829,7 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
   auto on_stack = [&](const Tensor& t) { for (auto& s : stack) if (s.p == t.p) return true; return false; };
 
   // gradient mode: what the backward pass needs from every node
-  struct Save { Tensor x, h1, qkv, sc; float* st1 = nullptr; float* st2 = nullptr; };
+  struct Save { Tensor x, h1, qkv, sc, o; float* st1 = nullptr; float* st2 = nullptr; };
   std::vector<Save> saves(m->nodes.size());
   int node_i = -1;
   for (const Node& nd : m->nodes) {
@@ -1868,6 +1873,7 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
         const int T = h.H * h.W, C = a.P;   // C: padded width of q / k / v (zero tail: no effect on Q K^T, zero rows of V^T)
         if (PL == 3) {
           // fp32-accurate mode: fp32 attention core on the CUDA cores over the split-f16 q | k | v planes
+          sv.o = o;                         // the backward's D = rowsum(dO o O)
           if (!dry) {
             const int Cr = a.C, dh = a.C / heads;
             if (sizeof(float) * 16 * (size_t)(dh + T) <= 160 * 1024 && qkv.C == 3 * C) {
@@ -2013,7 +2019,8 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
       }
       case N_UP: {
         sv.x = h;
-        if (up2_on && !keep && !h.alias && m->ups[nd.idx].w_up2 && h.H >= 64 && h.C == m->ups[nd.idx].cin_pad) {
+        // (the 16-bit backward keeps the separate upsample; the split forward of gradient mode stays that of forward-only mode)
+        if (up2_on && (!keep || PL == 3) && !h.alias && m->ups[nd.idx].w_up2 && h.H >= 64 && h.C == m->ups[nd.idx].cin_pad) {
           Tensor out;
           conv_up2(m->ups[nd.idx], h, &out);
           if (!on_stack(h)) tfree(h);
@@ -2076,7 +2083,10 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
       a.C = x.Cr; a.P = x.C; a.Pda = da.C; a.N = B; a.HW = x.H * x.W; a.G = G;
       a.gamma = L.g; a.beta = L.b; a.stats = stats; a.partial = gpart; a.chunks = gn_chunks(a.HW, a.C); a.silu = silu;
       if (add && add->C != x.C) { rc = B2E_INVALID_ARG; set_error("unet backward: residual pitch mismatch"); return; }
-      ops.push_back({[a](cudaStream_t st) { return gn_bwd_launch(a, st); }, 1, 0.0, 10.0 * B * a.HW * a.C, "groupnorm backward"});
+      // algorithmic traffic per element: both passes read x and da, the apply pass reads add and writes dx (split: two planes
+      // read, three written)
+      ops.push_back({[a, PL](cudaStream_t st) { return gn_bwd_launch(a, st, PL); }, 1, 0.0, (PL == 3 ? 26.0 : 10.0) * B * a.HW * a.C,
+                     PL == 3 ? "groupnorm backward (fp32, split-f16)" : "groupnorm backward"});
     };
     // gradient w.r.t. the image arrives as fp32 NCHW: pack to f16 NHWC with 64 (zero-padded) channels
     Tensor gy = talloc(B, So, So, kConvBlockK, c.out_channels);
@@ -2086,8 +2096,8 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
       cudaMemset(gs, 0, sizeof(float) * 4);
       ops.push_back({[m, gs, B, Co, So](cudaStream_t st) { return grad_scale_launch(m->in_dy, (int64_t)B * Co * So * So, gs, 1.f, st); },
                      3, 0.0, 4.0 * B * Co * So * So, "max|d(image)| -> power-of-two gradient scale"});
-      ops.push_back({[m, gy, gs, B, Co, So](cudaStream_t st) { return pack_input_launch(m->in_dy, gy.p, B, Co, So, So, kConvBlockK, false, st, 1, gs); },
-                     3, 0.0, (double)B * So * So * (4.0 * Co + 2.0 * kConvBlockK), "pack d(image)"});
+      ops.push_back({[m, gy, gs, B, Co, So, PL](cudaStream_t st) { return pack_input_launch(m->in_dy, gy.p, B, Co, So, So, kConvBlockK, false, st, PL, gs); },
+                     3, 0.0, (double)B * So * So * (4.0 * Co + 2.0 * PL * kConvBlockK), "pack d(image)"});
     }
     Tensor d_an, g;
     conv(m->dgrads[m->conv_out_dg], gy, nullptr, 1, ConvEpilogue{}, &d_an, nullptr, nullptr, nullptr, false);
@@ -2114,41 +2124,59 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
         case N_ATTN: {
           const AttnL& a = m->attns[nd.idx];
           const int T = sv.x.H * sv.x.W, P = a.P, Hh = sv.x.H, Ww = sv.x.W;
-          if (!sv.sc.p && !dry) { rc = B2E_UNSUPPORTED_SHAPE; set_error("unet backward: attention needs the tensor-core path"); break; }
+          if (PL == 1 && !sv.sc.p && !dry) { rc = B2E_UNSUPPORTED_SHAPE; set_error("unet backward: attention needs the tensor-core path"); break; }
           Tensor dO, dV, dP, dQ, dK, d_an2, gin;
           conv(m->dgrads[a.proj.dg], g, nullptr, 1, ConvEpilogue{}, &dO, nullptr, nullptr, nullptr, false);
-          Tensor Pt = talloc(B, Hh, Ww, T), dSt = talloc(B, Hh, Ww, T);
-          Tensor dOt = talloc(B, 1, P, T), Kt = talloc(B, 1, P, T), Qt = talloc(B, 1, P, T);
-          dV = talloc(B, Hh, Ww, P, a.C); dP = talloc(B, Hh, Ww, T); dQ = talloc(B, Hh, Ww, P, a.C); dK = talloc(B, Hh, Ww, P, a.C);
-          if (!dry) {
-            auto gemm = [&](const Tensor& A, int K, const f16* Bop, int brows, int bpitch, int Cout, const Tensor& out,
-                            const char* what) {
-              // out[n][t][co] = sum_k A[n][t][k] * Bop[n*brows + co][k]
-              ConvDesc d;
-              d.s0.ptr = A.p; d.s0.C = K; if (A.C != K) d.s0.pitch = A.C;
-              d.N = B; d.H = Hh; d.W = Ww; d.ksize = 1; d.stride = 1;
-              d.w_packed = Bop; d.b_batch_rows = brows; d.b_pitch = bpitch; d.Cout = Cout; d.out_f16 = out.p;
-              ConvPlan pl;
-              if (!rc) rc = conv_plan_build(&pl, d);
-              if (!rc) { ops.push_back({[pl](cudaStream_t st) { return conv_launch(pl, ConvEpilogue{}, st); }, 0, pl.flops, 0.0, what}); flops += pl.flops; }
-            };
-            const Tensor sc = sv.sc, qkv = sv.qkv;
-            const float scale = 1.0f / sqrtf((float)a.C);
-            const int64_t rows = (int64_t)B * T;
-            // dV = P^T dO
-            ops.push_back({[sc, Pt, B, T](cudaStream_t st) { return transpose_window_launch(sc.p, Pt.p, B, T, T, T, 0, st); }, 3, 0.0, 4.0 * B * T * T, "P^T"});
-            ops.push_back({[dO, dOt, B, T, P](cudaStream_t st) { return transpose_window_launch(dO.p, dOt.p, B, T, P, P, 0, st); }, 3, 0.0, 4.0 * B * T * P, "dO^T"});
-            gemm(Pt, T, dOt.p, P, T, P, dV, "attention backward dV = P^T dO");
-            // dP = dO V^T ; dS = scale * P o (dP - rowsum(dP o P))  (in place)
-            gemm(dO, P, qkv.p + 2 * P, T, 3 * P, T, dP, "attention backward dP = dO V^T");
-            ops.push_back({[sc, dP, rows, T, scale](cudaStream_t st) { return softmax_bwd_rows_launch(sc.p, dP.p, rows, T, scale, st); },
-                           3, 0.0, 6.0 * rows * T, "softmax backward"});
-            // dQ = dS K ; dK = dS^T Q
-            ops.push_back({[qkv, Kt, B, T, P](cudaStream_t st) { return transpose_window_launch(qkv.p, Kt.p, B, T, P, 3 * P, P, st); }, 3, 0.0, 4.0 * B * T * P, "K^T"});
-            gemm(dP, T, Kt.p, P, T, P, dQ, "attention backward dQ = dS K");
-            ops.push_back({[dP, dSt, B, T](cudaStream_t st) { return transpose_window_launch(dP.p, dSt.p, B, T, T, T, 0, st); }, 3, 0.0, 4.0 * B * T * T, "dS^T"});
-            ops.push_back({[qkv, Qt, B, T, P](cudaStream_t st) { return transpose_window_launch(qkv.p, Qt.p, B, T, P, 3 * P, 0, st); }, 3, 0.0, 4.0 * B * T * P, "Q^T"});
-            gemm(dSt, T, Qt.p, P, T, P, dK, "attention backward dK = dS^T Q");
+          if (PL == 3) {
+            // fp32 flash-style backward on the CUDA cores from the saved split q | k | v and O: split dQ, dK, dV
+            dV = talloc(B, Hh, Ww, P, a.C); dQ = talloc(B, Hh, Ww, P, a.C); dK = talloc(B, Hh, Ww, P, a.C);
+            float* ast = (float*)ar.alloc(sizeof(float) * 4 * (size_t)B * T);
+            const double fl = B * attention_split_bwd_flops(T, a.C);
+            flops += fl;
+            if (!dry && !rc) {
+              if (dO.C != P || sv.o.C != P || sv.qkv.C != 3 * P) { rc = B2E_INVALID_ARG; set_error("unet backward: attention operand pitch mismatch"); break; }
+              const Tensor qkv = sv.qkv, o = sv.o;
+              const int Cr = a.C;
+              // bytes: the split q, k, v and dO rows are re-read from L2 per tile; counted once here (algorithmic traffic)
+              ops.push_back({[qkv, o, dO, dQ, dK, dV, ast, B, T, Cr, P](cudaStream_t st) {
+                               return attention_split_bwd_launch(qkv.p, o.p, dO.p, dQ.p, dK.p, dV.p, ast, B, T, Cr, P, st); },
+                             2, fl, (double)B * T * P * 2.0 * (9.0 + 3.0 + 3.0 + 9.0),
+                             "attention backward (fp32, flash-style: stats, dK / dV, dQ; split-f16 operands)"});
+            }
+          } else {
+            Tensor Pt = talloc(B, Hh, Ww, T), dSt = talloc(B, Hh, Ww, T);
+            Tensor dOt = talloc(B, 1, P, T), Kt = talloc(B, 1, P, T), Qt = talloc(B, 1, P, T);
+            dV = talloc(B, Hh, Ww, P, a.C); dP = talloc(B, Hh, Ww, T); dQ = talloc(B, Hh, Ww, P, a.C); dK = talloc(B, Hh, Ww, P, a.C);
+            if (!dry) {
+              auto gemm = [&](const Tensor& A, int K, const f16* Bop, int brows, int bpitch, int Cout, const Tensor& out,
+                              const char* what) {
+                // out[n][t][co] = sum_k A[n][t][k] * Bop[n*brows + co][k]
+                ConvDesc d;
+                d.s0.ptr = A.p; d.s0.C = K; if (A.C != K) d.s0.pitch = A.C;
+                d.N = B; d.H = Hh; d.W = Ww; d.ksize = 1; d.stride = 1;
+                d.w_packed = Bop; d.b_batch_rows = brows; d.b_pitch = bpitch; d.Cout = Cout; d.out_f16 = out.p;
+                ConvPlan pl;
+                if (!rc) rc = conv_plan_build(&pl, d);
+                if (!rc) { ops.push_back({[pl](cudaStream_t st) { return conv_launch(pl, ConvEpilogue{}, st); }, 0, pl.flops, 0.0, what}); flops += pl.flops; }
+              };
+              const Tensor sc = sv.sc, qkv = sv.qkv;
+              const float scale = 1.0f / sqrtf((float)a.C);
+              const int64_t rows = (int64_t)B * T;
+              // dV = P^T dO
+              ops.push_back({[sc, Pt, B, T](cudaStream_t st) { return transpose_window_launch(sc.p, Pt.p, B, T, T, T, 0, st); }, 3, 0.0, 4.0 * B * T * T, "P^T"});
+              ops.push_back({[dO, dOt, B, T, P](cudaStream_t st) { return transpose_window_launch(dO.p, dOt.p, B, T, P, P, 0, st); }, 3, 0.0, 4.0 * B * T * P, "dO^T"});
+              gemm(Pt, T, dOt.p, P, T, P, dV, "attention backward dV = P^T dO");
+              // dP = dO V^T ; dS = scale * P o (dP - rowsum(dP o P))  (in place)
+              gemm(dO, P, qkv.p + 2 * P, T, 3 * P, T, dP, "attention backward dP = dO V^T");
+              ops.push_back({[sc, dP, rows, T, scale](cudaStream_t st) { return softmax_bwd_rows_launch(sc.p, dP.p, rows, T, scale, st); },
+                             3, 0.0, 6.0 * rows * T, "softmax backward"});
+              // dQ = dS K ; dK = dS^T Q
+              ops.push_back({[qkv, Kt, B, T, P](cudaStream_t st) { return transpose_window_launch(qkv.p, Kt.p, B, T, P, 3 * P, P, st); }, 3, 0.0, 4.0 * B * T * P, "K^T"});
+              gemm(dP, T, Kt.p, P, T, P, dQ, "attention backward dQ = dS K");
+              ops.push_back({[dP, dSt, B, T](cudaStream_t st) { return transpose_window_launch(dP.p, dSt.p, B, T, T, T, 0, st); }, 3, 0.0, 4.0 * B * T * T, "dS^T"});
+              ops.push_back({[qkv, Qt, B, T, P](cudaStream_t st) { return transpose_window_launch(qkv.p, Qt.p, B, T, P, 3 * P, 0, st); }, 3, 0.0, 4.0 * B * T * P, "Q^T"});
+              gemm(dSt, T, Qt.p, P, T, P, dK, "attention backward dK = dS^T Q");
+            }
           }
           // d(normed input) = Wq^T dQ + Wk^T dK + Wv^T dV: one 1x1 convolution drawing K from three tensors
           conv(m->dgrads[a.qkv_dg], dQ, &dK, 1, ConvEpilogue{}, &d_an2, nullptr, &dV, nullptr, false);
@@ -2160,8 +2188,8 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
           Tensor d_up, gin = talloc(B, sv.x.H, sv.x.W, sv.x.C, sv.x.Cr);
           conv(m->dgrads[m->ups[nd.idx].dg], g, nullptr, 1, ConvEpilogue{}, &d_up, nullptr, nullptr, nullptr, false);
           if (!dry) {
-            ops.push_back({[d_up, gin, B](cudaStream_t st) { return downsum2x_launch(d_up.p, gin.p, B, gin.H, gin.W, gin.C, st); },
-                           3, 0.0, 10.0 * B * gin.H * gin.W * gin.C, "upsample backward"});
+            ops.push_back({[d_up, gin, B, PL](cudaStream_t st) { return downsum2x_launch(d_up.p, gin.p, B, gin.H, gin.W, gin.C, st, PL); },
+                           3, 0.0, (PL == 3 ? 22.0 : 10.0) * B * gin.H * gin.W * gin.C, "upsample backward"});
           }
           g = gin;
           break;
@@ -2174,8 +2202,9 @@ int build_program(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* need) {
       conv(m->dgrads[m->conv_in_dg], g, nullptr, 1, ConvEpilogue{}, &dcols, nullptr, nullptr, nullptr, false);
       if (!dry && !rc) {
         const int L = c.in_channels;
-        ops.push_back({[m, dcols, gs, B, L, S](cudaStream_t st) { return vq_col2im_bwd_launch(dcols.p, m->pq_w, m->out_dz, B, L, S, S, st, gs); },
-                       3, 0.0, (double)B * S * S * (128.0 + 4.0 * L), "col2im + post_quant_conv backward (straight-through)"});
+        ops.push_back({[m, dcols, gs, B, L, S, PL](cudaStream_t st) {
+                         return vq_col2im_bwd_launch(dcols.p, m->pq_w, m->out_dz, B, L, S, S, st, gs, nullptr, 0, PL); },
+                       3, 0.0, (double)B * S * S * (128.0 * (PL == 3 ? 2 : 1) + 4.0 * L), "col2im + post_quant_conv backward (straight-through)"});
       }
     }
     cur = &ops_fwd;
@@ -2520,7 +2549,6 @@ int b2e_unet_enable_grad(b2e_unet* m, int enable) {
   B2E_REQUIRE(m, B2E_INVALID_ARG, "unet_enable_grad: null handle");
   B2E_REQUIRE(!enable || m->decoder || m->resnet || m->lpips, B2E_UNSUPPORTED_SHAPE,
               "unet_enable_grad: gradient mode is implemented for the VQ / KL decoder, the classifier and LPIPS");
-  B2E_REQUIRE(!enable || m->PL == 1 || m->resnet || m->lpips, B2E_UNSUPPORTED_SHAPE, "unet_enable_grad: the fp32-accurate mode is forward-only");
   if ((enable != 0) == m->grad) return B2E_OK;
   m->grad = enable != 0;
   m->cur_B = -1; m->fwd_B = -1; m->ws = nullptr; m->ws_bytes = 0;   // the workspace must be re-queried and re-bound

@@ -441,7 +441,7 @@ int gn_launch(const GNArgs& a_in, cudaStream_t st) {
               "groupnorm: unsupported channels %d+%d / groups %d", a.C0, a.C1, a.G);
   B2E_REQUIRE(a.P0 >= a.C0 && a.P1 >= a.C1 && a.Pout >= C && a.P0 % 8 == 0 && a.P1 % 8 == 0 && a.Pout % 8 == 0,
               B2E_INVALID_ARG, "groupnorm: bad channel pitches %d/%d -> %d", a.P0, a.P1, a.Pout);
-  B2E_REQUIRE(a.planes == 1 || (a.planes == 3 && !a.cs0 && !a.ts0 && !a.save_stats), B2E_INVALID_ARG,
+  B2E_REQUIRE(a.planes == 1 || (a.planes == 3 && !a.cs0 && !a.ts0), B2E_INVALID_ARG,
               "groupnorm: split-f16 tensors take their statistics from the stand-alone pass");
   int rc = B2E_OK;
   if (!a.cs0 && !a.ts0) {
@@ -724,10 +724,150 @@ __global__ void __launch_bounds__(kGNThreads) gn_bwd_apply_bulk_kernel(GNBwdArgs
   }
 }
 
-int gn_bwd_launch(const GNBwdArgs& a, cudaStream_t st) {
+// ---- fp32-accurate mode (planes = 3): x, da, add and dx are split tensors ([hi | lo | hi] planes, value hi + lo).  The same
+// two passes in fp32 with the forward's exact SiLU (expf, not the tanh.approx of the 16-bit kernels); dx is re-split.
+__device__ __forceinline__ void load_split8(const f16* p, int lo_off, float* f) {
+  float l[8];
+  unpack8(__ldg(reinterpret_cast<const uint4*>(p)), f);
+  unpack8(__ldg(reinterpret_cast<const uint4*>(p + lo_off)), l);
+#pragma unroll
+  for (int j = 0; j < 8; ++j) f[j] += l[j];
+}
+__device__ __forceinline__ void store_split8(f16* p, int lo_off, const float* f) {
+  float l[8];
+  const uint4 hi = pack8(f);
+  float h[8];
+  unpack8(hi, h);
+#pragma unroll
+  for (int j = 0; j < 8; ++j) l[j] = __fsub_rn(f[j], h[j]);
+  *reinterpret_cast<uint4*>(p) = hi;
+  *reinterpret_cast<uint4*>(p + lo_off) = pack8(l);
+  *reinterpret_cast<uint4*>(p + 2 * lo_off) = hi;
+}
+// d silu(y) / dy with the forward's sigmoid (gn_apply_kernel<true>: y / (1 + expf(-y)))
+__device__ __forceinline__ float silu_grad_exact(float y) {
+  const float sg = 1.f / (1.f + expf(-y));
+  return sg * fmaf(y, 1.f - sg, 1.f);
+}
+
+__global__ void __launch_bounds__(kGNThreads) gn_bwd_partial_split_kernel(GNBwdArgs a) {
+  pdl_wait();
+  __shared__ float s_a[2048], s_b[2048];
+  const int C = a.C, slots = C >> 3, ppi = kGNThreads / slots;
+  const int n = blockIdx.y, chunk = blockIdx.x, tid = threadIdx.x;
+  const int s = tid % slots, pl = tid / slots;
+  const int per = (a.HW + a.chunks - 1) / a.chunks;
+  const int p0 = chunk * per, p1 = min(a.HW, p0 + per);
+  const int cpg = C / a.G;
+  if (pl < ppi) {
+    float sa[8], sb[8], sc[8], sh[8], r[8], mr[8], gam[8];
+    const int c = s * 8;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      sa[j] = sb[j] = 0.f;
+      const float2 st = *reinterpret_cast<const float2*>(a.stats + ((int64_t)n * a.G + (c + j) / cpg) * 2);
+      gam[j] = __ldg(a.gamma + c + j);
+      r[j] = st.y; mr[j] = -st.x * st.y;
+      sc[j] = gam[j] * st.y; sh[j] = __ldg(a.beta + c + j) - st.x * sc[j];   // the forward's affine (gn_apply_kernel)
+    }
+    const f16* xs = a.x + (int64_t)n * a.HW * 3 * a.P + c;
+    const f16* ds = a.da + (int64_t)n * a.HW * 3 * a.Pda + c;
+    for (int p = p0 + pl; p < p1; p += ppi) {
+      float xf[8], df[8];
+      load_split8(xs + (int64_t)p * 3 * a.P, a.P, xf);
+      load_split8(ds + (int64_t)p * 3 * a.Pda, a.Pda, df);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        float dy = df[j];
+        if (a.silu) dy *= silu_grad_exact(fmaf(xf[j], sc[j], sh[j]));
+        const float dxh = dy * gam[j];
+        sa[j] += dxh; sb[j] = fmaf(dxh, fmaf(xf[j], r[j], mr[j]), sb[j]);
+      }
+    }
+#pragma unroll
+    for (int j = 0; j < 8; ++j) { s_a[pl * C + c + j] = sa[j]; s_b[pl * C + c + j] = sb[j]; }
+  }
+  __syncthreads();
+  if (tid < a.G) {
+    float ta = 0.f, tb = 0.f;
+    for (int q = 0; q < ppi; ++q)
+      for (int c = tid * cpg; c < (tid + 1) * cpg; ++c) { ta += s_a[q * C + c]; tb += s_b[q * C + c]; }
+    float* o = a.partial + (((int64_t)n * a.chunks + chunk) * a.G + tid) * 2;
+    o[0] = ta; o[1] = tb;
+  }
+}
+
+__global__ void __launch_bounds__(kGNThreads) gn_bwd_apply_split_kernel(GNBwdArgs a, int pix_per_block) {
+  pdl_wait();
+  __shared__ float s_ma[64], s_mb[64];
+  const int C = a.C, slots = a.P >> 3, ppi = kGNThreads / slots;
+  const int n = blockIdx.y, tid = threadIdx.x;
+  const int cpg = C / a.G;
+  if (tid < a.G) {
+    double ta = 0.0, tb = 0.0;
+    for (int ch = 0; ch < a.chunks; ++ch) {
+      const float* o = a.partial + (((int64_t)n * a.chunks + ch) * a.G + tid) * 2;
+      ta += (double)o[0]; tb += (double)o[1];
+    }
+    const double cnt = (double)a.HW * cpg;
+    s_ma[tid] = (float)(ta / cnt); s_mb[tid] = (float)(tb / cnt);
+  }
+  __syncthreads();
+  const int s = tid % slots, pl = tid / slots;
+  if (pl >= ppi) return;
+  const int c = s * 8;
+  const int p0 = blockIdx.x * pix_per_block, p1 = min(a.HW, p0 + pix_per_block);
+  const int64_t px = 3 * (int64_t)a.P;
+  f16* dst = a.dx + (int64_t)n * a.HW * px + c;
+  if (c >= C) {   // zero tail of the pitch, all planes
+    for (int p = p0 + pl; p < p1; p += ppi)
+      for (int k = 0; k < 3; ++k) *reinterpret_cast<uint4*>(dst + (int64_t)p * px + k * a.P) = make_uint4(0, 0, 0, 0);
+    return;
+  }
+  float sc[8], sh[8], gr[8], k1[8], k0[8];
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    const int g = (c + j) / cpg;
+    const float2 st = *reinterpret_cast<const float2*>(a.stats + ((int64_t)n * a.G + g) * 2);
+    const float gam = __ldg(a.gamma + c + j), rstd = st.y, mr = -st.x * st.y;
+    sc[j] = gam * rstd; sh[j] = __ldg(a.beta + c + j) - st.x * sc[j];
+    gr[j] = gam * rstd;
+    k1[j] = -rstd * rstd * s_mb[g];
+    k0[j] = -rstd * fmaf(mr, s_mb[g], s_ma[g]);
+  }
+  const f16* xs = a.x + (int64_t)n * a.HW * px + c;
+  const f16* ds = a.da + (int64_t)n * a.HW * 3 * a.Pda + c;
+  const f16* as = a.add ? a.add + (int64_t)n * a.HW * px + c : nullptr;
+  for (int p = p0 + pl; p < p1; p += ppi) {
+    float xf[8], df[8], af[8];
+    load_split8(xs + (int64_t)p * px, a.P, xf);
+    load_split8(ds + (int64_t)p * 3 * a.Pda, a.Pda, df);
+    if (as) load_split8(as + (int64_t)p * px, a.P, af);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      float dy = df[j];
+      if (a.silu) dy *= silu_grad_exact(fmaf(xf[j], sc[j], sh[j]));
+      float dx = fmaf(dy, gr[j], fmaf(xf[j], k1[j], k0[j]));
+      if (as) dx += af[j];
+      xf[j] = dx;
+    }
+    store_split8(dst + (int64_t)p * px, a.P, xf);
+  }
+}
+
+int gn_bwd_launch(const GNBwdArgs& a, cudaStream_t st, int planes) {
   B2E_REQUIRE(a.C % 8 == 0 && a.P >= a.C && a.Pda >= a.C && a.P % 8 == 0 && a.Pda % 8 == 0 && a.P <= 2048 && a.G <= 64 &&
-                  a.C % a.G == 0 && a.x && a.da && a.dx && a.stats && a.partial,
+                  a.C % a.G == 0 && a.x && a.da && a.dx && a.stats && a.partial && (planes == 1 || planes == 3),
               B2E_UNSUPPORTED_SHAPE, "groupnorm backward: unsupported channels %d (pitch %d) / groups %d", a.C, a.P, a.G);
+  if (planes == 3) {
+    launch_pdl(gn_bwd_partial_split_kernel, dim3(a.chunks, a.N), dim3(kGNThreads), 0, st, a);
+    int rc = check_launch("gn_bwd_partial_split");
+    if (rc) return rc;
+    const int ppi = kGNThreads / (a.P / 8);
+    const int ppb = ppi * 8 > a.HW ? a.HW : ppi * 8;
+    launch_pdl(gn_bwd_apply_split_kernel, dim3((a.HW + ppb - 1) / ppb, a.N), dim3(kGNThreads), 0, st, a, ppb);
+    return check_launch("gn_bwd_apply_split");
+  }
   const int slots = a.P / 8, ppi = kGNThreads / slots;
   int ppb = ppi * kGNBwdUnroll * 2;   // two unrolled sweeps per thread
   if (ppb > a.HW) ppb = a.HW;
@@ -882,6 +1022,24 @@ __global__ void pack_input_kernel(const float* __restrict__ x, f16* __restrict__
   }
 }
 
+// split-f16 output (fp32-accurate mode: the d(image) entry of the decoder backward): [hi | lo | hi] planes of cpad channels
+__global__ void pack_input_split_kernel(const float* __restrict__ x, f16* __restrict__ out, int B, int C, int HW, int cpad,
+                                        const float* __restrict__ gs) {
+  pdl_wait();
+  const float sc = gs ? gs[0] : 1.f;
+  const int64_t total = (int64_t)B * HW;
+  for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < total; p += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t b = p / HW, q = p % HW;
+    float f[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    for (int c = 0; c < C && c < 8; ++c) f[c] = x[(b * C + c) * HW + q] * sc;   // power-of-two scale: exact
+    f16* o = out + p * 3 * cpad;
+    const uint4 z = make_uint4(0, 0, 0, 0);
+    for (int k = 0; k < 3; ++k)
+      for (int i = 1; i < cpad / 8; ++i) reinterpret_cast<uint4*>(o + k * cpad)[i] = z;
+    store_split8(o, cpad, f);
+  }
+}
+
 // im2col variant: one thread per pixel gathers its 9 x C neighbourhood (coalesced across the warp, neighbours hit
 // L1) and writes the pixel's 64 channels (128 B)
 // mask / shift: the optional input transform (1 - mask * x, then (v - shift) / scale) of pack_input_launch; none of it
@@ -947,7 +1105,11 @@ int pack_input_launch(const float* x, f16* out, int B, int C, int H, int W, int 
     return check_launch("pack_input_im2col");
   }
   B2E_REQUIRE(C <= 8 && cpad % 8 == 0, B2E_UNSUPPORTED_SHAPE, "pack_input: in_channels must be <= 8");
-  B2E_REQUIRE(planes == 1, B2E_UNSUPPORTED_SHAPE, "pack_input: split-f16 output needs the im2col layout");
+  B2E_REQUIRE(planes == 1 || planes == 3, B2E_UNSUPPORTED_SHAPE, "pack_input: planes must be 1 or 3");
+  if (planes == 3) {
+    launch_pdl(pack_input_split_kernel, dim3(grid), dim3(256), 0, st, x, out, B, C, HW, cpad, gs);
+    return check_launch("pack_input_split");
+  }
   launch_pdl(pack_input_kernel, dim3(grid), dim3(256), 0, st, x, out, B, C, HW, cpad, gs);
   return check_launch("pack_input");
 }
@@ -1647,11 +1809,41 @@ __global__ void __launch_bounds__(256) downsum2x_kernel(const uint4* __restrict_
   }
 }
 
-int downsum2x_launch(const f16* dy, f16* dx, int N, int H, int W, int C, cudaStream_t st) {
-  B2E_REQUIRE(C % 8 == 0, B2E_UNSUPPORTED_SHAPE, "downsum2x: C %% 8");
+// split-f16 gradients: the four hi + lo values summed in fp32 and re-split (the hi planes summed as plain channels would
+// round their sum to 16 bits)
+__global__ void __launch_bounds__(256) downsum2x_split_kernel(const f16* __restrict__ dy, f16* __restrict__ dx, int N, int H,
+                                                              int W, int C) {
+  pdl_wait();
+  const int C8 = C / 8;
+  const int64_t total = (int64_t)N * H * W * C8;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int c = (int)(i % C8) * 8;
+    const int64_t p = i / C8;
+    const int w = (int)(p % W), h = (int)((p / W) % H);
+    const int64_t n = p / ((int64_t)W * H);
+    float acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+#pragma unroll
+    for (int dh = 0; dh < 2; ++dh)
+#pragma unroll
+      for (int dw = 0; dw < 2; ++dw) {
+        float f[8];
+        load_split8(dy + ((n * 2 * H + 2 * h + dh) * 2 * W + 2 * w + dw) * 3 * C + c, C, f);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) acc[j] += f[j];
+      }
+    store_split8(dx + p * 3 * C + c, C, acc);
+  }
+}
+
+int downsum2x_launch(const f16* dy, f16* dx, int N, int H, int W, int C, cudaStream_t st, int planes) {
+  B2E_REQUIRE(C % 8 == 0 && (planes == 1 || planes == 3), B2E_UNSUPPORTED_SHAPE, "downsum2x: C %% 8 / planes");
   const int64_t total = (int64_t)N * H * W * (C / 8);
   int grid = (int)((total + 255) / 256);
   if (grid > kNumSMs * 32) grid = kNumSMs * 32;
+  if (planes == 3) {
+    launch_pdl(downsum2x_split_kernel, dim3(grid), dim3(256), 0, st, dy, dx, N, H, W, C);
+    return check_launch("downsum2x_split");
+  }
   launch_pdl(downsum2x_kernel, dim3(grid), dim3(256), 0, st, (const uint4*)dy, (uint4*)dx, N, H, W, C / 8);
   return check_launch("downsum2x");
 }
@@ -1737,6 +1929,7 @@ int softmax_bwd_rows_launch(const f16* p, f16* dp, int64_t rows, int T, float sc
 
 // backward of (nearest code [straight-through] -> post_quant_conv -> im2col): dcols f16 [B][H][W][64] holds the gradient
 // w.r.t. im2col column t*L + c of every pixel; dz[b][k][h][w] = sum_c pq_w[c][k] * sum_t dcols[(h,w) - tap_t][t*L + c]
+template <bool SPLIT>   // split-f16 dcols ([hi | lo | hi] planes of 64 columns): value hi + lo
 __global__ void __launch_bounds__(256) vq_col2im_bwd_kernel(const f16* __restrict__ dcols, const float* __restrict__ pq_w,
                                                             float* __restrict__ dz, int B, int L, int H, int W,
                                                             const float* __restrict__ gs, const float* __restrict__ mask,
@@ -1753,8 +1946,8 @@ __global__ void __launch_bounds__(256) vq_col2im_bwd_kernel(const f16* __restric
     // forward: cols[(hh, ww)][t*L + c] = x[c][hh + t/3 - 1][ww + t%3 - 1]  ->  (hh, ww) = (h, w) - tap
     const int hh = h - (t / 3 - 1), ww = w - (t % 3 - 1);
     if (hh < 0 || hh >= H || ww < 0 || ww >= W) continue;
-    const f16* src = dcols + (((int64_t)b * H + hh) * W + ww) * 64 + t * L;
-    for (int c = 0; c < L; ++c) g[c] += f16_to_float(src[c]);
+    const f16* src = dcols + (((int64_t)b * H + hh) * W + ww) * (SPLIT ? 192 : 64) + t * L;
+    for (int c = 0; c < L; ++c) g[c] += SPLIT ? f16_to_float(src[c]) + f16_to_float(src[64 + c]) : f16_to_float(src[c]);
   }
   for (int k = 0; k < L; ++k) {
     float acc = 0.f;
@@ -1766,10 +1959,13 @@ __global__ void __launch_bounds__(256) vq_col2im_bwd_kernel(const f16* __restric
 }
 
 int vq_col2im_bwd_launch(const f16* dcols, const float* pq_w, float* dz, int B, int L, int H, int W, cudaStream_t st,
-                         const float* gs, const float* mask, int mask_batched) {
-  B2E_REQUIRE(L >= 1 && L <= 4 && 9 * L <= 64, B2E_UNSUPPORTED_SHAPE, "vq_col2im_bwd: latent channels %d", L);
+                         const float* gs, const float* mask, int mask_batched, int planes) {
+  B2E_REQUIRE(L >= 1 && L <= 4 && 9 * L <= 64 && (planes == 1 || planes == 3), B2E_UNSUPPORTED_SHAPE,
+              "vq_col2im_bwd: latent channels %d / planes %d", L, planes);
   const int64_t total = (int64_t)B * H * W;
-  launch_pdl(vq_col2im_bwd_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, st, dcols, pq_w, dz, B, L, H, W, gs, mask, mask_batched);
+  const dim3 grid((unsigned)((total + 255) / 256));
+  if (planes == 3) launch_pdl(vq_col2im_bwd_kernel<true>, grid, dim3(256), 0, st, dcols, pq_w, dz, B, L, H, W, gs, mask, mask_batched);
+  else launch_pdl(vq_col2im_bwd_kernel<false>, grid, dim3(256), 0, st, dcols, pq_w, dz, B, L, H, W, gs, mask, mask_batched);
   return check_launch("vq_col2im_bwd");
 }
 
@@ -2396,6 +2592,289 @@ int attention_split_tiled_launch(const f16* q, int q_plane, int q_col, const f16
   }
   launch_pdl(attention_split_tiled_kernel<false>, grid, dim3(kTaThreads), smem, st, a);
   return check_launch("attention_split_tiled");
+}
+
+// ------------------------------------------------------------------ fp32-accurate attention backward (single head)
+// Flash-style, fp32 on the CUDA cores, S = (q / sqrt(C)) k^T recomputed from the split q | k | v planes as the tiled forward
+// computes it (query pre-scaled in fp32), P = exp(S - m) / l never stored:
+//   stats kernel   (32-query blocks):  m, 1 / l over every key; D = rowsum(dO o O)
+//   dK / dV kernel (16-key blocks, every query tile):  dV += P^T dO ; dK += dS^T (q / sqrt(C)),  dS = P o (dO V^T - D)
+//   dQ kernel      (32-query blocks, every key tile):  dQ += dS K, times 1 / sqrt(C) at the end
+// Every output element belongs to one thread and sums in a fixed order: deterministic, no atomics.
+constexpr int kAbQ = 32, kAbK = 16, kAbThreads = 256;
+
+// rows [row0, row0 + rows) of a split tensor (value = plane 0 + plane 1, `plane` channels apart) -> fp32 smem [rows][ds]
+__device__ __forceinline__ void ab_load_tile(float* dst, int ds, const f16* src, int64_t row_pitch, int plane, int row0,
+                                             int rows, int d, float mul) {
+  const int d8 = d >> 3;
+  for (int i = threadIdx.x; i < rows * d8; i += blockDim.x) {
+    const int r = i / d8, c = (i - r * d8) * 8;
+    float f[8];
+    load_split8(src + (int64_t)(row0 + r) * row_pitch + c, plane, f);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) dst[r * ds + c + j] = f[j] * mul;
+  }
+}
+
+// the (32 query x 16 key) tile: P and dS = P o (dP - D) into smem [32][kAbK + 1]; st = per-query (m, 1 / l, D) in smem
+__device__ __forceinline__ void ab_scores(const float* Qs, const float* dOs, const float* Ks, const float* Vs, const float4* st,
+                                          float* Ps, float* dSs, int ds, int d) {
+  const int q = threadIdx.x >> 3, kk = (threadIdx.x & 7) * 2;
+  float s0 = 0.f, s1 = 0.f, p0 = 0.f, p1 = 0.f;
+  const float* qr = Qs + q * ds;
+  const float* orow = dOs + q * ds;
+  const float* k0 = Ks + kk * ds;
+  const float* v0 = Vs + kk * ds;
+  for (int c = 0; c < d; ++c) {
+    const float qv = qr[c], ov = orow[c];
+    s0 += qv * k0[c]; s1 += qv * k0[ds + c];
+    p0 += ov * v0[c]; p1 += ov * v0[ds + c];
+  }
+  const float4 r = st[q];
+  const float e0 = expf(s0 - r.x) * r.y, e1 = expf(s1 - r.x) * r.y;
+  Ps[q * (kAbK + 1) + kk] = e0; Ps[q * (kAbK + 1) + kk + 1] = e1;
+  dSs[q * (kAbK + 1) + kk] = e0 * (p0 - r.z); dSs[q * (kAbK + 1) + kk + 1] = e1 * (p1 - r.z);
+}
+
+// fp32 value pair -> split f16x2 planes at o, o + plane, o + 2 plane
+__device__ __forceinline__ void ab_store_pair(f16* o, int plane, float x, float y) {
+  const f16x2 hi = floats_to_f16x2(x, y);
+  const float2 hf = f16x2_to_float2(hi);
+  *reinterpret_cast<f16x2*>(o) = hi;
+  *reinterpret_cast<f16x2*>(o + plane) = floats_to_f16x2(__fsub_rn(x, hf.x), __fsub_rn(y, hf.y));
+  *reinterpret_cast<f16x2*>(o + 2 * plane) = hi;
+}
+// zero tail [C, P) of rows [row0, row0 + rows) of a split tensor, all planes
+__device__ __forceinline__ void ab_zero_tail(f16* base, int P, int C, int row0, int rows) {
+  const int pad = P - C;
+  for (int i = threadIdx.x; i < rows * pad * 3; i += blockDim.x) {
+    const int k = i % 3, r = i / 3, q = r / pad, c = r % pad;
+    base[(int64_t)(row0 + q) * 3 * P + k * P + C + c] = float_to_f16(0.f);
+  }
+}
+
+struct AttnBwdArgs {
+  const f16* qkv; const f16* o; const f16* d_o;
+  f16 *dq, *dk, *dv;
+  float4* stats;     // [N][T] (m, 1 / l, D, -)
+  int T, C, P;
+  float scale;
+};
+
+// 32 queries per block: online max / sum over 32-key tiles exactly as attention_split_tiled_kernel, then D
+__global__ void __launch_bounds__(kAbThreads) attention_split_bwd_stats_kernel(AttnBwdArgs a) {
+  pdl_wait();
+  extern __shared__ __align__(16) uint8_t ab_smem[];
+  const int d = a.C, ds = d + 1, n = blockIdx.z, q0 = blockIdx.x * kAbQ, tid = threadIdx.x;
+  float* Qs = reinterpret_cast<float*>(ab_smem);     // [32][ds]
+  float* Ks = Qs + kAbQ * ds;                        // [32][ds]
+  float* S = Ks + kAbQ * ds;                         // [32][33]
+  float* rowm = S + kAbQ * 33;
+  float* rowl = rowm + kAbQ;
+  const int64_t row = 9 * (int64_t)a.P;
+  const f16* base = a.qkv + (int64_t)n * a.T * row;
+  ab_load_tile(Qs, ds, base, row, 3 * a.P, q0, kAbQ, d, a.scale);
+  if (tid < kAbQ) { rowm[tid] = -INFINITY; rowl[tid] = 0.f; }
+  for (int k0 = 0; k0 < a.T; k0 += 32) {
+    __syncthreads();
+    ab_load_tile(Ks, ds, base + a.P, row, 3 * a.P, k0, 32, d, 1.f);
+    __syncthreads();
+    {
+      const int q = tid >> 3, kk = (tid & 7) * 4;
+      float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
+      const float* qr = Qs + q * ds;
+      const float* kr = Ks + kk * ds;
+      for (int c = 0; c < d; ++c) {
+        const float qv = qr[c];
+        s0 += qv * kr[c]; s1 += qv * kr[ds + c]; s2 += qv * kr[2 * ds + c]; s3 += qv * kr[3 * ds + c];
+      }
+      float* sr = S + q * 33 + kk;
+      sr[0] = s0; sr[1] = s1; sr[2] = s2; sr[3] = s3;
+    }
+    __syncthreads();
+    const int warp = tid >> 5, lane = tid & 31;
+    for (int q = warp; q < kAbQ; q += kAbThreads / 32) {
+      const float sv = S[q * 33 + lane];
+      float mx = sv;
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+      const float mold = rowm[q], mnew = fmaxf(mold, mx);
+      const float ps = warp_sum(expf(sv - mnew));
+      if (lane == 0) { rowl[q] = rowl[q] * (mold == -INFINITY ? 0.f : expf(mold - mnew)) + ps; rowm[q] = mnew; }
+    }
+  }
+  __syncthreads();
+  // D = rowsum(dO o O): one warp per query row
+  const int warp = tid >> 5, lane = tid & 31;
+  const int64_t orow = 3 * (int64_t)a.P;
+  for (int q = warp; q < kAbQ; q += kAbThreads / 32) {
+    const f16* op = a.o + ((int64_t)n * a.T + q0 + q) * orow;
+    const f16* gp = a.d_o + ((int64_t)n * a.T + q0 + q) * orow;
+    float acc = 0.f;
+    for (int c = lane * 8; c < d; c += 256) {
+      float of[8], gf[8];
+      load_split8(op + c, a.P, of);
+      load_split8(gp + c, a.P, gf);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) acc = fmaf(of[j], gf[j], acc);
+    }
+    acc = warp_sum(acc);
+    if (lane == 0) a.stats[(int64_t)n * a.T + q0 + q] = make_float4(rowm[q], 1.f / rowl[q], acc, 0.f);
+  }
+}
+
+// smem of the dK / dV and dQ kernels: q, dO tiles [32][ds], k, v tiles [16][ds], P and dS [32][17], stats [32]
+__host__ __device__ inline size_t ab_tile_smem(int d) {
+  return sizeof(float) * ((size_t)(2 * kAbQ + 2 * kAbK) * (d + 1) + 2 * kAbQ * (kAbK + 1)) + sizeof(float4) * kAbQ;
+}
+
+// 16 keys per block; a thread owns a column pair of dK and dV for a group of keys
+__global__ void __launch_bounds__(kAbThreads, 1) attention_split_bwd_dkv_kernel(AttnBwdArgs a) {
+  pdl_wait();
+  extern __shared__ __align__(16) uint8_t ab_smem[];
+  const int d = a.C, ds = d + 1, n = blockIdx.z, k0 = blockIdx.x * kAbK, tid = threadIdx.x;
+  float4* st = reinterpret_cast<float4*>(ab_smem);
+  float* Qs = reinterpret_cast<float*>(st + kAbQ);
+  float* dOs = Qs + kAbQ * ds;
+  float* Ks = dOs + kAbQ * ds;
+  float* Vs = Ks + kAbK * ds;
+  float* Ps = Vs + kAbK * ds;
+  float* dSs = Ps + kAbQ * (kAbK + 1);
+  const int64_t row = 9 * (int64_t)a.P, orow = 3 * (int64_t)a.P;
+  const f16* base = a.qkv + (int64_t)n * a.T * row;
+  ab_load_tile(Ks, ds, base + a.P, row, 3 * a.P, k0, kAbK, d, 1.f);
+  ab_load_tile(Vs, ds, base + 2 * a.P, row, 3 * a.P, k0, kAbK, d, 1.f);
+  const int half = d >> 1, ngroups = half >= kAbThreads ? 1 : kAbThreads / half;
+  const int cp = tid % half, kg = tid / half, kper = (kAbK + ngroups - 1) / ngroups;
+  const bool owner = kg < ngroups;
+  const int c0 = 2 * cp;
+  float dvx[kAbK], dvy[kAbK], dkx[kAbK], dky[kAbK];
+#pragma unroll
+  for (int i = 0; i < kAbK; ++i) dvx[i] = dvy[i] = dkx[i] = dky[i] = 0.f;
+  for (int q0 = 0; q0 < a.T; q0 += kAbQ) {
+    __syncthreads();
+    ab_load_tile(Qs, ds, base, row, 3 * a.P, q0, kAbQ, d, a.scale);
+    ab_load_tile(dOs, ds, a.d_o + (int64_t)n * a.T * orow, orow, a.P, q0, kAbQ, d, 1.f);
+    if (tid < kAbQ) st[tid] = a.stats[(int64_t)n * a.T + q0 + tid];
+    __syncthreads();
+    ab_scores(Qs, dOs, Ks, Vs, st, Ps, dSs, ds, d);
+    __syncthreads();
+    if (owner) {
+      for (int q = 0; q < kAbQ; ++q) {
+        const float ox = dOs[q * ds + c0], oy = dOs[q * ds + c0 + 1];
+        const float qx = Qs[q * ds + c0], qy = Qs[q * ds + c0 + 1];
+#pragma unroll
+        for (int i = 0; i < kAbK; ++i) {
+          const int k = kg * kper + i;
+          if (i < kper && k < kAbK) {
+            const float p = Ps[q * (kAbK + 1) + k], s = dSs[q * (kAbK + 1) + k];
+            dvx[i] = fmaf(p, ox, dvx[i]); dvy[i] = fmaf(p, oy, dvy[i]);
+            dkx[i] = fmaf(s, qx, dkx[i]); dky[i] = fmaf(s, qy, dky[i]);
+          }
+        }
+      }
+    }
+  }
+  if (owner) {
+#pragma unroll
+    for (int i = 0; i < kAbK; ++i) {
+      const int k = kg * kper + i;
+      if (i < kper && k < kAbK) {
+        const int64_t r = ((int64_t)n * a.T + k0 + k) * orow + c0;
+        ab_store_pair(a.dv + r, a.P, dvx[i], dvy[i]);
+        ab_store_pair(a.dk + r, a.P, dkx[i], dky[i]);
+      }
+    }
+  }
+  if (a.P > a.C) {
+    ab_zero_tail(a.dk + (int64_t)n * a.T * orow, a.P, a.C, k0, kAbK);
+    ab_zero_tail(a.dv + (int64_t)n * a.T * orow, a.P, a.C, k0, kAbK);
+  }
+}
+
+// 32 queries per block; a thread owns a column pair of dQ for a group of queries
+__global__ void __launch_bounds__(kAbThreads, 1) attention_split_bwd_dq_kernel(AttnBwdArgs a) {
+  pdl_wait();
+  extern __shared__ __align__(16) uint8_t ab_smem[];
+  const int d = a.C, ds = d + 1, n = blockIdx.z, q0 = blockIdx.x * kAbQ, tid = threadIdx.x;
+  float4* st = reinterpret_cast<float4*>(ab_smem);
+  float* Qs = reinterpret_cast<float*>(st + kAbQ);
+  float* dOs = Qs + kAbQ * ds;
+  float* Ks = dOs + kAbQ * ds;
+  float* Vs = Ks + kAbK * ds;
+  float* Ps = Vs + kAbK * ds;
+  float* dSs = Ps + kAbQ * (kAbK + 1);
+  const int64_t row = 9 * (int64_t)a.P, orow = 3 * (int64_t)a.P;
+  const f16* base = a.qkv + (int64_t)n * a.T * row;
+  ab_load_tile(Qs, ds, base, row, 3 * a.P, q0, kAbQ, d, a.scale);
+  ab_load_tile(dOs, ds, a.d_o + (int64_t)n * a.T * orow, orow, a.P, q0, kAbQ, d, 1.f);
+  if (tid < kAbQ) st[tid] = a.stats[(int64_t)n * a.T + q0 + tid];
+  const int half = d >> 1, ngroups = half >= kAbThreads ? 1 : kAbThreads / half;
+  const int cp = tid % half, qg = tid / half, qper = (kAbQ + ngroups - 1) / ngroups;
+  const bool owner = qg < ngroups;
+  const int c0 = 2 * cp;
+  float ax[kAbQ], ay[kAbQ];
+#pragma unroll
+  for (int i = 0; i < kAbQ; ++i) ax[i] = ay[i] = 0.f;
+  for (int k0 = 0; k0 < a.T; k0 += kAbK) {
+    __syncthreads();
+    ab_load_tile(Ks, ds, base + a.P, row, 3 * a.P, k0, kAbK, d, 1.f);
+    ab_load_tile(Vs, ds, base + 2 * a.P, row, 3 * a.P, k0, kAbK, d, 1.f);
+    __syncthreads();
+    ab_scores(Qs, dOs, Ks, Vs, st, Ps, dSs, ds, d);
+    __syncthreads();
+    if (owner) {
+      for (int k = 0; k < kAbK; ++k) {
+        const float kx = Ks[k * ds + c0], ky = Ks[k * ds + c0 + 1];
+#pragma unroll
+        for (int i = 0; i < kAbQ; ++i) {
+          const int q = qg * qper + i;
+          if (i < qper && q < kAbQ) {
+            const float s = dSs[q * (kAbK + 1) + k];
+            ax[i] = fmaf(s, kx, ax[i]); ay[i] = fmaf(s, ky, ay[i]);
+          }
+        }
+      }
+    }
+  }
+  if (owner) {
+#pragma unroll
+    for (int i = 0; i < kAbQ; ++i) {
+      const int q = qg * qper + i;
+      if (i < qper && q < kAbQ) ab_store_pair(a.dq + ((int64_t)n * a.T + q0 + q) * orow + c0, a.P, ax[i] * a.scale, ay[i] * a.scale);
+    }
+  }
+  if (a.P > a.C) ab_zero_tail(a.dq + (int64_t)n * a.T * orow, a.P, a.C, q0, kAbQ);
+}
+
+int attention_split_bwd_launch(const f16* qkv, const f16* o, const f16* d_o, f16* dq, f16* dk, f16* dv, float* stats, int N,
+                               int T, int C, int P, cudaStream_t st) {
+  B2E_REQUIRE(N >= 1 && T >= kAbQ && T % kAbQ == 0 && C % 8 == 0 && C >= 8 && C <= 512 && P >= C && P % 8 == 0,
+              B2E_UNSUPPORTED_SHAPE, "attention backward (fp32-accurate): unsupported T=%d C=%d P=%d", T, C, P);
+  B2E_REQUIRE(qkv && o && d_o && dq && dk && dv && stats, B2E_INVALID_ARG, "attention backward (fp32-accurate): null pointer");
+  AttnBwdArgs a;
+  a.qkv = qkv; a.o = o; a.d_o = d_o; a.dq = dq; a.dk = dk; a.dv = dv; a.stats = reinterpret_cast<float4*>(stats);
+  a.T = T; a.C = C; a.P = P; a.scale = 1.0f / sqrtf((float)C);
+  const size_t smem_st = sizeof(float) * ((size_t)2 * kAbQ * (C + 1) + kAbQ * 33 + 2 * kAbQ);
+  const size_t smem_t = ab_tile_smem(C);
+  static size_t attr[3] = {0, 0, 0};
+  if (smem_st > attr[0]) {
+    B2E_CUDA(cudaFuncSetAttribute(attention_split_bwd_stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_st));
+    attr[0] = smem_st;
+  }
+  if (smem_t > attr[1]) {
+    B2E_CUDA(cudaFuncSetAttribute(attention_split_bwd_dkv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_t));
+    B2E_CUDA(cudaFuncSetAttribute(attention_split_bwd_dq_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_t));
+    attr[1] = smem_t;
+  }
+  launch_pdl(attention_split_bwd_stats_kernel, dim3(T / kAbQ, 1, N), dim3(kAbThreads), smem_st, st, a);
+  int rc = check_launch("attention_split_bwd_stats");
+  if (rc) return rc;
+  launch_pdl(attention_split_bwd_dkv_kernel, dim3(T / kAbK, 1, N), dim3(kAbThreads), smem_t, st, a);
+  rc = check_launch("attention_split_bwd_dkv");
+  if (rc) return rc;
+  launch_pdl(attention_split_bwd_dq_kernel, dim3(T / kAbQ, 1, N), dim3(kAbThreads), smem_t, st, a);
+  return check_launch("attention_split_bwd_dq");
 }
 
 int attention_launch(const f16* qkv, f16* out, int N, int T, int C, int P, int heads, cudaStream_t st) {

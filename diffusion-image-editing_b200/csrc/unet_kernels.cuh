@@ -47,7 +47,9 @@ struct GNBwdArgs {
   int chunks;
   int silu;
 };
-int gn_bwd_launch(const GNBwdArgs& a, cudaStream_t st);
+// planes = 3: x / da / add / dx are split-f16 tensors of the fp32-accurate mode ([hi | lo | hi] planes of P / Pda channels,
+// value hi + lo), read in fp32, dx re-split
+int gn_bwd_launch(const GNBwdArgs& a, cudaStream_t st, int planes = 1);
 int gn_chunks(int HW, int C);
 int gn_launch(const GNArgs& a, cudaStream_t st);
 // fused GroupNorm: only the (scale, shift) coefficients, float2 [N][P0 + P1]; the consumer convolution applies them to its
@@ -59,7 +61,7 @@ int gn_finalize_launch(const float* tile_stats, float* chan_stats, int N, int C,
 
 // x fp32 NCHW (B,C,H,W) -> f16 NHWC (B,H,W,cpad), zero padded channels; im2col: channel t*C + c of a pixel holds
 // x[c] at 3x3 tap t (zero outside the image), so that a 3x3 convolution becomes a 1x1 one
-// planes = 3 (im2col only): split-f16 output [hi | lo | hi] of cpad channels each (fp32-accurate mode)
+// planes = 3: split-f16 output [hi | lo | hi] of cpad channels each (fp32-accurate mode)
 // gs (plain layout only): gradient scale record of grad_scale_launch, x is multiplied by gs[0]
 // im2col only: mask (fp32 (1 | B, C, H, W), mask_batched) replaces x by 1 - mask * x, and shift / scale (C floats each,
 // device) apply (v - shift[c]) / scale[c] (the LPIPS scaling layer) before the zero padding of the taps
@@ -108,13 +110,14 @@ int clip_embed_launch(const int64_t* ids, const float* tok, const float* pos, f1
 int quick_gelu_launch(const f16* in, f16* out, int64_t numel, cudaStream_t st, int planes = 1, int C = 0);
 int unpad_rows_f32_launch(const f16* x, float* out, int B, int L, int Lpad, int D, cudaStream_t st, int planes = 1);
 
-// backward helpers of the decoder (f16 NHWC gradients)
-int downsum2x_launch(const f16* dy, f16* dx, int N, int H, int W, int C, cudaStream_t st);
+// backward helpers of the decoder (f16 NHWC gradients; planes = 3: split-f16 gradients of the fp32-accurate mode,
+// [hi | lo | hi] planes of C (dcols: 64) channels per pixel, summed in fp32 and re-split)
+int downsum2x_launch(const f16* dy, f16* dx, int N, int H, int W, int C, cudaStream_t st, int planes = 1);
 int transpose_window_launch(const f16* src, f16* dst, int N, int R, int Cc, int src_pitch, int col0, cudaStream_t st);
 int softmax_bwd_rows_launch(const f16* p, f16* dp, int64_t rows, int T, float scale, cudaStream_t st);
 // mask (fp32 (1 | B, L, H, W), mask_batched): the chain of an input x -> 1 - mask * x, dz *= -mask
 int vq_col2im_bwd_launch(const f16* dcols, const float* pq_w, float* dz, int B, int L, int H, int W, cudaStream_t st,
-                         const float* gs = nullptr, const float* mask = nullptr, int mask_batched = 0);
+                         const float* gs = nullptr, const float* mask = nullptr, int mask_batched = 0, int planes = 1);
 
 // VQModel.decode front: nearest codebook entry + 1x1 post_quant_conv; z, out fp32 NCHW (B, L <= 4, HW)
 int vq_quantize_launch(const float* z, const float* codebook, int n_codes, const float* pq_w, const float* pq_b, float* out,
@@ -186,5 +189,14 @@ int attention_split_launch(const f16* qkv, f16* out, int N, int T, int C, int P,
 int attention_split_tiled_launch(const f16* q, int q_plane, int q_col, const f16* kv, int k_plane, int k_col, int v_col, f16* out,
                                  int o_plane, int o_real, int N, int Tq, int Tk_rows, int valid_k, int heads, int d, cudaStream_t st,
                                  int causal = 0);
+// backward of the single-head fp32-accurate self-attention O = softmax(Q K^T / sqrt(C)) V, fp32 on the CUDA cores, flash
+// style (S recomputed, P never stored): qkv [N][T] rows of [hi | lo | hi] planes of 3P channels (q | k | v blocks of P
+// columns), o / d_o / dq / dk / dv [N][T] rows of [hi | lo | hi] planes of P channels (C real; the tails of dq / dk / dv are
+// zeroed).  stats: scratch of 4 floats per query row (row max, 1 / row sum, D = rowsum(dO o O)).  Deterministic: every
+// output element is owned by one thread, no atomics.  T % 32 == 0, C % 8 == 0, 8 <= C <= 512.
+int attention_split_bwd_launch(const f16* qkv, const f16* o, const f16* d_o, f16* dq, f16* dk, f16* dv, float* stats, int N,
+                               int T, int C, int P, cudaStream_t st);
+// FLOPs of attention_split_bwd_launch per image: the stats pass (S), dK / dV (S, dP, dV, dK) and dQ (S, dP, dQ)
+inline double attention_split_bwd_flops(int T, int C) { return 8.0 * 2.0 * (double)T * T * C; }
 
 }  // namespace b2e

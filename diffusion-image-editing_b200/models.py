@@ -27,19 +27,30 @@ def create_diffusion_model(name: str, sample_clipping: bool = True, *, max_batch
                            vq_config: Optional[dict] = None, vq_state_dict: Optional[dict] = None, guidance_module=None,
                            decoder_grad: bool = True, tokenizer=None, text_encoder=None, precision: Optional[str] = None,
                            with_encoder: bool = True, text_encoder_config: Optional[dict] = None,
-                           text_encoder_state_dict: Optional[dict] = None, encoder_precision: Optional[str] = None):
+                           text_encoder_state_dict: Optional[dict] = None, encoder_precision: Optional[str] = None,
+                           decoder_grad_precision: Optional[str] = None):
     """``name``: "ddpm" (google/ddpm-celebahq-256 layout), "sd" (Stable Diffusion 1.x layout: native conditional UNet
     + native KL decoder with gradient; ``vqvae=`` substitutes the vae, ``tokenizer=`` / ``text_encoder=`` are the
     caller's CLIP modules) or "ldm" (CompVis/ldm-celebahq-256 layout: native UNet on
     the 64x64x3 latent + native VQ decoder (forward + latent gradient) and encoder; ``vqvae=`` substitutes the caller's VQ autoencoder module
     (encode().latents / decode().sample, as in the reference's pipeline object); ``guidance_module=`` is the
     differentiable decoder used when guidance runs through decode).  ``precision="fp32"`` selects the fp32-accurate
-    (split-f16) noise predictor (all three families) and VQ / KL decoder (forward only: guidance through the decoder uses the fp16 engine).  ``with_encoder`` (default) also builds the native VQ / KL encoder behind
+    (split-f16) noise predictor (all three families) and VQ / KL decoder.  Guidance through that decoder
+    (``decoder_grad=True``) follows ``decoder_grad_precision``: ``None`` (default) keeps the split decoder forward-only
+    and differentiates a second, 16-bit decoder engine with the same weights (``guidance_vqvae`` / ``guidance_vae``,
+    gradient within 3e-3 relative RMS of fp32); ``"fp32"`` (needs ``precision="fp32"``) puts the split decoder itself in
+    gradient mode - an fp32-accurate guidance gradient, no second engine.  ``with_encoder`` (default) also builds the native VQ / KL encoder behind
     ``LDM.encode`` / ``SD.encode``.  ``encoder_precision="fp32"`` selects the fp32-accurate native VQ / KL encoder and
     native CLIP text encoder (the inputs of a real-image or prompt-conditioned edit); it does not apply to a caller's
     ``vqvae=`` / ``text_encoder=`` and does not follow ``precision`` (``None``: the 16-bit type)."""
     if encoder_precision is not None:
         _C.resolve_precision(encoder_precision, "create_diffusion_model(encoder_precision)")   # refuse before building anything
+    split_grad = False
+    if decoder_grad_precision is not None:
+        split_grad = _C.resolve_precision(decoder_grad_precision, "create_diffusion_model(decoder_grad_precision)")[0] == "fp32"
+        if not split_grad or precision != "fp32":
+            raise ValueError(f"create_diffusion_model: decoder_grad_precision must be None or 'fp32' with precision='fp32' "
+                             f"(got {decoder_grad_precision!r} with precision={precision!r})")
     device = get_device()
     if name == "ddpm":
         unet = UNet2DModel(**(unet_config or DDPM256_CONFIG), max_batch=max_batch, device=device, precision=precision)
@@ -69,8 +80,8 @@ def create_diffusion_model(name: str, sample_clipping: bool = True, *, max_batch
                 vqvae.init_random(seed + 1)
             # decoder weights for a gradient twin (random init: the decoder part of what init_random just loaded)
             vq_sd = vq_state_dict if vq_state_dict is not None else vqvae.random_state_dict(seed + 1)
-            if decoder_grad and precision == "fp32":
-                # the fp32-accurate (split-operand) decoder is forward-only: guidance THROUGH the decoder runs on a second,
+            if decoder_grad and precision == "fp32" and not split_grad:
+                # default of the fp32-accurate (split-operand) decoder: guidance THROUGH the decoder runs on a second,
                 # f16-operand engine with the same weights (decoder gradient within 3e-3 relative RMS of fp32 autograd)
                 guidance_vqvae = VQModel(**(vq_config or LDM_VQ_CONFIG), max_batch=max_batch, device=device, with_encoder=False,
                                          precision="fp16")
@@ -103,7 +114,7 @@ def create_diffusion_model(name: str, sample_clipping: bool = True, *, max_batch
                 vae.init_random(seed + 1)
             vq_sd = vq_state_dict if vq_state_dict is not None else vae.random_state_dict(seed + 1)
             guidance_vae = None
-            if decoder_grad and precision == "fp32":      # see the "ldm" branch: f16-operand gradient twin
+            if decoder_grad and precision == "fp32" and not split_grad:      # see the "ldm" branch: f16-operand gradient twin
                 guidance_vae = AutoencoderKL(**(vq_config or SD_VAE_CONFIG), max_batch=max_batch, device=device, with_encoder=False,
                                              precision="fp16")
                 guidance_vae.load_state_dict(vq_sd, strict=False)

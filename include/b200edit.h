@@ -490,6 +490,16 @@ int b2e_attention_f16(const void* q, int64_t q_pitch, int64_t q_col, const void*
                       int64_t valid_k, int64_t heads, int64_t head_dim, int causal, int path, int softmax_warps,
                       void* stream);
 
+/* Test hook for the backward of the fp32-accurate single-head self-attention O = softmax(Q K^T / sqrt(C)) V (the VQ / KL
+ * decoders' mid-block attention in gradient mode): the flash-style fp32 kernels of the decoder backward alone.  All tensors
+ * are split rows of the fp32-accurate mode, [hi | lo | hi] planes of `pitch` channels each (value hi + lo), b2e_act_dtype:
+ *   qkv  (B, T, 9 * pitch): q | k | v blocks at columns 0 / pitch / 2 * pitch of every plane (C real channels each);
+ *   o    (B, T, 3 * pitch): the forward output; d_o (B, T, 3 * pitch): d(loss)/dO;
+ *   dq, dk, dv (B, T, 3 * pitch): the split gradients, tails [C, pitch) written with zeros.
+ * T % 32 == 0, C % 8 == 0, 8 <= C <= 512.  Deterministic (no atomics).  Allocates its scratch itself and synchronises. */
+int b2e_attention_bwd_fp32(const void* qkv, const void* o, const void* d_o, void* dq, void* dk, void* dv, int64_t B, int64_t T,
+                           int64_t C, int64_t pitch, void* stream);
+
 /* Test hook for the face parser's label kernel: x (N,Hi,Wi,planes*P) 16-bit NHWC (b2e_act_dtype; planes = 3: split
  * [hi | lo | hi] channel planes, value hi + lo) -> labels int64 (N,S,S), the argmax over the first K channels of the
  * align_corners bilinear upsampling to S x S. */
