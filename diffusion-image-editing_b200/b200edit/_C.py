@@ -64,11 +64,11 @@ class ClipConfig(C.Structure):
 class ResNetConfig(C.Structure):
     _fields_ = [("input_size", C.c_int32), ("in_channels", C.c_int32), ("bottleneck", C.c_int32),
                 ("layers", C.c_int32 * 4), ("width", C.c_int32), ("num_classes", C.c_int32), ("head", C.c_int32),
-                ("precision", C.c_int32)]
+                ("precision", C.c_int32), ("grad_precision", C.c_int32)]
 
 
 class LpipsConfig(C.Structure):
-    _fields_ = [("input_size", C.c_int32), ("precision", C.c_int32)]
+    _fields_ = [("input_size", C.c_int32), ("precision", C.c_int32), ("grad_precision", C.c_int32)]
 
 
 _P, _I64, _I, _F, _SZ = C.c_void_p, C.c_int64, C.c_int, C.c_float, C.c_size_t
@@ -211,3 +211,16 @@ def resolve_precision(precision, who: str):
                              f"(use precision=None / {fast!r} / 'fp32')")
         return fast, 0
     raise ValueError(f"{who}: precision must be '{fast}' or 'fp32' (got {precision!r})")
+
+
+def resolve_grad_precision(grad_precision, precision, who: str) -> int:
+    """-> b2e config value of a loss network's ``grad_precision``.  None: 0, the 16-bit backward; "fp32": 1, the
+    fp32-accurate backward (split hi + lo gradients and dgrad weights), which needs the fp32-accurate forward
+    (``precision`` "fp32", as resolve_precision names it).  Anything else raises ValueError."""
+    if grad_precision is None:
+        return 0
+    if grad_precision != "fp32":
+        raise ValueError(f"{who}: grad_precision must be None or 'fp32' (got {grad_precision!r})")
+    if precision != "fp32":
+        raise ValueError(f"{who}: grad_precision='fp32' needs precision='fp32' (got precision={precision!r})")
+    return 1

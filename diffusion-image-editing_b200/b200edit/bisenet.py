@@ -28,19 +28,21 @@ def _fold(w, sd, bn, eps=1e-5):
 class BiSeNet(Engine):
     differentiable = False
 
-    def __init__(self, n_classes=19, input_size=512, max_batch=1, device="cuda", precision=None):
+    def __init__(self, n_classes=19, input_size=512, max_batch=1, device="cuda", precision=None, grad_precision=None):
         """precision: None / "fp16" - f16 operands throughout; "fp32" - fp32-accurate FORWARD (split f16 operands), so
-        the ReLU / max-pool masks the backward pass routes gradients with are those of the fp32 network (see
-        b200edit.resnet.ResNet)."""
-        _C.require_device()
+        the ReLU / max-pool masks the backward pass routes gradients with are those of the fp32 network.  grad_precision:
+        None - 16-bit backward; "fp32" (needs precision="fp32") - fp32-accurate backward (see b200edit.resnet.ResNet)."""
         self.precision, precision_cfg = _C.resolve_precision(precision, "BiSeNet")
+        grad_cfg = _C.resolve_grad_precision(grad_precision, self.precision, "BiSeNet")
+        _C.require_device()
+        self.grad_precision = grad_precision
         self.config = SimpleNamespace(n_classes=n_classes, input_size=input_size, in_channels=3, sample_size=input_size,
                                       out_channels=n_classes)
         cfg = ResNetConfig()
         cfg.input_size, cfg.in_channels, cfg.bottleneck, cfg.width, cfg.num_classes, cfg.head = input_size, 3, 0, 64, n_classes, 1
         for i in range(4):
             cfg.layers[i] = 2
-        cfg.precision = precision_cfg
+        cfg.precision, cfg.grad_precision = precision_cfg, grad_cfg
         self._create(lib.b2e_resnet_create, cfg, max_batch, device)
 
     def enable_grad(self, enable: bool = True):
@@ -148,13 +150,16 @@ class MultiResBiSeNet:
 
     ``precision``: None - forward-only engines (mask creation: an argmax) run f16 operands, the differentiated engines
     the fp32-accurate forward ("fp32"), so the guidance gradient has the fp32 network's ReLU / max-pool masks;
-    "fp16" / "fp32" force one mode for both."""
+    "fp16" / "fp32" force one mode for both.  ``grad_precision`` applies to the differentiated engines only: None - their
+    backward runs on 16-bit operands; "fp32" - fp32-accurate backward (needs their forward to be fp32-accurate, i.e.
+    ``precision`` None or "fp32")."""
 
-    def __init__(self, n_classes=19, max_batch=1, device="cuda", seed=0, precision=None):
+    def __init__(self, n_classes=19, max_batch=1, device="cuda", seed=0, precision=None, grad_precision=None):
         self.n_classes, self.max_batch, self.device, self.seed = n_classes, int(max_batch), device, seed
         if precision not in (None, "fp16", "fp32"):
             raise ValueError(f"MultiResBiSeNet: precision must be None, 'fp16' or 'fp32' (got {precision!r})")
-        self.precision = precision
+        _C.resolve_grad_precision(grad_precision, precision or "fp32", "MultiResBiSeNet")
+        self.precision, self.grad_precision = precision, grad_precision
         self._folded = None      # engine-format state dict (BatchNorm folded); None -> seeded random init
         self._engines = {}
 
@@ -171,7 +176,8 @@ class MultiResBiSeNet:
             if size % 32 or size < 64:
                 raise ValueError(f"BiSeNet: input resolution must be a multiple of 32 and >= 64 (got {size})")
             precision = self.precision or ("fp32" if grad else "fp16")
-            e = BiSeNet(self.n_classes, size, max_batch=self.max_batch, device=self.device, precision=precision)
+            e = BiSeNet(self.n_classes, size, max_batch=self.max_batch, device=self.device, precision=precision,
+                        grad_precision=self.grad_precision if grad else None)
             if self._folded is not None:
                 e.load_state_dict(self._folded)
             else:

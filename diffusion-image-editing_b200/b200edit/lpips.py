@@ -32,17 +32,20 @@ class LPIPS(Engine):
     _ref = None             # the reference tensor whose features the engine holds (kept alive: identity check)
     _mask = None            # the mask the engine reads in the backward of the last forward (kept alive)
 
-    def __init__(self, net="vgg", input_size=256, max_batch=1, device="cuda", precision="fp32"):
+    def __init__(self, net="vgg", input_size=256, max_batch=1, device="cuda", precision="fp32", grad_precision=None):
         """precision: "fp32" (default) - fp32-accurate FORWARD (split 16-bit operands, three tensor-core products per
         GEMM), so that the ReLU / max-pool masks of the input gradient agree with an fp32 evaluation; None / "fp16" - 16-bit
-        operands throughout.  The backward pass runs on 16-bit operands either way."""
+        operands throughout.  grad_precision: None - the backward pass runs on 16-bit operands; "fp32" (needs
+        precision="fp32") - fp32-accurate backward (split gradients and dgrad weights); the distance is the same either way."""
         if net != "vgg":
             raise ValueError(f"LPIPS: only net='vgg' is implemented (got {net!r})")
-        _C.require_device()
         self.precision, precision_cfg = _C.resolve_precision(precision, "LPIPS")
+        grad_cfg = _C.resolve_grad_precision(grad_precision, self.precision, "LPIPS")
+        _C.require_device()
+        self.grad_precision = grad_precision
         self.config = SimpleNamespace(net=net, input_size=input_size, sample_size=input_size, in_channels=3, out_channels=1)
         cfg = LpipsConfig()
-        cfg.input_size, cfg.precision = input_size, precision_cfg
+        cfg.input_size, cfg.precision, cfg.grad_precision = input_size, precision_cfg, grad_cfg
         self._create(lib.b2e_lpips_create, cfg, max_batch, device)
 
     # ------------------------------------------------------------------ parameters

@@ -22,12 +22,16 @@ class ResNet(Engine):
     """``logits = net(image)``; image (B, C, S, S) fp32 CUDA, S a power of two >= 64."""
 
     def __init__(self, block="bottleneck", layers=RESNET50_LAYERS, num_classes=80, input_size=256, in_channels=3, width=64,
-                 max_batch=8, device="cuda", precision=None):
+                 max_batch=8, device="cuda", precision=None, grad_precision=None):
         """precision: None / "fp16" - f16 operands throughout; "fp32" - fp32-accurate FORWARD (split f16 operands, three
         tensor-core products per GEMM) so that the ReLU / max-pool masks of the input gradient agree with an fp32 evaluation
-        of the network; the backward pass stays on f16 operands."""
-        _C.require_device()
+        of the network.  grad_precision: None - the backward pass stays on f16 operands; "fp32" (needs precision="fp32") -
+        fp32-accurate backward too (split gradients through split dgrad weights, fp32 element-wise backward kernels); the
+        forward is the same either way."""
         self.precision, precision_cfg = _C.resolve_precision(precision, "ResNet")
+        grad_cfg = _C.resolve_grad_precision(grad_precision, self.precision, "ResNet")
+        _C.require_device()
+        self.grad_precision = grad_precision
         if block not in ("bottleneck", "basic"):
             raise ValueError("ResNet: block must be 'bottleneck' or 'basic'")
         self.config = SimpleNamespace(block=block, layers=tuple(layers), num_classes=num_classes, input_size=input_size,
@@ -37,7 +41,7 @@ class ResNet(Engine):
         for i in range(4):
             cfg.layers[i] = layers[i]
         cfg.width, cfg.num_classes = width, num_classes
-        cfg.precision = precision_cfg
+        cfg.precision, cfg.grad_precision = precision_cfg, grad_cfg
         self._create(lib.b2e_resnet_create, cfg, max_batch, device)
 
     # ------------------------------------------------------------------ parameters
@@ -103,9 +107,10 @@ class ResNet(Engine):
         return self._profile(x, None, torch.empty(self._out_shape(x.shape[0]), dtype=torch.float32, device=x.device))
 
 
-def resnet50_predictor(num_classes=80, input_size=256, max_batch=8, state_dict=None, seed=0, precision=None):
+def resnet50_predictor(num_classes=80, input_size=256, max_batch=8, state_dict=None, seed=0, precision=None, grad_precision=None):
     """The attribute predictor of src/models.py:69-77 (``models.resnet50()`` with ``fc = Linear(2048, 40 * 2)``)."""
-    net = ResNet("bottleneck", RESNET50_LAYERS, num_classes, input_size, max_batch=max_batch, precision=precision)
+    net = ResNet("bottleneck", RESNET50_LAYERS, num_classes, input_size, max_batch=max_batch, precision=precision,
+                 grad_precision=grad_precision)
     if state_dict is not None:
         net.load_torchvision_state_dict(state_dict)
     else:

@@ -80,7 +80,10 @@ int maxpool2x2_launch(const f16* x, f16* y, uint16_t* idx, int N, int H, int W, 
   return check_launch("maxpool2x2");
 }
 
-// gx[p] = (x[p] > 0) * (gy[window of p] if p is the window's recorded arg-max else 0); x = the pooled (ReLU) activation
+// gx[p] = (x[p] > 0) * (gy[window of p] if p is the window's recorded arg-max else 0); x = the pooled (ReLU) activation.
+// SPLIT_G: gy / gx are split gradients [hi | lo | hi] (pixel pitch 3 C); every input takes at most one window's value, so
+// the planes are selected as they are (exact)
+template <bool SPLIT_G>
 __global__ void __launch_bounds__(256) maxpool2x2_bwd_kernel(const f16* __restrict__ x, const uint16_t* __restrict__ idx,
                                                              const f16* __restrict__ gy, f16* __restrict__ gx, int N, int H,
                                                              int W, int C8, int xplanes) {
@@ -96,8 +99,14 @@ __global__ void __launch_bounds__(256) maxpool2x2_bwd_kernel(const f16* __restri
     const int64_t o = (((int64_t)n * Ho + (ih >> 1)) * Wo + (iw >> 1)) * C8 + s;
     const uint32_t a = __ldg(idx + o);
     const uint32_t t = (uint32_t)((ih & 1) * 2 + (iw & 1));
-    float g[8], xv[8];
-    unpack8l(__ldg(reinterpret_cast<const uint4*>(gy) + o), g);
+    float g[8], xv[8], gl[8];
+    if (SPLIT_G) {
+      const int64_t po = (o / C8) * 3 * C8 + s;
+      unpack8l(__ldg(reinterpret_cast<const uint4*>(gy) + po), g);
+      unpack8l(__ldg(reinterpret_cast<const uint4*>(gy) + po + C8), gl);
+    } else {
+      unpack8l(__ldg(reinterpret_cast<const uint4*>(gy) + o), g);
+    }
     const f16* xp = x + ((i / C8) * (int64_t)(xplanes * C8) + s) * 8;
     unpack8l(__ldg(reinterpret_cast<const uint4*>(xp)), xv);
     if (xplanes == 3) {
@@ -107,16 +116,29 @@ __global__ void __launch_bounds__(256) maxpool2x2_bwd_kernel(const f16* __restri
       for (int j = 0; j < 8; ++j) xv[j] += l[j];
     }
 #pragma unroll
-    for (int j = 0; j < 8; ++j) g[j] = (((a >> (2 * j)) & 3u) == t && xv[j] > 0.f) ? g[j] : 0.f;
-    *reinterpret_cast<uint4*>(gx + i * 8) = pack8l(g);
+    for (int j = 0; j < 8; ++j) {
+      const bool on = ((a >> (2 * j)) & 3u) == t && xv[j] > 0.f;
+      g[j] = on ? g[j] : 0.f;
+      if (SPLIT_G) gl[j] = on ? gl[j] : 0.f;
+    }
+    if (SPLIT_G) {
+      uint4* d = reinterpret_cast<uint4*>(gx) + (i / C8) * 3 * C8 + s;
+      const uint4 hv = pack8l(g);
+      d[0] = hv;
+      d[C8] = pack8l(gl);
+      d[2 * C8] = hv;
+    } else {
+      *reinterpret_cast<uint4*>(gx + i * 8) = pack8l(g);
+    }
   }
 }
 
 int maxpool2x2_bwd_launch(const f16* x, const uint16_t* idx, const f16* gy, f16* gx, int N, int H, int W, int C, cudaStream_t st,
-                          int xplanes) {
-  B2E_REQUIRE(C % 8 == 0 && H % 2 == 0 && W % 2 == 0, B2E_UNSUPPORTED_SHAPE, "maxpool2x2_bwd: bad shape");
+                          int xplanes, int gplanes) {
+  B2E_REQUIRE(C % 8 == 0 && H % 2 == 0 && W % 2 == 0 && (gplanes == 1 || gplanes == 3), B2E_UNSUPPORTED_SHAPE, "maxpool2x2_bwd: bad shape");
   const int64_t total = (int64_t)N * H * W * (C / 8);
-  launch_pdl(maxpool2x2_bwd_kernel, dim3(grid_for(total)), dim3(256), 0, st, x, idx, gy, gx, N, H, W, C / 8, xplanes);
+  if (gplanes == 3) launch_pdl(maxpool2x2_bwd_kernel<true>, dim3(grid_for(total)), dim3(256), 0, st, x, idx, gy, gx, N, H, W, C / 8, xplanes);
+  else launch_pdl(maxpool2x2_bwd_kernel<false>, dim3(grid_for(total)), dim3(256), 0, st, x, idx, gy, gx, N, H, W, C / 8, xplanes);
   return check_launch("maxpool2x2_bwd");
 }
 
@@ -295,8 +317,9 @@ int lpips_grad_scale_launch(const float* d_dist, const float* hmax, float* prod,
 // ---- head backward.  s = ||f||, k = 1 / (s + eps), u0 = k f, g = 2 w (u0 - u1) d_dist[b] / HW:
 //   d/df = k g - k^2 (f.g) / s f        (fp32; 0 where s = 0)
 // then + the gradient arriving from the pooled path (gp, already scaled), ReLU mask of the tap, x gs[0], f16 store.
-// The mask is applied BEFORE the f16 store: on an all-zero pixel the exact Jacobian is I / eps.
-template <int NCH>
+// The mask is applied BEFORE the f16 store: on an all-zero pixel the exact Jacobian is I / eps.  SPLIT_G: gp and gout are
+// split gradients [hi | lo | hi] (pixel pitch 3 C): gp read as hi + lo, gout re-split.
+template <int NCH, bool SPLIT_G>
 __global__ void __launch_bounds__(256) lpips_head_bwd_kernel(const f16* __restrict__ x, int C, int HW, int planes, const float* __restrict__ w,
                                                              const float* __restrict__ ref, int ref_batched, const float* __restrict__ d_dist,
                                                              const float* __restrict__ gs, const f16* __restrict__ gp, f16* __restrict__ gout,
@@ -348,9 +371,15 @@ __global__ void __launch_bounds__(256) lpips_head_bwd_kernel(const f16* __restri
     const float t = s > 0.f ? k * k * fg / s : 0.f;
 #pragma unroll
     for (int c = 0; c < NCH; ++c) {
-      const int64_t off = pix * C + (c * LP + lg) * 8;
+      const int64_t off = SPLIT_G ? pix * 3 * C + (c * LP + lg) * 8 : pix * C + (c * LP + lg) * 8;
       float add[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
       if (gp) unpack8l(__ldg(reinterpret_cast<const uint4*>(gp + off)), add);
+      if (gp && SPLIT_G) {
+        float l[8];
+        unpack8l(__ldg(reinterpret_cast<const uint4*>(gp + off + C)), l);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) add[j] += l[j];
+      }
       float o[8];
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
@@ -358,21 +387,36 @@ __global__ void __launch_bounds__(256) lpips_head_bwd_kernel(const f16* __restri
         const float dh = s > 0.f ? k * gv[8 * c + j] - t * v : 0.f;
         o[j] = v > 0.f ? dh * sc + add[j] : 0.f;
       }
-      *reinterpret_cast<uint4*>(gout + off) = pack8l(o);
+      const uint4 hv = pack8l(o);
+      *reinterpret_cast<uint4*>(gout + off) = hv;
+      if (SPLIT_G) {
+        float h[8];
+        unpack8l(hv, h);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) h[j] = __fsub_rn(o[j], h[j]);
+        *reinterpret_cast<uint4*>(gout + off + C) = pack8l(h);
+        *reinterpret_cast<uint4*>(gout + off + 2 * C) = hv;
+      }
     }
   }
 }
 
 int lpips_head_bwd_launch(const f16* x, int B, int C, int HW, int planes, const float* w, const float* ref, int ref_batched,
-                          const float* d_dist, const float* gs, const f16* gp, f16* gout, cudaStream_t st) {
+                          const float* d_dist, const float* gs, const f16* gp, f16* gout, cudaStream_t st, int gplanes) {
   B2E_REQUIRE(C == 64 || C == 128 || C == 256 || C == 512, B2E_UNSUPPORTED_SHAPE, "lpips_head_bwd: %d channels", C);
+  B2E_REQUIRE(gplanes == 1 || gplanes == 3, B2E_UNSUPPORTED_SHAPE, "lpips_head_bwd: planes");
   const int groups = 256 / (C == 512 ? 32 : C / 8);
   int64_t blocks = ((int64_t)B * HW + groups - 1) / groups;
   if (blocks > (int64_t)kNumSMs * 16) blocks = (int64_t)kNumSMs * 16;
-  if (C == 512)
-    launch_pdl(lpips_head_bwd_kernel<2>, dim3((unsigned)blocks), dim3(256), 0, st, x, C, HW, planes, w, ref, ref_batched, d_dist, gs, gp, gout, B);
+  const dim3 grid((unsigned)blocks);
+  if (C == 512 && gplanes == 3)
+    launch_pdl(lpips_head_bwd_kernel<2, true>, grid, dim3(256), 0, st, x, C, HW, planes, w, ref, ref_batched, d_dist, gs, gp, gout, B);
+  else if (C == 512)
+    launch_pdl(lpips_head_bwd_kernel<2, false>, grid, dim3(256), 0, st, x, C, HW, planes, w, ref, ref_batched, d_dist, gs, gp, gout, B);
+  else if (gplanes == 3)
+    launch_pdl(lpips_head_bwd_kernel<1, true>, grid, dim3(256), 0, st, x, C, HW, planes, w, ref, ref_batched, d_dist, gs, gp, gout, B);
   else
-    launch_pdl(lpips_head_bwd_kernel<1>, dim3((unsigned)blocks), dim3(256), 0, st, x, C, HW, planes, w, ref, ref_batched, d_dist, gs, gp, gout, B);
+    launch_pdl(lpips_head_bwd_kernel<1, false>, grid, dim3(256), 0, st, x, C, HW, planes, w, ref, ref_batched, d_dist, gs, gp, gout, B);
   return check_launch("lpips_head_bwd");
 }
 

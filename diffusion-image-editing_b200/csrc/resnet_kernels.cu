@@ -25,6 +25,25 @@ inline int grid_for(int64_t total, int per_sm = 32) {
   if (g > (int64_t)kNumSMs * per_sm) g = (int64_t)kNumSMs * per_sm;
   return (int)(g < 1 ? 1 : g);
 }
+// split gradients (grad_precision = 1): 8 channels of a [hi | lo | hi] tensor whose planes are lo_off elements apart; read
+// as hi + lo, written as hi = f16(v), lo = f16(v - hi)
+__device__ __forceinline__ void load_split8r(const f16* p, int lo_off, float* f) {
+  float l[8];
+  unpack8r(__ldg(reinterpret_cast<const uint4*>(p)), f);
+  unpack8r(__ldg(reinterpret_cast<const uint4*>(p + lo_off)), l);
+#pragma unroll
+  for (int j = 0; j < 8; ++j) f[j] += l[j];
+}
+__device__ __forceinline__ void store_split8r(f16* p, int lo_off, const float* f) {
+  const uint4 hi = pack8r(f);
+  float h[8];
+  unpack8r(hi, h);
+#pragma unroll
+  for (int j = 0; j < 8; ++j) h[j] = __fsub_rn(f[j], h[j]);
+  *reinterpret_cast<uint4*>(p) = hi;
+  *reinterpret_cast<uint4*>(p + lo_off) = pack8r(h);
+  *reinterpret_cast<uint4*>(p + 2 * lo_off) = hi;
+}
 }  // namespace
 
 // ---- stem: x fp32 NCHW (B,C,H,W) -> f16 (B,H/2,W/2,KP): column (kh*7 + kw)*C + c = x[c][2oh + kh - 3][2ow + kw - 3]
@@ -76,7 +95,9 @@ int im2col7s2_launch(const float* x, f16* out, int B, int C, int H, int W, int K
 }
 
 // gradient of the stem w.r.t. the image: dx[b][c][ih][iw] = sum over taps with 2oh + kh - 3 = ih, 2ow + kw - 3 = iw of
-// dcols[b][oh][ow][(kh*7 + kw)*C + c]; dcols f16 (B,H/2,W/2,KP), dx fp32 NCHW
+// dcols[b][oh][ow][(kh*7 + kw)*C + c]; dcols f16 (B,H/2,W/2,KP), dx fp32 NCHW.  SPLIT: dcols holds [hi | lo | hi] planes of
+// KP columns, value hi + lo
+template <bool SPLIT>
 __global__ void __launch_bounds__(256) col2im7s2_kernel(const f16* __restrict__ dcols, float* __restrict__ dx, int B, int C,
                                                         int H, int W, int KP, const float* __restrict__ gs) {
   pdl_wait();
@@ -94,17 +115,18 @@ __global__ void __launch_bounds__(256) col2im7s2_kernel(const f16* __restrict__ 
       for (int kw = (iw + 3) & 1; kw < 7; kw += 2) {
         const int ow = (iw + 3 - kw) >> 1;
         if (ow < 0 || ow >= Wo) continue;
-        const f16* p = dcols + (((int64_t)b * Ho + oh) * Wo + ow) * KP + (kh * 7 + kw) * C;
-        for (int c = 0; c < C; ++c) acc[c] += f16_to_float(p[c]);
+        const f16* p = dcols + (((int64_t)b * Ho + oh) * Wo + ow) * (SPLIT ? 3 * KP : KP) + (kh * 7 + kw) * C;
+        for (int c = 0; c < C; ++c) acc[c] += SPLIT ? f16_to_float(p[c]) + f16_to_float(p[KP + c]) : f16_to_float(p[c]);
       }
     }
     for (int c = 0; c < C; ++c) dx[(((int64_t)b * C + c) * H + ih) * W + iw] = acc[c] * unscale;
   }
 }
 
-int col2im7s2_launch(const f16* dcols, float* dx, int B, int C, int H, int W, int KP, cudaStream_t st, const float* gs) {
-  B2E_REQUIRE(C >= 1 && C <= 4 && 49 * C <= KP, B2E_UNSUPPORTED_SHAPE, "col2im7s2: bad shape");
-  launch_pdl(col2im7s2_kernel, dim3(grid_for((int64_t)B * H * W)), dim3(256), 0, st, dcols, dx, B, C, H, W, KP, gs);
+int col2im7s2_launch(const f16* dcols, float* dx, int B, int C, int H, int W, int KP, cudaStream_t st, const float* gs, int planes) {
+  B2E_REQUIRE(C >= 1 && C <= 4 && 49 * C <= KP && (planes == 1 || planes == 3), B2E_UNSUPPORTED_SHAPE, "col2im7s2: bad shape");
+  if (planes == 3) launch_pdl(col2im7s2_kernel<true>, dim3(grid_for((int64_t)B * H * W)), dim3(256), 0, st, dcols, dx, B, C, H, W, KP, gs);
+  else launch_pdl(col2im7s2_kernel<false>, dim3(grid_for((int64_t)B * H * W)), dim3(256), 0, st, dcols, dx, B, C, H, W, KP, gs);
   return check_launch("col2im7s2");
 }
 
@@ -170,7 +192,9 @@ int maxpool3s2_launch(const f16* x, f16* y, uint8_t* idx, int N, int H, int W, i
 }
 
 // gx[p] = (x[p] > 0) * sum over the (<= 4) windows whose recorded argmax is p of gy[window]   (the x > 0 factor is the
-// backward of the ReLU that produced x)
+// backward of the ReLU that produced x).  SPLIT_G: gy and gx are split gradients; the overlapping windows' hi + lo
+// contributions are summed in fp32 and re-split
+template <bool SPLIT_G>
 __global__ void __launch_bounds__(256) maxpool3s2_bwd_kernel(const f16* __restrict__ x, const uint8_t* __restrict__ idx,
                                                              const f16* __restrict__ gy, f16* __restrict__ gx, int N, int H,
                                                              int W, int C8, int xplanes) {
@@ -206,7 +230,8 @@ __global__ void __launch_bounds__(256) maxpool3s2_bwd_kernel(const f16* __restri
         const int64_t o = ((((int64_t)n * Ho + oh) * Wo + ow) * C8 + s) * 8;
         const uint2 a = __ldg(reinterpret_cast<const uint2*>(idx + o));
         float g[8];
-        unpack8r(__ldg(reinterpret_cast<const uint4*>(gy + o)), g);
+        if (SPLIT_G) load_split8r(gy + ((((int64_t)n * Ho + oh) * Wo + ow) * 3 * C8 + s) * 8, C8 * 8, g);
+        else unpack8r(__ldg(reinterpret_cast<const uint4*>(gy + o)), g);
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
           const uint32_t aj = ((j < 4 ? a.x : a.y) >> (8 * (j & 3))) & 0xffu;
@@ -216,14 +241,17 @@ __global__ void __launch_bounds__(256) maxpool3s2_bwd_kernel(const f16* __restri
     }
 #pragma unroll
     for (int j = 0; j < 8; ++j) acc[j] = xv[j] > 0.f ? acc[j] : 0.f;
-    *reinterpret_cast<uint4*>(gx + i * 8) = pack8r(acc);
+    if (SPLIT_G) store_split8r(gx + ((i / C8) * 3 * C8 + s) * 8, C8 * 8, acc);
+    else *reinterpret_cast<uint4*>(gx + i * 8) = pack8r(acc);
   }
 }
 
 int maxpool3s2_bwd_launch(const f16* x, const uint8_t* idx, const f16* gy, f16* gx, int N, int H, int W, int C,
-                          cudaStream_t st, int xplanes) {
+                          cudaStream_t st, int xplanes, int gplanes) {
+  B2E_REQUIRE(gplanes == 1 || (gplanes == 3 && xplanes == 3), B2E_UNSUPPORTED_SHAPE, "maxpool3s2_bwd: split gradients need a split forward");
   const int64_t total = (int64_t)N * H * W * (C / 8);
-  launch_pdl(maxpool3s2_bwd_kernel, dim3(grid_for(total)), dim3(256), 0, st, x, idx, gy, gx, N, H, W, C / 8, xplanes);
+  if (gplanes == 3) launch_pdl(maxpool3s2_bwd_kernel<true>, dim3(grid_for(total)), dim3(256), 0, st, x, idx, gy, gx, N, H, W, C / 8, xplanes);
+  else launch_pdl(maxpool3s2_bwd_kernel<false>, dim3(grid_for(total)), dim3(256), 0, st, x, idx, gy, gx, N, H, W, C / 8, xplanes);
   return check_launch("maxpool3s2_bwd");
 }
 
@@ -241,13 +269,22 @@ __global__ void __launch_bounds__(256) relu_bwd_kernel(const uint4* __restrict__
   }
 }
 
-// the same with y a split tensor [hi | lo | hi] of the fp32-accurate forward (pixel pitch 3 C): mask = (hi + lo > 0)
+// the same with y a split tensor [hi | lo | hi] of the fp32-accurate forward (pixel pitch 3 C): mask = (hi + lo > 0).
+// SPLIT_G: g / out are split gradients too (pixel pitch 3 C); the one mask zeroes all three planes, which is exact
+template <bool SPLIT_G>
 __global__ void __launch_bounds__(256) relu_bwd_split_kernel(const uint4* __restrict__ g, const uint4* __restrict__ y,
                                                              uint4* __restrict__ out, int64_t n8, int C8) {
   pdl_wait();
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += (int64_t)gridDim.x * blockDim.x) {
-    const int64_t row = i / C8;
-    const int s = (int)(i - row * C8);
+    int64_t row;
+    int s;
+    if (SPLIT_G) {
+      row = i / (3 * C8);
+      s = (int)((i - row * 3 * C8) % C8);
+    } else {
+      row = i / C8;
+      s = (int)(i - row * C8);
+    }
     float gv[8], yv[8], lv[8];
     unpack8r(g[i], gv);
     unpack8r(__ldg(y + row * 3 * C8 + s), yv);
@@ -258,12 +295,17 @@ __global__ void __launch_bounds__(256) relu_bwd_split_kernel(const uint4* __rest
   }
 }
 
-int relu_bwd_launch(const f16* g, const f16* y, f16* out, int64_t numel, cudaStream_t st, int yplanes, int C) {
+int relu_bwd_launch(const f16* g, const f16* y, f16* out, int64_t numel, cudaStream_t st, int yplanes, int C, int gplanes) {
   B2E_REQUIRE(numel % 8 == 0, B2E_UNSUPPORTED_SHAPE, "relu_bwd: numel %% 8 != 0");
+  B2E_REQUIRE(gplanes == 1 || (gplanes == 3 && yplanes == 3), B2E_UNSUPPORTED_SHAPE, "relu_bwd: split gradients need a split forward");
   if (yplanes == 3) {
     B2E_REQUIRE(C > 0 && C % 8 == 0, B2E_UNSUPPORTED_SHAPE, "relu_bwd: split activation needs the channel count");
-    launch_pdl(relu_bwd_split_kernel, dim3(grid_for(numel / 8)), dim3(256), 0, st, (const uint4*)g, (const uint4*)y, (uint4*)out,
-               numel / 8, C / 8);
+    if (gplanes == 3)
+      launch_pdl(relu_bwd_split_kernel<true>, dim3(grid_for(numel / 8)), dim3(256), 0, st, (const uint4*)g, (const uint4*)y, (uint4*)out,
+                 numel / 8, C / 8);
+    else
+      launch_pdl(relu_bwd_split_kernel<false>, dim3(grid_for(numel / 8)), dim3(256), 0, st, (const uint4*)g, (const uint4*)y, (uint4*)out,
+                 numel / 8, C / 8);
     return check_launch("relu_bwd_split");
   }
   launch_pdl(relu_bwd_kernel, dim3(grid_for(numel / 8)), dim3(256), 0, st, (const uint4*)g, (const uint4*)y, (uint4*)out, numel / 8);
@@ -369,6 +411,7 @@ __global__ void __launch_bounds__(256) fc_bwd_kernel(const float* __restrict__ d
   dfeat[(int64_t)n * C + c] = s * scale;
 }
 
+template <bool SPLIT_G>   // g a split gradient (pixel pitch 3 C)
 __global__ void __launch_bounds__(256) avgpool_bwd_kernel(const float* __restrict__ dfeat, const f16* __restrict__ y,
                                                           f16* __restrict__ g, int HW, int C8, int yplanes) {
   pdl_wait();
@@ -388,17 +431,22 @@ __global__ void __launch_bounds__(256) avgpool_bwd_kernel(const float* __restric
     const float* d = dfeat + (int64_t)n * C8 * 8 + s * 8;
 #pragma unroll
     for (int j = 0; j < 8; ++j) o[j] = yv[j] > 0.f ? d[j] : 0.f;
-    *reinterpret_cast<uint4*>(g + ((int64_t)n * total + i) * 8) = pack8r(o);
+    if (SPLIT_G) store_split8r(g + (((int64_t)n * HW + i / C8) * 3 * C8 + s) * 8, C8 * 8, o);
+    else *reinterpret_cast<uint4*>(g + ((int64_t)n * total + i) * 8) = pack8r(o);
   }
 }
 
 int avgpool_fc_bwd_launch(const float* dlogits, const float* w, float* dfeat, const f16* y, f16* g, int N, int HW, int C, int K,
-                          cudaStream_t st, const float* gs, int yplanes) {
+                          cudaStream_t st, const float* gs, int yplanes, int gplanes) {
+  B2E_REQUIRE(gplanes == 1 || (gplanes == 3 && yplanes == 3), B2E_UNSUPPORTED_SHAPE, "avgpool_fc_bwd: split gradients need a split forward");
   launch_pdl(fc_bwd_kernel, dim3((C + 255) / 256, N), dim3(256), 0, st, dlogits, w, dfeat, C, K, 1.0f / (float)HW, gs);
   int rc = check_launch("fc_bwd");
   if (rc) return rc;
   const int64_t total = (int64_t)HW * (C / 8);
-  launch_pdl(avgpool_bwd_kernel, dim3((unsigned)((total + 255) / 256), N), dim3(256), 0, st, (const float*)dfeat, y, g, HW, C / 8, yplanes);
+  if (gplanes == 3)
+    launch_pdl(avgpool_bwd_kernel<true>, dim3((unsigned)((total + 255) / 256), N), dim3(256), 0, st, (const float*)dfeat, y, g, HW, C / 8, yplanes);
+  else
+    launch_pdl(avgpool_bwd_kernel<false>, dim3((unsigned)((total + 255) / 256), N), dim3(256), 0, st, (const float*)dfeat, y, g, HW, C / 8, yplanes);
   return check_launch("avgpool_bwd");
 }
 
@@ -491,6 +539,8 @@ int chan_affine_launch(const f16* x, const float* a, const float* b, const f16* 
 
 // ---- backward helpers of the face parser
 // out[n][c] = scale * sum_p x[n][p][c] * (y ? y[n][p][c] : 1)   (gradient of a per-channel attention / broadcast vector)
+// SPLIT_X: x is a split gradient (pixel pitch 3 C), value hi + lo
+template <bool SPLIT_X>
 __global__ void __launch_bounds__(256) chan_dot_kernel(const f16* __restrict__ x, const f16* __restrict__ y,
                                                        float* __restrict__ out, int HW, int C, float scale, int yplanes) {
   pdl_wait();
@@ -501,7 +551,8 @@ __global__ void __launch_bounds__(256) chan_dot_kernel(const f16* __restrict__ x
   if (c < C)
     for (int p = row; p < HW; p += 8) {
       const int64_t o = ((int64_t)n * HW + p) * C + c;
-      const float xv = f16_to_float(x[o]);
+      const float xv = SPLIT_X ? f16_to_float(x[((int64_t)n * HW + p) * 3 * C + c]) + f16_to_float(x[((int64_t)n * HW + p) * 3 * C + C + c])
+                               : f16_to_float(x[o]);
       if (y) {
         const f16* yp = y + ((int64_t)n * HW + p) * (yplanes * C) + c;     // yplanes = 3: split forward activation, hi + lo
         s += xv * (yplanes == 3 ? f16_to_float(yp[0]) + f16_to_float(yp[C]) : f16_to_float(yp[0]));
@@ -518,8 +569,11 @@ __global__ void __launch_bounds__(256) chan_dot_kernel(const f16* __restrict__ x
   }
 }
 
-int chan_dot_launch(const f16* x, const f16* y, float* out, int N, int HW, int C, float scale, cudaStream_t st, int yplanes) {
-  launch_pdl(chan_dot_kernel, dim3((C + 31) / 32, N), dim3(256), 0, st, x, y, out, HW, C, scale, yplanes);
+int chan_dot_launch(const f16* x, const f16* y, float* out, int N, int HW, int C, float scale, cudaStream_t st, int yplanes,
+                    int xplanes) {
+  B2E_REQUIRE(xplanes == 1 || xplanes == 3, B2E_UNSUPPORTED_SHAPE, "chan_dot: planes");
+  if (xplanes == 3) launch_pdl(chan_dot_kernel<true>, dim3((C + 31) / 32, N), dim3(256), 0, st, x, y, out, HW, C, scale, yplanes);
+  else launch_pdl(chan_dot_kernel<false>, dim3((C + 31) / 32, N), dim3(256), 0, st, x, y, out, HW, C, scale, yplanes);
   return check_launch("chan_dot");
 }
 
@@ -546,7 +600,9 @@ int vec_act_bwd_launch(const float* g, const float* a, float* out, int n, int mo
 }
 
 // out[r][c] = (g[r][c] + e[r * e_pitch + e_off + c]) * (y ? y[r][c] > 0 : 1): gradient accumulation from a second
-// consumer (a channel window of a wider tensor) followed by the ReLU mask of the tensor both consumers read
+// consumer (a channel window of a wider tensor) followed by the ReLU mask of the tensor both consumers read.  SPLIT_G: g, e
+// and out are split gradients (planes C / e_pitch channels apart), summed in fp32 and re-split
+template <bool SPLIT_G>
 __global__ void __launch_bounds__(256) grad_merge_kernel(const f16* __restrict__ g, const f16* __restrict__ e, int e_pitch,
                                                          int e_off, const f16* __restrict__ y, f16* __restrict__ out,
                                                          int64_t rows, int C8, int yplanes) {
@@ -556,13 +612,15 @@ __global__ void __launch_bounds__(256) grad_merge_kernel(const f16* __restrict__
     const int s = (int)(i % C8);
     const int64_t r = i / C8;
     float gv[8], ev[8], yv[8];
-    if (g) unpack8r(*reinterpret_cast<const uint4*>(g + i * 8), gv);
+    if (g && SPLIT_G) load_split8r(g + (r * 3 * C8 + s) * 8, C8 * 8, gv);
+    else if (g) unpack8r(*reinterpret_cast<const uint4*>(g + i * 8), gv);
     else {
 #pragma unroll
       for (int j = 0; j < 8; ++j) gv[j] = 0.f;
     }
     if (e) {
-      unpack8r(__ldg(reinterpret_cast<const uint4*>(e + r * e_pitch + e_off + s * 8)), ev);
+      if (SPLIT_G) load_split8r(e + r * 3 * e_pitch + e_off + s * 8, e_pitch, ev);
+      else unpack8r(__ldg(reinterpret_cast<const uint4*>(e + r * e_pitch + e_off + s * 8)), ev);
 #pragma unroll
       for (int j = 0; j < 8; ++j) gv[j] += ev[j];
     }
@@ -578,18 +636,25 @@ __global__ void __launch_bounds__(256) grad_merge_kernel(const f16* __restrict__
 #pragma unroll
       for (int j = 0; j < 8; ++j) gv[j] = yv[j] > 0.f ? gv[j] : 0.f;
     }
-    *reinterpret_cast<uint4*>(out + i * 8) = pack8r(gv);
+    if (SPLIT_G) store_split8r(out + (r * 3 * C8 + s) * 8, C8 * 8, gv);
+    else *reinterpret_cast<uint4*>(out + i * 8) = pack8r(gv);
   }
 }
 
 int grad_merge_launch(const f16* g, const f16* e, int e_pitch, int e_off, const f16* y, f16* out, int64_t rows, int C,
-                      cudaStream_t st, int yplanes) {
+                      cudaStream_t st, int yplanes, int gplanes) {
   B2E_REQUIRE(C % 8 == 0 && e_pitch % 8 == 0 && e_off % 8 == 0, B2E_UNSUPPORTED_SHAPE, "grad_merge: alignment");
-  launch_pdl(grad_merge_kernel, dim3(grid_for(rows * (C / 8))), dim3(256), 0, st, g, e, e_pitch, e_off, y, out, rows, C / 8, yplanes);
+  B2E_REQUIRE(gplanes == 1 || gplanes == 3, B2E_UNSUPPORTED_SHAPE, "grad_merge: planes");
+  if (gplanes == 3)
+    launch_pdl(grad_merge_kernel<true>, dim3(grid_for(rows * (C / 8))), dim3(256), 0, st, g, e, e_pitch, e_off, y, out, rows, C / 8, yplanes);
+  else
+    launch_pdl(grad_merge_kernel<false>, dim3(grid_for(rows * (C / 8))), dim3(256), 0, st, g, e, e_pitch, e_off, y, out, rows, C / 8, yplanes);
   return check_launch("grad_merge");
 }
 
-// adjoint of the align_corners bilinear upsampling: g (N,K,Ho,Wo) fp32 NCHW -> dx f16 NHWC (N,Hi,Wi,P), channels >= K zero
+// adjoint of the align_corners bilinear upsampling: g (N,K,Ho,Wo) fp32 NCHW -> dx f16 NHWC (N,Hi,Wi,P), channels >= K zero.
+// SPLIT: dx is a split gradient [hi | lo | hi] (pixel pitch 3 P)
+template <bool SPLIT>
 __global__ void __launch_bounds__(128) bilinear_ac_bwd_kernel(const float* __restrict__ g, f16* __restrict__ dx, int N, int Hi,
                                                               int Wi, int P, int K, int Ho, int Wo, float sh, float sw,
                                                               const float* __restrict__ gs) {
@@ -623,7 +688,16 @@ __global__ void __launch_bounds__(128) bilinear_ac_bwd_kernel(const float* __res
       }
       acc += wh * rowacc;
     }
-    dx[(((int64_t)n * Hi + h) * Wi + w) * P + k] = float_to_f16(acc * sc);
+    if (SPLIT) {
+      const float v = acc * sc;
+      const f16 hi = float_to_f16(v);
+      f16* d = dx + (((int64_t)n * Hi + h) * Wi + w) * 3 * P + k;
+      d[0] = hi;
+      d[P] = float_to_f16(__fsub_rn(v, f16_to_float(hi)));
+      d[2 * P] = hi;
+    } else {
+      dx[(((int64_t)n * Hi + h) * Wi + w) * P + k] = float_to_f16(acc * sc);
+    }
   }
 }
 
@@ -635,14 +709,20 @@ __global__ void __launch_bounds__(256) zero_tail_kernel(f16* __restrict__ x, int
 }
 
 int bilinear_ac_bwd_launch(const float* g, f16* dx, int N, int Hi, int Wi, int P, int K, int Ho, int Wo, cudaStream_t st,
-                           const float* gs) {
+                           const float* gs, int planes) {
+  B2E_REQUIRE(planes == 1 || planes == 3, B2E_UNSUPPORTED_SHAPE, "bilinear_ac_bwd: planes");
   const float sh = Ho > 1 ? (float)(Hi - 1) / (float)(Ho - 1) : 0.f, sw = Wo > 1 ? (float)(Wi - 1) / (float)(Wo - 1) : 0.f;
   if (P > K) {
-    launch_pdl(zero_tail_kernel, dim3(grid_for((int64_t)N * Hi * Wi * (P - K))), dim3(256), 0, st, dx, (int64_t)N * Hi * Wi, P, K);
+    // (split: every plane of P channels has its tail zeroed - the pixel's three planes are three rows of P)
+    const int64_t rows = (int64_t)N * Hi * Wi * planes;
+    launch_pdl(zero_tail_kernel, dim3(grid_for(rows * (P - K))), dim3(256), 0, st, dx, rows, P, K);
     int rc = check_launch("zero_tail");
     if (rc) return rc;
   }
-  launch_pdl(bilinear_ac_bwd_kernel, dim3(grid_for((int64_t)N * Hi * Wi * K, 64)), dim3(128), 0, st, g, dx, N, Hi, Wi, P, K, Ho, Wo, sh, sw, gs);
+  if (planes == 3)
+    launch_pdl(bilinear_ac_bwd_kernel<true>, dim3(grid_for((int64_t)N * Hi * Wi * K, 64)), dim3(128), 0, st, g, dx, N, Hi, Wi, P, K, Ho, Wo, sh, sw, gs);
+  else
+    launch_pdl(bilinear_ac_bwd_kernel<false>, dim3(grid_for((int64_t)N * Hi * Wi * K, 64)), dim3(128), 0, st, g, dx, N, Hi, Wi, P, K, Ho, Wo, sh, sw, gs);
   return check_launch("bilinear_ac_bwd");
 }
 

@@ -160,6 +160,7 @@ struct b2e_unet {
   std::vector<ConvL> dgrads;
   int conv_in_dg = -1, conv_out_dg = -1;
   bool grad = false;
+  bool split_grad = false;   // classifier / face parser / LPIPS with grad_precision = 1: fp32-accurate backward
   const float* in_dy = nullptr; float* out_dz = nullptr;   // per-call
   int64_t fwd_B = -1;                                      // batch of the forward whose activations are live
   NormL norm_out;
@@ -265,8 +266,9 @@ struct b2e_unet {
     return c;
   }
   // planes of the dgrad twins: the split decoder's gradient is fp32-accurate (split gradients, [W'_hi | W'_hi | W'_lo] x 2^10
-  // weights); the classifier and LPIPS keep a 16-bit backward under their fp32-accurate forward
-  int dgrad_planes() const { return decoder ? PL : 1; }
+  // weights); the classifier, face parser and LPIPS keep a 16-bit backward under their fp32-accurate forward unless they
+  // were created with grad_precision = 1
+  int dgrad_planes() const { return decoder || split_grad ? PL : 1; }
   static float dgrad_wscale(int planes) { return planes == 3 ? kSplitWScale : 1.f; }
   // dgrad twin of a stride-1 convolution with `cin` input channels whose output tensor has pitch `dy_pitch`:
   // a convolution dy (dy_pitch channels) -> dx (cin channels), zero bias; the weights are packed by the caller
@@ -539,8 +541,9 @@ int build_model_resnet(b2e_unet* m) {
     // fp32-accurate forward (rcfg.precision == 1, PL = 3): forward activations are split tensors [hi | lo | hi] and the
     // forward weights are packed [W_hi | W_hi | W_lo] (x 2^10, undone in the epilogue) exactly as in the UNet's split mode,
     // so ReLU / max-pool masks agree with the fp32 reference; the backward pass (dgrad twins, gradients) stays on plain
-    // f16 operands and reads its masks from the split activations.
-    const int PL = m->PL;
+    // f16 operands and reads its masks from the split activations - unless grad_precision = 1 (DPL = 3): then the dgrad
+    // twins are split too and the gradients travel as split tensors.
+    const int PL = m->PL, DPL = m->dgrad_planes();
     ConvL s;
     const int KP = pad64(49 * Cin);
     s.cin = s.cin_pad = KP; s.cout = W0; s.k = 1; s.cout_pad = conv_cout_pad(W0); s.row_len = KP * PL;
@@ -548,12 +551,12 @@ int build_model_resnet(b2e_unet* m) {
     s.b = m->dmalloc<float>(s.cout_pad);
     m->stem_dg = m->make_dgrad(KP, s.cout_pad, 1);   // gradient w.r.t. the im2col columns
     const ConvL sd = m->dgrads[m->stem_dg];
-    m->add_param(pre + "conv1.weight", (int64_t)W0 * Cin * 49, (int64_t)Cin * 49, [s, sd, Cin, PL, KP](const float* src, cudaStream_t st) {
+    m->add_param(pre + "conv1.weight", (int64_t)W0 * Cin * 49, (int64_t)Cin * 49, [s, sd, Cin, PL, DPL, KP](const float* src, cudaStream_t st) {
       const float ws = PL == 3 ? b2e_unet::kSplitWScale : 1.f;
       int rc = conv_pack_weight(src, s.w, s.cout, Cin, 7, Cin, s.row_len, 0, st, 0, 0, 0, ws);
       if (!rc && PL == 3) rc = conv_pack_weight(src, s.w, s.cout, Cin, 7, Cin, s.row_len, KP, st, 0, 0, 0, ws);
       if (!rc && PL == 3) rc = conv_pack_weight(src, s.w, s.cout, Cin, 7, Cin, s.row_len, 2 * KP, st, 0, 0, 1, ws);
-      if (!rc) rc = conv_pack_weight_im2col_T(src, sd.w, s.cout, Cin, sd.row_len, st, 49);
+      if (!rc) rc = conv_pack_weight_im2col_T(src, sd.w, s.cout, Cin, sd.row_len, st, 49, DPL, b2e_unet::dgrad_wscale(DPL));
       return rc;
     });
     m->add_f32(pre + "conv1.bias", s.b, W0, (int64_t)Cin * 49);
@@ -589,10 +592,10 @@ int build_model_resnet(b2e_unet* m) {
         const int extra = j == 0 ? pad64(rb.cout) : 0;
         rb.dg[j] = m->make_dgrad(cs[j].cin, L.cout_pad, L.k, extra);
         const ConvL D = m->dgrads[rb.dg[j]];
-        const int PLc = m->PL;
-        m->add_param(nm + ".weight", (int64_t)L.cout * L.cin * L.k * L.k, (int64_t)L.cin * L.k * L.k, [L, D, PLc](const float* src, cudaStream_t st) {
+        const int PLc = m->PL, DPL = m->dgrad_planes();
+        m->add_param(nm + ".weight", (int64_t)L.cout * L.cin * L.k * L.k, (int64_t)L.cin * L.k * L.k, [L, D, PLc, DPL](const float* src, cudaStream_t st) {
           int rc = b2e_unet::pack_w(PLc, src, L.w, L.cout, L.cin, L.k, L.cin_pad, L.row_len, 0, L.cin_pad, st);
-          if (!rc) rc = conv_pack_weight_dgrad(src, D.w, L.cout, L.cin, L.k, D.cin_pad, D.row_len, 0, st);
+          if (!rc) rc = conv_pack_weight_dgrad(src, D.w, L.cout, L.cin, L.k, D.cin_pad, D.row_len, 0, st, DPL, b2e_unet::dgrad_wscale(DPL));
           return rc;
         });
         m->add_f32(nm + ".bias", L.b, L.cout, (int64_t)L.cin * L.k * L.k);
@@ -601,20 +604,20 @@ int build_model_resnet(b2e_unet* m) {
       {
         const ConvL L = rb.c[rb.nconv - 1];
         const ConvL D0 = m->dgrads[rb.dg[0]];
-        const int PLc = m->PL;
+        const int PLc = m->PL, DPL = m->dgrad_planes();
         const int seg = PLc * L.k * L.k * L.cin_pad;            // forward: residual segment starts here (all planes of the taps first)
-        const int dseg = D0.k * D0.k * D0.cin_pad;              // backward twin of conv1: shortcut-gradient segment
+        const int dseg = DPL * D0.k * D0.k * D0.cin_pad;        // backward twin of conv1: shortcut-gradient segment
         if (rb.has_ds) {
           rb.c[rb.nconv - 1].b2 = m->dmalloc<float>(L.cout_pad);
           const int cin = inpl, cout = rb.cout;
-          m->add_param(base + ".downsample.0.weight", (int64_t)cout * cin, cin, [L, D0, seg, dseg, cin, cout, PLc](const float* src, cudaStream_t st) {
+          m->add_param(base + ".downsample.0.weight", (int64_t)cout * cin, cin, [L, D0, seg, dseg, cin, cout, PLc, DPL](const float* src, cudaStream_t st) {
             int rc = b2e_unet::pack_w(PLc, src, L.w, cout, cin, 1, cin, L.row_len, seg, pad64(cin), st);
-            if (!rc) rc = conv_pack_weight_dgrad(src, D0.w, cout, cin, 1, pad64(cout), D0.row_len, dseg, st);
+            if (!rc) rc = conv_pack_weight_dgrad(src, D0.w, cout, cin, 1, pad64(cout), D0.row_len, dseg, st, DPL, b2e_unet::dgrad_wscale(DPL));
             return rc;
           });
           m->add_f32(base + ".downsample.0.bias", rb.c[rb.nconv - 1].b2, cout, cin);
         } else if (L.w && D0.w) {
-          if (b2e_unet::fill_id(PLc, L.w, rb.cout, L.row_len, seg, pad64(inpl)) || conv_fill_identity(D0.w, rb.cout, D0.row_len, dseg, 0))
+          if (b2e_unet::fill_id(PLc, L.w, rb.cout, L.row_len, seg, pad64(inpl)) || b2e_unet::fill_id(DPL, D0.w, rb.cout, D0.row_len, dseg, pad64(rb.cout)))
             m->build_error = B2E_CUDA_ERROR;
         }
       }
@@ -665,7 +668,8 @@ int build_program_resnet(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* 
   std::vector<b2e_unet::Op>* cur = &fwd;
   double flops = 0;
   int rc = B2E_OK;
-  const int PL = m->PL;     // planes of the FORWARD activations (3: split tensors of the fp32-accurate forward); gradients: 1
+  const int PL = m->PL;     // planes of the FORWARD activations (3: split tensors of the fp32-accurate forward)
+  const int GP = m->dgrad_planes();   // planes of the gradients (3: split gradients of grad_precision = 1)
   auto talloc = [&](int N, int H, int W, int C, int planes = 1) {
     Tensor t; t.N = N; t.H = H; t.W = W; t.C = C; t.Cr = C; t.bytes = (size_t)N * H * W * C * planes * sizeof(f16);
     t.p = (f16*)ar.alloc(t.bytes);
@@ -839,38 +843,42 @@ int build_program_resnet(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* 
     // key = index of the block whose INPUT is that feature; value = (tensor, channel offset of the window)
     std::map<int, std::pair<Tensor, int>> extra;
     auto dconv = [&](int dg, const Tensor& dy, const Tensor* r0, Tensor* dx, const char* what) {
-      // dx = conv_{k, stride 1}(dy; flipped / transposed weights) [+ residual segment r0]
+      // dx = conv_{k, stride 1}(dy; flipped / transposed weights) [+ residual segment r0]; GP = 3: split dy, r0 and dx
       if (rc) return;
       const ConvL& D = m->dgrads[dg];
-      *dx = talloc(B, dy.H, dy.W, D.cout_pad);
+      *dx = talloc(B, dy.H, dy.W, D.cout_pad, GP);
       const double fl = 2.0 * B * dy.H * dy.W * (double)D.cout_pad * D.row_len;
       flops += fl;
       if (dry) return;
-      if (D.k * D.k * dy.C + D.res_c != D.row_len || (r0 ? r0->C : 0) != D.res_c) {
+      if (GP * (D.k * D.k * dy.C + D.res_c) != D.row_len || (r0 ? r0->C : 0) != D.res_c) {
         rc = B2E_INVALID_ARG; set_error("resnet backward: operand widths do not match (%s)", what); return;
       }
       ConvDesc d;
-      d.s0 = ConvSrc{dy.p, dy.C};
-      if (r0) d.r0 = ConvSrc{r0->p, r0->C};
+      d.s0 = ConvSrc{dy.p, dy.C * GP};
+      if (r0) d.r0 = ConvSrc{r0->p, r0->C * GP};
+      d.out_planes = GP;
       d.N = B; d.H = dy.H; d.W = dy.W; d.ksize = D.k; d.stride = 1;
       d.w_packed = D.w; d.Cout = D.cout_pad; d.out_f16 = dx->p;
       d.split_ws = split_ws; d.split_ws_bytes = split_bytes; d.split_counters = split_cnt;
       ConvPlan pl;
       rc = conv_plan_build(&pl, d);
       if (rc) return;
+      ConvEpilogue ep;
+      if (GP == 3) ep.acc_scale = 1.f / b2e_unet::kSplitWScale;
       char desc[160];
-      snprintf(desc, sizeof(desc), "%s: dgrad conv%dx%d %dx%d cin%d res%d cout%d", what, D.k, D.k, dy.H, dy.W, dy.C, D.res_c, D.cout);
-      cur->push_back({[pl](cudaStream_t st) { return conv_launch(pl, ConvEpilogue{}, st); }, 0, pl.flops, 0.0, desc});
+      snprintf(desc, sizeof(desc), "%s: dgrad conv%dx%d %dx%d cin%d res%d cout%d%s", what, D.k, D.k, dy.H, dy.W, dy.C, D.res_c, D.cout,
+               GP == 3 ? " split" : "");
+      cur->push_back({[pl, ep](cudaStream_t st) { return conv_launch(pl, ep, st); }, 0, pl.flops, 0.0, desc});
     };
     auto relu_mask = [&](Tensor& gt, const Tensor& y) {   // in place: gt *= (y > 0); y = forward activation (PL planes)
       const Tensor gg = gt, yy = y;
-      ew([gg, yy, PL](cudaStream_t st) { return relu_bwd_launch(gg.p, yy.p, gg.p, (int64_t)(gg.bytes / sizeof(f16)), st, PL, gg.C); },
+      ew([gg, yy, PL, GP](cudaStream_t st) { return relu_bwd_launch(gg.p, yy.p, gg.p, (int64_t)(gg.bytes / sizeof(f16)), st, PL, gg.C, GP); },
          3.0 * (double)gt.bytes, "relu backward");
     };
-    auto zero_up = [&](const Tensor& t) {
-      Tensor u = talloc(B, t.H * 2, t.W * 2, t.C);
+    auto zero_up = [&](const Tensor& t) {   // (split gradients: the [hi | lo | hi] planes of a pixel move as one 3C-channel row)
+      Tensor u = talloc(B, t.H * 2, t.W * 2, t.C, GP);
       const Tensor tt = t;
-      ew([tt, u, B](cudaStream_t st) { return zero_upsample2x_launch(tt.p, u.p, B, tt.H, tt.W, tt.C, st); }, 1.25 * (double)u.bytes,
+      ew([tt, u, B, GP](cudaStream_t st) { return zero_upsample2x_launch(tt.p, u.p, B, tt.H, tt.W, tt.C * GP, st); }, 1.25 * (double)u.bytes,
          "zero insertion (stride-2 gradient)");
       return u;
     };
@@ -887,10 +895,10 @@ int build_program_resnet(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* 
     }
     if (c.head == 0) {
       float* dfeat = (float*)ar.alloc(sizeof(float) * B * Cl);
-      g = talloc(B, h.H, h.W, h.C);
+      g = talloc(B, h.H, h.W, h.C, GP);
       const Tensor hl = h, gg = g;
-      ew([m, hl, gg, dfeat, gsc, B, HWl, Cl, K, PL](cudaStream_t st) {
-           return avgpool_fc_bwd_launch(m->in_dlogits, m->fc_w, dfeat, hl.p, gg.p, B, HWl, Cl, K, st, gsc, PL); },
+      ew([m, hl, gg, dfeat, gsc, B, HWl, Cl, K, PL, GP](cudaStream_t st) {
+           return avgpool_fc_bwd_launch(m->in_dlogits, m->fc_w, dfeat, hl.p, gg.p, B, HWl, Cl, K, st, gsc, PL, GP); },
          2.0 * (double)hl.bytes, "fc + average pool backward (+ relu mask)");
     } else {
       // ---- face parser head backward: d(logits) (B, K, S, S) -> gradients at feat8 / feat16 / feat32
@@ -899,7 +907,7 @@ int build_program_resnet(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* 
       auto dot = [&](const Tensor& x, const Tensor* y, float* out, float scale, const char* what) {
         const Tensor xx = x;
         const f16* yp = y ? y->p : nullptr;
-        ew([xx, yp, out, B, scale, PL](cudaStream_t st) { return chan_dot_launch(xx.p, yp, out, B, xx.H * xx.W, xx.C, scale, st, PL); },
+        ew([xx, yp, out, B, scale, PL, GP](cudaStream_t st) { return chan_dot_launch(xx.p, yp, out, B, xx.H * xx.W, xx.C, scale, st, PL, GP); },
            (y ? 2.0 : 1.0) * (double)xx.bytes, what);
       };
       auto vact = [&](const float* gv, const float* a, float* out, int n, int mode) {
@@ -909,31 +917,31 @@ int build_program_resnet(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* 
         ew([gv, w, out, B, C, Kk, scale](cudaStream_t st) { return fc_t_launch(gv, w, out, B, C, Kk, scale, st); }, 4.0 * C * Kk, "transposed 1x1 on pooled vector");
       };
       auto affine = [&](const Tensor& x, const float* a, const float* b, Tensor* out, const char* what) {
-        *out = talloc(B, x.H, x.W, x.C);
+        *out = talloc(B, x.H, x.W, x.C, GP);
         const Tensor xx = x, oo = *out;
-        ew([xx, a, b, oo, B](cudaStream_t st) { return chan_affine_launch(xx.p, a, b, nullptr, oo.p, B, xx.H * xx.W, xx.C, st); },
+        ew([xx, a, b, oo, B, GP](cudaStream_t st) { return chan_affine_launch(xx.p, a, b, nullptr, oo.p, B, xx.H * xx.W, xx.C, st, GP); },
            2.0 * (double)xx.bytes, what);
       };
       auto merge = [&](const Tensor* gt, const Tensor* e, int e_off, const Tensor* y, Tensor* out, int C, int H, int W, const char* what) {
-        *out = talloc(B, H, W, C);
+        *out = talloc(B, H, W, C, GP);
         const Tensor oo = *out;
         const f16* gp = gt ? gt->p : nullptr; const f16* ep = e ? e->p : nullptr; const f16* yp = y ? y->p : nullptr;
         const int epitch = e ? e->C : 0;
-        ew([gp, ep, epitch, e_off, yp, oo, B, PL](cudaStream_t st) {
-             return grad_merge_launch(gp, ep, epitch, e_off, yp, oo.p, (int64_t)B * oo.H * oo.W, oo.C, st, PL); }, 3.0 * (double)oo.bytes, what);
+        ew([gp, ep, epitch, e_off, yp, oo, B, PL, GP](cudaStream_t st) {
+             return grad_merge_launch(gp, ep, epitch, e_off, yp, oo.p, (int64_t)B * oo.H * oo.W, oo.C, st, PL, GP); }, 3.0 * (double)oo.bytes, what);
       };
       auto down2 = [&](const Tensor& dy, Tensor* dx) {
-        *dx = talloc(B, dy.H / 2, dy.W / 2, dy.C);
+        *dx = talloc(B, dy.H / 2, dy.W / 2, dy.C, GP);
         const Tensor dd = dy, xx = *dx;
-        ew([dd, xx, B](cudaStream_t st) { return downsum2x_launch(dd.p, xx.p, B, xx.H, xx.W, xx.C, st); }, 1.25 * (double)dd.bytes, "nearest upsample backward");
+        ew([dd, xx, B, GP](cudaStream_t st) { return downsum2x_launch(dd.p, xx.p, B, xx.H, xx.W, xx.C, st, GP); }, 1.25 * (double)dd.bytes, "nearest upsample backward");
       };
       const int mid = 128;
       const float i8 = 1.f / (float)(hs.ff.H * hs.ff.W), i16 = 1.f / (float)(hs.f16.H * hs.f16.W), i32 = 1.f / (float)(hs.f32.H * hs.f32.W);
-      Tensor g_o2 = talloc(B, hs.o2.H, hs.o2.W, hs.o2.C), g_o1, g_fo, g_ff, g_cat, g_cp8, g_up16, g_sum16, g_h32, g_f16, e16, g_up32,
+      Tensor g_o2 = talloc(B, hs.o2.H, hs.o2.W, hs.o2.C, GP), g_o1, g_fo, g_ff, g_cat, g_cp8, g_up16, g_sum16, g_h32, g_f16, e16, g_up32,
              g_sum32, g_f32, e32, g32;
       {
         const Tensor oo = g_o2;
-        ew([m, oo, gsc, B, K, S](cudaStream_t st) { return bilinear_ac_bwd_launch(m->in_dlogits, oo.p, B, oo.H, oo.W, oo.C, K, S, S, st, gsc); },
+        ew([m, oo, gsc, B, K, S, GP](cudaStream_t st) { return bilinear_ac_bwd_launch(m->in_dlogits, oo.p, B, oo.H, oo.W, oo.C, K, S, S, st, gsc, GP); },
            4.0 * B * K * S * S, "bilinear upsample backward");
       }
       dconv(bs.out_cls.dg, g_o2, nullptr, &g_o1, "conv_out.conv_out");
@@ -1011,9 +1019,9 @@ int build_program_resnet(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* 
         if (ex != extra.end() && !rc) {
           const Tensor gd = dx, ee = ex->second.first, yy = sv.x;
           const int eoff = ex->second.second;
-          Tensor merged = talloc(B, dx.H, dx.W, dx.C);
-          ew([gd, ee, eoff, yy, merged, B, PL](cudaStream_t st) {
-               return grad_merge_launch(gd.p, ee.p, ee.C, eoff, yy.p, merged.p, (int64_t)B * merged.H * merged.W, merged.C, st, PL); },
+          Tensor merged = talloc(B, dx.H, dx.W, dx.C, GP);
+          ew([gd, ee, eoff, yy, merged, B, PL, GP](cudaStream_t st) {
+               return grad_merge_launch(gd.p, ee.p, ee.C, eoff, yy.p, merged.p, (int64_t)B * merged.H * merged.W, merged.C, st, PL, GP); },
              4.0 * (double)merged.bytes, "gradient merge (second consumer) + relu mask");
           dx = merged;
         } else if (bi > 0) {
@@ -1024,14 +1032,14 @@ int build_program_resnet(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* 
     }
     if (!rc) {
       // max pool (+ the stem's ReLU mask) -> stem dgrad w.r.t. the im2col columns -> col2im -> fp32 NCHW image gradient
-      Tensor gy1 = talloc(B, y1.H, y1.W, y1.C), dcols;
+      Tensor gy1 = talloc(B, y1.H, y1.W, y1.C, GP), dcols;
       const Tensor gg = g;
-      ew([y1, pool_idx, gg, gy1, B, PL](cudaStream_t st) { return maxpool3s2_bwd_launch(y1.p, pool_idx, gg.p, gy1.p, B, y1.H, y1.W, y1.C, st, PL); },
+      ew([y1, pool_idx, gg, gy1, B, PL, GP](cudaStream_t st) { return maxpool3s2_bwd_launch(y1.p, pool_idx, gg.p, gy1.p, B, y1.H, y1.W, y1.C, st, PL, GP); },
          3.0 * (double)y1.bytes, "maxpool backward (+ stem relu mask)");
       dconv(m->stem_dg, gy1, nullptr, &dcols, "stem");
       if (!rc) {
         const Tensor dc = dcols;
-        ew([m, dc, gsc, B, Cin, S, KP](cudaStream_t st) { return col2im7s2_launch(dc.p, m->out_dz, B, Cin, S, S, KP, st, gsc); },
+        ew([m, dc, gsc, B, Cin, S, KP, GP](cudaStream_t st) { return col2im7s2_launch(dc.p, m->out_dz, B, Cin, S, S, KP, st, gsc, GP); },
            (double)dc.bytes + 4.0 * B * Cin * S * S, "stem col2im (image gradient)");
       }
     }
@@ -1072,12 +1080,13 @@ int build_model_lpips(b2e_unet* m) {
         ci.b = m->dmalloc<float>(ci.cout_pad);
         ci.dg = m->make_dgrad(kConvBlockK, ci.cout_pad, 1);   // gradient w.r.t. the 64 im2col columns
         const ConvL cd = m->dgrads[ci.dg];
-        m->add_param(name + ".weight", (int64_t)cout * 27, 27, [ci, cd, PL](const float* src, cudaStream_t st) {
+        const int DPL = m->dgrad_planes();
+        m->add_param(name + ".weight", (int64_t)cout * 27, 27, [ci, cd, PL, DPL](const float* src, cudaStream_t st) {
           const float ws = PL == 3 ? b2e_unet::kSplitWScale : 1.f;
           int rc = conv_pack_weight(src, ci.w, ci.cout, 3, 3, 3, ci.row_len, 0, st, 0, 0, 0, ws);
           if (!rc && PL == 3) rc = conv_pack_weight(src, ci.w, ci.cout, 3, 3, 3, ci.row_len, kConvBlockK, st, 0, 0, 0, ws);
           if (!rc && PL == 3) rc = conv_pack_weight(src, ci.w, ci.cout, 3, 3, 3, ci.row_len, 2 * kConvBlockK, st, 0, 0, 1, ws);
-          if (!rc) rc = conv_pack_weight_im2col_T(src, cd.w, ci.cout, 3, cd.row_len, st);
+          if (!rc) rc = conv_pack_weight_im2col_T(src, cd.w, ci.cout, 3, cd.row_len, st, 9, DPL, b2e_unet::dgrad_wscale(DPL));
           return rc;
         });
         m->add_f32(name + ".bias", ci.b, cout, 27);
@@ -1115,6 +1124,7 @@ int build_program_lpips(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* n
   double flops = 0;
   int rc = B2E_OK;
   const int PL = m->PL, S = m->lcfg.input_size;
+  const int GP = m->dgrad_planes();   // planes of the gradients (3: split gradients of grad_precision = 1)
   int tap_hw[kVggStages];
   for (int k = 0; k < kVggStages; ++k) tap_hw[k] = (S >> k) * (S >> k);
   // the reference cache comes first, sized for max_batch: same offset for every batch the program is rebuilt for
@@ -1212,21 +1222,24 @@ int build_program_lpips(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* n
     auto dconv = [&](const ConvL& L, const Tensor& dy, Tensor* dx) {
       if (rc) return;
       const ConvL& D = m->dgrads[L.dg];
-      *dx = talloc(B, dy.H, dy.W, D.cout_pad);
+      *dx = talloc(B, dy.H, dy.W, D.cout_pad, GP);
       flops += 2.0 * B * dy.H * dy.W * (double)D.cout_pad * D.row_len;
       if (dry) return;
-      if (D.k * D.k * dy.C != D.row_len) { rc = B2E_INVALID_ARG; set_error("lpips backward: operand widths do not match"); return; }
+      if (GP * D.k * D.k * dy.C != D.row_len) { rc = B2E_INVALID_ARG; set_error("lpips backward: operand widths do not match"); return; }
       ConvDesc d;
-      d.s0 = ConvSrc{dy.p, dy.C};
+      d.s0 = ConvSrc{dy.p, dy.C * GP};
+      d.out_planes = GP;
       d.N = B; d.H = dy.H; d.W = dy.W; d.ksize = D.k; d.stride = 1;
       d.w_packed = D.w; d.Cout = D.cout_pad; d.out_f16 = dx->p;
       d.split_ws = split_ws; d.split_ws_bytes = split_bytes; d.split_counters = split_cnt;
       ConvPlan pl;
       rc = conv_plan_build(&pl, d);
       if (rc) return;
+      ConvEpilogue ep;
+      if (GP == 3) ep.acc_scale = 1.f / b2e_unet::kSplitWScale;
       char desc[160];
-      snprintf(desc, sizeof(desc), "vgg: dgrad conv%dx%d %dx%d cin%d cout%d", D.k, D.k, dy.H, dy.W, dy.C, D.cout);
-      cur->push_back({[pl](cudaStream_t st) { return conv_launch(pl, ConvEpilogue{}, st); }, 0, pl.flops, 0.0, desc});
+      snprintf(desc, sizeof(desc), "vgg: dgrad conv%dx%d %dx%d cin%d cout%d%s", D.k, D.k, dy.H, dy.W, dy.C, D.cout, GP == 3 ? " split" : "");
+      cur->push_back({[pl, ep](cudaStream_t st) { return conv_launch(pl, ep, st); }, 0, pl.flops, 0.0, desc});
     };
     // gradient scale record (grad_scale_launch) from the largest head-gradient element the forward measured (it includes
     // the 1 / ||f|| of the normalisation Jacobian, so the scale follows the feature norms of the actual weights)
@@ -1239,18 +1252,18 @@ int build_program_lpips(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* n
     li = (int)m->vgg.size() - 1;
     for (int s = kVggStages - 1; s >= 0 && !rc; --s) {
       const Tensor t = tap[s];
-      Tensor g = talloc(B, t.H, t.W, t.C);
+      Tensor g = talloc(B, t.H, t.W, t.C, GP);
       const f16* gpp = s == kVggStages - 1 ? nullptr : gp.p;
       float* rk = ref + m->lp_ref_off[s];
-      ew([m, t, s, rk, gsc, gpp, g, B, PL](cudaStream_t st) {
-           return lpips_head_bwd_launch(t.p, B, t.C, t.H * t.W, PL, m->lin_w[s], rk, m->lp_ref_B != 1, m->in_dlogits, gsc, gpp, g.p, st); },
+      ew([m, t, s, rk, gsc, gpp, g, B, PL, GP](cudaStream_t st) {
+           return lpips_head_bwd_launch(t.p, B, t.C, t.H * t.W, PL, m->lin_w[s], rk, m->lp_ref_B != 1, m->in_dlogits, gsc, gpp, g.p, st, GP); },
          (double)t.bytes + 4.0 * B * t.H * t.W * t.C + 2.0 * (double)g.bytes, "lpips head backward (+ pooled path, relu mask)");
       for (int j = kVggConvs[s] - 1; j >= 0 && !rc; --j, --li) {
         Tensor dx;
         dconv(m->vgg[li], g, &dx);
         if (j > 0) {
           const Tensor gg = dx, yy = acts[li - 1];
-          ew([gg, yy, PL](cudaStream_t st) { return relu_bwd_launch(gg.p, yy.p, gg.p, (int64_t)(gg.bytes / sizeof(f16)), st, PL, gg.C); },
+          ew([gg, yy, PL, GP](cudaStream_t st) { return relu_bwd_launch(gg.p, yy.p, gg.p, (int64_t)(gg.bytes / sizeof(f16)), st, PL, gg.C, GP); },
              3.0 * (double)gg.bytes, "relu backward");
         }
         g = dx;
@@ -1259,15 +1272,15 @@ int build_program_lpips(b2e_unet* m, int B, void* ws, size_t ws_bytes, size_t* n
       if (s > 0) {
         // g = d(pool output): to the arg-max positions of the tap below (+ its ReLU mask)
         const Tensor tb = tap[s - 1], gy = g;
-        gp = talloc(B, tb.H, tb.W, tb.C);
+        gp = talloc(B, tb.H, tb.W, tb.C, GP);
         const Tensor gx = gp;
         uint16_t* ix = pidx[s - 1];
-        ew([tb, ix, gy, gx, B, PL](cudaStream_t st) { return maxpool2x2_bwd_launch(tb.p, ix, gy.p, gx.p, B, tb.H, tb.W, tb.C, st, PL); },
+        ew([tb, ix, gy, gx, B, PL, GP](cudaStream_t st) { return maxpool2x2_bwd_launch(tb.p, ix, gy.p, gx.p, B, tb.H, tb.W, tb.C, st, PL, GP); },
            2.5 * (double)gx.bytes, "maxpool 2x2 backward (+ relu mask)");
       } else {
         const Tensor dc = g;
-        ew([m, dc, gsc, B, S](cudaStream_t st) {
-             return vq_col2im_bwd_launch(dc.p, m->lp_const + 6, m->out_dz, B, 3, S, S, st, gsc, m->lp_mask, m->lp_mask_batched); },
+        ew([m, dc, gsc, B, S, GP](cudaStream_t st) {
+             return vq_col2im_bwd_launch(dc.p, m->lp_const + 6, m->out_dz, B, 3, S, S, st, gsc, m->lp_mask, m->lp_mask_batched, GP); },
            (double)dc.bytes + 12.0 * B * S * S, "col2im + scaling layer + input mask backward");
       }
     }
@@ -2378,6 +2391,9 @@ int b2e_resnet_create(const b2e_resnet_config* cfg, int64_t max_batch, b2e_unet*
   B2E_REQUIRE(cfg->width >= 64 && cfg->width % 64 == 0 && cfg->num_classes >= 1 && cfg->num_classes <= 4096, B2E_UNSUPPORTED_SHAPE,
               "resnet_create: width must be a multiple of 64, 1..4096 classes");
   for (int i = 0; i < 4; ++i) B2E_REQUIRE(cfg->layers[i] >= 1 && cfg->layers[i] <= 64, B2E_UNSUPPORTED_SHAPE, "resnet_create: layers");
+  B2E_REQUIRE(cfg->grad_precision == 0 || (cfg->grad_precision == 1 && cfg->precision == 1), B2E_INVALID_ARG,
+              "resnet_create: grad_precision must be 0, or 1 with precision = 1 (got %d with precision %d)", cfg->grad_precision,
+              cfg->precision);
   b2e_unet* m = new b2e_unet();
   m->resnet = true;
   B2E_REQUIRE(cfg->head == 0 || (cfg->head == 1 && !cfg->bottleneck && cfg->width == 64 && cfg->num_classes <= 64),
@@ -2385,6 +2401,7 @@ int b2e_resnet_create(const b2e_resnet_config* cfg, int64_t max_batch, b2e_unet*
   m->grad = cfg->head == 0;   // the classifier exists for its input gradient (classifier guidance)
   B2E_REQUIRE(cfg->precision == 0 || cfg->precision == 1, B2E_INVALID_ARG, "resnet_create: precision must be 0 or 1");
   m->PL = cfg->precision == 1 ? 3 : 1;
+  m->split_grad = cfg->grad_precision == 1;
   m->rcfg = *cfg;
   m->cfg = b2e_unet_config{};
   m->cfg.sample_size = cfg->input_size; m->cfg.in_channels = cfg->in_channels; m->cfg.out_channels = cfg->num_classes;
@@ -2419,10 +2436,14 @@ int b2e_lpips_create(const b2e_lpips_config* cfg, int64_t max_batch, b2e_unet** 
   B2E_REQUIRE(cfg->input_size >= 32 && cfg->input_size % 16 == 0 && cfg->input_size <= 4096, B2E_UNSUPPORTED_SHAPE,
               "lpips_create: input_size must be a multiple of 16 in 32..4096 (got %d)", cfg->input_size);
   B2E_REQUIRE(cfg->precision == 0 || cfg->precision == 1, B2E_INVALID_ARG, "lpips_create: precision must be 0 or 1");
+  B2E_REQUIRE(cfg->grad_precision == 0 || (cfg->grad_precision == 1 && cfg->precision == 1), B2E_INVALID_ARG,
+              "lpips_create: grad_precision must be 0, or 1 with precision = 1 (got %d with precision %d)", cfg->grad_precision,
+              cfg->precision);
   b2e_unet* m = new b2e_unet();
   m->lpips = true;
   m->grad = true;    // the regulariser exists for its input gradient
   m->PL = cfg->precision == 1 ? 3 : 1;
+  m->split_grad = cfg->grad_precision == 1;
   m->lcfg = *cfg;
   m->cfg = b2e_unet_config{};
   m->cfg.sample_size = cfg->input_size; m->cfg.in_channels = 3; m->cfg.out_channels = 1;

@@ -128,24 +128,30 @@ int pointwise_conv_f32_launch(const float* x, const float* w, const float* b, fl
                               cudaStream_t st);
 
 // classifier network (torchvision ResNet) kernels, csrc/resnet_kernels.cu
-// planes = 3 / xplanes / yplanes = 3: split tensors [hi | lo | hi] of the fp32-accurate forward (pixel pitch 3 C)
+// planes = 3 / xplanes / yplanes = 3: split tensors [hi | lo | hi] of the fp32-accurate forward (pixel pitch 3 C).
+// Backward kernels: gplanes = 3 (col2im7s2, bilinear_ac_bwd: planes; chan_dot: xplanes) - the gradients are split tensors
+// of the fp32-accurate backward (grad_precision = 1), read as hi + lo, computed in fp32 and re-split; they need the split
+// forward's activations for their masks.
 int im2col7s2_launch(const float* x, f16* out, int B, int C, int H, int W, int KP, cudaStream_t st, int planes = 1);
-int col2im7s2_launch(const f16* dcols, float* dx, int B, int C, int H, int W, int KP, cudaStream_t st, const float* gs = nullptr);
+int col2im7s2_launch(const f16* dcols, float* dx, int B, int C, int H, int W, int KP, cudaStream_t st, const float* gs = nullptr,
+                     int planes = 1);
 int maxpool3s2_launch(const f16* x, f16* y, uint8_t* idx, int N, int H, int W, int C, cudaStream_t st, int planes = 1);
 int maxpool3s2_bwd_launch(const f16* x, const uint8_t* idx, const f16* gy, f16* gx, int N, int H, int W, int C, cudaStream_t st,
-                          int xplanes = 1);
-int relu_bwd_launch(const f16* g, const f16* y, f16* out, int64_t numel, cudaStream_t st, int yplanes = 1, int C = 0);
+                          int xplanes = 1, int gplanes = 1);
+// numel counts every plane of g (gplanes = 3: 3 C channels per pixel)
+int relu_bwd_launch(const f16* g, const f16* y, f16* out, int64_t numel, cudaStream_t st, int yplanes = 1, int C = 0, int gplanes = 1);
 int subsample2x_launch(const f16* in, f16* out, int N, int Ho, int Wo, int C, cudaStream_t st);
+// (split gradients: C = 3 x the channels per plane - the planes of a pixel move together)
 int zero_upsample2x_launch(const f16* in, f16* out, int N, int Hi, int Wi, int C, cudaStream_t st);
 int avgpool_fc_launch(const f16* x, float* feat, const float* w, const float* b, float* logits, int N, int HW, int C, int K,
                       cudaStream_t st, int planes = 1);
 int avgpool_fc_bwd_launch(const float* dlogits, const float* w, float* dfeat, const f16* y, f16* g, int N, int HW, int C, int K,
-                          cudaStream_t st, const float* gs = nullptr, int yplanes = 1);
+                          cudaStream_t st, const float* gs = nullptr, int yplanes = 1, int gplanes = 1);
 
 // LPIPS (VGG-16) kernels, csrc/lpips_kernels.cu; planes / xplanes = 3: split tensors of the fp32-accurate forward
 int maxpool2x2_launch(const f16* x, f16* y, uint16_t* idx, int N, int H, int W, int C, cudaStream_t st, int planes = 1);
 int maxpool2x2_bwd_launch(const f16* x, const uint16_t* idx, const f16* gy, f16* gx, int N, int H, int W, int C, cudaStream_t st,
-                          int xplanes = 1);
+                          int xplanes = 1, int gplanes = 1);
 struct LpipsTaps { int n[5], off[5], hw[5]; };   // partial slots per tap, their offset in a row of partials, pixels per image
 int lpips_head_blocks(int HW);
 // mode 0: ref <- normalised features of x; mode 1: partial[b][slot0 ..] <- distance partial sums against ref
@@ -156,7 +162,7 @@ int lpips_head_launch(const f16* x, int B, int C, int HW, int planes, const floa
 int lpips_grad_scale_launch(const float* d_dist, const float* hmax, float* prod, int B, float* gs, cudaStream_t st);
 int lpips_finalize_launch(const double* partial, int part_pitch, const LpipsTaps& taps, float* dist, int B, cudaStream_t st);
 int lpips_head_bwd_launch(const f16* x, int B, int C, int HW, int planes, const float* w, const float* ref, int ref_batched,
-                          const float* d_dist, const float* gs, const f16* gp, f16* gout, cudaStream_t st);
+                          const float* d_dist, const float* gs, const f16* gp, f16* gout, cudaStream_t st, int gplanes = 1);
 
 // face parser (BiSeNet) helpers
 int avgpool_launch(const f16* x, float* feat, int N, int HW, int C, cudaStream_t st, int planes = 1);
@@ -168,12 +174,13 @@ int bilinear_ac_launch(const f16* x, float* out, int N, int Hi, int Wi, int P, i
 int bilinear_ac_argmax_launch(const f16* x, int64_t* labels, int N, int Hi, int Wi, int P, int K, int Ho, int Wo, cudaStream_t st,
                               int planes = 1);
 int bilinear_ac_bwd_launch(const float* g, f16* dx, int N, int Hi, int Wi, int P, int K, int Ho, int Wo, cudaStream_t st,
-                           const float* gs = nullptr);
-int chan_dot_launch(const f16* x, const f16* y, float* out, int N, int HW, int C, float scale, cudaStream_t st, int yplanes = 1);
+                           const float* gs = nullptr, int planes = 1);
+int chan_dot_launch(const f16* x, const f16* y, float* out, int N, int HW, int C, float scale, cudaStream_t st, int yplanes = 1,
+                    int xplanes = 1);
 int fc_t_launch(const float* g, const float* w, float* out, int N, int C, int K, float scale, cudaStream_t st);
 int vec_act_bwd_launch(const float* g, const float* a, float* out, int n, int mode, cudaStream_t st);
 int grad_merge_launch(const f16* g, const f16* e, int e_pitch, int e_off, const f16* y, f16* out, int64_t rows, int C,
-                      cudaStream_t st, int yplanes = 1);
+                      cudaStream_t st, int yplanes = 1, int gplanes = 1);
 
 // multi-head tensor-core attention: head-major operands (virtual image v = n*heads + h, head_dim padded to 64)
 int split_heads_launch(const f16* qkv, f16* qh, f16* kh, f16* vht, int N, int T, int P, int heads, int d, cudaStream_t st);

@@ -143,32 +143,41 @@ def create_diffusion_model(name: str, sample_clipping: bool = True, *, max_batch
 
 
 def get_pretrained_anyGAN(input_size: int = 256, max_batch: int = 1, state_dict_path: str = "../attribute_predictor.pt",
-                          seed: int = 0, precision: Optional[str] = "fp32"):
+                          seed: int = 0, precision: Optional[str] = "fp32", grad_precision: Optional[str] = None):
     """The attribute predictor of ClassifierAttrFunc (src/models.py:69-77: ``models.resnet50()`` with an 80-way ``fc``
     loaded from ../attribute_predictor.pt) on the native engine: forward AND input gradient on the tcgen05 kernels, so
     classifier guidance needs no torch network.  ``input_size`` is the resolution of the decoded images it will see (256
     for DDPM / LDM, 512 for SD).  Offline (no checkpoint file) the weights are random-init (seeded).  ``precision``:
     "fp32" (default) runs the fp32-accurate forward, so the guidance gradient is routed through the fp32 network's
     ReLU / max-pool masks (input gradient within 1e-2 relative RMS of fp32 autograd); "fp16" is the f16-operand forward
-    (3x fewer forward flops, gradient 0.15 relative RMS from fp32)."""
+    (3x fewer forward flops, gradient 0.15 relative RMS from fp32).  ``grad_precision="fp32"`` (with ``precision="fp32"``)
+    also runs the backward on split operands, for an fp32-accurate guidance gradient; None (default) keeps it 16-bit."""
     import os
+    from b200edit import _C
     from b200edit.resnet import resnet50_predictor
+    _C.resolve_grad_precision(grad_precision, _C.resolve_precision(precision, "get_pretrained_anyGAN")[0], "get_pretrained_anyGAN")
     sd = None
     if state_dict_path and os.path.exists(state_dict_path):
         sd = torch.load(state_dict_path, map_location="cpu")
         sd = sd.get("state_dict", sd)
-    return resnet50_predictor(80, input_size, max_batch=max_batch, state_dict=sd, seed=seed, precision=precision)
+    return resnet50_predictor(80, input_size, max_batch=max_batch, state_dict=sd, seed=seed, precision=precision,
+                              grad_precision=grad_precision)
 
 
 def get_lpips(input_size: int = 256, max_batch: int = 1, state_dict: Optional[dict] = None, seed: int = 0,
-              precision: Optional[str] = "fp32"):
+              precision: Optional[str] = "fp32", grad_precision: Optional[str] = None):
     """The LPIPS (vgg) distance of ``use_lpips`` guidance and ``metrics.lpips`` (the reference's ``lpips.LPIPS(net='vgg')``)
     on the native engine: forward and input gradient on the tcgen05 kernels.  ``state_dict``: the full
     ``lpips.LPIPS(net='vgg').state_dict()``; without it the weights are seeded random (no pretrained VGG offline).
     ``precision`` "fp32" (default) runs the fp32-accurate forward because guidance differentiates the network (the
-    ReLU / max-pool masks of the input gradient then agree with an fp32 evaluation); "fp16" is the 16-bit forward."""
+    ReLU / max-pool masks of the input gradient then agree with an fp32 evaluation); "fp16" is the 16-bit forward.
+    ``grad_precision="fp32"`` (with ``precision="fp32"``) also runs the backward on split operands (fp32-accurate input
+    gradient); None (default) keeps it 16-bit."""
+    from b200edit import _C
     from b200edit.lpips import LPIPS
-    net = LPIPS("vgg", input_size=input_size, max_batch=max_batch, device=get_device(), precision=precision)
+    _C.resolve_grad_precision(grad_precision, _C.resolve_precision(precision, "get_lpips")[0], "get_lpips")   # before building
+    net = LPIPS("vgg", input_size=input_size, max_batch=max_batch, device=get_device(), precision=precision,
+                grad_precision=grad_precision)
     if state_dict is not None:
         net.load_state_dict(state_dict)
     else:
@@ -183,10 +192,18 @@ class SegmentationModel:
     this one object as in the reference - loaded from ``ckpt`` (the reference's Segmentation/res/cp/79999_iter.pth, a blob
     missing from the checkout) when the file exists, else seeded random-init weights.  ``net=`` (keyword-only)
     substitutes any callable mapping a (1,3,S,S) image to ([1,19,S,S] logits, ...).  ``max_batch`` (keyword-only) is the
-    largest batch the default parser differentiates at once (``NetAttrFunc(per_sample=True)`` on a batch of images)."""
+    largest batch the default parser differentiates at once (``NetAttrFunc(per_sample=True)`` on a batch of images).
+    ``grad_precision`` (keyword-only) is that parser's backward: None - 16-bit, "fp32" - fp32-accurate (split operands;
+    needs ``precision`` None or "fp32"); it does not touch the forward-only engine of mask creation."""
 
     def __init__(self, ckpt: str = "Segmentation/res/cp/79999_iter.pth", n_classes: int = 19, image_size: tuple = (512, 512),
-                 *, net=None, seed: int = 0, precision: Optional[str] = None, max_batch: int = 1) -> None:
+                 *, net=None, seed: int = 0, precision: Optional[str] = None, max_batch: int = 1,
+                 grad_precision: Optional[str] = None) -> None:
+        if grad_precision is not None:
+            from b200edit import _C
+            if net is not None:
+                raise ValueError("SegmentationModel: grad_precision applies to the native parser; a net= sets its own")
+            _C.resolve_grad_precision(grad_precision, precision or "fp32", "SegmentationModel")   # before building anything
         self.device = get_device()
         if not (ckpt is None or isinstance(ckpt, (str, bytes)) or hasattr(ckpt, "__fspath__")):
             raise TypeError("SegmentationModel: the first argument is the checkpoint path (as in the reference); pass a "
@@ -194,7 +211,8 @@ class SegmentationModel:
         if net is None:
             import os
             from b200edit.bisenet import MultiResBiSeNet
-            net = MultiResBiSeNet(n_classes, max_batch=max_batch, device=self.device, seed=seed, precision=precision)
+            net = MultiResBiSeNet(n_classes, max_batch=max_batch, device=self.device, seed=seed, precision=precision,
+                                  grad_precision=grad_precision)
             if ckpt and os.path.exists(ckpt):
                 net.load_reference_state_dict(torch.load(ckpt, map_location="cpu"))
         self.net = net

@@ -402,7 +402,8 @@ typedef struct {
   /* 0: classifier (global average pool + fc -> logits (B, num_classes)).
    * 1: face parser: BiSeNet (src/Segmentation/model.py:234-262, the network of SegmentationModel, src/models.py:80-118) on a
    *    basic-block backbone - context path with attention refinement, feature fusion, output head, bilinear
-   *    (align_corners) upsampling: output = out[0] of the reference, logits (B, num_classes, S, S) fp32; forward only.
+   *    (align_corners) upsampling: output = out[0] of the reference, logits (B, num_classes, S, S) fp32.  Created with
+   *    gradient mode off (b2e_unet_enable_grad turns it on; b2e_resnet_backward then gives d(logits) -> d(image)).
    *    Parameters under the reference's names with BatchNorm folded ("cp.resnet.layer1.0.conv1.weight/.bias",
    *    "cp.arm16.conv.*", "cp.arm16.conv_atten.*", "cp.conv_head32.*", "cp.conv_avg.*", "ffm.convblk.*", "ffm.conv1.weight",
    *    "ffm.conv2.weight", "conv_out.conv.*", "conv_out.conv_out.*"). */
@@ -410,8 +411,13 @@ typedef struct {
   /* 0: f16 operands throughout.  1 (head 0): fp32-accurate FORWARD - split f16 operands hi + lo, three tensor-core products
    * per GEMM, as b2e_unet_config.precision - so the ReLU / max-pool masks the backward pass reads agree with an fp32
    * evaluation of the network (a 16-bit forward flips the masks of near-zero activations, which dominates the error of
-   * the INPUT GRADIENT); the backward pass itself stays on f16 operands. */
+   * the INPUT GRADIENT); the backward pass stays on f16 operands unless grad_precision = 1. */
   int32_t precision;
+  /* 0 (default): 16-bit backward - f16 gradients through f16 dgrad weights.  1 (needs precision = 1): fp32-accurate
+   * backward - split gradients hi + lo through split dgrad weights [W'_hi | W'_hi | W'_lo] x 2^10 (three tensor-core
+   * products per GEMM), every element-wise backward kernel in fp32.  The forward is the same either way.  Any other value,
+   * or 1 with precision = 0: B2E_INVALID_ARG. */
+  int32_t grad_precision;
 } b2e_resnet_config;
 int b2e_resnet_create(const b2e_resnet_config* cfg, int64_t max_batch, b2e_unet** out);
 int b2e_resnet_backward(b2e_unet* m, const float* d_logits, float* d_image, int64_t B, void* stream);
@@ -437,7 +443,9 @@ int b2e_resnet_forward_labels(b2e_unet* m, const float* x, int64_t* labels, int6
  * Workspace, parameters and profiling through the b2e_unet_* entry points. */
 typedef struct {
   int32_t input_size;   /* image height = width: a multiple of 16, >= 32 */
-  int32_t precision;    /* 0: f16 operands; 1: fp32-accurate forward (backward on f16 operands), as b2e_resnet_config */
+  int32_t precision;    /* 0: f16 operands; 1: fp32-accurate forward (backward on f16 operands unless grad_precision = 1),
+                         * as b2e_resnet_config */
+  int32_t grad_precision;   /* 0: 16-bit backward; 1 (needs precision = 1): fp32-accurate backward, as b2e_resnet_config */
 } b2e_lpips_config;
 int b2e_lpips_create(const b2e_lpips_config* cfg, int64_t max_batch, b2e_unet** out);
 int b2e_lpips_set_reference(b2e_unet* m, const float* x_ref, int64_t B_ref, void* stream);
